@@ -221,6 +221,44 @@ int64_t sai_gzip_inflate(const uint8_t* data, int64_t len, uint8_t* out, int64_t
 int32_t sai_inflate_raw(const uint8_t* in, int64_t in_len, uint8_t* out, int64_t out_len);
 uint32_t sai_crc32(const uint8_t* data, int64_t len, int32_t isa);
 
+/* ---- device VCF ingest: VCF text in HBM -> tiled bit-planes ----------------
+ * The same records and values as sai_vcf_parse_gt (the host parser is the specification), written
+ * straight into the packed layout: population p of `lay` takes its n_samples individuals from the
+ * VCF sample columns sample_column[first_p .. first_p + n_samples), first_p = sum of the earlier
+ * populations' n_samples, with the population's ploidy.  Values are coded in the population's
+ * bit-planes (negative = missing); a value that does not fit is recorded in vmax and the call still
+ * succeeds -- sai_vcf_state tells the caller to repeat with a wider layout. */
+typedef struct {
+  sai_layout lay;
+  const int32_t* sample_column; /* DEVICE, one VCF sample column per individual (see above) */
+  const int32_t* anc_pos;       /* DEVICE, sorted; n_anc == 0: no ancestral-allele table   */
+  const char* anc_allele;       /* DEVICE, 8 bytes per entry, NUL padded                    */
+  int64_t n_anc;
+  int64_t start, end;           /* start <= POS <= end; no region filter when start > end   */
+  int32_t max_column;           /* largest entry of sample_column                          */
+  int32_t chrom_len;            /* 1..255                                                  */
+  char chrom[256];
+} sai_vcf_query;
+
+/* Device-side running state of one parse (zero it before the first slice). */
+typedef struct {
+  int64_t n_sites;              /* sites found so far: slice k numbers its records from here  */
+  int32_t overflow;             /* 1: more sites than site_cap (those beyond it not written) */
+  int32_t pad_;
+  int32_t vmax[SAI_MAX_POPS];   /* largest value above the population's ploidy, else 0     */
+} sai_vcf_state;
+
+/* Device scratch one slice of `len` bytes needs (bytes, 256-byte aligned base). */
+uint64_t sai_vcf_scratch_bytes(const sai_vcf_query* q, int64_t len);
+/* Parses one slice of complete lines d_text[0, len) (16-byte aligned, len < 2^31), stream-ordered:
+ * kept records become sites d_state->n_sites, d_state->n_sites + 1, ... of d_tiles (tile 0 based,
+ * site_cap sites = a multiple of 32) and d_pos; the sites behind the last one, to the end of its
+ * tile, are coded all-missing, so after every call the tiles equal sai_pack_i8_all's over the
+ * sites so far.  Never synchronises the host. */
+int sai_vcf_tiles_device(const sai_vcf_query* q, const char* d_text, int64_t len, void* d_scratch,
+                         uint64_t scratch_bytes, void* d_tiles, int32_t* d_pos, int64_t site_cap,
+                         sai_vcf_state* d_state, void* stream);
+
 /* ---- K1: site counts (replaces calc_freq's passes, stat_utils.py:45-49) --- */
 /* For tiles [tile0, tile0+n_tiles): per population p and site s
  *     num[p*stride + s]    = sum of called values      (stat_utils.py:48)
@@ -487,6 +525,53 @@ int sai_engine_dd_sums(sai_engine* e, const sai_layout* lay, int32_t ref_pop, in
                        const int32_t* src_pops, int32_t n_src, const int64_t* neg_off,
                        const int32_t* neg_site, const int32_t* neg_ind, const int32_t* neg_val,
                        int64_t* ref_sum, int64_t* tgt_sum, int32_t m_max);
+
+/* ---- engine ingest session: a VCF parsed on the device, tiles left resident -------------------
+ * sai_engine_vcf_begin: populations of `lay` as in sai_vcf_query (sample_column, n_out = sum of
+ * n_samples, HOST), the ancestral-allele table (HOST, as sai_vcf_parse_gt), n_file_samples = sample
+ * columns of the #CHROM line and text_bytes_hint = text bytes expected (0: unknown) size the tile
+ * buffer (records are >= 2 * n_file_samples + 18 bytes; it grows with the text fed), min_sites = a
+ * lower bound of its capacity (a repeat after SAI_E_CAPACITY).
+ * sai_engine_vcf_feed: host text of any size; the complete lines are consumed (*consumed), the
+ * rest is the caller's to carry -- the contract of a `_scan_text` on_lines callback.  Host threads
+ * copy slices of complete lines into a ring of pinned buffers; each slice goes to the device with
+ * cudaMemcpyAsync on the copy stream and is parsed on the compute stream while the next ones are
+ * staged.  Returns once the bytes are staged.
+ * sai_engine_vcf_finish: synchronises once; *n_sites, max_value[p] = max(ploidy, largest value of
+ * population p), positions copied to pos_out when pos_cap >= *n_sites.  SAI_E_DOMAIN: a value does
+ * not fit its population's bit-planes (begin again with bits = sai_bits_for_max_value(max_value[p]));
+ * SAI_E_CAPACITY: more records than the tile buffer held (begin again with min_sites = *n_sites).
+ * sai_engine_score_loaded: K1 + K4 on the tiles the session left resident; afterwards
+ * sai_engine_score_resident / _rescore_windows / _pattern_sums work on them unchanged. */
+int sai_engine_vcf_begin(sai_engine* e, const sai_layout* lay, const char* chrom, int64_t start, int64_t end,
+                         const int32_t* sample_column, int32_t n_out, const int32_t* anc_pos,
+                         const char* anc_allele, int64_t n_anc, int32_t n_file_samples, int64_t text_bytes_hint,
+                         int64_t min_sites);
+int sai_engine_vcf_feed(sai_engine* e, const char* text, int64_t len, int64_t* consumed);
+/* The bgzip counterpart: blocks [0, n_blocks) as indexed by sai_bgzf_scan over the whole rest of the
+ * file (out_off[0] = 0), records from text offset `skip` on (the byte behind the #CHROM line).  The
+ * staging threads inflate groups of blocks (CRC checked, sai_bgzf_inflate) straight into the pinned
+ * ring slots -- the text never exists as a whole -- and the incomplete last line of a slot is carried
+ * into the next one; a last line without a newline is complete. */
+int sai_engine_vcf_feed_bgzf(sai_engine* e, const uint8_t* data, const int64_t* block_off, const int64_t* out_off,
+                             int64_t n_blocks, int64_t skip);
+int sai_engine_vcf_finish(sai_engine* e, int64_t* n_sites, int32_t* max_value, int32_t* pos_out, int64_t pos_cap);
+int sai_engine_score_loaded(sai_engine* e, const int64_t* win_start, const int64_t* win_end, int64_t n_windows,
+                            const sai_job* jobs, int32_t n_jobs, sai_host_results* out);
+/* Slice size (bytes, >= 64) and ring depth (>= 2) of the ingest session; <= 0 keeps the default
+ * (32 MB, 4).  Tests use tiny slices to make records and tiles straddle slices.
+ * sai_engine_vcf_slices: slices the last session parsed (tests). */
+int sai_engine_set_vcf_slicing(sai_engine* e, int64_t slice_bytes, int32_t ring);
+int64_t sai_engine_vcf_slices(const sai_engine* e);
+/* Stages of the last finished session: out[0] host seconds staging / inflating into the ring, [1] host
+ * seconds waiting for a free slot, [2] H2D and [3] parse seconds summed over the slices (CUDA events),
+ * [4] seconds from the first slice's H2D start to the last slice's parse end (events), [5] slices,
+ * [6] text bytes, [7] host seconds finish waited for the device, [8] host seconds enqueueing copies and
+ * kernels, [9] host seconds inside the feed calls (all of the above host times and the slicing).
+ * n <= 10 values are written. */
+int sai_engine_vcf_stats(const sai_engine* e, double* out, int32_t n);
+/* The resident tiles of the finished session (sai_packed_bytes(lay, n_sites) bytes) into HOST `out`. */
+int sai_engine_loaded_tiles(sai_engine* e, uint8_t* out, uint64_t cap);
 
 /* ---- synthetic genotypes (bench / tests only) ---------------------------- */
 /* Fills tiles [tile0, tile0+n_tiles) of a packed matrix directly on the device

@@ -80,6 +80,30 @@ class HostResults(C.Structure):
     ]
 
 
+class VcfQuery(C.Structure):
+    _fields_ = [
+        ("lay", Layout),
+        ("sample_column", C.c_void_p),
+        ("anc_pos", C.c_void_p),
+        ("anc_allele", C.c_void_p),
+        ("n_anc", C.c_int64),
+        ("start", C.c_int64),
+        ("end", C.c_int64),
+        ("max_column", C.c_int32),
+        ("chrom_len", C.c_int32),
+        ("chrom", C.c_char * 256),
+    ]
+
+
+class VcfState(C.Structure):
+    _fields_ = [
+        ("n_sites", C.c_int64),
+        ("overflow", C.c_int32),
+        ("pad_", C.c_int32),
+        ("vmax", C.c_int32 * MAX_POPS),
+    ]
+
+
 #: every symbol include/sai_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 _I32, _I64, _U64 = C.c_int32, C.c_int64, C.c_uint64
@@ -164,6 +188,18 @@ SYMBOLS = {
     "sai_zt_decode_host": (C.c_int, [_LAY, _P, _P, _I64, _P]),
     "sai_zt_decode": (C.c_int, [_LAY, _P, _U64, _P, _I64, _I64, _P, _P]),
     "sai_synth_fill": (C.c_int, [_LAY, _P, _I64, _I64, _I64, _P, _U64, C.c_double, _P]),
+    "sai_vcf_scratch_bytes": (_U64, [C.POINTER(VcfQuery), _I64]),
+    "sai_vcf_tiles_device": (C.c_int, [C.POINTER(VcfQuery), _P, _I64, _P, _U64, _P, _P, _I64, _P, _P]),
+    "sai_engine_vcf_begin": (
+        C.c_int, [_P, _LAY, C.c_char_p, _I64, _I64, _P, _I32, _P, _P, _I64, _I32, _I64, _I64]),
+    "sai_engine_vcf_feed": (C.c_int, [_P, _P, _I64, C.POINTER(_I64)]),
+    "sai_engine_vcf_feed_bgzf": (C.c_int, [_P, _P, _P, _P, _I64, _I64]),
+    "sai_engine_vcf_stats": (C.c_int, [_P, _P, _I32]),
+    "sai_engine_vcf_finish": (C.c_int, [_P, C.POINTER(_I64), _P, _P, _I64]),
+    "sai_engine_score_loaded": (C.c_int, [_P, _P, _P, _I64, _JOB, _I32, C.POINTER(HostResults)]),
+    "sai_engine_set_vcf_slicing": (C.c_int, [_P, _I64, _I32]),
+    "sai_engine_vcf_slices": (_I64, [_P]),
+    "sai_engine_loaded_tiles": (C.c_int, [_P, _P, _U64]),
 }
 
 _lib = None

@@ -12,17 +12,86 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <array>
 #include <condition_variable>
+#include <functional>
 #include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
+#include <tuple>
 #include <vector>
 
 #include "common.cuh"
 #include "host_pack.h"
 #include "zt_format.cuh"
 #include "zt_simd.h"
+
+// Persistent host threads of the ingest session: a call hands out tasks [0, n) and returns once all
+// of them have run (the caller works too).  Threads are created once per engine, not per slice.
+struct StagePool {
+  std::vector<std::thread> th;
+  std::mutex mu;
+  std::condition_variable wake, idle;
+  const std::function<void(int64_t)>* job = nullptr;
+  int64_t n_tasks = 0, finished = 0;
+  std::atomic<int64_t> next{0};
+  uint64_t gen = 0;
+  int active = 0;  // workers inside a generation's task loop
+  bool stop = false;
+
+  void work_loop(int64_t n, const std::function<void(int64_t)>& f) {
+    int64_t mine = 0;
+    for (int64_t i = next.fetch_add(1); i < n; i = next.fetch_add(1), ++mine) f(i);
+    std::lock_guard<std::mutex> lk(mu);
+    finished += mine;
+    if (finished == n_tasks) idle.notify_all();
+  }
+  void worker() {
+    uint64_t seen = 0;
+    std::unique_lock<std::mutex> lk(mu);
+    for (;;) {
+      wake.wait(lk, [&] { return stop || (gen != seen && job != nullptr); });
+      if (stop) return;
+      seen = gen;
+      const auto* f = job;
+      const int64_t n = n_tasks;
+      ++active;
+      lk.unlock();
+      work_loop(n, *f);
+      lk.lock();
+      if (--active == 0) idle.notify_all();
+    }
+  }
+  void run(int n_threads, int64_t n, const std::function<void(int64_t)>& f) {
+    if (n <= 0) return;
+    n_threads = std::max(1, n_threads);
+    {
+      std::unique_lock<std::mutex> lk(mu);
+      while ((int)th.size() < n_threads - 1) th.emplace_back([this] { worker(); });
+      job = &f;
+      n_tasks = n;
+      finished = 0;
+      next.store(0);
+      ++gen;
+    }
+    wake.notify_all();
+    work_loop(n, f);
+    std::unique_lock<std::mutex> lk(mu);
+    // every task has run and no worker is still inside this generation's loop (it would take the
+    // next generation's indices with this generation's job)
+    idle.wait(lk, [&] { return finished == n_tasks && active == 0; });
+    job = nullptr;
+  }
+  ~StagePool() {
+    {
+      std::lock_guard<std::mutex> lk(mu);
+      stop = true;
+    }
+    wake.notify_all();
+    for (auto& t : th) t.join();
+  }
+};
 
 struct sai_engine {
   int device = 0;
@@ -47,6 +116,27 @@ struct sai_engine {
   int32_t n_jobs = 0;
   sai_job jobs[SAI_MAX_JOBS];
   sai_layout lay{};  // layout of the resident tiles (sai_engine_score_resident)
+  // ingest session (sai_engine_vcf_*): text ring (pinned + device), the query and its tables
+  struct Vcf {
+    int state = 0;                    // 0 none, 1 feeding, 2 finished (tiles resident)
+    sai_vcf_query q{};
+    int64_t site_cap = 0;             // sites the tile / position buffers hold (multiple of 32)
+    int64_t row_bytes = 64;           // lower bound of a record's length: sizes the tile buffer
+    int64_t fed = 0, n_slices = 0;
+    int64_t slice_bytes = 32ll << 20; // sai_engine_set_vcf_slicing
+    int ring = 4;
+    size_t slot_bytes = 0;            // capacity of one ring slot (pinned and device)
+    char* h_ring = nullptr;
+    std::vector<cudaEvent_t> copied, parsed;  // per slot: H2D done (host slot free), parse done (device slot free)
+    std::vector<std::array<cudaEvent_t, 4>> tev;  // per slice: H2D start / end, parse start / end (stage timing)
+    std::vector<char> carry;          // bgzip feed: the incomplete line at the end of the last slot
+    double t_stage = 0, t_wait = 0;   // host seconds: staging / inflating into the ring, waiting for a free slot
+    double t_launch = 0, t_feed = 0;  // host seconds: enqueueing copies and kernels, inside the feed calls
+    double stats[10] = {0};           // sai_engine_vcf_stats of the last finished session
+    int sticky_rc = SAI_OK;           // first failure of the session, reported by finish
+    StagePool pool;
+  } vcf;
+  Buf vtext, vscratch, vcols, vanc_pos, vanc_all, vstate;
 };
 
 namespace sai {
@@ -174,10 +264,17 @@ int sai_engine_create(int32_t device, sai_engine** out) {
 void sai_engine_destroy(sai_engine* e) {
   if (!e) return;
   cudaSetDevice(e->device);
-  for (auto* b : {&e->packed, &e->pos, &e->win, &e->mask, &e->qval, &e->res, &e->cand, &e->counts, &e->sums, &e->hist, &e->neg, &e->dd, &e->zt, &e->ztoff})
+  for (auto* b : {&e->packed, &e->pos, &e->win, &e->mask, &e->qval, &e->res, &e->cand, &e->counts, &e->sums, &e->hist,
+                  &e->neg, &e->dd, &e->zt, &e->ztoff, &e->vtext, &e->vscratch, &e->vcols, &e->vanc_pos, &e->vanc_all,
+                  &e->vstate})
     if (b->p) cudaFree(b->p);
   for (auto ev : e->ev) cudaEventDestroy(ev);
   for (auto ev : e->ev_dec) cudaEventDestroy(ev);
+  for (auto ev : e->vcf.copied) cudaEventDestroy(ev);
+  for (auto ev : e->vcf.parsed) cudaEventDestroy(ev);
+  for (auto& t : e->vcf.tev)
+    for (auto ev : t) cudaEventDestroy(ev);
+  if (e->vcf.h_ring) cudaFreeHost(e->vcf.h_ring);
   if (e->ring) cudaFreeHost(e->ring);
   if (e->h_ztoff) cudaFreeHost(e->h_ztoff);
   if (e->s_copy) cudaStreamDestroy(e->s_copy);
@@ -433,6 +530,7 @@ static int score_host_impl(sai_engine* e, const sai_layout* lay, const uint8_t* 
   SAI_REQUIRE(n_windows == 0 || (win_start && win_end), "NULL windows");
   if (int rc = check_results(out)) return rc;
   SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  e->vcf.state = 0;  // the tiles of an ingest session are replaced
   const int64_t W = n_windows;
   const int64_t n_tiles = sai_num_tiles(n_sites);
   const int64_t stride = n_tiles * kTile;
@@ -714,6 +812,461 @@ int sai_engine_rescore_windows(sai_engine* e, sai_host_results* out) {
   if (int rc = check_results(out)) return rc;
   SAI_CUDA_CHECK(cudaSetDevice(e->device));
   return run_windows(e, out);
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// Ingest session (sai_engine_vcf_*): VCF text -> pinned ring slot (host threads) -> cudaMemcpyAsync on
+// the copy stream -> sai_vcf_tiles_device on the compute stream, straight into the engine's tile and
+// position buffers.  A host slot is rewritten once its copy has landed (`copied`), a device slot once
+// the slice in it has been parsed (`parsed`).
+namespace sai {
+
+// tile / position buffers for `cap` sites; `keep`: the sites parsed so far move along
+static int vcf_grow_sites(sai_engine* e, int64_t cap, bool keep) {
+  auto& V = e->vcf;
+  cap = (cap + kTile - 1) / kTile * kTile;
+  if (cap <= V.site_cap) return SAI_OK;
+  const size_t tb = sai_packed_bytes(&V.q.lay, cap), pb = sizeof(int32_t) * (size_t)cap;
+  if (keep) SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));
+  const size_t old_tb = sai_packed_bytes(&V.q.lay, V.site_cap), old_pb = sizeof(int32_t) * (size_t)V.site_cap;
+  for (auto [b, bytes, old] : {std::make_tuple(&e->packed, tb, old_tb), std::make_tuple(&e->pos, pb, old_pb)}) {
+    if (bytes + 256 <= b->cap) continue;
+    void* p = nullptr;
+    cudaError_t ce = cudaMalloc(&p, bytes + 256);
+    if (ce != cudaSuccess) {
+      set_error("cudaMalloc(%zu) failed: %s", bytes + 256, cudaGetErrorString(ce));
+      return SAI_E_NOMEM;
+    }
+    if (keep && old > 0 && b->p) SAI_CUDA_CHECK(cudaMemcpyAsync(p, b->p, old, cudaMemcpyDeviceToDevice, e->s_comp));
+    if (keep) SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));
+    if (b->p) SAI_CUDA_CHECK(cudaFree(b->p));
+    b->p = p;
+    b->cap = bytes + 256;
+  }
+  V.site_cap = cap;
+  return SAI_OK;
+}
+
+// waits until `ev` has completed; any other answer than "not ready" is fatal
+static int vcf_wait(cudaEvent_t ev) {
+  for (;;) {
+    const cudaError_t r = cudaEventQuery(ev);
+    if (r == cudaSuccess) return SAI_OK;
+    if (r != cudaErrorNotReady) {
+      set_error("ingest ring: cudaEventQuery failed: %s", cudaGetErrorString(r));
+      return SAI_E_CUDA;
+    }
+    std::this_thread::sleep_for(std::chrono::microseconds(20));
+  }
+}
+
+static int stage_threads(const sai_engine* e) {
+  return std::min(16, e->host_threads > 0 ? e->host_threads : (int)std::max(1u, std::thread::hardware_concurrency()));
+}
+
+static double now_s() {
+  return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
+}
+
+// The host slot of the next slice, with room for `n` bytes (the ring grows -- after a drain -- when a
+// slice is larger than its slots) and free: the H2D copy of the slice that used it last has landed.
+static int vcf_acquire_slot(sai_engine* e, int64_t n, char** h) {
+  auto& V = e->vcf;
+  if ((size_t)n + 16 > V.slot_bytes) {
+    SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_copy));
+    SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));
+    const size_t want = std::max<size_t>((size_t)n + 16, std::min<size_t>((size_t)V.slice_bytes + 16, 2 * V.slot_bytes + (1u << 20)));
+    const size_t slot = align256(want);
+    if (V.h_ring) SAI_CUDA_CHECK(cudaFreeHost(V.h_ring));
+    V.h_ring = nullptr;
+    V.slot_bytes = 0;
+    SAI_CUDA_CHECK(cudaHostAlloc(reinterpret_cast<void**>(&V.h_ring), slot * V.ring, cudaHostAllocDefault));
+    if (int rc = grow(e->vtext, slot * V.ring)) return rc;
+    if (int rc = grow(e->vscratch, sai_vcf_scratch_bytes(&V.q, (int64_t)slot))) return rc;
+    V.slot_bytes = slot;
+  }
+  while ((int)V.copied.size() < V.ring) {
+    cudaEvent_t a, b;
+    SAI_CUDA_CHECK(cudaEventCreateWithFlags(&a, cudaEventDisableTiming));
+    SAI_CUDA_CHECK(cudaEventCreateWithFlags(&b, cudaEventDisableTiming));
+    V.copied.push_back(a);
+    V.parsed.push_back(b);
+  }
+  const int slot = (int)(V.n_slices % V.ring);
+  if (V.n_slices >= V.ring) {
+    const double t0 = now_s();
+    const int rc = vcf_wait(V.copied[slot]);
+    V.t_wait += now_s() - t0;
+    if (rc) return rc;
+  }
+  *h = V.h_ring + (size_t)slot * V.slot_bytes;
+  return SAI_OK;
+}
+
+// Bytes [off, off + n) of the acquired slot (complete lines) -> device slot (copy stream) -> parse (compute stream).
+static int vcf_launch_slot_impl(sai_engine* e, int64_t off, int64_t n);
+static int vcf_launch_slot(sai_engine* e, int64_t off, int64_t n) {
+  const double t0 = now_s();
+  const int rc = vcf_launch_slot_impl(e, off, n);
+  e->vcf.t_launch += now_s() - t0;
+  return rc;
+}
+static int vcf_launch_slot_impl(sai_engine* e, int64_t off, int64_t n) {
+  auto& V = e->vcf;
+  V.fed += n;
+  const int64_t need = V.fed / V.row_bytes + V.n_slices + 1 + 1024;  // records of normal width in the text so far
+  if (need > V.site_cap)
+    if (int rc = vcf_grow_sites(e, std::max(need, 2 * V.site_cap), true)) return rc;
+  while ((int64_t)V.tev.size() <= V.n_slices) {
+    std::array<cudaEvent_t, 4> t;
+    for (auto& x : t) SAI_CUDA_CHECK(cudaEventCreate(&x));
+    V.tev.push_back(t);
+  }
+  const auto& T = V.tev[V.n_slices];
+  const int slot = (int)(V.n_slices % V.ring);
+  const char* h = V.h_ring + (size_t)slot * V.slot_bytes + off;
+  char* d = static_cast<char*>(e->vtext.p) + (size_t)slot * V.slot_bytes;
+  if (V.n_slices >= V.ring) SAI_CUDA_CHECK(cudaStreamWaitEvent(e->s_copy, V.parsed[slot], 0));
+  SAI_CUDA_CHECK(cudaEventRecord(T[0], e->s_copy));
+  SAI_CUDA_CHECK(cudaMemcpyAsync(d, h, (size_t)n, cudaMemcpyHostToDevice, e->s_copy));
+  SAI_CUDA_CHECK(cudaEventRecord(T[1], e->s_copy));
+  SAI_CUDA_CHECK(cudaEventRecord(V.copied[slot], e->s_copy));
+  SAI_CUDA_CHECK(cudaStreamWaitEvent(e->s_comp, V.copied[slot], 0));
+  SAI_CUDA_CHECK(cudaEventRecord(T[2], e->s_comp));
+  if (int rc = sai_vcf_tiles_device(&V.q, d, n, e->vscratch.p, e->vscratch.cap, e->packed.p, static_cast<int32_t*>(e->pos.p),
+                                    V.site_cap, static_cast<sai_vcf_state*>(e->vstate.p), e->s_comp))
+    return rc;
+  SAI_CUDA_CHECK(cudaEventRecord(T[3], e->s_comp));
+  SAI_CUDA_CHECK(cudaEventRecord(V.parsed[slot], e->s_comp));
+  ++V.n_slices;
+  return SAI_OK;
+}
+
+// host text -> pinned slot, 1 MB parts over the staging threads
+static void staged_copy(sai_engine* e, char* dst, const char* src, size_t n) {
+  const size_t part = 1u << 20;
+  const double t0 = now_s();
+  const std::function<void(int64_t)> f = [&](int64_t i) {
+    const size_t a = (size_t)i * part;
+    memcpy(dst + a, src + a, std::min(part, n - a));
+  };
+  e->vcf.pool.run(stage_threads(e), (int64_t)((n + part - 1) / part), f);
+  e->vcf.t_stage += now_s() - t0;
+}
+
+}  // namespace sai
+
+extern "C" {
+
+int sai_engine_vcf_begin(sai_engine* e, const sai_layout* lay, const char* chrom, int64_t start, int64_t end,
+                         const int32_t* sample_column, int32_t n_out, const int32_t* anc_pos,
+                         const char* anc_allele, int64_t n_anc, int32_t n_file_samples, int64_t text_bytes_hint,
+                         int64_t min_sites) {
+  SAI_REQUIRE(e && lay && chrom && sample_column, "sai_engine_vcf_begin: NULL argument");
+  if (int rc = validate_layout(lay)) return rc;
+  int64_t total = 0;
+  for (int p = 0; p < lay->n_pops; ++p) total += lay->pop[p].n_samples;
+  SAI_REQUIRE(total == n_out, "sai_engine_vcf_begin: n_out %d != individuals of the layout %lld", n_out, (long long)total);
+  const size_t clen = strlen(chrom);
+  SAI_REQUIRE(clen >= 1 && clen < sizeof(sai_vcf_query::chrom), "sai_engine_vcf_begin: chromosome name of %zu bytes (1..255)", clen);
+  SAI_REQUIRE(n_anc >= 0 && (n_anc == 0 || (anc_pos && anc_allele)), "sai_engine_vcf_begin: bad ancestral-allele table");
+  SAI_REQUIRE(n_file_samples >= 0 && text_bytes_hint >= 0 && min_sites >= 0, "sai_engine_vcf_begin: negative size");
+  int32_t max_col = 0;
+  for (int i = 0; i < n_out; ++i) {
+    SAI_REQUIRE(sample_column[i] >= 0, "sai_engine_vcf_begin: negative sample column");
+    max_col = std::max(max_col, sample_column[i]);
+  }
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  auto& V = e->vcf;
+  if (V.state == 1) {  // an unfinished session: let its work drain before its buffers are reused
+    SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_copy));
+    SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));
+  }
+  V.state = 0;
+  e->n_jobs = 0;  // the resident chunk is replaced
+  sai_vcf_query& q = V.q;
+  q = sai_vcf_query{};
+  q.lay = *lay;
+  q.start = start;
+  q.end = end;
+  q.n_anc = n_anc;
+  q.max_column = max_col;
+  q.chrom_len = (int32_t)clen;
+  memcpy(q.chrom, chrom, clen);
+  if (int rc = grow(e->vcols, sizeof(int32_t) * (size_t)n_out)) return rc;
+  SAI_CUDA_CHECK(cudaMemcpy(e->vcols.p, sample_column, sizeof(int32_t) * (size_t)n_out, cudaMemcpyHostToDevice));
+  q.sample_column = static_cast<const int32_t*>(e->vcols.p);
+  if (n_anc > 0) {
+    if (int rc = grow(e->vanc_pos, sizeof(int32_t) * (size_t)n_anc)) return rc;
+    if (int rc = grow(e->vanc_all, 8 * (size_t)n_anc)) return rc;
+    SAI_CUDA_CHECK(cudaMemcpy(e->vanc_pos.p, anc_pos, sizeof(int32_t) * (size_t)n_anc, cudaMemcpyHostToDevice));
+    SAI_CUDA_CHECK(cudaMemcpy(e->vanc_all.p, anc_allele, 8 * (size_t)n_anc, cudaMemcpyHostToDevice));
+    q.anc_pos = static_cast<const int32_t*>(e->vanc_pos.p);
+    q.anc_allele = static_cast<const char*>(e->vanc_all.p);
+  }
+  if (int rc = grow(e->vstate, sizeof(sai_vcf_state))) return rc;
+  SAI_CUDA_CHECK(cudaMemsetAsync(e->vstate.p, 0, sizeof(sai_vcf_state), e->s_comp));
+  V.row_bytes = std::max<int64_t>(64, 2 * (int64_t)n_file_samples + 18);
+  V.site_cap = 0;  // the buffers' content is not kept from an earlier chunk
+  if (int rc = vcf_grow_sites(e, std::max(text_bytes_hint / V.row_bytes + 1024, min_sites), false)) return rc;
+  if (V.slot_bytes > 0)  // the scratch depends on the query (max_column): resize for the ring's slots
+    if (int rc = grow(e->vscratch, sai_vcf_scratch_bytes(&q, (int64_t)V.slot_bytes))) return rc;
+  V.fed = V.n_slices = 0;
+  V.t_stage = V.t_wait = V.t_launch = V.t_feed = 0;
+  V.carry.clear();
+  V.sticky_rc = SAI_OK;
+  V.state = 1;
+  return SAI_OK;
+}
+
+static int vcf_feed_impl(sai_engine* e, const char* text, int64_t len, int64_t* consumed);
+int sai_engine_vcf_feed(sai_engine* e, const char* text, int64_t len, int64_t* consumed) {
+  const double t0 = now_s();
+  const int rc = vcf_feed_impl(e, text, len, consumed);
+  if (e) e->vcf.t_feed += now_s() - t0;
+  return rc;
+}
+static int vcf_feed_impl(sai_engine* e, const char* text, int64_t len, int64_t* consumed) {
+  SAI_REQUIRE(e && consumed && len >= 0 && (len == 0 || text), "sai_engine_vcf_feed: bad argument");
+  *consumed = 0;
+  auto& V = e->vcf;
+  SAI_REQUIRE(V.state == 1, "sai_engine_vcf_feed: no ingest session (sai_engine_vcf_begin)");
+  if (V.sticky_rc) return V.sticky_rc;
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  const void* last = len > 0 ? memrchr(text, '\n', (size_t)len) : nullptr;
+  if (!last) return SAI_OK;
+  const int64_t complete = static_cast<const char*>(last) - text + 1;
+  int64_t at = 0;
+  while (at < complete) {
+    const int64_t want = std::min<int64_t>(complete - at, V.slice_bytes);
+    int64_t cut = at + want;
+    if (cut < complete) {  // end the slice after its last complete line; a longer line makes a longer slice
+      const void* nl = memrchr(text + at, '\n', (size_t)want);
+      if (!nl) nl = memchr(text + cut, '\n', (size_t)(complete - cut));
+      cut = static_cast<const char*>(nl) - text + 1;
+    }
+    if (cut - at >= (int64_t(1) << 31)) {
+      set_error("sai_engine_vcf_feed: a line of more than 2 GB");
+      V.sticky_rc = SAI_E_ARG;
+      return SAI_E_ARG;
+    }
+    char* h = nullptr;
+    int rc = vcf_acquire_slot(e, cut - at, &h);
+    if (rc == SAI_OK) {
+      staged_copy(e, h, text + at, (size_t)(cut - at));
+      rc = vcf_launch_slot(e, 0, cut - at);
+    }
+    if (rc) {
+      V.sticky_rc = rc;
+      return rc;
+    }
+    at = cut;
+  }
+  *consumed = complete;
+  return SAI_OK;
+}
+
+int sai_engine_vcf_finish(sai_engine* e, int64_t* n_sites, int32_t* max_value, int32_t* pos_out, int64_t pos_cap) {
+  SAI_REQUIRE(e && n_sites && max_value, "sai_engine_vcf_finish: NULL argument");
+  auto& V = e->vcf;
+  SAI_REQUIRE(V.state == 1, "sai_engine_vcf_finish: no ingest session (sai_engine_vcf_begin)");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  V.state = 0;
+  const double t_sync = now_s();
+  const cudaError_t c1 = cudaStreamSynchronize(e->s_copy), c2 = cudaStreamSynchronize(e->s_comp);
+  double h2d = 0, parse = 0, span = 0;
+  float ms = 0;
+  for (int64_t k = 0; c1 == cudaSuccess && c2 == cudaSuccess && k < V.n_slices; ++k) {
+    const auto& T = V.tev[k];
+    if (cudaEventElapsedTime(&ms, T[0], T[1]) == cudaSuccess) h2d += ms / 1e3;
+    if (cudaEventElapsedTime(&ms, T[2], T[3]) == cudaSuccess) parse += ms / 1e3;
+  }
+  if (c1 == cudaSuccess && c2 == cudaSuccess && V.n_slices > 0 &&
+      cudaEventElapsedTime(&ms, V.tev[0][0], V.tev[V.n_slices - 1][3]) == cudaSuccess)
+    span = ms / 1e3;
+  const double stats[10] = {V.t_stage, V.t_wait, h2d, parse, span, (double)V.n_slices, (double)V.fed, now_s() - t_sync,
+                            V.t_launch, V.t_feed};
+  memcpy(V.stats, stats, sizeof(stats));
+  if (V.sticky_rc) {
+    set_error("ingest session failed earlier (code %d)", V.sticky_rc);
+    return V.sticky_rc;
+  }
+  if (c1 != cudaSuccess || c2 != cudaSuccess) {
+    set_error("ingest session: %s", cudaGetErrorString(c1 != cudaSuccess ? c1 : c2));
+    return SAI_E_CUDA;
+  }
+  sai_vcf_state st;
+  SAI_CUDA_CHECK(cudaMemcpy(&st, e->vstate.p, sizeof(st), cudaMemcpyDeviceToHost));
+  *n_sites = st.n_sites;
+  const sai_layout& lay = V.q.lay;
+  bool fits = true;
+  for (int p = 0; p < lay.n_pops; ++p) {
+    max_value[p] = std::max(lay.pop[p].ploidy, st.vmax[p]);
+    if (max_value[p] > (1 << lay.pop[p].bits) - 2) fits = false;
+  }
+  if (st.overflow) {
+    set_error("more records than the ingest buffers hold (%lld sites, room for %lld)", (long long)st.n_sites,
+              (long long)V.site_cap);
+    return SAI_E_CAPACITY;
+  }
+  if (!fits) {
+    set_error("a genotype value does not fit the bit-planes of its population");
+    return SAI_E_DOMAIN;
+  }
+  if (pos_out && pos_cap >= st.n_sites && st.n_sites > 0)
+    SAI_CUDA_CHECK(cudaMemcpy(pos_out, e->pos.p, sizeof(int32_t) * (size_t)st.n_sites, cudaMemcpyDeviceToHost));
+  e->n_sites = st.n_sites;
+  e->lay = lay;
+  e->n_jobs = 0;
+  e->W = 0;
+  V.state = 2;
+  return SAI_OK;
+}
+
+int sai_engine_score_loaded(sai_engine* e, const int64_t* win_start, const int64_t* win_end, int64_t n_windows,
+                            const sai_job* jobs, int32_t n_jobs, sai_host_results* out) {
+  SAI_REQUIRE(e && e->vcf.state == 2, "sai_engine_score_loaded: no finished ingest session");
+  if (int rc = validate_jobs(&e->lay, jobs, n_jobs)) return rc;
+  if (int rc = check_results(out)) return rc;
+  SAI_REQUIRE(n_windows >= 0 && (n_windows == 0 || (win_start && win_end)), "NULL windows");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  const int64_t W = n_windows;
+  const int64_t n_tiles = sai_num_tiles(e->n_sites);
+  const int64_t stride = n_tiles * kTile;
+  const ResLayout rl = res_layout(W, n_jobs);
+  if (int rc = grow(e->win, sizeof(int64_t) * 2 * (size_t)W + 256)) return rc;
+  if (int rc = grow(e->mask, sizeof(uint32_t) * 2 * (size_t)n_jobs * n_tiles + 256)) return rc;
+  if (int rc = grow(e->qval, sizeof(double) * (size_t)n_jobs * stride + 256)) return rc;
+  if (int rc = grow(e->res, rl.total + 256)) return rc;
+  e->W = W;
+  e->n_jobs = n_jobs;
+  for (int j = 0; j < n_jobs; ++j) e->jobs[j] = jobs[j];
+  int64_t* d_ws = static_cast<int64_t*>(e->win.p);
+  if (W > 0) {
+    SAI_CUDA_CHECK(cudaMemcpyAsync(d_ws, win_start, sizeof(int64_t) * W, cudaMemcpyHostToDevice, e->s_comp));
+    SAI_CUDA_CHECK(cudaMemcpyAsync(d_ws + W, win_end, sizeof(int64_t) * W, cudaMemcpyHostToDevice, e->s_comp));
+  }
+  uint32_t* d_mask_u = static_cast<uint32_t*>(e->mask.p);
+  if (n_tiles > 0)
+    if (int rc = sai_site_flags(&e->lay, e->packed.p, 0, n_tiles, n_tiles, jobs, n_jobs, d_mask_u,
+                                d_mask_u + (size_t)n_jobs * n_tiles, static_cast<double*>(e->qval.p), stride, nullptr,
+                                nullptr, 0, 0, e->s_comp))
+      return rc;
+  return run_windows(e, out);
+}
+
+static int vcf_feed_bgzf_impl(sai_engine* e, const uint8_t* data, const int64_t* block_off, const int64_t* out_off,
+                              int64_t n_blocks, int64_t skip);
+int sai_engine_vcf_feed_bgzf(sai_engine* e, const uint8_t* data, const int64_t* block_off, const int64_t* out_off,
+                             int64_t n_blocks, int64_t skip) {
+  const double t0 = now_s();
+  const int rc = vcf_feed_bgzf_impl(e, data, block_off, out_off, n_blocks, skip);
+  if (e) e->vcf.t_feed += now_s() - t0;
+  return rc;
+}
+static int vcf_feed_bgzf_impl(sai_engine* e, const uint8_t* data, const int64_t* block_off, const int64_t* out_off,
+                              int64_t n_blocks, int64_t skip) {
+  SAI_REQUIRE(e && n_blocks >= 0 && skip >= 0 && (n_blocks == 0 || (data && block_off && out_off)),
+              "sai_engine_vcf_feed_bgzf: bad argument");
+  auto& V = e->vcf;
+  SAI_REQUIRE(V.state == 1, "sai_engine_vcf_feed_bgzf: no ingest session (sai_engine_vcf_begin)");
+  if (V.sticky_rc) return V.sticky_rc;
+  if (n_blocks == 0) return SAI_OK;
+  SAI_REQUIRE(out_off[0] == 0 && skip <= out_off[n_blocks], "sai_engine_vcf_feed_bgzf: bad text offsets");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  auto fail = [&](int rc) {
+    V.sticky_rc = rc;
+    return rc;
+  };
+  // the block that holds text offset `skip`
+  int64_t b = std::upper_bound(out_off, out_off + n_blocks + 1, skip) - out_off - 1;
+  int64_t from = skip;  // first text offset of the records (inside block b)
+  V.carry.clear();
+  while (b < n_blocks) {
+    // a group of blocks with at most slice_bytes of text (at least one block), inflated by the staging
+    // threads straight into the slot behind the incomplete line carried from the previous group
+    // (carry + text + 1 within the slice size: the ring slots are not reallocated slice after slice)
+    const int64_t c = (int64_t)V.carry.size();
+    int64_t b1 = b + 1;
+    while (b1 < n_blocks && c + out_off[b1 + 1] - out_off[b] + 1 <= V.slice_bytes) ++b1;
+    SAI_REQUIRE(out_off[b1] >= out_off[b], "sai_engine_vcf_feed_bgzf: text offsets are not monotonic");
+    const int64_t text = out_off[b1] - out_off[b];
+    SAI_REQUIRE(c + text + 1 < (int64_t(1) << 31), "sai_engine_vcf_feed_bgzf: a line of more than 2 GB");
+    char* h = nullptr;
+    if (int rc = vcf_acquire_slot(e, c + text + 1, &h)) return fail(rc);
+    if (c) memcpy(h, V.carry.data(), (size_t)c);
+    const double t0 = now_s();
+    constexpr int64_t kGroup = 16;  // blocks per task (~1 MB of text)
+    std::atomic<int> bad_rc{SAI_OK};
+    std::mutex msg_mu;
+    std::string msg;
+    const std::function<void(int64_t)> f = [&](int64_t i) {
+      const int64_t g0 = b + i * kGroup, g1 = std::min(b1, g0 + kGroup);
+      int64_t rel[kGroup + 1];
+      for (int64_t k = g0; k <= g1; ++k) rel[k - g0] = out_off[k] - out_off[b] + c;
+      const int rc = sai_bgzf_inflate(data, block_off + g0, rel, g1 - g0, reinterpret_cast<uint8_t*>(h), 1);
+      if (rc != SAI_OK) {
+        std::lock_guard<std::mutex> lk(msg_mu);
+        if (bad_rc.load() == SAI_OK) msg = sai_last_error();
+        bad_rc.store(rc);
+      }
+    };
+    V.pool.run(stage_threads(e), (b1 - b + kGroup - 1) / kGroup, f);
+    V.t_stage += now_s() - t0;
+    if (bad_rc.load() != SAI_OK) {
+      set_error("%s", msg.c_str());
+      return fail(bad_rc.load());
+    }
+    const int64_t lo = c == 0 && from > out_off[b] ? from - out_off[b] : 0;  // the header stays behind
+    int64_t end = c + text;
+    if (b1 == n_blocks && end > lo && h[end - 1] != '\n') h[end++] = '\n';  // last line without a newline
+    const void* nl = end > lo ? memrchr(h + lo, '\n', (size_t)(end - lo)) : nullptr;
+    const int64_t cut = nl ? static_cast<const char*>(nl) - h + 1 : lo;
+    std::vector<char> rest(h + cut, h + end);  // the incomplete last line, carried into the next slot
+    if (cut > lo)
+      if (int rc = vcf_launch_slot(e, lo, cut - lo)) return fail(rc);
+    V.carry.swap(rest);
+    b = b1;
+    from = out_off[b];
+  }
+  return SAI_OK;
+}
+
+int sai_engine_vcf_stats(const sai_engine* e, double* out, int32_t n) {
+  SAI_REQUIRE(e && out && n >= 0, "sai_engine_vcf_stats: bad argument");
+  for (int i = 0; i < n && i < 10; ++i) out[i] = e->vcf.stats[i];
+  return SAI_OK;
+}
+
+int sai_engine_set_vcf_slicing(sai_engine* e, int64_t slice_bytes, int32_t ring) {
+  SAI_REQUIRE(e, "NULL engine");
+  auto& V = e->vcf;
+  SAI_REQUIRE(V.state != 1, "sai_engine_set_vcf_slicing: an ingest session is feeding");
+  SAI_REQUIRE(slice_bytes <= 0 || (slice_bytes >= 64 && slice_bytes < (int64_t(1) << 30)), "slice size outside [64, 2^30)");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  V.slice_bytes = slice_bytes > 0 ? slice_bytes : (32ll << 20);
+  const int r = ring > 0 ? std::max(2, (int)ring) : 4;
+  // new geometry: the slots are reallocated by the next slice
+  SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_copy));
+  SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));
+  if (V.h_ring) SAI_CUDA_CHECK(cudaFreeHost(V.h_ring));
+  V.h_ring = nullptr;
+  V.slot_bytes = 0;
+  V.ring = r;
+  return SAI_OK;
+}
+
+int64_t sai_engine_vcf_slices(const sai_engine* e) { return e ? e->vcf.n_slices : 0; }
+
+int sai_engine_loaded_tiles(sai_engine* e, uint8_t* out, uint64_t cap) {
+  SAI_REQUIRE(e && e->vcf.state == 2, "sai_engine_loaded_tiles: no finished ingest session");
+  const uint64_t bytes = sai_packed_bytes(&e->lay, e->n_sites);
+  SAI_REQUIRE(cap >= bytes && (bytes == 0 || out), "sai_engine_loaded_tiles: %llu bytes needed", (unsigned long long)bytes);
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  if (bytes) SAI_CUDA_CHECK(cudaMemcpy(out, e->packed.p, bytes, cudaMemcpyDeviceToHost));
+  return SAI_OK;
 }
 
 }  // extern "C"

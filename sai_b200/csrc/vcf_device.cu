@@ -1,0 +1,497 @@
+// Device VCF genotype parser: VCF text resident in HBM -> tiled bit-planes + positions.
+//
+// The host parser (vcf_parse.cu: GtParser::scan / parse_record / gt_sum) is the specification; this
+// file reproduces it record for record and value for value on one text slice (any run of complete
+// lines) per sai_vcf_tiles_device call:
+//   1. newline index: per 8 KB segment a newline count, an exclusive scan, then the line ends in
+//      file order (per-thread counts, warp ballot / popc ranks, block scan);
+//   2. record pass, one warp per line: empty and '#' lines skipped, a trailing '\r' stripped, the
+//      first nine tabs found with ballots, then CHROM / POS / region / REF / first ALT /
+//      ancestral-allele table (binary search, flip when ALT is ancestral) / GT index in FORMAT;
+//      a record without a sample column (fewer than nine tabs) is dropped, as the host drops it;
+//   3. site numbering: per 1024 lines a keep count, an exclusive scan that also advances the
+//      device-side site counter of sai_vcf_state (slices chain without a host sync), then the
+//      kept lines in file order and pos[site];
+//   4. genotype pass, one warp per kept record: lane j parses individual 32g + j of every group of
+//      every population into the allele sum (gt_sum semantics), one __ballot_sync per bit-plane
+//      gives the plane word.  A record whose fields are all three characters wide (the regular
+//      `x|y` diploid record, GT first) is addressed directly at samples + 4*col; any other record
+//      first has its field offsets written to the warp's scratch row by a cooperative tab scan;
+//   5. the sites behind the last one written, up to the end of its tile, are coded all-missing --
+//      so after every call the tiles are exactly what sai_pack_i8_all writes for the sites so far.
+#include <string.h>
+
+#include "common.cuh"
+
+namespace sai {
+
+namespace {
+
+constexpr int kSegBytes = 8192;       // newline pass: bytes per block (256 threads x 32 bytes)
+constexpr int kLinesPerChunk = 1024;  // site numbering: lines per block
+constexpr int kWarpsPerBlock = 8;
+
+struct SliceInfo {
+  int32_t n_lines;
+  int32_t n_kept;
+  int64_t site_base;
+};
+
+struct Scratch {
+  SliceInfo* info;
+  int32_t* seg_cnt;   // [n_seg]
+  int32_t* seg_off;   // [n_seg]
+  int32_t* line_end;  // [len]
+  int32_t* rec_samp;  // [len] offset of the first sample field
+  int32_t* rec_end;   // [len] end of the line ('\r' stripped)
+  int32_t* rec_pos;   // [len]
+  int32_t* rec_meta;  // [len] bit 0 keep, bit 1 flip, bits 2.. GT index
+  int32_t* chunk_cnt; // [n_chunk]
+  int32_t* chunk_off; // [n_chunk]
+  int32_t* kept;      // line index of the slice's k-th kept record: reuses line_end, which only the record pass reads
+  int32_t* fields;    // [n_geno_warps][max_column + 1] field offsets of irregular records
+};
+
+inline size_t al(size_t x) { return (x + 255) & ~size_t(255); }
+
+int geno_warps() { return sm_count() * 4 * kWarpsPerBlock; }
+
+// byte size of the scratch and, when base != null, its carving
+size_t carve(const sai_vcf_query& q, int64_t len, char* base, Scratch* s) {
+  const size_t n_seg = (size_t)((len + kSegBytes - 1) / kSegBytes) + 1;
+  const size_t n_line = (size_t)len + 1;
+  const size_t n_chunk = n_line / kLinesPerChunk + 2;
+  size_t at = 0;
+  auto take = [&](size_t bytes) {
+    char* p = base ? base + at : nullptr;
+    at += al(bytes);
+    return p;
+  };
+  Scratch t;
+  t.info = reinterpret_cast<SliceInfo*>(take(sizeof(SliceInfo)));
+  t.seg_cnt = reinterpret_cast<int32_t*>(take(4 * n_seg));
+  t.seg_off = reinterpret_cast<int32_t*>(take(4 * n_seg));
+  t.line_end = reinterpret_cast<int32_t*>(take(4 * n_line));
+  t.rec_samp = reinterpret_cast<int32_t*>(take(4 * n_line));
+  t.rec_end = reinterpret_cast<int32_t*>(take(4 * n_line));
+  t.rec_pos = reinterpret_cast<int32_t*>(take(4 * n_line));
+  t.rec_meta = reinterpret_cast<int32_t*>(take(4 * n_line));
+  t.chunk_cnt = reinterpret_cast<int32_t*>(take(4 * n_chunk));
+  t.chunk_off = reinterpret_cast<int32_t*>(take(4 * n_chunk));
+  t.kept = t.line_end;
+  t.fields = reinterpret_cast<int32_t*>(take(4 * (size_t)geno_warps() * (size_t)(q.max_column + 1)));
+  if (s) *s = t;
+  return at;
+}
+
+// ---- block-wide exclusive scan of one int per thread (blockDim.x multiple of 32, <= 1024) ----
+__device__ int block_excl_scan(int v, int* total) {
+  __shared__ int warp_sum[32];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  int x = v;
+  for (int d = 1; d < 32; d <<= 1) {
+    const int y = __shfl_up_sync(0xffffffffu, x, d);
+    if (lane >= d) x += y;
+  }
+  if (lane == 31) warp_sum[w] = x;
+  __syncthreads();
+  if (w == 0) {
+    int s = lane < nw ? warp_sum[lane] : 0;
+    for (int d = 1; d < 32; d <<= 1) {
+      const int y = __shfl_up_sync(0xffffffffu, s, d);
+      if (lane >= d) s += y;
+    }
+    if (lane < nw) warp_sum[lane] = s;  // inclusive
+  }
+  __syncthreads();
+  const int before = (w > 0 ? warp_sum[w - 1] : 0) + x - v;
+  *total = warp_sum[nw - 1];
+  __syncthreads();  // warp_sum is reused by the next call
+  return before;
+}
+
+// ---- 1. newline index ----------------------------------------------------------------------
+// 32 bytes per thread: bitmask of '\n' (the slot base is 256-byte aligned and segments are 8 KB,
+// so the two 16-byte loads are aligned)
+__device__ inline uint32_t nl_mask32(const char* text, int64_t len, int64_t at) {
+  uint32_t m = 0;
+  if (at + 32 <= len) {
+    const uint4* p = reinterpret_cast<const uint4*>(text + at);
+    const uint4 a = __ldg(p), b = __ldg(p + 1);
+    const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+#pragma unroll
+    for (int k = 0; k < 8; ++k)
+#pragma unroll
+      for (int c = 0; c < 4; ++c)
+        if (((w[k] >> (8 * c)) & 0xff) == '\n') m |= 1u << (4 * k + c);
+  } else {
+    for (int k = 0; k < 32 && at + k < len; ++k)
+      if (text[at + k] == '\n') m |= 1u << k;
+  }
+  return m;
+}
+
+__global__ void __launch_bounds__(256) k_nl_count(const char* __restrict__ text, int64_t len, Scratch s) {
+  const int64_t at = (int64_t)blockIdx.x * kSegBytes + 32 * threadIdx.x;
+  const int c = at < len ? __popc(nl_mask32(text, len, at)) : 0;
+  int total;
+  block_excl_scan(c, &total);
+  if (threadIdx.x == 0) s.seg_cnt[blockIdx.x] = total;
+}
+
+// exclusive scan of n ints by one block; *total (optional) = sum
+__device__ void scan_one_block(const int32_t* in, int32_t* out, int n, int32_t* total) {
+  int carry = 0;
+  for (int base = 0; base < n; base += blockDim.x) {
+    const int i = base + threadIdx.x;
+    const int v = i < n ? in[i] : 0;
+    int sum;
+    const int ex = block_excl_scan(v, &sum);
+    if (i < n) out[i] = carry + ex;
+    carry += sum;
+  }
+  if (total && threadIdx.x == 0) *total = carry;
+}
+
+__global__ void __launch_bounds__(1024) k_seg_scan(int n_seg, Scratch s) {
+  scan_one_block(s.seg_cnt, s.seg_off, n_seg, &s.info->n_lines);
+}
+
+__global__ void __launch_bounds__(256) k_nl_write(const char* __restrict__ text, int64_t len, Scratch s) {
+  const int64_t at = (int64_t)blockIdx.x * kSegBytes + 32 * threadIdx.x;
+  uint32_t m = at < len ? nl_mask32(text, len, at) : 0;
+  int total;
+  int r = s.seg_off[blockIdx.x] + block_excl_scan(__popc(m), &total);
+  while (m) {
+    const int b = __ffs(m) - 1;
+    m &= m - 1;
+    s.line_end[r++] = (int32_t)(at + b);
+  }
+}
+
+// ---- 2. record pass ---------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) k_records(const char* __restrict__ text, const __grid_constant__ sai_vcf_query q,
+                                                 Scratch s) {
+  __shared__ int32_t tabs[kWarpsPerBlock][9];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int n_lines = s.info->n_lines;
+  const int64_t n_warps = (int64_t)gridDim.x * kWarpsPerBlock;
+  for (int64_t i = (int64_t)blockIdx.x * kWarpsPerBlock + wib; i < n_lines; i += n_warps) {
+    const int32_t ls = i > 0 ? s.line_end[i - 1] + 1 : 0;
+    int32_t le = s.line_end[i];
+    if (le > ls && text[le - 1] == '\r') --le;
+    int meta = 0, samp = 0, pos32 = 0;
+    if (le > ls && text[ls] != '#') {
+      // the first nine tabs of the line
+      int n_tab = 0;
+      for (int32_t c = ls; c < le && n_tab < 9; c += 32) {
+        const bool t = c + lane < le && text[c + lane] == '\t';
+        const uint32_t m = __ballot_sync(0xffffffffu, t);
+        const int r = n_tab + __popc(m & ((1u << lane) - 1));
+        if (t && r < 9) tabs[wib][r] = c + lane;
+        n_tab += __popc(m);
+      }
+      __syncwarp();
+      if (lane == 0 && n_tab >= 9) {
+        const int32_t* T = tabs[wib];
+        bool keep = T[0] - ls == q.chrom_len;
+        for (int k = 0; keep && k < q.chrom_len; ++k) keep = text[ls + k] == q.chrom[k];
+        int64_t pos = 0;
+        for (int32_t p = T[0] + 1; p < T[1]; ++p)
+          pos = (int64_t)((uint64_t)pos * 10u + (uint64_t)(int64_t)((signed char)text[p] - '0'));
+        if (keep && q.start <= q.end && (pos < q.start || pos > q.end)) keep = false;
+        bool flip = false;
+        if (keep && q.n_anc > 0) {
+          const int32_t key = (int32_t)pos;
+          int64_t lo = 0, hi = q.n_anc;  // lower_bound
+          while (lo < hi) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (q.anc_pos[mid] < key) lo = mid + 1; else hi = mid;
+          }
+          if (lo == q.n_anc || q.anc_pos[lo] != key) {
+            keep = false;
+          } else {
+            const char* a = q.anc_allele + 8 * lo;
+            int alen = 0;
+            while (alen < 8 && a[alen]) ++alen;
+            const int32_t ref = T[2] + 1, ref_len = T[3] - ref;
+            const int32_t alt = T[3] + 1;
+            int32_t alt_end = T[4];
+            for (int32_t p = alt; p < T[4]; ++p)
+              if (text[p] == ',') {
+                alt_end = p;
+                break;
+              }
+            bool is_ref = ref_len == alen, is_alt = alt_end - alt == alen;
+            for (int k = 0; k < alen; ++k) {
+              is_ref = is_ref && text[ref + k] == a[k];
+              is_alt = is_alt && text[alt + k] == a[k];
+            }
+            if (!is_ref && !is_alt) keep = false;
+            flip = is_alt;
+          }
+        }
+        int gi = 0;
+        if (keep) {  // index of the first FORMAT key that is exactly "GT" (0 if none)
+          int k = 0;
+          for (int32_t p = T[7] + 1; p < T[8];) {
+            int32_t ke = p;
+            while (ke < T[8] && text[ke] != ':') ++ke;
+            if (ke - p == 2 && text[p] == 'G' && text[p + 1] == 'T') {
+              gi = k;
+              break;
+            }
+            p = ke + 1;
+            ++k;
+          }
+        }
+        meta = keep ? (1 | (flip ? 2 : 0) | (gi << 2)) : 0;
+        samp = T[8] + 1;
+        pos32 = (int32_t)pos;
+      }
+    }
+    if (lane == 0) {
+      s.rec_meta[i] = meta;
+      s.rec_samp[i] = samp;
+      s.rec_end[i] = le;
+      s.rec_pos[i] = pos32;
+    }
+    __syncwarp();
+  }
+}
+
+// ---- 3. site numbering ------------------------------------------------------------------------
+__global__ void __launch_bounds__(kLinesPerChunk) k_keep_count(Scratch s) {
+  const int n_lines = s.info->n_lines;
+  const int n_chunk = (n_lines + kLinesPerChunk - 1) / kLinesPerChunk;
+  for (int c = blockIdx.x; c < n_chunk; c += gridDim.x) {
+    const int i = c * kLinesPerChunk + threadIdx.x;
+    int total;
+    block_excl_scan(i < n_lines ? (s.rec_meta[i] & 1) : 0, &total);
+    if (threadIdx.x == 0) s.chunk_cnt[c] = total;
+  }
+}
+
+__global__ void __launch_bounds__(1024) k_keep_scan(Scratch s, sai_vcf_state* st, int64_t site_cap) {
+  const int n_chunk = (s.info->n_lines + kLinesPerChunk - 1) / kLinesPerChunk;
+  scan_one_block(s.chunk_cnt, s.chunk_off, n_chunk, &s.info->n_kept);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    const int64_t base = st->n_sites;
+    s.info->site_base = base;
+    st->n_sites = base + s.info->n_kept;
+    if (base + s.info->n_kept > site_cap) st->overflow = 1;
+  }
+}
+
+__global__ void __launch_bounds__(kLinesPerChunk) k_keep_write(Scratch s, int32_t* __restrict__ pos, int64_t site_cap) {
+  const int n_lines = s.info->n_lines;
+  const int n_chunk = (n_lines + kLinesPerChunk - 1) / kLinesPerChunk;
+  const int64_t base = s.info->site_base;
+  for (int c = blockIdx.x; c < n_chunk; c += gridDim.x) {
+    const int i = c * kLinesPerChunk + threadIdx.x;
+    const int keep = i < n_lines ? (s.rec_meta[i] & 1) : 0;
+    int total;
+    const int k = s.chunk_off[c] + block_excl_scan(keep, &total);
+    if (keep) {
+      s.kept[k] = i;
+      if (base + k < site_cap) pos[base + k] = s.rec_pos[i];
+    }
+  }
+}
+
+// ---- 4. genotype pass -------------------------------------------------------------------------
+// gt_sum of vcf_parse.cu: GT sub-field of the field at p (ends at a tab or at lend), cut / padded
+// to `ploidy` alleles, "." and junk = -1, flipped |a - 1|, summed, clamped to int8
+__device__ inline int gt_sum_dev(const char* p, const char* lend, int gt_index, int ploidy, bool flip) {
+  for (int k = 0; k < gt_index; ++k) {
+    while (p < lend && *p != ':' && *p != '\t') ++p;
+    if (p < lend && *p == ':') ++p;
+  }
+  int sum = 0;
+  bool open = p < lend && *p != '\t' && *p != ':';
+  for (int n = 0; n < ploidy; ++n) {
+    int a = -1;
+    if (open) {
+      int v = 0;
+      bool digits = false, junk = false;
+      while (p < lend) {
+        const char c = *p;
+        if (c == '/' || c == '|' || c == ':' || c == '\t') break;
+        if (c >= '0' && c <= '9' && !junk) {
+          v = v * 10 + (c - '0');
+          digits = true;
+        } else {
+          junk = true;
+        }
+        ++p;
+      }
+      if (digits && !junk) a = v;
+      if (p < lend && (*p == '/' || *p == '|'))
+        ++p;
+      else
+        open = false;
+    }
+    if (flip) a = a > 0 ? a - 1 : 1 - a;
+    sum += a;
+  }
+  return sum < -128 ? -128 : (sum > 127 ? 127 : sum);
+}
+
+__device__ inline uint32_t* word_at(void* tiles, int pps, int64_t site, int w) {
+  const int64_t T = site >> 5;
+  const int sl = (int)(site & 31);
+  return reinterpret_cast<uint32_t*>(static_cast<char*>(tiles) + ((T * pps + (w >> 1)) * 32 + sl) * 8 + (w & 1) * 4);
+}
+
+__global__ void __launch_bounds__(256) k_genotypes(const char* __restrict__ text, const __grid_constant__ sai_vcf_query q,
+                                                   Scratch s, void* __restrict__ tiles, int64_t site_cap,
+                                                   sai_vcf_state* st) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = (int64_t)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
+  const int64_t n_warps = (int64_t)gridDim.x * kWarpsPerBlock;
+  const int n_kept = s.info->n_kept;
+  const int64_t base = s.info->site_base;
+  const int row = q.max_column + 1;
+  int32_t* fo = s.fields + warp * row;
+  const int pps = q.lay.pairs_per_site;
+  for (int64_t k = warp; k < n_kept; k += n_warps) {
+    const int64_t site = base + k;
+    if (site >= site_cap) break;  // reported through st->overflow
+    const int line = s.kept[k];
+    const int meta = s.rec_meta[line];
+    const bool flip = (meta & 2) != 0;
+    const int gi = meta >> 2;
+    const char* S = text + s.rec_samp[line];
+    const int32_t L = s.rec_end[line] - s.rec_samp[line];  // bytes of the sample columns (>= 0)
+    const char* lend = S + L;
+    // regular record: tabs exactly at offsets 3, 7, 11, ... -> field c at 4c
+    bool regular = gi == 0 && L > 0 && ((L + 1) & 3) == 0;
+    for (int32_t c = 0; regular && c < L; c += 32) {
+      const int32_t i = c + lane;
+      const bool bad = i < L && ((S[i] == '\t') != ((i & 3) == 3));
+      if (__any_sync(0xffffffffu, bad)) regular = false;
+    }
+    int32_t n_fields;
+    if (regular) {
+      n_fields = (L + 1) >> 2;
+    } else {
+      // field offsets of columns 0..max_column; a field exists behind every tab (possibly empty)
+      n_fields = L > 0 ? 1 : 0;
+      if (lane == 0 && L > 0) fo[0] = 0;
+      for (int32_t c = 0; c < L && n_fields < row; c += 32) {
+        const int32_t i = c + lane;
+        const bool t = i < L && S[i] == '\t';
+        const uint32_t m = __ballot_sync(0xffffffffu, t);
+        const int r = n_fields + __popc(m & ((1u << lane) - 1));
+        if (t && r < row) fo[r] = i + 1;
+        n_fields += __popc(m);
+      }
+      __syncwarp();
+    }
+    int col_base = 0;
+    for (int p = 0; p < q.lay.n_pops; ++p) {
+      const sai_pop_layout& P = q.lay.pop[p];
+      const int B = P.bits, miss = (1 << B) - 1;
+      int vmax = 0;
+      for (int g = 0; g < P.n_groups; ++g) {
+        const int ind = 32 * g + lane;
+        uint32_t code = (uint32_t)miss;
+        if (ind < P.n_samples) {
+          const int col = q.sample_column[col_base + ind];
+          int v;
+          if (col >= n_fields) {
+            v = -P.ploidy;  // column absent: all alleles missing, never flipped
+          } else {
+            const int32_t f = regular ? 4 * col : fo[col];
+            v = gt_sum_dev(S + f, lend, gi, P.ploidy, flip);
+          }
+          if (v >= 0) {
+            code = (uint32_t)v;
+            vmax = max(vmax, v);
+          }
+        }
+        const int w0 = 2 * P.pair_off + g * B;
+        for (int b = 0; b < B; ++b) {
+          const uint32_t word = __ballot_sync(0xffffffffu, (code >> b) & 1u);
+          if (lane == b) *word_at(tiles, pps, site, w0 + b) = word;
+        }
+      }
+      if ((P.n_groups * B) & 1)
+        if (lane == 0) *word_at(tiles, pps, site, 2 * P.pair_off + P.n_groups * B) = 0u;  // the pad word
+      for (int d = 16; d > 0; d >>= 1) vmax = max(vmax, __shfl_xor_sync(0xffffffffu, vmax, d));
+      if (lane == 0 && vmax > P.ploidy) atomicMax(&st->vmax[p], vmax);
+      col_base += P.n_samples;
+    }
+  }
+}
+
+// ---- 5. padding sites behind the last site, to the end of its tile -----------------------------
+__global__ void k_pad_tail(const __grid_constant__ sai_layout lay, void* tiles, const sai_vcf_state* st, int64_t site_cap) {
+  const int64_t n = st->n_sites;
+  if (n > site_cap) return;
+  const int64_t end = (n + 31) & ~int64_t(31);
+  const int n_words = 2 * lay.pairs_per_site;
+  for (int64_t x = threadIdx.x; x < (end - n) * n_words; x += blockDim.x) {
+    const int64_t site = n + x / n_words;
+    const int w = (int)(x % n_words);
+    int p = 0;
+    while (p + 1 < lay.n_pops && w >= 2 * lay.pop[p + 1].pair_off) ++p;
+    const sai_pop_layout& P = lay.pop[p];
+    *word_at(tiles, lay.pairs_per_site, site, w) = (w - 2 * P.pair_off) < P.n_groups * P.bits ? 0xffffffffu : 0u;
+  }
+}
+
+}  // namespace
+
+}  // namespace sai
+
+using namespace sai;
+
+extern "C" {
+
+uint64_t sai_vcf_scratch_bytes(const sai_vcf_query* q, int64_t len) {
+  if (!q || len < 0) return 0;
+  return (uint64_t)carve(*q, len, nullptr, nullptr) + 256;
+}
+
+int sai_vcf_tiles_device(const sai_vcf_query* q, const char* d_text, int64_t len, void* d_scratch,
+                         uint64_t scratch_bytes, void* d_tiles, int32_t* d_pos, int64_t site_cap,
+                         sai_vcf_state* d_state, void* stream) {
+  SAI_REQUIRE(q && d_state && d_scratch && d_tiles && d_pos, "sai_vcf_tiles_device: NULL argument");
+  if (int rc = validate_layout(&q->lay)) return rc;
+  SAI_REQUIRE(len >= 0 && len < (int64_t(1) << 31), "sai_vcf_tiles_device: slice of %lld bytes (at most 2^31 - 1)",
+              (long long)len);
+  SAI_REQUIRE(len == 0 || d_text, "sai_vcf_tiles_device: NULL text");
+  SAI_REQUIRE(q->chrom_len >= 1 && q->chrom_len < (int)sizeof(q->chrom), "sai_vcf_tiles_device: bad chromosome name");
+  SAI_REQUIRE(q->max_column >= 0 && q->sample_column, "sai_vcf_tiles_device: bad sample columns");
+  SAI_REQUIRE(q->n_anc == 0 || (q->anc_pos && q->anc_allele), "sai_vcf_tiles_device: bad ancestral-allele table");
+  SAI_REQUIRE(site_cap >= 0 && site_cap % kTile == 0, "sai_vcf_tiles_device: site_cap must be a multiple of 32");
+  SAI_REQUIRE((reinterpret_cast<uintptr_t>(d_text) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_scratch) & 255) == 0,
+              "sai_vcf_tiles_device: text must be 16-byte and scratch 256-byte aligned");
+  Scratch s;
+  const size_t need = carve(*q, len, static_cast<char*>(d_scratch), &s);
+  SAI_REQUIRE(scratch_bytes >= need, "sai_vcf_tiles_device: scratch of %llu bytes, %zu needed",
+              (unsigned long long)scratch_bytes, need);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int n_seg = (int)((len + kSegBytes - 1) / kSegBytes);
+  const int grid = sm_count() * 4;
+  if (n_seg > 0) {
+    k_nl_count<<<n_seg, 256, 0, st>>>(d_text, len, s);
+    SAI_CUDA_CHECK(cudaGetLastError());
+    k_seg_scan<<<1, 1024, 0, st>>>(n_seg, s);
+    k_nl_write<<<n_seg, 256, 0, st>>>(d_text, len, s);
+  } else {
+    SAI_CUDA_CHECK(cudaMemsetAsync(&s.info->n_lines, 0, sizeof(int32_t), st));
+  }
+  k_records<<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, *q, s);
+  k_keep_count<<<grid, kLinesPerChunk, 0, st>>>(s);
+  k_keep_scan<<<1, 1024, 0, st>>>(s, d_state, site_cap);
+  k_keep_write<<<grid, kLinesPerChunk, 0, st>>>(s, d_pos, site_cap);
+  k_genotypes<<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, *q, s, d_tiles, site_cap, d_state);
+  k_pad_tail<<<1, 256, 0, st>>>(q->lay, d_tiles, d_state, site_cap);
+  SAI_CUDA_CHECK(cudaGetLastError());
+  return SAI_OK;
+}
+
+}  // extern "C"

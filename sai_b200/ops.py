@@ -123,3 +123,53 @@ def column_quantiles(cols: Tensor, quantile: float, out: Tensor) -> None:
     with torch.cuda.device(cols.device):
         _cabi.check(_cabi.load().sai_column_quantiles(cols.data_ptr(), n_cols, n_chunks, n_cols * length, length, length,
                                                       float(quantile), out.data_ptr(), _stream(cols)))
+
+
+def vcf_query_tensor(layout, chrom: str, start: int = 1, end: int = 0) -> Tensor:
+    """A ``sai_vcf_query`` (the device tables and ``max_column`` are filled in by ``vcf_tiles`` from its
+    tensor arguments) as a CPU uint8 tensor; ``start > end`` = no region filter."""
+    q = _cabi.VcfQuery()
+    q.lay = layout
+    q.start, q.end = int(start), int(end)
+    name = chrom.encode()
+    if not 1 <= len(name) <= 255:
+        raise ValueError("chromosome name must be 1..255 bytes")
+    q.chrom_len, q.chrom = len(name), name
+    return struct_tensor(q)
+
+
+def vcf_scratch_bytes(query: Tensor, text_bytes: int, sample_column: Tensor) -> int:
+    """Bytes of the ``scratch`` tensor ``vcf_tiles`` needs for a text of ``text_bytes`` with these
+    sample columns (the genotype pass keeps a row of field offsets up to the largest column)."""
+    q = _cabi.VcfQuery.from_buffer_copy(query.numpy().tobytes())
+    q.max_column = int(sample_column.max().item()) if sample_column.numel() else 0
+    return int(_cabi.load().sai_vcf_scratch_bytes(C.byref(q), int(text_bytes)))
+
+
+@torch.library.custom_op("sai_b200::vcf_tiles", mutates_args=("scratch", "tiles", "pos", "state"), device_types="cuda")
+def vcf_tiles(text: Tensor, query: Tensor, sample_column: Tensor, anc_pos: Tensor, anc_allele: Tensor, scratch: Tensor,
+              tiles: Tensor, pos: Tensor, state: Tensor) -> None:
+    """Device VCF parse of one slice of complete lines (sai_vcf_tiles_device): ``text`` uint8 CUDA,
+    ``query`` from ``vcf_query_tensor``, ``sample_column`` int32 (one VCF column per individual of
+    the layout), ``anc_pos`` int32 / ``anc_allele`` uint8 ``[n, 8]`` (empty: no table), ``tiles``
+    uint8 of ``sai_packed_bytes`` for ``pos.numel()`` sites (a multiple of 32), ``state`` the 88-byte
+    ``sai_vcf_state`` as uint8 (zeroed before the first slice; slices chain through it)."""
+    q = _cabi.VcfQuery.from_buffer_copy(query.numpy().tobytes())
+    if text.dtype != torch.uint8 or sample_column.dtype != torch.int32 or pos.dtype != torch.int32:
+        raise ValueError("text uint8, sample_column / pos int32")
+    if state.numel() != C.sizeof(_cabi.VcfState) or sample_column.numel() < 1:
+        raise ValueError("state must hold one sai_vcf_state; sample_column one column per individual")
+    n_ind = sum(int(q.lay.pop[p].n_samples) for p in range(q.lay.n_pops))
+    if sample_column.numel() != n_ind:
+        raise ValueError("sample_column must hold one column per individual of the layout")
+    q.sample_column = sample_column.data_ptr()
+    q.max_column = int(sample_column.max().item())
+    q.n_anc = int(anc_pos.numel())
+    if q.n_anc:
+        if anc_pos.dtype != torch.int32 or anc_allele.numel() != 8 * q.n_anc:
+            raise ValueError("anc_pos int32 and anc_allele 8 bytes per entry")
+        q.anc_pos, q.anc_allele = anc_pos.data_ptr(), anc_allele.data_ptr()
+    with torch.cuda.device(text.device):
+        _cabi.check(_cabi.load().sai_vcf_tiles_device(
+            C.byref(q), text.data_ptr() if text.numel() else None, text.numel(), scratch.data_ptr(), scratch.numel(),
+            tiles.data_ptr(), pos.data_ptr(), pos.numel(), state.data_ptr(), _stream(text)))

@@ -52,13 +52,18 @@ def score_populations(
     engine: HostEngine,
     out_data: Optional[dict[str, PopData]] = None,
     num_src: Optional[int] = None,
+    loaded=None,
 ) -> list[dict[str, Any]]:
     """Item dicts for every (ref, tgt, src-combination, outgroup) x window.
 
     When every population sits on the same positions and every target population has the same
     windows (always the case for ``ChunkPreprocessor.run(chr, start, end)`` on one VCF), ALL
     populations are packed once and the population product becomes up to ``SAI_MAX_JOBS`` jobs per
-    genotype pass, instead of one pack + one transfer + one pass per combination."""
+    genotype pass, instead of one pack + one transfer + one pass per combination.
+
+    ``loaded`` (a ``vcf_device.LoadedChunk``): the populations were parsed on the device into one
+    layout resident in ``engine``; the ``*_data`` dicts then only name the populations (their
+    values are not read) and every combination is scored from that layout."""
     stats = [s for s in stat_config.root.keys() if s in ("U", "Q")]
     four = [s for s in stat_config.root.keys() if s in ("Danc", "Dplus", "df", "fd") and stat_config.root[s] is True]
     dd = any(s == "DD" and stat_config.root[s] is True for s in stat_config.root.keys())
@@ -166,7 +171,7 @@ def score_populations(
     if use_out:
         everyone += list(out_data.values())
     win_lists = list(windows_by_tgt.values())
-    fused = (
+    fused = loaded is not None or (
         len(combos) > 1
         and len(src_combos) == 1
         and len(everyone) <= _cabi.MAX_POPS
@@ -174,7 +179,9 @@ def score_populations(
         and all(w == win_lists[0] for w in win_lists[1:])
         and (stats or four or dd)
     )
-    if fused:
+    if loaded is not None:
+        index, pos, pg = loaded.index, loaded.pos, loaded
+    elif fused:
         index, mats, ploidy = {}, [], []
         for group, data in (("ref", ref_data), ("tgt", tgt_data)):
             for name, d in data.items():
@@ -192,21 +199,29 @@ def score_populations(
                 mats.append(d.GT)
                 ploidy.append(ploidy_config.get_ploidy("outgroup", name))
         pos = everyone[0].POS
-        windows = win_lists[0]
-        src_idx = [index[("src", s)] for s in src_comb]
         pg = None
+    if fused:
+        windows = win_lists[0]
+        n_of = lambda i: int(pg.layout.pop[i].n_samples)
         for b0 in range(0, len(combos), _cabi.MAX_JOBS):
             batch = combos[b0 : b0 + _cabi.MAX_JOBS]
-            jobs = [job_for(r, t, index[("ref", r)], index[("tgt", t)], src_idx) for r, t, _, _ in batch]
-            if pg is None:  # int8 matrices -> pack | copy | genotype pass, pipelined; ONE upload for all batches
+            jobs = []
+            for r, t, sc, _ in batch:
+                if loaded is not None:
+                    src_ploidy_list(len(sc))  # same check as the host path
+                jobs.append(job_for(r, t, index[("ref", r)], index[("tgt", t)], [index[("src", s)] for s in sc]))
+            if b0 == 0 and loaded is not None:  # the device-parsed tiles are already resident
+                res = engine.score_loaded(windows, jobs)
+            elif pg is None:  # int8 matrices -> pack | copy | genotype pass, pipelined; ONE upload for all batches
                 res, pg = engine.score_matrices(mats, ploidy, pos, windows, jobs, keep_negatives=dd)
             else:
                 res = engine.score_resident(jobs)
             for j, combo in enumerate(batch):
-                r, t, _, o = combo
+                r, t, sc, o = combo
+                src_idx = [index[("src", s)] for s in sc]
                 four_vals, dd_vals = extras(
                     pg, index[("ref", r)], index[("tgt", t)], src_idx, index[("out", o)] if (use_out and o is not None) else -1,
-                    ref_data[r].GT.shape[1], tgt_data[t].GT.shape[1], [src_data[s].GT.shape[1] for s in src_comb])
+                    n_of(index[("ref", r)]), n_of(index[("tgt", t)]), [n_of(i) for i in src_idx])
                 emit(combo, windows, pos, res, j, four_vals, dd_vals)
         return items
 
@@ -293,8 +308,18 @@ class ChunkPreprocessor:
         anc_allele_file: Optional[str] = None,
         num_src: int = 1,
         device: int = 0,
+        ingest: str = "host",
     ):
+        """``ingest="device"`` parses the VCF on the GPU (``vcf_device``): the text is copied to the
+        device and parsed there straight into the packed tiles, which all combinations are scored
+        from.  The items are identical to ``"host"``; chunks the device reader does not cover (DD,
+        more than 16 populations, ancestral alleles longer than 7 bytes, source ploidies that differ
+        from their positions in a combination) are read on the host automatically."""
         from .vcf import parse_ind_file
+
+        if ingest not in ("host", "device"):
+            raise ValueError(f"ingest must be 'host' or 'device', not {ingest!r}")
+        self.ingest = ingest
 
         self.vcf_file = vcf_file
         self.ref_ind_file = ref_ind_file
@@ -318,6 +343,10 @@ class ChunkPreprocessor:
             raise ValueError("`win_len` must be greater than 0.")
         if self.win_step < 0:
             raise ValueError("`win_step` must be non-negative.")
+        if self.ingest == "device":
+            items = self._run_device(chr_name, start, end)
+            if items is not None:
+                return items
         groups = read_data(
             vcf_file=self.vcf_file,
             chr_name=chr_name,
@@ -344,6 +373,55 @@ class ChunkPreprocessor:
         return score_populations(
             chr_name, windows, ref_data, tgt_data, src_data, self.ploidy_config, self.stat_config,
             self.anc_allele_available, self.engine, out_data=out_data, num_src=self.num_src,
+        )
+
+    def device_fallback(self, chr_name: str, start=None, end=None) -> Optional[str]:
+        """Why ``run(chr_name, start, end)`` reads this chunk on the host although ``ingest="device"``
+        (``None``: it is read on the device)."""
+        from .vcf import read_anc_or_error
+        from .vcf_device import fallback_reason, read_plan
+
+        plan, _, _ = read_plan(self.vcf_file, chr_name, self.ploidy_config, self.ref_ind_file, self.tgt_ind_file,
+                               self.src_ind_file, self.out_ind_file)
+        anc, _ = read_anc_or_error(self.anc_allele_file, chr_name, start, end)
+        return fallback_reason(self.stat_config, self.ploidy_config, plan, anc, chr_name, self.num_src)
+
+    def _run_device(self, chr_name, start, end):
+        import warnings
+
+        from .vcf import read_anc_or_error
+        from .vcf_device import _wants_outgroup, fallback_reason, read_loaded, read_plan
+
+        with warnings.catch_warnings(record=True) as caught:  # warned once, by the read that is used
+            warnings.simplefilter("always")
+            plan, requests, out = read_plan(self.vcf_file, chr_name, self.ploidy_config, self.ref_ind_file,
+                                            self.tgt_ind_file, self.src_ind_file, self.out_ind_file)
+        anc, anc_error = read_anc_or_error(self.anc_allele_file, chr_name, start, end)
+        if fallback_reason(self.stat_config, self.ploidy_config, plan, anc, chr_name, self.num_src) is not None:
+            return None
+        for w in caught:
+            warnings.warn_explicit(w.message, w.category, w.filename, w.lineno)
+        try:
+            loaded = read_loaded(self.engine, self.vcf_file, chr_name, plan, requests, out, anc, anc_error, start, end,
+                                 with_outgroup=_wants_outgroup(self.stat_config))
+        except (KeyError, OSError) as e:
+            region = chr_name if start is None and end is None else f"{chr_name}:{start}-{end}"
+            raise ValueError(f"Failed to read VCF file {self.vcf_file} from {region}: {e}") from e
+        if loaded is None:  # no #CHROM line: the host reader decides what that means
+            return None
+        (ref_pops, ref_samples), (tgt_pops, tgt_samples) = loaded.groups["ref"], loaded.groups["tgt"]
+        (src_pops, src_samples), (out_pops, out_samples) = loaded.groups["src"], loaded.groups["outgroup"]
+        if start is None and end is None:
+            windows = {t: split_genome(loaded.pos, self.win_len, self.win_step) for t in tgt_samples}
+        else:
+            wins = chunk_windows(start, end, self.win_len, self.win_step)
+            windows = {t: wins for t in tgt_samples}
+        if ref_pops is None or tgt_pops is None or src_pops is None:
+            return self._empty_items(chr_name, windows, ref_samples, tgt_samples, src_samples, out_samples)
+        names = lambda pops: {p: None for p in pops} if pops else None
+        return score_populations(
+            chr_name, windows, names(ref_pops), names(tgt_pops), names(src_pops), self.ploidy_config, self.stat_config,
+            self.anc_allele_available, self.engine, out_data=names(out_pops), num_src=self.num_src, loaded=loaded,
         )
 
     def _empty_items(self, chr_name, windows, ref_samples, tgt_samples, src_samples, out_samples=None):

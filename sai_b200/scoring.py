@@ -234,9 +234,48 @@ class HostEngine:
         _cabi.check(rc)
         return r
 
+    def set_vcf_slicing(self, slice_bytes: int = 0, ring: int = 0) -> None:
+        """Slice size and ring depth of device ingest (<= 0: default).  Tests force many slices."""
+        _cabi.check(_cabi.load().sai_engine_set_vcf_slicing(self._handle(), int(slice_bytes), int(ring)))
+
+    def vcf_stats(self) -> dict:
+        """Stages of the last finished device ingest (``sai_engine_vcf_stats``): host seconds staging /
+        inflating into the pinned ring and waiting for a free slot, H2D and parse seconds summed over
+        the slices (CUDA events), the device span from the first copy to the last parse, slices,
+        text bytes, the seconds the final synchronise waited, host seconds enqueueing copies and
+        kernels, and host seconds inside the feed calls."""
+        out = (C.c_double * 10)()
+        _cabi.check(_cabi.load().sai_engine_vcf_stats(self._handle(), out, 10))
+        keys = ("stage_s", "wait_s", "h2d_s", "parse_s", "device_span_s", "slices", "text_bytes", "finish_wait_s",
+                "launch_s", "feed_s")
+        return dict(zip(keys, list(out)))
+
+    def vcf_slices(self) -> int:
+        """Text slices the last device ingest parsed."""
+        return int(_cabi.load().sai_engine_vcf_slices(self._handle()))
+
+    def loaded_tiles(self, layout, n_sites: int) -> np.ndarray:
+        """Host copy of the tiles the last device ingest left resident (tests, tools)."""
+        lib = _cabi.load()
+        out = np.empty(max(1, int(lib.sai_packed_bytes(C.byref(layout), int(n_sites)))), dtype=np.uint8)
+        _cabi.check(lib.sai_engine_loaded_tiles(self._handle(), out.ctypes.data, out.nbytes))
+        return out[: int(lib.sai_packed_bytes(C.byref(layout), int(n_sites)))]
+
+    def score_loaded(self, windows, jobs, cap_u=None, cap_q=None) -> WindowResults:
+        """K1 + K4 on the chunk the last device ingest (``vcf_device.read_loaded``) left resident;
+        ``score_resident`` / ``pattern_sums`` then work on it like after ``score``."""
+        ws = np.ascontiguousarray([w[0] for w in windows], dtype=np.int64)
+        we = np.ascontiguousarray([w[1] for w in windows], dtype=np.int64)
+        self._last_W = int(ws.shape[0])
+        return self._resident_call("sai_engine_score_loaded", jobs, cap_u, cap_q,
+                                   ws.ctypes.data if ws.size else None, we.ctypes.data if we.size else None, int(ws.shape[0]))
+
     def score_resident(self, jobs, cap_u=None, cap_q=None) -> WindowResults:
         """Another batch of jobs over the chunk of the last ``score*`` call, still resident on the
         device (no upload): a population product of more than 8 combinations costs one transfer."""
+        return self._resident_call("sai_engine_score_resident", jobs, cap_u, cap_q)
+
+    def _resident_call(self, entry: str, jobs, cap_u, cap_q, *head) -> WindowResults:
         lib = _cabi.load()
         J, W = len(jobs), self._last_W
         cap_u = max(1, 4 * W + 1024) if cap_u is None else int(cap_u)
@@ -257,7 +296,7 @@ class HostEngine:
             return h
 
         res = c_results()
-        rc = lib.sai_engine_score_resident(self._handle(), _job_array(jobs), J, C.byref(res))
+        rc = getattr(lib, entry)(self._handle(), *head, _job_array(jobs), J, C.byref(res))
         if rc == _cabi.E_CAPACITY:
             r.u_cand = np.zeros((J, max(1, int(r.totals[:, 0].max()))), dtype=np.int32)
             r.q_cand = np.zeros((J, max(1, int(r.totals[:, 1].max()))), dtype=np.int32)

@@ -765,6 +765,19 @@ def chromosome_span(vcf_file: str, chr_name: str, n_threads: int = 0):
     return None if first is None else (first, last, n)
 
 
+def anc_table(anc):
+    """The native parsers' form of an ancestral-allele table (``AncAlleles`` or ``{pos: allele}``):
+    ``(pos int32, alleles as 8-byte NUL-padded records, n)``, or ``None`` when an allele is longer
+    than 7 bytes (the native parsers' limit)."""
+    if isinstance(anc, dict):
+        keys = sorted(anc)
+        anc = AncAlleles(np.asarray(keys, dtype=np.int64), np.asarray([anc[k] for k in keys], dtype=object))
+    table = np.char.encode(anc.allele.astype(str), "utf-8")  # fixed-width bytes, NUL padded
+    if table.dtype.itemsize > 7:
+        return None
+    return np.ascontiguousarray(anc.pos, dtype=np.int32), np.ascontiguousarray(table.astype("S8")).tobytes(), len(anc)
+
+
 def _native_read(vcf_file, chr_name, start, end, requests, anc, n_threads=0, chunk_bytes=64 << 20,
                  batch_bytes=256 << 20, fused_bgzf=True, group_blocks=0):
     """One pass of the native parser (``sai_vcf_parse_gt``) over the file.
@@ -778,15 +791,10 @@ def _native_read(vcf_file, chr_name, start, end, requests, anc, n_threads=0, chu
     anc_pos = anc_buf = None
     n_anc = 0
     if anc is not None:
-        if isinstance(anc, dict):
-            keys = sorted(anc)
-            anc = AncAlleles(np.asarray(keys, dtype=np.int64), np.asarray([anc[k] for k in keys], dtype=object))
-        table = np.char.encode(anc.allele.astype(str), "utf-8")  # fixed-width bytes, NUL padded
-        if table.dtype.itemsize > 7:
+        table = anc_table(anc)
+        if table is None:
             return None  # long alleles: use the Python reader
-        anc_pos = np.ascontiguousarray(anc.pos, dtype=np.int32)
-        anc_buf = np.ascontiguousarray(table.astype("S8")).tobytes()
-        n_anc = len(anc)
+        anc_pos, anc_buf, n_anc = table
     cols = ploidies = None
     n_out = len(requests)
     consumed = C.c_int64(0)
@@ -923,51 +931,12 @@ def _is_gzip(path: str) -> bool:
         return f.read(2) == b"\x1f\x8b"
 
 
-def read_data(
-    vcf_file: str,
-    chr_name: str,
-    ploidy_config,
-    ref_ind_file: Optional[str],
-    tgt_ind_file: Optional[str],
-    src_ind_file: Optional[str],
-    out_ind_file: Optional[str],
-    anc_allele_file: Optional[str],
-    start: Optional[int] = None,
-    end: Optional[int] = None,
-    native: bool = True,
-):
-    """``{"ref": (data, samples), "tgt": ..., "src": ..., "outgroup": ...}``
-    (sai/utils/utils.py:215-356 with the WindowGenerator's fixed flags:
-    ``is_phased=False``, no fixed-variant / missing filters).  ``native=True``
-    parses the file once for all populations with ``sai_vcf_parse_gt``;
-    ``native=False`` is the pure-Python reader kept as a cross-check."""
-    # The reference reads the VCF region first and returns None (-> NaN rows) when it holds no
-    # record, BEFORE it looks at the ancestral-allele table (utils.py:123-141 then :152-158): a
-    # chunk that falls into a gap (centromere) must not fail because the table is empty there too.
-    # So an empty table is only an error once the region turns out to have records.
-    anc, anc_error = None, None
-    if anc_allele_file:
-        try:
-            anc = read_anc_arrays(anc_allele_file, chr_name, start, end)
-        except ValueError as e:
-            if "No ancestral allele is found" not in str(e):
-                raise
-            anc_error = e
-    groups = (("ref", ref_ind_file), ("tgt", tgt_ind_file), ("src", src_ind_file), ("outgroup", out_ind_file))
-    if not native:
-        anc = anc.as_dict() if anc is not None else None
-        region = VcfRegion(vcf_file, chr_name, start, end)
-        if anc_error is not None and region.pos.size:
-            raise anc_error
-        out = {}
-        for group, ind_file in groups:
-            if ind_file is None or (group == "outgroup" and group not in ploidy_config.root):
-                out[group] = (None, None)
-                continue
-            out[group] = load_population_group(region, ind_file, group, ploidy_config, anc)
-        return out
-
-    # plan: one output column per (population, sample) with the population's ploidy
+def population_plan(groups, ploidy_config):
+    """One output column per (population, sample) with the population's ploidy, for the groups
+    ``((group, ind_file), ...)``: ``(plan, requests, out)`` with ``plan = [(group, samples,
+    [(population, first request, end request), ...]), ...]``, ``requests = [(sample name, ploidy),
+    ...]`` and ``out[group] = (None, None)`` for the groups without a sample file.  Raises and warns
+    like ``_load_population_data`` (sai/utils/utils.py:649-761)."""
     plan, requests, out = [], [], {}
     for group, ind_file in groups:
         if ind_file is None or (group == "outgroup" and group not in ploidy_config.root):
@@ -994,6 +963,58 @@ def read_data(
             requests += [(n, ploidies[population]) for n in names]
             pops.append((population, a, len(requests)))
         plan.append((group, samples, pops))
+    return plan, requests, out
+
+
+def read_anc_or_error(anc_allele_file, chr_name, start, end):
+    """``(table, error)``: the reference reads the VCF region first and returns None (-> NaN rows)
+    when it holds no record, BEFORE it looks at the ancestral-allele table (utils.py:123-141 then
+    :152-158), so an empty table is only an error once the region turns out to have records."""
+    if not anc_allele_file:
+        return None, None
+    try:
+        return read_anc_arrays(anc_allele_file, chr_name, start, end), None
+    except ValueError as e:
+        if "No ancestral allele is found" not in str(e):
+            raise
+        return None, e
+
+
+def read_data(
+    vcf_file: str,
+    chr_name: str,
+    ploidy_config,
+    ref_ind_file: Optional[str],
+    tgt_ind_file: Optional[str],
+    src_ind_file: Optional[str],
+    out_ind_file: Optional[str],
+    anc_allele_file: Optional[str],
+    start: Optional[int] = None,
+    end: Optional[int] = None,
+    native: bool = True,
+):
+    """``{"ref": (data, samples), "tgt": ..., "src": ..., "outgroup": ...}``
+    (sai/utils/utils.py:215-356 with the WindowGenerator's fixed flags:
+    ``is_phased=False``, no fixed-variant / missing filters).  ``native=True``
+    parses the file once for all populations with ``sai_vcf_parse_gt``;
+    ``native=False`` is the pure-Python reader kept as a cross-check."""
+    # a chunk that falls into a gap (centromere) must not fail because the table is empty there too
+    anc, anc_error = read_anc_or_error(anc_allele_file, chr_name, start, end)
+    groups = (("ref", ref_ind_file), ("tgt", tgt_ind_file), ("src", src_ind_file), ("outgroup", out_ind_file))
+    if not native:
+        anc = anc.as_dict() if anc is not None else None
+        region = VcfRegion(vcf_file, chr_name, start, end)
+        if anc_error is not None and region.pos.size:
+            raise anc_error
+        out = {}
+        for group, ind_file in groups:
+            if ind_file is None or (group == "outgroup" and group not in ploidy_config.root):
+                out[group] = (None, None)
+                continue
+            out[group] = load_population_group(region, ind_file, group, ploidy_config, anc)
+        return out
+
+    plan, requests, out = population_plan(groups, ploidy_config)
     if not requests:
         return out
     try:

@@ -1,0 +1,174 @@
+"""Device VCF ingest: the VCF text goes to the GPU and is parsed there straight into the packed
+tiles (``sai_engine_vcf_*``, ``vcf_device.cu``), which stay resident in the engine for scoring.
+
+The host only reads or inflates bytes and copies them: ``_scan_text`` / ``_scan_sorted_region``
+hand their text buffers to ``sai_engine_vcf_feed`` exactly as they hand them to the host parser,
+so plain, bgzip and gzip files and region reads all work the same way.  The records and values
+are those of ``read_data`` (the host parser is the specification); the layout is the one the host
+path packs, so the tiles are comparable byte for byte.
+"""
+
+from __future__ import annotations
+
+import ctypes as C
+from typing import Optional
+
+import numpy as np
+
+from . import _cabi
+from .encode import make_layout
+from .vcf import _scan_sorted_region, _scan_text, anc_table, population_plan, read_anc_or_error
+
+GROUPS = ("ref", "tgt", "src", "outgroup")
+
+
+class LoadedChunk:
+    """One VCF region parsed on the device: its tiles, positions and windows live in ``engine``.
+    ``index[(group, population)]`` = population index in ``layout``; ``groups[group] =
+    (population names or None, samples)`` mirrors what ``read_data`` returns per group."""
+
+    def __init__(self, layout, pos, index, groups):
+        self.layout, self.pos, self.index, self.groups = layout, pos, index, groups
+
+    @property
+    def n_sites(self) -> int:
+        return int(self.pos.shape[0])
+
+
+def fallback_reason(stat_config, ploidy_config, plan, anc, chr_name: str, num_src: int) -> Optional[str]:
+    """Why a chunk has to be read on the host (``None``: it can be read on the device).
+    DD needs the raw values of missing calls, a table the host builds; one layout holds at most
+    ``SAI_MAX_POPS`` populations; the native parsers take ancestral alleles of at most 7 bytes;
+    a source population is scored with the ploidy of its position in the combination
+    (feature_preprocessor.py:160,168-170), which one layout can only hold when that is its own."""
+    if any(s == "DD" and stat_config.root[s] is True for s in stat_config.root):
+        return "DD is enabled"
+    if sum(len(pops) for group, _, pops in plan if group != "outgroup" or _wants_outgroup(stat_config)) > _cabi.MAX_POPS:
+        return f"more than {_cabi.MAX_POPS} populations"
+    if anc is not None and anc_table(anc) is None:
+        return "an ancestral allele is longer than 7 bytes"
+    if not 1 <= len(chr_name.encode()) <= 255:
+        return "chromosome name outside 1..255 bytes"
+    src = [pops for group, _, pops in plan if group == "src"]
+    if src:
+        from itertools import combinations
+
+        positional = list(ploidy_config.get_ploidy("src"))
+        for comb in combinations([p for p, _, _ in src[0]], num_src):
+            if [ploidy_config.get_ploidy("src", name) for name in comb] != positional[: len(comb)]:
+                return "source ploidies differ from their positions in a combination"
+    return None
+
+
+def _wants_outgroup(stat_config) -> bool:
+    return any(s in ("Danc", "Dplus", "df", "fd") and stat_config.root[s] is True for s in stat_config.root)
+
+
+def read_plan(vcf_file, chr_name, ploidy_config, ref_ind_file, tgt_ind_file, src_ind_file, out_ind_file):
+    """The population plan of ``read_data`` (same errors and warnings)."""
+    files = (ref_ind_file, tgt_ind_file, src_ind_file, out_ind_file)
+    return population_plan(tuple(zip(GROUPS, files)), ploidy_config)
+
+
+def read_loaded(engine, vcf_file: str, chr_name: str, plan, requests, out, anc, anc_error, start=None, end=None,
+                with_outgroup: bool = True) -> Optional[LoadedChunk]:
+    """Parses the records of ``chr_name`` (``start <= POS <= end`` when both are given) on the
+    device into ``engine``'s resident tiles, one layout for every population of ``plan`` (the
+    outgroup only with ``with_outgroup``).  ``None`` when the file has no ``#CHROM`` line."""
+    lib = _cabi.load()
+    pops = [(group, name, a, b) for group, _, gp in plan for name, a, b in gp
+            if group != "outgroup" or with_outgroup]
+    groups = dict(out)
+    for group, samples, gp in plan:
+        groups[group] = ([name for name, _, _ in gp] or None, samples)
+    index = {(group if group != "outgroup" else "out", name): i for i, (group, name, _, _) in enumerate(pops)}
+    empty = np.empty(0, dtype=np.int32)
+    if not pops:
+        return LoadedChunk(None, empty, index, groups)
+    n_samples = [b - a for _, _, a, b in pops]
+    ploidy = [requests[a][1] for _, _, a, _ in pops]
+    anc_pos, anc_buf, n_anc = (None, None, 0) if anc is None else anc_table(anc)
+    bits, min_sites = None, 0
+    for _attempt in range(4):
+        lay = make_layout(n_samples, ploidy, bits)
+        state = {"cols": None, "n_file": 0, "hint": 0, "begun": False, "fed": 0}
+        consumed = C.c_int64(0)
+
+        def on_header(line: bytes):
+            names = line.decode().rstrip("\r").split("\t")[9:]
+            col = {n: i for i, n in enumerate(names)}
+            try:
+                every = [col[name] for name, _ in requests]  # every population's samples, parsed or not (read_data's errors)
+                state["cols"] = np.ascontiguousarray([every[i] for _, _, a, b in pops for i in range(a, b)],
+                                                     dtype=np.int32)
+            except KeyError as e:
+                region = chr_name if start is None and end is None else f"{chr_name}:{start}-{end}"
+                raise ValueError(f"Failed to read VCF file {vcf_file} from {region}: {e}") from e
+            state["n_file"] = len(names)
+
+        def on_size_hint(text_bytes: int):
+            state["hint"] = int(text_bytes)
+
+        def begin(length: int) -> None:
+            if not state["begun"]:
+                _cabi.check(lib.sai_engine_vcf_begin(
+                    engine._handle(), C.byref(lay), chr_name.encode(), region[0], region[1], state["cols"].ctypes.data,
+                    int(state["cols"].shape[0]), anc_pos.ctypes.data if n_anc else None, anc_buf if n_anc else None,
+                    n_anc, state["n_file"], max(state["hint"], length), min_sites))
+                state["begun"] = True
+
+        def on_lines(addr: int, length: int) -> int:
+            begin(length)
+            _cabi.check(lib.sai_engine_vcf_feed(engine._handle(), addr, length, C.byref(consumed)))
+            state["fed"] += int(consumed.value)
+            return int(consumed.value)
+
+        def on_bgzf(base: int, block_off, out_off, n_blocks: int, skip: int) -> None:
+            """A whole bgzip file: inflated by the engine's threads straight into its pinned ring."""
+            text = int(out_off[n_blocks]) - skip
+            begin(text)
+            _cabi.check(lib.sai_engine_vcf_feed_bgzf(engine._handle(), base, block_off.ctypes.data, out_off.ctypes.data,
+                                                     n_blocks, skip))
+            state["fed"] += text + 1
+
+        region = (int(start), int(end)) if (start is not None and end is not None) else (1, 0)
+        handled = False
+        if start is not None and end is not None:
+            handled = _scan_sorted_region(vcf_file, chr_name, int(start), int(end), on_header, on_lines)
+        if not handled:
+            _scan_text(vcf_file, on_header, on_lines, on_size_hint=on_size_hint, on_bgzf=on_bgzf)
+        if state["cols"] is None:
+            return None
+        if not state["begun"]:  # no record lines at all
+            pos = empty
+            break
+        n_sites, vmax = C.c_int64(0), (C.c_int32 * len(pops))()
+        # a kept record is >= 11 bytes (CHROM, nine tabs, newline): room for every one (np.empty commits no pages)
+        pos = np.empty(state["fed"] // 11 + 1024, dtype=np.int32)
+        rc = lib.sai_engine_vcf_finish(engine._handle(), C.byref(n_sites), vmax, pos.ctypes.data, pos.shape[0])
+        if rc == _cabi.E_DOMAIN:  # the host path's retry rule (encode.bits_for)
+            bits = [int(lib.sai_bits_for_max_value(int(v))) for v in vmax]
+            continue
+        if rc == _cabi.E_CAPACITY:
+            min_sites = int(n_sites.value)
+            continue
+        _cabi.check(rc)
+        n = int(n_sites.value)
+        pos = pos[:n].copy() if n * 4 < pos.shape[0] else pos[:n]
+        break
+    else:
+        raise _cabi.SaiError("device ingest did not converge on a layout")
+    if anc_error is not None and pos.size:  # records but no ancestral allele in the region: the reference raises
+        raise anc_error
+    if pos.size == 0:
+        groups = {g: (None, v[1]) for g, v in groups.items()}
+    return LoadedChunk(lay, pos, index, groups)
+
+
+def read_region(engine, vcf_file, chr_name, ploidy_config, ref_ind_file, tgt_ind_file, src_ind_file, out_ind_file,
+                anc_allele_file, start=None, end=None, with_outgroup=True):
+    """Plan, ancestral-allele table and device parse in one call (tests, tools)."""
+    plan, requests, out = read_plan(vcf_file, chr_name, ploidy_config, ref_ind_file, tgt_ind_file, src_ind_file,
+                                    out_ind_file)
+    anc, anc_error = read_anc_or_error(anc_allele_file, chr_name, start, end)
+    return read_loaded(engine, vcf_file, chr_name, plan, requests, out, anc, anc_error, start, end, with_outgroup)
