@@ -65,7 +65,8 @@ enum {
   SAI_E_CUDA = -2,     /* CUDA runtime error; see sai_last_error()              */
   SAI_E_DOMAIN = -3,   /* genotype value does not fit the bit-planes            */
   SAI_E_CAPACITY = -4, /* candidate buffers too small; totals were written      */
-  SAI_E_NOMEM = -5
+  SAI_E_NOMEM = -5,
+  SAI_E_CORRUPT = -6   /* a bgzip block inflated on the device is corrupt; see sai_last_error() */
 };
 
 /* comparator of a source population, `"=", "<", ">", "<=", ">="`
@@ -220,6 +221,30 @@ int64_t sai_gzip_inflate(const uint8_t* data, int64_t len, uint8_t* out, int64_t
  * when the CPU has it, 1 = slicing tables). */
 int32_t sai_inflate_raw(const uint8_t* in, int64_t in_len, uint8_t* out, int64_t out_len);
 uint32_t sai_crc32(const uint8_t* data, int64_t len, int32_t isa);
+
+/* Device inflate of BGZF blocks (all of RFC 1951, CRC-32 checked).  One descriptor per block,
+ * built on the host from sai_bgzf_scan's table: the raw deflate payload of comp_bytes bytes at
+ * d_comp + comp_off (behind the gzip header, FEXTRA included), inflated into exactly isize (<= 65536)
+ * bytes at d_out + text_off, whose CRC-32 must equal crc (the member's trailer).  Stream-ordered,
+ * never synchronises the host.  d_status[i] = 0 when block i decoded to exactly isize bytes with a
+ * matching CRC; 1 an invalid stream, 2 too much or too little output, 3 a CRC mismatch -- and then
+ * its output range holds '\n' bytes only.  Blocks never write outside their own output range. */
+typedef struct {
+  int64_t comp_off;   /* payload offset in the device compressed buffer */
+  int64_t text_off;   /* offset of the block's text in the device output */
+  int32_t comp_bytes; /* payload bytes (the member minus header and the 8-byte trailer) */
+  int32_t isize;      /* text bytes (the trailer's ISIZE) */
+  uint32_t crc;       /* expected CRC-32 of the text (the trailer's CRC32) */
+  int32_t pad_;
+} sai_bgzf_block;
+int sai_bgzf_inflate_device(const uint8_t* d_comp, const sai_bgzf_block* d_blocks, int64_t n_blocks,
+                            uint8_t* d_out, int32_t* d_status, void* stream);
+/* The descriptors of blocks [0, n_blocks) of a sai_bgzf_scan table (HOST data, block_off, out_off)
+ * when the members from block_off[0] on are copied, as they lie, to d_comp + comp_base and the text
+ * of block 0 goes to d_out + text_base: the payload offset from the gzip header walk (FEXTRA may
+ * hold more than BC), isize = out_off[j + 1] - out_off[j], crc from the member's trailer. */
+int sai_bgzf_descriptors(const uint8_t* data, const int64_t* block_off, const int64_t* out_off, int64_t n_blocks,
+                         int64_t comp_base, int64_t text_base, sai_bgzf_block* out);
 
 /* ---- device VCF ingest: VCF text in HBM -> tiled bit-planes ----------------
  * The same records and values as sai_vcf_parse_gt (the host parser is the specification), written
@@ -555,6 +580,17 @@ int sai_engine_vcf_feed(sai_engine* e, const char* text, int64_t len, int64_t* c
  * into the next one; a last line without a newline is complete. */
 int sai_engine_vcf_feed_bgzf(sai_engine* e, const uint8_t* data, const int64_t* block_off, const int64_t* out_off,
                              int64_t n_blocks, int64_t skip);
+/* The same with the blocks inflated on the device (sai_bgzf_inflate_device): the staging threads copy
+ * each group's compressed members (whole-file reads and region reads alike: block_off may index any
+ * contiguous run of blocks, out_off[0] = 0) into a pinned ring, one cudaMemcpyAsync moves them to the
+ * device, and the kernel inflates them into the slot that is parsed.  The host inflates only a group's
+ * last block(s) to find its last newline; the incomplete line behind it travels in front of the next
+ * group.  A group without any newline is staged with host inflate.  at_eof != 0: the blocks end the
+ * file, so a last line without a newline is complete; otherwise that line is dropped (a region read
+ * that stops inside the file).  A corrupt block makes sai_engine_vcf_finish return SAI_E_CORRUPT and
+ * name the first one (its index in block_off) in sai_last_error(). */
+int sai_engine_vcf_feed_bgzf_device(sai_engine* e, const uint8_t* data, const int64_t* block_off,
+                                    const int64_t* out_off, int64_t n_blocks, int64_t skip, int32_t at_eof);
 int sai_engine_vcf_finish(sai_engine* e, int64_t* n_sites, int32_t* max_value, int32_t* pos_out, int64_t pos_cap);
 int sai_engine_score_loaded(sai_engine* e, const int64_t* win_start, const int64_t* win_end, int64_t n_windows,
                             const sai_job* jobs, int32_t n_jobs, sai_host_results* out);
@@ -567,8 +603,10 @@ int64_t sai_engine_vcf_slices(const sai_engine* e);
  * seconds waiting for a free slot, [2] H2D and [3] parse seconds summed over the slices (CUDA events),
  * [4] seconds from the first slice's H2D start to the last slice's parse end (events), [5] slices,
  * [6] text bytes, [7] host seconds finish waited for the device, [8] host seconds enqueueing copies and
- * kernels, [9] host seconds inside the feed calls (all of the above host times and the slicing).
- * n <= 10 values are written. */
+ * kernels, [9] host seconds inside the feed calls (all of the above host times and the slicing),
+ * [10] device inflate seconds summed over the slices (CUDA events), [11] compressed bytes copied for
+ * device inflate (descriptors included), [12] host seconds inflating the boundary blocks of
+ * device-inflated groups, [13] slices inflated on the device.  n <= 14 values are written. */
 int sai_engine_vcf_stats(const sai_engine* e, double* out, int32_t n);
 /* The resident tiles of the finished session (sai_packed_bytes(lay, n_sites) bytes) into HOST `out`. */
 int sai_engine_loaded_tiles(sai_engine* e, uint8_t* out, uint64_t cap);

@@ -16,7 +16,7 @@ MAX_SRC = 8
 MAX_JOBS = 8
 TILE_SITES = 32
 
-OK, E_ARG, E_CUDA, E_DOMAIN, E_CAPACITY, E_NOMEM = 0, -1, -2, -3, -4, -5
+OK, E_ARG, E_CUDA, E_DOMAIN, E_CAPACITY, E_NOMEM, E_CORRUPT = 0, -1, -2, -3, -4, -5, -6
 OPS = {"=": 0, "<": 1, ">": 2, "<=": 3, ">=": 4}
 
 
@@ -134,6 +134,8 @@ SYMBOLS = {
     "sai_gzip_inflate": (_I64, [_P, _I64, _P, _I64]),
     "sai_inflate_raw": (_I32, [_P, _I64, _P, _I64]),
     "sai_crc32": (C.c_uint32, [_P, _I64, _I32]),
+    "sai_bgzf_inflate_device": (C.c_int, [_P, _P, _I64, _P, _P, _P]),
+    "sai_bgzf_descriptors": (C.c_int, [_P, _P, _P, _I64, _I64, _I64, _P]),
     "sai_site_counts": (C.c_int, [_LAY, _P, _I64, _I64, _P, _P, _I64, _I32, _P]),
     "sai_site_flags": (
         C.c_int,
@@ -194,6 +196,7 @@ SYMBOLS = {
         C.c_int, [_P, _LAY, C.c_char_p, _I64, _I64, _P, _I32, _P, _P, _I64, _I32, _I64, _I64]),
     "sai_engine_vcf_feed": (C.c_int, [_P, _P, _I64, C.POINTER(_I64)]),
     "sai_engine_vcf_feed_bgzf": (C.c_int, [_P, _P, _P, _P, _I64, _I64]),
+    "sai_engine_vcf_feed_bgzf_device": (C.c_int, [_P, _P, _P, _P, _I64, _I64, _I32]),
     "sai_engine_vcf_stats": (C.c_int, [_P, _P, _I32]),
     "sai_engine_vcf_finish": (C.c_int, [_P, C.POINTER(_I64), _P, _P, _I64]),
     "sai_engine_score_loaded": (C.c_int, [_P, _P, _P, _I64, _JOB, _I32, C.POINTER(HostResults)]),

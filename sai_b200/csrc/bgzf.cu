@@ -24,8 +24,10 @@ namespace sai {
 static inline uint32_t le16(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8); }
 static inline uint32_t le32(const uint8_t* p) { return le16(p) | (le16(p + 2) << 16); }
 
-// total size of the block at p (0: not a complete / valid BGZF block within `avail` bytes)
-static int64_t block_size(const uint8_t* p, int64_t avail, int64_t* payload_off) {
+// total size of the block at p (0: not a complete / valid BGZF block within `avail` bytes);
+// *payload_off = where its raw deflate data starts (behind the whole FEXTRA field); the one walk of the
+// gzip header, also behind the device inflater's descriptors (sai_bgzf_descriptors)
+static int64_t bgzf_block_size(const uint8_t* p, int64_t avail, int64_t* payload_off) {
   if (avail < 18) return 0;
   if (p[0] != 31 || p[1] != 139 || p[2] != 8 || !(p[3] & 4)) return -1;
   const int64_t xlen = le16(p + 10);
@@ -51,7 +53,7 @@ static int64_t block_size(const uint8_t* p, int64_t avail, int64_t* payload_off)
 // the block is called corrupt.
 static bool inflate_one(const uint8_t* p, uint8_t* out, int64_t want, z_stream* zs) {
   int64_t payload = 0;
-  const int64_t bs = block_size(p, (int64_t)1 << 20, &payload);
+  const int64_t bs = bgzf_block_size(p, (int64_t)1 << 20, &payload);
   if (bs <= 0) return false;
   if (want == 0) return true;  // empty block (the EOF marker)
   const uint32_t want_crc = le32(p + bs - 8);
@@ -74,7 +76,7 @@ extern "C" {
 
 int32_t sai_is_bgzf(const uint8_t* data, int64_t len) {
   int64_t off = 0;
-  return data && block_size(data, len, &off) > 0 ? 1 : 0;
+  return data && bgzf_block_size(data, len, &off) > 0 ? 1 : 0;
 }
 
 int64_t sai_bgzf_scan(const uint8_t* data, int64_t len, int64_t max_blocks, int64_t max_out_bytes,
@@ -87,7 +89,7 @@ int64_t sai_bgzf_scan(const uint8_t* data, int64_t len, int64_t max_blocks, int6
   out_off[0] = 0;
   while (n < max_blocks && at < len) {
     int64_t payload = 0;
-    const int64_t bs = block_size(data + at, len - at, &payload);
+    const int64_t bs = bgzf_block_size(data + at, len - at, &payload);
     if (bs < 0) {
       set_error("not a BGZF block at offset %lld", (long long)at);
       return SAI_E_ARG;
@@ -106,6 +108,31 @@ int64_t sai_bgzf_scan(const uint8_t* data, int64_t len, int64_t max_blocks, int6
   }
   *consumed = at;
   return n;
+}
+
+int sai_bgzf_descriptors(const uint8_t* data, const int64_t* block_off, const int64_t* out_off, int64_t n_blocks,
+                         int64_t comp_base, int64_t text_base, sai_bgzf_block* out) {
+  if (!data || n_blocks < 0 || (n_blocks > 0 && (!block_off || !out_off || !out))) {
+    set_error("sai_bgzf_descriptors: bad argument");
+    return SAI_E_ARG;
+  }
+  for (int64_t j = 0; j < n_blocks; ++j) {
+    int64_t payload = 0;
+    const int64_t bs = bgzf_block_size(data + block_off[j], (int64_t)1 << 20, &payload);
+    const int64_t isize = out_off[j + 1] - out_off[j];
+    if (bs <= 0 || isize < 0 || isize > (1 << 16)) {
+      set_error("sai_bgzf_descriptors: no BGZF block of <= 64 KB of text at offset %lld", (long long)block_off[j]);
+      return SAI_E_ARG;
+    }
+    sai_bgzf_block& d = out[j];
+    d.comp_off = comp_base + (block_off[j] - block_off[0]) + payload;
+    d.text_off = text_base + out_off[j] - out_off[0];
+    d.comp_bytes = (int32_t)(bs - payload - 8);
+    d.isize = (int32_t)isize;
+    d.crc = le32(data + block_off[j] + bs - 8);
+    d.pad_ = 0;
+  }
+  return SAI_OK;
 }
 
 int sai_bgzf_inflate(const uint8_t* data, const int64_t* block_off, const int64_t* out_off, int64_t n_blocks,

@@ -36,6 +36,11 @@ int sm_count();
 
 constexpr int kTile = SAI_TILE_SITES;  // sites per tile == warp width
 
+// inflate_device.cu: sai_bgzf_inflate_device that also lowers *d_first_bad to first_index + i for
+// every failed block i (d_first_bad may be NULL).
+int bgzf_inflate_launch(const uint8_t* d_comp, const sai_bgzf_block* d_blocks, int64_t n_blocks, uint8_t* d_out,
+                        int32_t* d_status, unsigned long long* d_first_bad, int64_t first_index, cudaStream_t stream);
+
 // Kernel-parameter block shared by the site kernels (passed __grid_constant__).
 struct JobBlock {
   int32_t n_jobs;

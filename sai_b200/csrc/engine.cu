@@ -128,15 +128,23 @@ struct sai_engine {
     size_t slot_bytes = 0;            // capacity of one ring slot (pinned and device)
     char* h_ring = nullptr;
     std::vector<cudaEvent_t> copied, parsed;  // per slot: H2D done (host slot free), parse done (device slot free)
-    std::vector<std::array<cudaEvent_t, 4>> tev;  // per slice: H2D start / end, parse start / end (stage timing)
+    // per slice: H2D start / end, parse start / end, device inflate start / end (stage timing)
+    std::vector<std::array<cudaEvent_t, 6>> tev;
+    std::vector<char> inflated;       // per slice: its text was inflated on the device
     std::vector<char> carry;          // bgzip feed: the incomplete line at the end of the last slot
     double t_stage = 0, t_wait = 0;   // host seconds: staging / inflating into the ring, waiting for a free slot
     double t_launch = 0, t_feed = 0;  // host seconds: enqueueing copies and kernels, inside the feed calls
-    double stats[10] = {0};           // sai_engine_vcf_stats of the last finished session
+    double t_boundary = 0;            // host seconds inflating the boundary blocks of device-inflated groups
+    double comp_bytes = 0;            // compressed bytes (with descriptors) copied for device inflate
+    char* h_comp = nullptr;           // pinned ring of compressed groups (device inflate), comp_slot bytes a slot
+    size_t comp_slot = 0;             // 0: (re)built by the next device-inflated group, for `ring` slots
+    std::vector<cudaStream_t> s_infl; // per ring slot: the stream its inflates run on (slices inflate side by side)
+    double stats[14] = {0};           // sai_engine_vcf_stats of the last finished session
     int sticky_rc = SAI_OK;           // first failure of the session, reported by finish
     StagePool pool;
   } vcf;
   Buf vtext, vscratch, vcols, vanc_pos, vanc_all, vstate;
+  Buf vcomp, vbad;  // device inflate: ring of compressed groups (+ block statuses), first corrupt block
 };
 
 namespace sai {
@@ -266,7 +274,7 @@ void sai_engine_destroy(sai_engine* e) {
   cudaSetDevice(e->device);
   for (auto* b : {&e->packed, &e->pos, &e->win, &e->mask, &e->qval, &e->res, &e->cand, &e->counts, &e->sums, &e->hist,
                   &e->neg, &e->dd, &e->zt, &e->ztoff, &e->vtext, &e->vscratch, &e->vcols, &e->vanc_pos, &e->vanc_all,
-                  &e->vstate})
+                  &e->vstate, &e->vcomp, &e->vbad})
     if (b->p) cudaFree(b->p);
   for (auto ev : e->ev) cudaEventDestroy(ev);
   for (auto ev : e->ev_dec) cudaEventDestroy(ev);
@@ -275,6 +283,8 @@ void sai_engine_destroy(sai_engine* e) {
   for (auto& t : e->vcf.tev)
     for (auto ev : t) cudaEventDestroy(ev);
   if (e->vcf.h_ring) cudaFreeHost(e->vcf.h_ring);
+  if (e->vcf.h_comp) cudaFreeHost(e->vcf.h_comp);
+  for (auto s : e->vcf.s_infl) cudaStreamDestroy(s);
   if (e->ring) cudaFreeHost(e->ring);
   if (e->h_ztoff) cudaFreeHost(e->h_ztoff);
   if (e->s_copy) cudaStreamDestroy(e->s_copy);
@@ -905,35 +915,74 @@ static int vcf_acquire_slot(sai_engine* e, int64_t n, char** h) {
   return SAI_OK;
 }
 
+// A compressed group in the slot's part of the compressed ring (device inflate): `bytes` to copy,
+// starting with `n_desc` block descriptors; descriptor i is block first_block + i (the carry's
+// pseudo-blocks come last).
+struct DevGroup {
+  size_t bytes;
+  int64_t n_desc, first_block;
+};
+
 // Bytes [off, off + n) of the acquired slot (complete lines) -> device slot (copy stream) -> parse (compute stream).
-static int vcf_launch_slot_impl(sai_engine* e, int64_t off, int64_t n);
-static int vcf_launch_slot(sai_engine* e, int64_t off, int64_t n) {
+// With `g` the slot's compressed group goes over instead and is inflated into the device slot on the slot's
+// own inflate stream: one slice has too few blocks to fill the GPU, so the inflates of the slices in the
+// ring run side by side (and next to the parse); [off, off + n) is then the range of the inflated text
+// that is parsed.  The slot's inflate waits for its copy, which waited for the slot's previous parse.
+static int vcf_launch_slot_impl(sai_engine* e, int64_t off, int64_t n, const DevGroup* g);
+static int vcf_launch_slot(sai_engine* e, int64_t off, int64_t n, const DevGroup* g = nullptr) {
   const double t0 = now_s();
-  const int rc = vcf_launch_slot_impl(e, off, n);
+  const int rc = vcf_launch_slot_impl(e, off, n, g);
   e->vcf.t_launch += now_s() - t0;
   return rc;
 }
-static int vcf_launch_slot_impl(sai_engine* e, int64_t off, int64_t n) {
+static int vcf_launch_slot_impl(sai_engine* e, int64_t off, int64_t n, const DevGroup* g) {
   auto& V = e->vcf;
   V.fed += n;
   const int64_t need = V.fed / V.row_bytes + V.n_slices + 1 + 1024;  // records of normal width in the text so far
   if (need > V.site_cap)
     if (int rc = vcf_grow_sites(e, std::max(need, 2 * V.site_cap), true)) return rc;
   while ((int64_t)V.tev.size() <= V.n_slices) {
-    std::array<cudaEvent_t, 4> t;
+    std::array<cudaEvent_t, 6> t;
     for (auto& x : t) SAI_CUDA_CHECK(cudaEventCreate(&x));
     V.tev.push_back(t);
   }
+  V.inflated.resize((size_t)V.n_slices + 1);
+  V.inflated[V.n_slices] = g != nullptr;
   const auto& T = V.tev[V.n_slices];
   const int slot = (int)(V.n_slices % V.ring);
-  const char* h = V.h_ring + (size_t)slot * V.slot_bytes + off;
   char* d = static_cast<char*>(e->vtext.p) + (size_t)slot * V.slot_bytes;
   if (V.n_slices >= V.ring) SAI_CUDA_CHECK(cudaStreamWaitEvent(e->s_copy, V.parsed[slot], 0));
   SAI_CUDA_CHECK(cudaEventRecord(T[0], e->s_copy));
-  SAI_CUDA_CHECK(cudaMemcpyAsync(d, h, (size_t)n, cudaMemcpyHostToDevice, e->s_copy));
+  if (!g) {
+    SAI_CUDA_CHECK(cudaMemcpyAsync(d, V.h_ring + (size_t)slot * V.slot_bytes + off, (size_t)n, cudaMemcpyHostToDevice,
+                                   e->s_copy));
+  } else {
+    uint8_t* dc = static_cast<uint8_t*>(e->vcomp.p) + (size_t)slot * V.comp_slot;
+    SAI_CUDA_CHECK(cudaMemcpyAsync(dc, V.h_comp + (size_t)slot * V.comp_slot, g->bytes, cudaMemcpyHostToDevice, e->s_copy));
+    V.comp_bytes += (double)g->bytes;
+  }
   SAI_CUDA_CHECK(cudaEventRecord(T[1], e->s_copy));
   SAI_CUDA_CHECK(cudaEventRecord(V.copied[slot], e->s_copy));
-  SAI_CUDA_CHECK(cudaStreamWaitEvent(e->s_comp, V.copied[slot], 0));
+  if (g) {
+    uint8_t* dc = static_cast<uint8_t*>(e->vcomp.p) + (size_t)slot * V.comp_slot;
+    int32_t* status = reinterpret_cast<int32_t*>(dc + align256(g->bytes));
+    while ((int)V.s_infl.size() <= slot) {
+      cudaStream_t s;
+      SAI_CUDA_CHECK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+      V.s_infl.push_back(s);
+    }
+    cudaStream_t si = V.s_infl[slot];
+    SAI_CUDA_CHECK(cudaStreamWaitEvent(si, V.copied[slot], 0));
+    SAI_CUDA_CHECK(cudaEventRecord(T[4], si));
+    if (int rc = bgzf_inflate_launch(dc, reinterpret_cast<const sai_bgzf_block*>(dc), g->n_desc, reinterpret_cast<uint8_t*>(d),
+                                     status, static_cast<unsigned long long*>(e->vbad.p), g->first_block, si))
+      return rc;
+    SAI_CUDA_CHECK(cudaEventRecord(T[5], si));
+    SAI_CUDA_CHECK(cudaStreamWaitEvent(e->s_comp, T[5], 0));
+    d += off;
+  } else {
+    SAI_CUDA_CHECK(cudaStreamWaitEvent(e->s_comp, V.copied[slot], 0));
+  }
   SAI_CUDA_CHECK(cudaEventRecord(T[2], e->s_comp));
   if (int rc = sai_vcf_tiles_device(&V.q, d, n, e->vscratch.p, e->vscratch.cap, e->packed.p, static_cast<int32_t*>(e->pos.p),
                                     V.site_cap, static_cast<sai_vcf_state*>(e->vstate.p), e->s_comp))
@@ -1013,8 +1062,10 @@ int sai_engine_vcf_begin(sai_engine* e, const sai_layout* lay, const char* chrom
   if (int rc = vcf_grow_sites(e, std::max(text_bytes_hint / V.row_bytes + 1024, min_sites), false)) return rc;
   if (V.slot_bytes > 0)  // the scratch depends on the query (max_column): resize for the ring's slots
     if (int rc = grow(e->vscratch, sai_vcf_scratch_bytes(&q, (int64_t)V.slot_bytes))) return rc;
+  if (int rc = grow(e->vbad, sizeof(unsigned long long))) return rc;
+  SAI_CUDA_CHECK(cudaMemsetAsync(e->vbad.p, 0xff, sizeof(unsigned long long), e->s_copy));  // no corrupt block
   V.fed = V.n_slices = 0;
-  V.t_stage = V.t_wait = V.t_launch = V.t_feed = 0;
+  V.t_stage = V.t_wait = V.t_launch = V.t_feed = V.t_boundary = V.comp_bytes = 0;
   V.carry.clear();
   V.sticky_rc = SAI_OK;
   V.state = 1;
@@ -1076,18 +1127,23 @@ int sai_engine_vcf_finish(sai_engine* e, int64_t* n_sites, int32_t* max_value, i
   V.state = 0;
   const double t_sync = now_s();
   const cudaError_t c1 = cudaStreamSynchronize(e->s_copy), c2 = cudaStreamSynchronize(e->s_comp);
-  double h2d = 0, parse = 0, span = 0;
+  double h2d = 0, parse = 0, span = 0, infl = 0;
+  int64_t n_inflated = 0;
   float ms = 0;
   for (int64_t k = 0; c1 == cudaSuccess && c2 == cudaSuccess && k < V.n_slices; ++k) {
     const auto& T = V.tev[k];
     if (cudaEventElapsedTime(&ms, T[0], T[1]) == cudaSuccess) h2d += ms / 1e3;
     if (cudaEventElapsedTime(&ms, T[2], T[3]) == cudaSuccess) parse += ms / 1e3;
+    if (V.inflated[k]) {
+      ++n_inflated;
+      if (cudaEventElapsedTime(&ms, T[4], T[5]) == cudaSuccess) infl += ms / 1e3;
+    }
   }
   if (c1 == cudaSuccess && c2 == cudaSuccess && V.n_slices > 0 &&
       cudaEventElapsedTime(&ms, V.tev[0][0], V.tev[V.n_slices - 1][3]) == cudaSuccess)
     span = ms / 1e3;
-  const double stats[10] = {V.t_stage, V.t_wait, h2d, parse, span, (double)V.n_slices, (double)V.fed, now_s() - t_sync,
-                            V.t_launch, V.t_feed};
+  const double stats[14] = {V.t_stage, V.t_wait, h2d, parse, span, (double)V.n_slices, (double)V.fed, now_s() - t_sync,
+                            V.t_launch, V.t_feed, infl, V.comp_bytes, V.t_boundary, (double)n_inflated};
   memcpy(V.stats, stats, sizeof(stats));
   if (V.sticky_rc) {
     set_error("ingest session failed earlier (code %d)", V.sticky_rc);
@@ -1096,6 +1152,14 @@ int sai_engine_vcf_finish(sai_engine* e, int64_t* n_sites, int32_t* max_value, i
   if (c1 != cudaSuccess || c2 != cudaSuccess) {
     set_error("ingest session: %s", cudaGetErrorString(c1 != cudaSuccess ? c1 : c2));
     return SAI_E_CUDA;
+  }
+  if (n_inflated > 0) {
+    unsigned long long bad = 0;
+    SAI_CUDA_CHECK(cudaMemcpy(&bad, e->vbad.p, sizeof(bad), cudaMemcpyDeviceToHost));
+    if (bad != ~0ull) {
+      set_error("BGZF block %lld is corrupt", (long long)bad);
+      return SAI_E_CORRUPT;
+    }
   }
   sai_vcf_state st;
   SAI_CUDA_CHECK(cudaMemcpy(&st, e->vstate.p, sizeof(st), cudaMemcpyDeviceToHost));
@@ -1157,17 +1221,212 @@ int sai_engine_score_loaded(sai_engine* e, const int64_t* win_start, const int64
   return run_windows(e, out);
 }
 
+}  // extern "C"
+
+namespace sai {
+
+// The group of blocks [b, b1) that starts at block b: at most slice_bytes of text together with the
+// carried line and a newline (at least one block), so the ring slots are not reallocated slice after slice.
+static int64_t vcf_group_end(const sai_engine* e, const int64_t* out_off, int64_t n_blocks, int64_t b) {
+  const int64_t c = (int64_t)e->vcf.carry.size();
+  int64_t b1 = b + 1;
+  while (b1 < n_blocks && c + out_off[b1 + 1] - out_off[b] + 1 <= e->vcf.slice_bytes) ++b1;
+  return b1;
+}
+
+// Group [b, b1) inflated by the staging threads straight into the slot behind the carried line; the
+// incomplete last line is carried on.  `from`: text offset of the first record when it lies inside
+// block b; `eof`: the group ends the file, so a last line without a newline is complete.
+static int vcf_bgzf_group_host(sai_engine* e, const uint8_t* data, const int64_t* block_off, const int64_t* out_off,
+                               int64_t b, int64_t b1, int64_t from, bool eof) {
+  auto& V = e->vcf;
+  const int64_t c = (int64_t)V.carry.size();
+  const int64_t text = out_off[b1] - out_off[b];
+  char* h = nullptr;
+  if (int rc = vcf_acquire_slot(e, c + text + 1, &h)) return rc;
+  if (c) memcpy(h, V.carry.data(), (size_t)c);
+  const double t0 = now_s();
+  constexpr int64_t kGroup = 16;  // blocks per task (~1 MB of text)
+  std::atomic<int> bad_rc{SAI_OK};
+  std::mutex msg_mu;
+  std::string msg;
+  const std::function<void(int64_t)> f = [&](int64_t i) {
+    const int64_t g0 = b + i * kGroup, g1 = std::min(b1, g0 + kGroup);
+    int64_t rel[kGroup + 1];
+    for (int64_t k = g0; k <= g1; ++k) rel[k - g0] = out_off[k] - out_off[b] + c;
+    const int rc = sai_bgzf_inflate(data, block_off + g0, rel, g1 - g0, reinterpret_cast<uint8_t*>(h), 1);
+    if (rc != SAI_OK) {
+      std::lock_guard<std::mutex> lk(msg_mu);
+      if (bad_rc.load() == SAI_OK) msg = sai_last_error();
+      bad_rc.store(rc);
+    }
+  };
+  V.pool.run(stage_threads(e), (b1 - b + kGroup - 1) / kGroup, f);
+  V.t_stage += now_s() - t0;
+  if (bad_rc.load() != SAI_OK) {
+    set_error("%s", msg.c_str());
+    return bad_rc.load();
+  }
+  const int64_t lo = c == 0 && from > out_off[b] ? from - out_off[b] : 0;  // the header stays behind
+  int64_t end = c + text;
+  if (eof && end > lo && h[end - 1] != '\n') h[end++] = '\n';  // last line without a newline
+  const void* nl = end > lo ? memrchr(h + lo, '\n', (size_t)(end - lo)) : nullptr;
+  const int64_t cut = nl ? static_cast<const char*>(nl) - h + 1 : lo;
+  std::vector<char> rest(h + cut, h + end);  // the incomplete last line, carried into the next slot
+  if (cut > lo)
+    if (int rc = vcf_launch_slot(e, lo, cut - lo)) return rc;
+  V.carry.swap(rest);
+  return SAI_OK;
+}
+
+// The compressed ring (pinned + device) with slots of at least `bytes`; grows after a drain.
+static int vcf_comp_ring(sai_engine* e, size_t bytes) {
+  auto& V = e->vcf;
+  if (bytes <= V.comp_slot) return SAI_OK;  // comp_slot is 0 whenever the ring's depth changed
+  SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_copy));
+  SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));
+  const size_t slot = align256(std::max(bytes, std::max<size_t>(2 * V.comp_slot, 1u << 20)));
+  if (V.h_comp) SAI_CUDA_CHECK(cudaFreeHost(V.h_comp));
+  V.h_comp = nullptr;
+  V.comp_slot = 0;
+  SAI_CUDA_CHECK(cudaHostAlloc(reinterpret_cast<void**>(&V.h_comp), slot * V.ring, cudaHostAllocDefault));
+  if (int rc = grow(e->vcomp, slot * V.ring)) return rc;
+  V.comp_slot = slot;
+  return SAI_OK;
+}
+
+// Group [b, b1) inflated on the device.  The host inflates only the boundary: the group's last block
+// (and, when it holds no newline, the ones before it, up to kLookBack bytes of text) to find the last line
+// end `cut`; the bytes behind it are the next group's carry.  The slot then holds [carry | text of the
+// group's blocks] -- the carry travels as stored deflate pseudo-blocks in the same copy -- and [lo, cut)
+// is parsed.  A group whose last kLookBack bytes hold no newline (a line of about that length or longer)
+// is staged by vcf_bgzf_group_host.  The slot's text starts `pad` bytes in, so that the parsed range
+// begins 16-byte aligned as the parse kernels read it.
+static int vcf_bgzf_group_device(sai_engine* e, const uint8_t* data, const int64_t* block_off, const int64_t* out_off,
+                                 int64_t b, int64_t b1, int64_t from, bool eof) {
+  constexpr int64_t kLookBack = 1 << 20;
+  auto& V = e->vcf;
+  const int64_t c = (int64_t)V.carry.size();
+  const int64_t text = out_off[b1] - out_off[b];
+  const int64_t lo = c == 0 && from > out_off[b] ? from - out_off[b] : 0;
+  const int64_t pad = (16 - (lo & 15)) & 15;
+  const double t0 = now_s();
+  std::vector<std::vector<char>> tail;  // text of blocks b1 - 1, b1 - 2, ..., k inflated by the host
+  int64_t k = b1, cut = -1;
+  bool newline = false;  // a '\n' pseudo-block completes the file's last line
+  while (k > b && cut < 0 && out_off[b1] - out_off[k] < kLookBack) {
+    --k;
+    const int64_t isz = out_off[k + 1] - out_off[k];
+    const int64_t at = c + out_off[k] - out_off[b];  // slot offset of block k
+    tail.emplace_back((size_t)isz);
+    std::vector<char>& blk = tail.back();
+    if (isz > 0) {
+      const int64_t rel[2] = {0, isz};
+      if (sai_bgzf_inflate(data, block_off + k, rel, 1, reinterpret_cast<uint8_t*>(blk.data()), 1) != SAI_OK) {
+        V.t_boundary += now_s() - t0;
+        set_error("BGZF block %lld is corrupt", (long long)k);
+        return SAI_E_CORRUPT;
+      }
+      if (eof) {  // the range ends at the end of the file: its last line is complete
+        newline = blk.back() != '\n';
+        cut = c + text + (newline ? 1 : 0);
+      } else {
+        const int64_t from_k = std::max<int64_t>(0, lo - at);
+        const void* nl = from_k < isz ? memrchr(blk.data() + from_k, '\n', (size_t)(isz - from_k)) : nullptr;
+        if (nl) cut = at + (static_cast<const char*>(nl) - blk.data()) + 1;
+      }
+    }
+    if (at <= lo) break;  // nothing of the group's records lies before block k
+  }
+  if (cut < 0 && eof && c > lo && k == b) {  // only empty blocks behind the carried line: it is the file's last line
+    cut = c + text + 1;
+    newline = true;
+  }
+  V.t_boundary += now_s() - t0;
+  if (eof && c + text <= lo) return SAI_OK;  // nothing behind the header
+  if (cut <= lo) return vcf_bgzf_group_host(e, data, block_off, out_off, b, b1, from, eof);
+  // descriptors, the group's members as they lie in the file, then the pseudo-blocks
+  const int64_t n_real = b1 - b;
+  const int64_t n_carry = (c + 65534) / 65535;
+  const int64_t n_desc = n_real + n_carry + (newline ? 1 : 0);
+  std::vector<sai_bgzf_block> desc((size_t)n_desc);
+  const size_t desc_bytes = align256(sizeof(sai_bgzf_block) * (size_t)n_desc);
+  if (int rc = sai_bgzf_descriptors(data, block_off + b, out_off + b, n_real, (int64_t)desc_bytes, pad + c, desc.data()))
+    return rc;
+  for (int64_t j = 0; j + 1 < n_real; ++j) {  // the members are copied as one span of the file
+    const sai_bgzf_block& d = desc[(size_t)j];
+    const int64_t member_end = d.comp_off + d.comp_bytes + 8 - (int64_t)desc_bytes;
+    SAI_REQUIRE(block_off[b + j + 1] - block_off[b] == member_end, "sai_engine_vcf_feed_bgzf_device: blocks are not contiguous");
+  }
+  const int64_t span = desc[(size_t)n_real - 1].comp_off + desc[(size_t)n_real - 1].comp_bytes + 8 - (int64_t)desc_bytes;
+  const int64_t pseudo = c + 5 * n_carry + (newline ? 6 : 0);
+  const size_t bytes = desc_bytes + (size_t)span + (size_t)pseudo;
+  char* h = nullptr;
+  if (int rc = vcf_acquire_slot(e, pad + c + text + 1, &h)) return rc;
+  if (int rc = vcf_comp_ring(e, align256(bytes) + sizeof(int32_t) * (size_t)n_desc)) return rc;
+  uint8_t* hc = reinterpret_cast<uint8_t*>(V.h_comp) + (size_t)(V.n_slices % V.ring) * V.comp_slot;
+  uint8_t* ps = hc + desc_bytes + span;
+  int64_t ps_off = (int64_t)desc_bytes + span;
+  auto stored = [&](int64_t idx, const char* src, int64_t len, int64_t text_off) {  // BFINAL, BTYPE 00, LEN, NLEN, bytes
+    ps[0] = 1;
+    ps[1] = (uint8_t)(len & 0xff), ps[2] = (uint8_t)(len >> 8);
+    ps[3] = (uint8_t)(~len & 0xff), ps[4] = (uint8_t)((~len >> 8) & 0xff);
+    memcpy(ps + 5, src, (size_t)len);
+    sai_bgzf_block& d = desc[(size_t)idx];
+    d.comp_off = ps_off;
+    d.comp_bytes = (int32_t)(5 + len);
+    d.text_off = text_off;
+    d.isize = (int32_t)len;
+    d.crc = sai_crc32(reinterpret_cast<const uint8_t*>(src), len, 0);
+    ps += 5 + len;
+    ps_off += 5 + len;
+  };
+  for (int64_t i = 0; i < n_carry; ++i) {
+    const int64_t a = i * 65535, len = std::min<int64_t>(65535, c - a);
+    stored(n_real + i, V.carry.data() + a, len, pad + a);
+  }
+  if (newline) stored(n_desc - 1, "\n", 1, pad + c + text);
+  memcpy(hc, desc.data(), sizeof(sai_bgzf_block) * (size_t)n_desc);
+  staged_copy(e, reinterpret_cast<char*>(hc + desc_bytes), reinterpret_cast<const char*>(data + block_off[b]), (size_t)span);
+  const DevGroup g{bytes, n_desc, b};
+  if (int rc = vcf_launch_slot(e, pad + lo, cut - lo, &g)) return rc;
+  // the carry: slot bytes [cut, c + text) -- inside the blocks the host inflated (tail, last block first)
+  std::vector<char> rest;
+  if (!eof) {
+    int64_t skip = cut - (c + out_off[k] - out_off[b]);
+    rest.reserve((size_t)(c + text - cut));
+    for (auto it = tail.rbegin(); it != tail.rend(); ++it) {
+      const int64_t from_here = std::min<int64_t>(skip, (int64_t)it->size());
+      rest.insert(rest.end(), it->begin() + from_here, it->end());
+      skip -= from_here;
+    }
+  }
+  V.carry.swap(rest);
+  return SAI_OK;
+}
+
+}  // namespace sai
+
+extern "C" {
+
 static int vcf_feed_bgzf_impl(sai_engine* e, const uint8_t* data, const int64_t* block_off, const int64_t* out_off,
-                              int64_t n_blocks, int64_t skip);
+                              int64_t n_blocks, int64_t skip, int device, bool at_eof);
 int sai_engine_vcf_feed_bgzf(sai_engine* e, const uint8_t* data, const int64_t* block_off, const int64_t* out_off,
                              int64_t n_blocks, int64_t skip) {
   const double t0 = now_s();
-  const int rc = vcf_feed_bgzf_impl(e, data, block_off, out_off, n_blocks, skip);
+  const int rc = vcf_feed_bgzf_impl(e, data, block_off, out_off, n_blocks, skip, 0, true);
+  if (e) e->vcf.t_feed += now_s() - t0;
+  return rc;
+}
+int sai_engine_vcf_feed_bgzf_device(sai_engine* e, const uint8_t* data, const int64_t* block_off, const int64_t* out_off,
+                                    int64_t n_blocks, int64_t skip, int32_t at_eof) {
+  const double t0 = now_s();
+  const int rc = vcf_feed_bgzf_impl(e, data, block_off, out_off, n_blocks, skip, 1, at_eof != 0);
   if (e) e->vcf.t_feed += now_s() - t0;
   return rc;
 }
 static int vcf_feed_bgzf_impl(sai_engine* e, const uint8_t* data, const int64_t* block_off, const int64_t* out_off,
-                              int64_t n_blocks, int64_t skip) {
+                              int64_t n_blocks, int64_t skip, int device, bool at_eof) {
   SAI_REQUIRE(e && n_blocks >= 0 && skip >= 0 && (n_blocks == 0 || (data && block_off && out_off)),
               "sai_engine_vcf_feed_bgzf: bad argument");
   auto& V = e->vcf;
@@ -1176,58 +1435,22 @@ static int vcf_feed_bgzf_impl(sai_engine* e, const uint8_t* data, const int64_t*
   if (n_blocks == 0) return SAI_OK;
   SAI_REQUIRE(out_off[0] == 0 && skip <= out_off[n_blocks], "sai_engine_vcf_feed_bgzf: bad text offsets");
   SAI_CUDA_CHECK(cudaSetDevice(e->device));
-  auto fail = [&](int rc) {
-    V.sticky_rc = rc;
-    return rc;
-  };
   // the block that holds text offset `skip`
   int64_t b = std::upper_bound(out_off, out_off + n_blocks + 1, skip) - out_off - 1;
   int64_t from = skip;  // first text offset of the records (inside block b)
   V.carry.clear();
   while (b < n_blocks) {
-    // a group of blocks with at most slice_bytes of text (at least one block), inflated by the staging
-    // threads straight into the slot behind the incomplete line carried from the previous group
-    // (carry + text + 1 within the slice size: the ring slots are not reallocated slice after slice)
-    const int64_t c = (int64_t)V.carry.size();
-    int64_t b1 = b + 1;
-    while (b1 < n_blocks && c + out_off[b1 + 1] - out_off[b] + 1 <= V.slice_bytes) ++b1;
+    const int64_t b1 = vcf_group_end(e, out_off, n_blocks, b);
     SAI_REQUIRE(out_off[b1] >= out_off[b], "sai_engine_vcf_feed_bgzf: text offsets are not monotonic");
-    const int64_t text = out_off[b1] - out_off[b];
-    SAI_REQUIRE(c + text + 1 < (int64_t(1) << 31), "sai_engine_vcf_feed_bgzf: a line of more than 2 GB");
-    char* h = nullptr;
-    if (int rc = vcf_acquire_slot(e, c + text + 1, &h)) return fail(rc);
-    if (c) memcpy(h, V.carry.data(), (size_t)c);
-    const double t0 = now_s();
-    constexpr int64_t kGroup = 16;  // blocks per task (~1 MB of text)
-    std::atomic<int> bad_rc{SAI_OK};
-    std::mutex msg_mu;
-    std::string msg;
-    const std::function<void(int64_t)> f = [&](int64_t i) {
-      const int64_t g0 = b + i * kGroup, g1 = std::min(b1, g0 + kGroup);
-      int64_t rel[kGroup + 1];
-      for (int64_t k = g0; k <= g1; ++k) rel[k - g0] = out_off[k] - out_off[b] + c;
-      const int rc = sai_bgzf_inflate(data, block_off + g0, rel, g1 - g0, reinterpret_cast<uint8_t*>(h), 1);
-      if (rc != SAI_OK) {
-        std::lock_guard<std::mutex> lk(msg_mu);
-        if (bad_rc.load() == SAI_OK) msg = sai_last_error();
-        bad_rc.store(rc);
-      }
-    };
-    V.pool.run(stage_threads(e), (b1 - b + kGroup - 1) / kGroup, f);
-    V.t_stage += now_s() - t0;
-    if (bad_rc.load() != SAI_OK) {
-      set_error("%s", msg.c_str());
-      return fail(bad_rc.load());
+    SAI_REQUIRE((int64_t)V.carry.size() + out_off[b1] - out_off[b] + 1 < (int64_t(1) << 31),
+                "sai_engine_vcf_feed_bgzf: a line of more than 2 GB");
+    const bool eof = at_eof && b1 == n_blocks;
+    const int rc = device ? vcf_bgzf_group_device(e, data, block_off, out_off, b, b1, from, eof)
+                          : vcf_bgzf_group_host(e, data, block_off, out_off, b, b1, from, eof);
+    if (rc) {
+      V.sticky_rc = rc;
+      return rc;
     }
-    const int64_t lo = c == 0 && from > out_off[b] ? from - out_off[b] : 0;  // the header stays behind
-    int64_t end = c + text;
-    if (b1 == n_blocks && end > lo && h[end - 1] != '\n') h[end++] = '\n';  // last line without a newline
-    const void* nl = end > lo ? memrchr(h + lo, '\n', (size_t)(end - lo)) : nullptr;
-    const int64_t cut = nl ? static_cast<const char*>(nl) - h + 1 : lo;
-    std::vector<char> rest(h + cut, h + end);  // the incomplete last line, carried into the next slot
-    if (cut > lo)
-      if (int rc = vcf_launch_slot(e, lo, cut - lo)) return fail(rc);
-    V.carry.swap(rest);
     b = b1;
     from = out_off[b];
   }
@@ -1236,7 +1459,7 @@ static int vcf_feed_bgzf_impl(sai_engine* e, const uint8_t* data, const int64_t*
 
 int sai_engine_vcf_stats(const sai_engine* e, double* out, int32_t n) {
   SAI_REQUIRE(e && out && n >= 0, "sai_engine_vcf_stats: bad argument");
-  for (int i = 0; i < n && i < 10; ++i) out[i] = e->vcf.stats[i];
+  for (int i = 0; i < n && i < 14; ++i) out[i] = e->vcf.stats[i];
   return SAI_OK;
 }
 
@@ -1254,6 +1477,9 @@ int sai_engine_set_vcf_slicing(sai_engine* e, int64_t slice_bytes, int32_t ring)
   if (V.h_ring) SAI_CUDA_CHECK(cudaFreeHost(V.h_ring));
   V.h_ring = nullptr;
   V.slot_bytes = 0;
+  if (V.h_comp) SAI_CUDA_CHECK(cudaFreeHost(V.h_comp));  // the compressed ring has `ring` slots too
+  V.h_comp = nullptr;
+  V.comp_slot = 0;
   V.ring = r;
   return SAI_OK;
 }

@@ -13,6 +13,8 @@ directly through ctypes.
                                     u_start, q_start, totals, u_cand, q_cand)
     torch.ops.sai_b200.window_stats_pieces(pos, ws, we, first_site, last_site, jb, ...)   # several chromosomes, one launch
     torch.ops.sai_b200.column_quantiles(cols, 0.99, out)                                  # `sai outlier` thresholds
+    table, n_text = ops.bgzf_scan_table(bgzip_bytes)                                     # bgzip blocks in HBM
+    torch.ops.sai_b200.bgzf_inflate(comp, table, out, status)
 """
 
 from __future__ import annotations
@@ -123,6 +125,60 @@ def column_quantiles(cols: Tensor, quantile: float, out: Tensor) -> None:
     with torch.cuda.device(cols.device):
         _cabi.check(_cabi.load().sai_column_quantiles(cols.data_ptr(), n_cols, n_chunks, n_cols * length, length, length,
                                                       float(quantile), out.data_ptr(), _stream(cols)))
+
+
+BGZF_BLOCK = np.dtype([("comp_off", "<i8"), ("text_off", "<i8"), ("comp_bytes", "<i4"), ("isize", "<i4"), ("crc", "<u4"),
+                       ("pad_", "<i4")])  # sai_bgzf_block
+
+
+def bgzf_scan_table(data) -> tuple[Tensor, int]:
+    """Descriptors of every complete BGZF block at the start of ``data`` (bytes-like or a uint8 array:
+    the members as they lie in a bgzip file; ``comp`` = the same bytes on the device) and the bytes of
+    text they inflate to, laid out block after block.  Built by ``sai_bgzf_scan`` and
+    ``sai_bgzf_descriptors``: the payload offsets come from the library's gzip header walk."""
+    buf = np.frombuffer(data, dtype=np.uint8) if not isinstance(data, np.ndarray) else np.ascontiguousarray(data, np.uint8)
+    lib = _cabi.load()
+    tables, at, text = [], 0, 0
+    cap = 1 << 16
+    boff, ooff, used = np.empty(cap, np.int64), np.empty(cap + 1, np.int64), C.c_int64(0)
+    while at < buf.size:
+        n = int(lib.sai_bgzf_scan(buf.ctypes.data + at, buf.size - at, cap, 1 << 62, boff.ctypes.data, ooff.ctypes.data,
+                                  C.byref(used)))
+        _cabi.check(min(n, 0))
+        if n == 0:
+            break
+        t = np.zeros(n, dtype=BGZF_BLOCK)
+        _cabi.check(lib.sai_bgzf_descriptors(buf.ctypes.data + at, boff.ctypes.data, ooff.ctypes.data, n, at, text,
+                                             t.ctypes.data))
+        tables.append(t)
+        text += int(ooff[n])
+        at += used.value
+    t = np.concatenate(tables) if tables else np.zeros(0, dtype=BGZF_BLOCK)
+    return torch.from_numpy(t.view(np.uint8).copy()), text
+
+
+@torch.library.custom_op("sai_b200::bgzf_inflate", mutates_args=("out", "status"), device_types="cuda")
+def bgzf_inflate(comp: Tensor, blocks: Tensor, out: Tensor, status: Tensor) -> None:
+    """Device inflate of BGZF blocks (sai_bgzf_inflate_device): ``comp`` uint8 CUDA holds the raw
+    deflate payloads, ``blocks`` the CPU uint8 descriptor table of ``bgzf_scan_table`` (checked
+    against the buffers here), ``out`` uint8 CUDA receives the text, ``status`` int32 CUDA one value
+    per block (0 = exact size and matching CRC-32)."""
+    n, rem = divmod(blocks.numel(), BGZF_BLOCK.itemsize)
+    if blocks.device.type != "cpu" or blocks.dtype != torch.uint8 or rem:
+        raise ValueError("blocks must be a CPU uint8 tensor of sai_bgzf_block descriptors")
+    if comp.dtype != torch.uint8 or out.dtype != torch.uint8 or status.dtype != torch.int32 or status.numel() < n:
+        raise ValueError("comp / out uint8, status int32 with one value per block")
+    t = blocks.numpy().view(BGZF_BLOCK)
+    if n and ((t["comp_off"] < 0).any() or (t["comp_bytes"] < 0).any() or (t["isize"] < 0).any() or (t["isize"] > 65536).any()
+              or (t["text_off"] < 0).any() or (t["comp_off"] + t["comp_bytes"] > comp.numel()).any()
+              or (t["text_off"] + t["isize"] > out.numel()).any()):
+        raise ValueError("a block descriptor points outside comp / out or claims more than 64 KB of text")
+    if n == 0:
+        return
+    with torch.cuda.device(comp.device):
+        d_blocks = blocks.to(comp.device)
+        _cabi.check(_cabi.load().sai_bgzf_inflate_device(comp.data_ptr(), d_blocks.data_ptr(), n, out.data_ptr(),
+                                                         status.data_ptr(), _stream(comp)))
 
 
 def vcf_query_tensor(layout, chrom: str, start: int = 1, end: int = 0) -> Tensor:

@@ -309,17 +309,25 @@ class ChunkPreprocessor:
         num_src: int = 1,
         device: int = 0,
         ingest: str = "host",
+        inflate: str = "host",
     ):
         """``ingest="device"`` parses the VCF on the GPU (``vcf_device``): the text is copied to the
         device and parsed there straight into the packed tiles, which all combinations are scored
         from.  The items are identical to ``"host"``; chunks the device reader does not cover (DD,
         more than 16 populations, ancestral alleles longer than 7 bytes, source ploidies that differ
-        from their positions in a combination) are read on the host automatically."""
+        from their positions in a combination) are read on the host automatically.
+        ``inflate="device"`` (with ``ingest="device"``) also inflates a bgzip file on the GPU: only
+        the compressed blocks cross PCIe.  Plain text and single-member gzip are read as before."""
         from .vcf import parse_ind_file
 
         if ingest not in ("host", "device"):
             raise ValueError(f"ingest must be 'host' or 'device', not {ingest!r}")
+        if inflate not in ("host", "device"):
+            raise ValueError(f"inflate must be 'host' or 'device', not {inflate!r}")
+        if inflate == "device" and ingest != "device":
+            raise ValueError("inflate='device' needs ingest='device'")
         self.ingest = ingest
+        self.inflate = inflate
 
         self.vcf_file = vcf_file
         self.ref_ind_file = ref_ind_file
@@ -403,7 +411,7 @@ class ChunkPreprocessor:
             warnings.warn_explicit(w.message, w.category, w.filename, w.lineno)
         try:
             loaded = read_loaded(self.engine, self.vcf_file, chr_name, plan, requests, out, anc, anc_error, start, end,
-                                 with_outgroup=_wants_outgroup(self.stat_config))
+                                 with_outgroup=_wants_outgroup(self.stat_config), inflate=self.inflate)
         except (KeyError, OSError) as e:
             region = chr_name if start is None and end is None else f"{chr_name}:{start}-{end}"
             raise ValueError(f"Failed to read VCF file {self.vcf_file} from {region}: {e}") from e

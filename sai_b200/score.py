@@ -28,8 +28,10 @@ def score(
     num_workers: int = 1,
     device: int = 0,
     ingest: str = "host",
+    inflate: str = "host",
 ) -> None:
-    """``ingest="device"`` parses the VCF on the GPU (``ChunkPreprocessor(ingest=...)``); same output."""
+    """``ingest="device"`` parses the VCF on the GPU (``ChunkPreprocessor(ingest=...)``), and
+    ``inflate="device"`` also inflates a bgzip file there; same output."""
     cfg = load_config(config)
     stat_config, ploidy_config, pop_config = cfg.statistics, cfg.ploidies, cfg.populations
     others = [s for s in stat_config.root if s not in ("U", "Q", "Danc", "Dplus", "df", "fd", "DD") and stat_config.root[s] is not False]
@@ -62,6 +64,7 @@ def score(
         anc_allele_file=anc_allele_file,
         device=device,
         ingest=ingest,
+        inflate=inflate,
     )
     header = ["Chrom", "Start", "End", "Ref", "Tgt", "Src", "Outgroup", "N(Variants)"]
     src_pops = list(ploidy_config.root["src"].keys())

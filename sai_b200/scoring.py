@@ -243,11 +243,14 @@ class HostEngine:
         inflating into the pinned ring and waiting for a free slot, H2D and parse seconds summed over
         the slices (CUDA events), the device span from the first copy to the last parse, slices,
         text bytes, the seconds the final synchronise waited, host seconds enqueueing copies and
-        kernels, and host seconds inside the feed calls."""
-        out = (C.c_double * 10)()
-        _cabi.check(_cabi.load().sai_engine_vcf_stats(self._handle(), out, 10))
+        kernels, host seconds inside the feed calls; with ``inflate="device"`` also the inflate
+        kernel seconds (CUDA events), the compressed bytes copied and the host seconds spent
+        inflating the groups' boundary blocks, and the slices inflated on the device."""
+        out = (C.c_double * 14)()
+        _cabi.check(_cabi.load().sai_engine_vcf_stats(self._handle(), out, 14))
         keys = ("stage_s", "wait_s", "h2d_s", "parse_s", "device_span_s", "slices", "text_bytes", "finish_wait_s",
-                "launch_s", "feed_s")
+                "launch_s", "feed_s", "inflate_s", "comp_bytes", "boundary_s",
+                "inflated_slices")
         return dict(zip(keys, list(out)))
 
     def vcf_slices(self) -> int:

@@ -544,12 +544,17 @@ def _span_from_ends(vcf_file: str, chr_name: str, tail_bytes: int = 1 << 20):
     return head[1], tail[1], -1
 
 
-def _scan_sorted_region(vcf_file, chr_name, start, end, on_header, on_lines, n_threads=0, batch_bytes=256 << 20):
+def _scan_sorted_region(vcf_file, chr_name, start, end, on_header, on_lines, n_threads=0, batch_bytes=256 << 20,
+                        on_bgzf=None):
     """Region read without an index, for the usual one-chromosome, position-sorted file (plain text or
     bgzip): bisection over line starts / bgzip blocks finds the byte range that holds every record with
     ``start <= POS <= end`` (plus a little slack; the parser still filters by POS), and only that range is
     inflated and parsed -- a chunk of a sharded run costs its share of the file, not the whole file.
-    Returns False (nothing done) when the file does not qualify; the caller then scans everything."""
+    Returns False (nothing done) when the file does not qualify; the caller then scans everything.
+    ``on_bgzf(base_addr, block_off, out_off, n_blocks, skip, at_eof)``, when given, receives a bgzip
+    region as its blocks instead of text: ``block_off`` / ``out_off`` index the blocks found by the
+    bisection (``out_off[0] = 0``), the records start at text offset ``skip``, and ``at_eof`` says the
+    blocks end the file (else the last incomplete line is dropped, as the text path drops it)."""
     import ctypes as C
     import mmap
 
@@ -689,6 +694,24 @@ def _scan_sorted_region(vcf_file, chr_name, start, end, on_header, on_lines, n_t
                 probe += 1
             b_hi = n_blocks if p_hi is None else probe
             on_header(head[h:he])
+            if on_bgzf is not None:
+                blocks, texts = np.empty(b_hi - b_lo, np.int64), np.zeros(b_hi - b_lo + 1, np.int64)
+                n = int(lib.sai_bgzf_scan(base + int(boff[b_lo]), int(boff[b_hi] - boff[b_lo]), b_hi - b_lo, 1 << 62,
+                                          blocks.ctypes.data, texts.ctypes.data, C.byref(used))) if b_hi > b_lo else 0
+                if n != b_hi - b_lo:
+                    raise ValueError("bgzip block table changed under the reader")
+                blocks += int(boff[b_lo])
+                if b_lo == first_data_block:  # the records follow the header inside block b_lo
+                    skip = max(0, he + 1 - (len(head) - int(texts[1] - texts[0])))
+                else:  # behind the first newline from block b_lo on (a record that started before it)
+                    skip = int(texts[n]) if n else 0
+                    for b in range(b_lo, b_hi):
+                        nl = inflate(b, b + 1).find(b"\n")
+                        if nl >= 0:
+                            skip = int(texts[b - b_lo]) + nl + 1
+                            break
+                on_bgzf(base, blocks, texts, n, skip, b_hi == n_blocks)
+                return True
             # the records of the first data block follow the header inside `head`
             from_head = b_lo == first_data_block
             pending = head[he + 1 :] if from_head else b""

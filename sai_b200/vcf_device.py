@@ -3,7 +3,10 @@ tiles (``sai_engine_vcf_*``, ``vcf_device.cu``), which stay resident in the engi
 
 The host only reads or inflates bytes and copies them: ``_scan_text`` / ``_scan_sorted_region``
 hand their text buffers to ``sai_engine_vcf_feed`` exactly as they hand them to the host parser,
-so plain, bgzip and gzip files and region reads all work the same way.  The records and values
+so plain, bgzip and gzip files and region reads all work the same way.  With ``inflate="device"``
+a bgzip file's blocks go over compressed instead and are inflated on the device
+(``sai_engine_vcf_feed_bgzf_device``); a corrupt block repeats the read with host inflate, which
+raises the host path's error.  The records and values
 are those of ``read_data`` (the host parser is the specification); the layout is the one the host
 path packs, so the tiles are comparable byte for byte.
 """
@@ -71,10 +74,13 @@ def read_plan(vcf_file, chr_name, ploidy_config, ref_ind_file, tgt_ind_file, src
 
 
 def read_loaded(engine, vcf_file: str, chr_name: str, plan, requests, out, anc, anc_error, start=None, end=None,
-                with_outgroup: bool = True) -> Optional[LoadedChunk]:
+                with_outgroup: bool = True, inflate: str = "host") -> Optional[LoadedChunk]:
     """Parses the records of ``chr_name`` (``start <= POS <= end`` when both are given) on the
     device into ``engine``'s resident tiles, one layout for every population of ``plan`` (the
-    outgroup only with ``with_outgroup``).  ``None`` when the file has no ``#CHROM`` line."""
+    outgroup only with ``with_outgroup``).  ``None`` when the file has no ``#CHROM`` line.
+    ``inflate="device"``: bgzip blocks are inflated on the device."""
+    if inflate not in ("host", "device"):
+        raise ValueError(f"inflate must be 'host' or 'device', not {inflate!r}")
     lib = _cabi.load()
     pops = [(group, name, a, b) for group, _, gp in plan for name, a, b in gp
             if group != "outgroup" or with_outgroup]
@@ -89,7 +95,7 @@ def read_loaded(engine, vcf_file: str, chr_name: str, plan, requests, out, anc, 
     ploidy = [requests[a][1] for _, _, a, _ in pops]
     anc_pos, anc_buf, n_anc = (None, None, 0) if anc is None else anc_table(anc)
     bits, min_sites = None, 0
-    for _attempt in range(4):
+    for _attempt in range(5):
         lay = make_layout(n_samples, ploidy, bits)
         state = {"cols": None, "n_file": 0, "hint": 0, "begun": False, "fed": 0}
         consumed = C.c_int64(0)
@@ -125,16 +131,30 @@ def read_loaded(engine, vcf_file: str, chr_name: str, plan, requests, out, anc, 
 
         def on_bgzf(base: int, block_off, out_off, n_blocks: int, skip: int) -> None:
             """A whole bgzip file: inflated by the engine's threads straight into its pinned ring."""
+            if inflate == "device":
+                return on_bgzf_device(base, block_off, out_off, n_blocks, skip, True)
             text = int(out_off[n_blocks]) - skip
             begin(text)
             _cabi.check(lib.sai_engine_vcf_feed_bgzf(engine._handle(), base, block_off.ctypes.data, out_off.ctypes.data,
                                                      n_blocks, skip))
             state["fed"] += text + 1
 
+        def on_bgzf_device(base: int, block_off, out_off, n_blocks: int, skip: int, at_eof: bool) -> None:
+            """bgzip blocks (whole file or region): copied compressed and inflated on the device.  A
+            corrupt block fails in ``sai_engine_vcf_finish`` (SAI_E_CORRUPT), like one the device finds."""
+            text = int(out_off[n_blocks]) - skip
+            begin(text)
+            rc = lib.sai_engine_vcf_feed_bgzf_device(engine._handle(), base, block_off.ctypes.data, out_off.ctypes.data,
+                                                     n_blocks, skip, int(at_eof))
+            if rc != _cabi.E_CORRUPT:
+                _cabi.check(rc)
+            state["fed"] += text + 1
+
         region = (int(start), int(end)) if (start is not None and end is not None) else (1, 0)
         handled = False
         if start is not None and end is not None:
-            handled = _scan_sorted_region(vcf_file, chr_name, int(start), int(end), on_header, on_lines)
+            handled = _scan_sorted_region(vcf_file, chr_name, int(start), int(end), on_header, on_lines,
+                                          on_bgzf=on_bgzf_device if inflate == "device" else None)
         if not handled:
             _scan_text(vcf_file, on_header, on_lines, on_size_hint=on_size_hint, on_bgzf=on_bgzf)
         if state["cols"] is None:
@@ -151,6 +171,9 @@ def read_loaded(engine, vcf_file: str, chr_name: str, plan, requests, out, anc, 
             continue
         if rc == _cabi.E_CAPACITY:
             min_sites = int(n_sites.value)
+            continue
+        if rc == _cabi.E_CORRUPT:  # read again with host inflate: it raises the host path's error
+            inflate = "host"
             continue
         _cabi.check(rc)
         n = int(n_sites.value)

@@ -1,12 +1,13 @@
 #!/usr/bin/env python
 """Device VCF ingest against host ingest, file -> results (needs a GPU).
 
-    python tools/vcf_device_bench.py [--sites 600000] [--samples 2504] [--reps 2]
+    python tools/vcf_device_bench.py [--sites 600000] [--samples 2504] [--reps 2] [--level 6]
 
-Writes (untimed) a synthetic VCF of diploid, phased GT-only records in plain text and bgzip form,
-then times ``ChunkPreprocessor.run`` over the whole chromosome with ``ingest="host"`` and
-``ingest="device"`` (U and Q, one ref / tgt / src population each), checks that the items are
-identical, and breaks the device path into stages:
+Writes (untimed) a synthetic VCF of diploid, phased GT-only records in plain text and bgzip form
+(zlib level ``--level``), then times ``ChunkPreprocessor.run`` over the whole chromosome with
+``ingest="host"`` and ``ingest="device"`` -- for bgzip also ``ingest="device", inflate="device"``
+(U and Q, one ref / tgt / src population each), checks that the items are identical, and breaks the
+device path into stages:
   * the device session's own stages (``HostEngine.vcf_stats``): host seconds staging the text into
     the pinned ring (plain) or inflating the blocks into it (bgzip), host seconds waiting for a free
     ring slot, H2D and parse seconds summed over the real slices (CUDA events), the device span from
@@ -15,7 +16,9 @@ identical, and breaks the device path into stages:
   * parse: ``torch.ops.sai_b200.vcf_tiles`` on a device-resident 256 MB slice, CUDA events;
   * K1 + K4: ``score_loaded`` on the resident tiles;
   * the layout retry: the plain file with an ancestral table that flips every site (a flipped
-    missing call is 4 in a diploid: the parse is repeated with 3 planes) against one that flips none.
+    missing call is 4 in a diploid: the parse is repeated with 3 planes) against one that flips none;
+  * inflate: ``torch.ops.sai_b200.bgzf_inflate`` on every block of ~256 MB of text whose compressed
+    members are resident in HBM, CUDA events; GB/s of text out and of compressed bytes in.
 Prints one JSON line (GPU name and power limit included).
 """
 import argparse
@@ -98,6 +101,7 @@ def main():
     ap.add_argument("--sites", type=int, default=600000)
     ap.add_argument("--samples", type=int, default=2504)
     ap.add_argument("--reps", type=int, default=2)
+    ap.add_argument("--level", type=int, default=6, help="zlib level of the bgzip file")
     a = ap.parse_args()
     import torch
 
@@ -109,14 +113,15 @@ def main():
     from sai_b200.vcf_device import read_region
 
     n_ref, n_tgt = int(a.samples * 0.6), int(a.samples * 0.4) - 4
-    out = {"gpu": gpu_info(), "sites": a.sites, "samples": a.samples}
+    out = {"gpu": gpu_info(), "sites": a.sites, "samples": a.samples, "level": a.level}
     with tempfile.TemporaryDirectory() as tmp:
         vcf = os.path.join(tmp, "s.vcf")
         pos = write_vcf(vcf, a.sites, a.samples)
         bgz = os.path.join(tmp, "s.vcf.gz")
-        write_bgzf_parallel(bgz, open(vcf, "rb").read())
+        write_bgzf_parallel(bgz, open(vcf, "rb").read(), level=a.level)
         text_bytes = os.path.getsize(vcf)
         out["text_GB"] = round(text_bytes / 1e9, 3)
+        out["bgzip_GB"] = round(os.path.getsize(bgz) / 1e9, 3)
         groups = {"ref": (0, n_ref, "REF"), "tgt": (n_ref, n_ref + n_tgt, "TGT"), "src": (n_ref + n_tgt, a.samples, "SRC")}
         for g, (lo, hi, name) in groups.items():
             with open(os.path.join(tmp, f"{g}.list"), "w") as f:
@@ -128,18 +133,21 @@ def main():
         end = int(pos[-1]) + 1
         for kind, path in (("plain", vcf), ("bgzip", bgz)):
             items, times = {}, {}
-            for ingest in ("host", "device"):
+            legs = [("host", "host", "host"), ("device", "device", "host")]
+            if kind == "bgzip":
+                legs.append(("device_inflate", "device", "device"))
+            for leg, ingest, inflate in legs:
                 pre = ChunkPreprocessor(path, *lists, None, 50000, 10000, os.path.join(tmp, "o.tsv"), pc,
-                                        StatConfig(json.loads(json.dumps(stats))), ingest=ingest)
+                                        StatConfig(json.loads(json.dumps(stats))), ingest=ingest, inflate=inflate)
                 best = None
                 for _ in range(a.reps + 1):  # the first run warms the page cache and the engine's buffers
                     t0 = time.perf_counter()
-                    items[ingest] = pre.run("1", 1, end)
+                    items[leg] = pre.run("1", 1, end)
                     dt = time.perf_counter() - t0
                     best = dt if best is None else min(best, dt)
-                times[ingest] = best
+                times[leg] = best
                 if ingest == "device":
-                    out[kind + "_device_stages"] = {k: round(v, 4) for k, v in pre.engine.vcf_stats().items()}
+                    out[f"{kind}_{leg}_stages"] = {k: round(v, 4) for k, v in pre.engine.vcf_stats().items()}
                 pre.engine.close()
             out[kind] = {
                 "host_s": round(times["host"], 4), "device_s": round(times["device"], 4),
@@ -149,6 +157,13 @@ def main():
                 "host_text_GB_s": round(text_bytes / times["host"] / 1e9, 2),
                 "identical": same_items(items["host"], items["device"]),
             }
+            if kind == "bgzip":
+                out[kind].update({
+                    "device_inflate_s": round(times["device_inflate"], 4),
+                    "device_inflate_speedup": round(times["host"] / times["device_inflate"], 3),
+                    "device_inflate_vs_device": round(times["device"] / times["device_inflate"], 3),
+                    "device_inflate_identical": same_items(items["host"], items["device_inflate"]),
+                })
 
         # the layout retry: every site flipped (the rare missing calls become 4) against none flipped
         with open(os.path.join(tmp, "ref.bed"), "w") as f_ref, open(os.path.join(tmp, "alt.bed"), "w") as f_alt:
@@ -228,6 +243,35 @@ def main():
         out["parse_sites"] = n_parsed
         out["parse_TB_s"] = round(d_text.numel() / t_parse / 1e12, 3)
         eng.close()
+
+        # the inflate kernel alone: every block of the first ~256 MB of text, members resident in HBM
+        mm = np.memmap(bgz, dtype=np.uint8, mode="r")
+        table, _ = ops.bgzf_scan_table(mm)
+        n = min(table.numel() // ops.BGZF_BLOCK.itemsize, (256 << 20) // 0xFF00 + 1)
+        t = table.numpy().view(ops.BGZF_BLOCK)
+        comp_bytes = int(t["comp_bytes"][:n].sum())  # the deflate payloads the kernel reads
+        text_bytes = int(t["text_off"][n - 1] + t["isize"][n - 1])
+        raw = mm[: int(t["comp_off"][n - 1] + t["comp_bytes"][n - 1]) + 8].tobytes()
+        table = table[: n * ops.BGZF_BLOCK.itemsize].clone()
+        d_comp = torch.frombuffer(bytearray(raw), dtype=torch.uint8).cuda()
+        d_out = torch.empty(text_bytes, dtype=torch.uint8, device="cuda")
+        status = torch.empty(n, dtype=torch.int32, device="cuda")
+
+        def inflate():
+            torch.ops.sai_b200.bgzf_inflate(d_comp, table, d_out, status)
+
+        inflate()
+        torch.cuda.synchronize()
+        ok = bool((status == 0).all()) and d_out[: 1 << 20].cpu().numpy().tobytes() == open(vcf, "rb").read(1 << 20)
+        e0.record()
+        for _ in range(5):
+            inflate()
+        e1.record()
+        torch.cuda.synchronize()
+        t_inf = e0.elapsed_time(e1) / 1e3 / 5
+        out["inflate_kernel"] = {"blocks": n, "text_MB": round(text_bytes / 1e6, 1), "comp_MB": round(comp_bytes / 1e6, 1),
+                                 "s": round(t_inf, 5), "text_GB_s": round(text_bytes / t_inf / 1e9, 2),
+                                 "comp_GB_s": round(comp_bytes / t_inf / 1e9, 3), "ok": ok}
     print(json.dumps(out))
 
 
