@@ -183,6 +183,59 @@ __device__ __forceinline__ SiteFlags eval_site_fast(const JobFast& F, const sai_
   return out;
 }
 
+// ---------------------------------------------------------------------------
+// Gates of the staged genotype pass (k_site_gated).  A site is flagged only if its sources
+// match (op(src_freq, y), or op(src_freq, 1 - y) without ancestral alleles) and its possibly
+// inverted ref_freq < w, so the pass reads the sources first and the reference and target only
+// where a job can still hold.  Each factor below is evaluated per lane exactly as eval_site /
+// eval_site_fast evaluate it (interval test for a fully called population, the IEEE division
+// otherwise), so a gate is a superset of the final decision: it lets through every site that
+// will be flagged, and the flags themselves still come from eval_site_fast.
+// with_ref == false: sources only (the reference need not have been read yet).
+// ---------------------------------------------------------------------------
+template <typename NumFn, typename CalledFn>
+__device__ __forceinline__ void site_gate(const JobFast& F, const sai_job& J, const sai_layout& lay, bool with_ref,
+                                          NumFn num_of, CalledFn called_of, bool& gate_u, bool& gate_q) {
+  const bool fast = F.ok != 0;
+  bool valid = true, my_u = true, mf_u = true, my_q = true, mf_q = true;
+  for (int k = 0; k < J.n_src; ++k) {
+    const int sp = J.src_pop[k];
+    const int ns = num_of(sp);
+    const int ds = called_of(sp) * lay.pop[sp].ploidy;
+    valid = valid && ds > 0 && ns <= ds;
+    if (fast && ds == F.den_src[k]) {
+      my_u = my_u && ns >= F.u.y_lo[k] && ns <= F.u.y_hi[k];
+      mf_u = mf_u && ns >= F.u.f_lo[k] && ns <= F.u.f_hi[k];
+      my_q = my_q && ns >= F.q.y_lo[k] && ns <= F.q.y_hi[k];
+      mf_q = mf_q && ns >= F.q.f_lo[k] && ns <= F.q.f_hi[k];
+    } else {
+      const double fs = site_freq(ns, ds);
+      my_u = my_u && cmp_op(J.u.op[k], fs, J.u.y[k]);
+      mf_u = mf_u && cmp_op(J.u.op[k], fs, J.u.one_minus_y[k]);
+      my_q = my_q && cmp_op(J.q.op[k], fs, J.q.y[k]);
+      mf_q = mf_q && cmp_op(J.q.op[k], fs, J.q.one_minus_y[k]);
+    }
+  }
+  const bool anc = J.anc_allele_available != 0;
+  gate_u = valid && J.u.enabled && (my_u || (!anc && mf_u));
+  gate_q = valid && J.q.enabled && (my_q || (!anc && mf_q));
+  if (!with_ref || !(gate_u || gate_q)) return;
+  const int nr = num_of(J.ref_pop), dr = called_of(J.ref_pop) * lay.pop[J.ref_pop].ploidy;
+  if (!(dr > 0 && nr <= dr)) {
+    gate_u = gate_q = false;
+    return;
+  }
+  const bool full = fast && dr == F.den_ref;
+  const double fr = full ? 0.0 : site_freq(nr, dr);
+  // ref_freq < w, or 1 - ref_freq < w where the job inverts (as eval_cond)
+  auto ref_ok = [&](const CondFast& X, const sai_cond& C, bool inv) {
+    if (full) return inv ? nr >= X.ref_inv_min : nr <= X.ref_max;
+    return (inv ? __dsub_rn(1.0, fr) : fr) < C.w;
+  };
+  gate_u = gate_u && ref_ok(F.u, J.u, !anc && mf_u);
+  gate_q = gate_q && ref_ok(F.q, J.q, !anc && mf_q);
+}
+
 // host: interval ends for one job (plain IEEE double division / subtraction, as on the device)
 void build_job_fast(const sai_layout& lay, const sai_job& J, JobFast& F);
 

@@ -15,6 +15,7 @@
 
 #include "common.cuh"
 #include "popcount.cuh"
+#include "scratch.cuh"
 #include "site_cond.cuh"
 
 namespace sai {
@@ -174,6 +175,22 @@ __device__ __forceinline__ void count_wide(const uint2* __restrict__ col, int n_
   miss = accm;
 }
 
+// (num, called) of one population at the lane's site; col = the population's first pair of the tile
+template <int MODE>
+__device__ __forceinline__ void count_pop(const sai_pop_layout& L, const uint2* __restrict__ col, int& num,
+                                          int& called) {
+  int miss;
+  if (L.bits == 2)
+    count_b2<MODE>(col, L.n_pairs, num, miss);
+  else if (L.bits == 4)
+    count_b4(col, L.n_groups, num, miss);
+  else if (L.bits == 3)
+    count_b3(col, L.n_groups, num, miss);
+  else
+    count_wide(col, L.n_groups, L.bits, num, miss);
+  called = L.n_groups * 32 - miss;
+}
+
 // ---- host side of the integer fast path (site_cond.cuh) ----------------------------
 namespace {
 // first n in [0, d + 1] for which pred(n) holds; pred must be monotone (false ... false true ... true)
@@ -243,6 +260,10 @@ struct SiteParams {
   int32_t* num;
   int32_t* called;
   int64_t count_stride;
+  // k_site_gated only
+  unsigned long long* next_batch;  // batch counter, zero at launch
+  uint32_t gate_pops;              // populations that are a source of a job with U or Q enabled
+  int32_t batch_tiles;             // tiles per batch, 1..kGateTiles
 };
 
 constexpr int kSiteWarps = 8;
@@ -264,17 +285,8 @@ __global__ void __launch_bounds__(kSiteWarps * 32, MODE == 1 ? 3 : 4)
     const uint2* tile = P.packed + (size_t)T * pps * kTile + lane;
     for (int pi = 0; pi < n_pops; ++pi) {
       const sai_pop_layout& L = P.lay.pop[pi];
-      const uint2* col = tile + (size_t)L.pair_off * kTile;
-      int num, miss;
-      if (L.bits == 2)
-        count_b2<MODE>(col, L.n_pairs, num, miss);
-      else if (L.bits == 4)
-        count_b4(col, L.n_groups, num, miss);
-      else if (L.bits == 3)
-        count_b3(col, L.n_groups, num, miss);
-      else
-        count_wide(col, L.n_groups, L.bits, num, miss);
-      const int called = L.n_groups * 32 - miss;
+      int num, called;
+      count_pop<MODE>(L, tile + (size_t)L.pair_off * kTile, num, called);
       s_num[pi * kTile + lane] = num;
       s_cal[pi * kTile + lane] = called;
       if (P.num) {
@@ -297,6 +309,142 @@ __global__ void __launch_bounds__(kSiteWarps * 32, MODE == 1 ? 3 : 4)
           P.mask_q[(size_t)j * P.n_tiles_total + T] = mq;
         }
         if (f.q) P.qval[(size_t)j * P.qval_stride + site] = f.q_tgt_freq;
+      }
+    }
+  }
+}
+
+// K1 without stored counts: the staged pass.  A site can be flagged only where its sources match
+// and its reference frequency is below w (site_gate), and the sources are the smallest operand
+// (bench layout: 1 of 80 pairs), so a tile is read in three stages -- the source populations of
+// all jobs, the references of the jobs still live on the tile, the targets of those still live --
+// and each population at most once.  On the bench spectrum 77 % of the tiles stop after the
+// source pair and 4.8x fewer bytes are read.  Decisions are unchanged: a tile that reaches the
+// third stage has every count its live jobs need and runs eval_site_fast as k_site does; a job
+// dead on a tile stores zero mask words (and no qval, which exists only at Q-flagged sites).
+//
+// A warp claims batches of batch_tiles consecutive tiles from a global counter (live tiles fall at
+// random, and a static tile-to-warp map leaves the busiest warp with ~2x the mean bytes) and reads
+// the source pairs of the whole batch at once, so a 1-pair source still has one load per tile in
+// flight.  Shared memory holds the counts of every tile of the batch: [warp][tile][2][n_pops][32].
+// 4 tiles per batch: on one B200, 8 was slower on both the bench job and the all-live job, and 2
+// slower on the bench job (DESIGN section 4).
+constexpr int kGateTiles = 4;
+constexpr int kGateSmemPerWarp = 6144;  // 48 KB per 8-warp block: 4 blocks per SM
+
+__global__ void __launch_bounds__(kSiteWarps * 32, 4)
+    k_site_gated(const __grid_constant__ SiteParams P, const __grid_constant__ JobBlock JB,
+                 const __grid_constant__ JobFastBlock JF) {
+  extern __shared__ int s_counts[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int n_pops = P.lay.n_pops, G = P.batch_tiles;
+  const int per_tile = 2 * n_pops * kTile;
+  int* s_warp = s_counts + warp * G * per_tile;
+  const int64_t pps = P.lay.pairs_per_site;
+  const int64_t n_batches = (P.n_tiles + G - 1) / G;
+  // lane 0 claims; the claim of the next batch is in flight while this one is read
+  auto claim = [&]() { return lane == 0 ? atomicAdd(P.next_batch, 1ull) : 0ull; };
+  unsigned long long claimed = claim();
+  for (int64_t b = (int64_t)__shfl_sync(0xffffffffu, claimed, 0); b < n_batches;
+       b = (int64_t)__shfl_sync(0xffffffffu, claimed, 0)) {
+    claimed = claim();
+    const int64_t t0 = b * G;
+    const int n = (int)(P.n_tiles - t0 < G ? P.n_tiles - t0 : G);
+    const uint2* batch = P.packed + (size_t)(P.tile0 + t0) * pps * kTile + lane;
+
+    // stage 1: the source populations of the n tiles.  2 planes: pair by pair across the batch,
+    // n loads in flight per lane; other widths tile by tile.
+    for (uint32_t m = P.gate_pops; m; m &= m - 1) {
+      const int pi = __ffs(m) - 1;
+      const sai_pop_layout& L = P.lay.pop[pi];
+      int* s_num = s_warp + pi * kTile + lane;
+      int* s_cal = s_num + n_pops * kTile;
+      if (L.bits == 2) {
+        int num[kGateTiles], miss[kGateTiles];
+#pragma unroll
+        for (int g = 0; g < kGateTiles; ++g) num[g] = miss[g] = 0;
+        for (int i = 0; i < L.n_pairs; ++i) {
+          uint2 v[kGateTiles];
+#pragma unroll
+          for (int g = 0; g < kGateTiles; ++g)
+            v[g] = g < n ? ld_stream(batch + ((size_t)g * pps + L.pair_off + i) * kTile) : make_uint2(0u, 0u);
+#pragma unroll
+          for (int g = 0; g < kGateTiles; ++g) {
+            const int mm = __popc(v[g].x & v[g].y);
+            num[g] += __popc(v[g].x) + 2 * __popc(v[g].y) - 3 * mm;
+            miss[g] += mm;
+          }
+        }
+#pragma unroll
+        for (int g = 0; g < kGateTiles; ++g) {
+          if (g < n) {
+            s_num[g * per_tile] = num[g];
+            s_cal[g * per_tile] = L.n_groups * 32 - miss[g];
+          }
+        }
+      } else {
+        for (int g = 0; g < n; ++g)
+          count_pop<0>(L, batch + ((size_t)g * pps + L.pair_off) * kTile, s_num[g * per_tile], s_cal[g * per_tile]);
+      }
+    }
+
+    for (int g = 0; g < n; ++g) {
+      const int64_t T = P.tile0 + t0 + g;
+      const uint2* tile = batch + (size_t)g * pps * kTile;
+      int* s_num = s_warp + g * per_tile;
+      int* s_cal = s_num + n_pops * kTile;
+      auto num_of = [&](int pop) { return s_num[pop * kTile + lane]; };
+      auto called_of = [&](int pop) { return s_cal[pop * kTile + lane]; };
+      auto read = [&](uint32_t pops) {
+        for (; pops; pops &= pops - 1) {
+          const int pi = __ffs(pops) - 1;
+          const sai_pop_layout& L = P.lay.pop[pi];
+          count_pop<0>(L, tile + (size_t)L.pair_off * kTile, s_num[pi * kTile + lane], s_cal[pi * kTile + lane]);
+        }
+      };
+      // live: jobs whose U or Q can still hold at some site of the tile (warp-uniform)
+      uint32_t live = 0;
+      for (int j = 0; j < JB.n_jobs; ++j) {
+        bool u, q;
+        site_gate(JF.job[j], JB.job[j], P.lay, false, num_of, called_of, u, q);
+        live |= (uint32_t)(u || q) << j;
+      }
+      live = __reduce_or_sync(0xffffffffu, live);
+      uint32_t have = P.gate_pops;
+      // stage 2: the references of the live jobs, then the reference gate
+      if (live) {
+        uint32_t need = 0;
+        for (uint32_t m = live; m; m &= m - 1) need |= 1u << JB.job[__ffs(m) - 1].ref_pop;
+        read(need & ~have);
+        have |= need;
+        uint32_t still = 0;
+        for (uint32_t m = live; m; m &= m - 1) {
+          const int j = __ffs(m) - 1;
+          bool u, q;
+          site_gate(JF.job[j], JB.job[j], P.lay, true, num_of, called_of, u, q);
+          still |= (uint32_t)(u || q) << j;
+        }
+        live = __reduce_or_sync(0xffffffffu, still);
+      }
+      // stage 3: the targets of the jobs still live
+      if (live) {
+        uint32_t need = 0;
+        for (uint32_t m = live; m; m &= m - 1) need |= 1u << JB.job[__ffs(m) - 1].tgt_pop;
+        read(need & ~have);
+      }
+      const int64_t site = T * kTile + lane;
+      for (int j = 0; j < JB.n_jobs; ++j) {
+        uint32_t mu = 0, mq = 0;
+        if ((live >> j) & 1u) {
+          const SiteFlags f = eval_site_fast(JF.job[j], JB.job[j], P.lay, num_of, called_of);
+          mu = __ballot_sync(0xffffffffu, f.u);
+          mq = __ballot_sync(0xffffffffu, f.q);
+          if (f.q) P.qval[(size_t)j * P.qval_stride + site] = f.q_tgt_freq;
+        }
+        if (lane == 0) {
+          P.mask_u[(size_t)j * P.n_tiles_total + T] = mu;
+          P.mask_q[(size_t)j * P.n_tiles_total + T] = mq;
+        }
       }
     }
   }
@@ -411,6 +559,34 @@ static int launch_site(const SiteParams& P, const JobBlock& JB, cudaStream_t st)
   k_site<MODE, FUSED><<<grid, kSiteWarps * 32, smem, st>>>(P, JB, JF);
   SAI_CUDA_CHECK(cudaGetLastError());
   return SAI_OK;
+}
+
+static int launch_site_gated(SiteParams P, const JobBlock& JB, cudaStream_t st) {
+  if (P.n_tiles == 0) return SAI_OK;
+  P.gate_pops = 0;
+  for (int j = 0; j < JB.n_jobs; ++j) {
+    const sai_job& J = JB.job[j];
+    if (J.u.enabled || J.q.enabled)
+      for (int k = 0; k < J.n_src; ++k) P.gate_pops |= 1u << J.src_pop[k];
+  }
+  const int tile_bytes = 2 * P.lay.n_pops * kTile * (int)sizeof(int);
+  P.batch_tiles = std::max(1, std::min(kGateTiles, kGateSmemPerWarp / tile_bytes));
+  const size_t smem = (size_t)kSiteWarps * P.batch_tiles * tile_bytes;
+  int occ = 0;
+  SAI_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_site_gated, kSiteWarps * 32, smem));
+  if (occ < 1) occ = 1;
+  const int64_t n_batches = (P.n_tiles + P.batch_tiles - 1) / P.batch_tiles;
+  const int64_t want = (n_batches + kSiteWarps - 1) / kSiteWarps;
+  const int64_t cap = (int64_t)sm_count() * occ;
+  JobFastBlock JF;
+  fill_job_fast(P.lay, JB, JF);
+  void* counter = nullptr;
+  if (int rc = scratch_alloc(&counter, sizeof(unsigned long long), st)) return rc;
+  P.next_batch = static_cast<unsigned long long*>(counter);
+  SAI_CUDA_CHECK(cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
+  k_site_gated<<<(int)(want < cap ? want : cap), kSiteWarps * 32, smem, st>>>(P, JB, JF);
+  SAI_CUDA_CHECK(cudaGetLastError());
+  return scratch_free(counter, st);
 }
 
 
@@ -685,7 +861,9 @@ int sai_site_flags(const sai_layout* lay, const void* d_packed, int64_t tile0, i
 #else
   SAI_REQUIRE(variant == 0, "variant %d exists only in -DSAI_EXPERIMENTS builds", variant);
 #endif
-  return launch_site<0, true>(P, JB, st);
+  // stored counts: every population is read anyway
+  if (d_num) return launch_site<0, true>(P, JB, st);
+  return launch_site_gated(P, JB, st);
 }
 
 int sai_flags_from_counts(const sai_layout* lay, const int32_t* d_num, const int32_t* d_called,
