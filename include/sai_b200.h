@@ -29,8 +29,8 @@
  *    (2^B - 1) means missing.  B = 2 covers haploid/diploid data (0,1,2,missing); B up to 8
  *    holds every int8 value (multi-allelic GT indices are not recoded by the reference, and a
  *    flipped missing allele counts 2: sai/utils/utils.py:119-135, :555).  The genotype pass is
- *    at the HBM roofline for B = 2..4; B = 5..8 take a plain per-word path, and DD
- *    (sai_site_hist / sai_window_dd) is limited to B <= 4.
+ *    at the HBM roofline for B = 2..4; B = 5..8 take a plain per-word path (DD included:
+ *    sai_site_hist / sai_window_dd).
  *  - 32 individuals of one population form a *group*: B consecutive 32-bit
  *    words (plane 0 .. plane B-1), bit i of a word = individual 32*g + i.
  *    Unused individuals of the last group are coded missing.
@@ -397,14 +397,19 @@ int sai_window_patterns(const sai_layout* lay, const int32_t* d_pos, int64_t n_s
  * neg_off is host memory ([n_pops + 1], neg_off[0] = 0).
  *
  * sai_site_hist: one genotype pass over the listed populations; row r of population
- * pops[q] (rows of earlier populations first, 2^bits - 1 rows each, sai_hist_rows() in total)
- *     d_hist[r*stride + site] = number of individuals whose called value is r.
+ * pops[q] (rows of earlier populations first, sai_hist_rows() in total: 2^bits - 1 rows for
+ * bits <= 4, 16 rows for bits 5..8)
+ *     d_hist[r*stride + site] = number of individuals whose called value is r   (r <= 14),
+ * and for bits 5..8 row 15 = number of *wide* calls (called values >= 15), which
+ * sai_window_dd reads back from the bit-planes.
  * d_missing[q] (optional) = missing calls of pops[q] over sites < n_sites, padding excluded.
  *
  * sai_window_dd: d_hist must hold {ref_pop, tgt_pop} in this order.  Per source population k,
  * window i and source individual a (exact integers)
  *     d_ref_sum[(k*W + i)*m_max + a] = sum_j sum_sites |src_a - ref_j|        (tgt likewise)
- * *d_err is set to 1 if a missing source call has no table entry.  The caller forms
+ * *d_err is set to 1 if a missing source call has no table entry.  Per-site distances are int32:
+ * ref and tgt may hold at most 8 454 660 individuals each (254 per individual and site).
+ * The caller forms
  *     DD_k = mean_a( ref_sum/n_ref - tgt_sum/n_tgt )           dd_statistic.py:74-77 */
 int64_t sai_hist_rows(const sai_layout* lay, const int32_t* pops, int32_t n);
 int sai_site_hist(const sai_layout* lay, const void* d_packed, int64_t n_sites, const int32_t* pops,

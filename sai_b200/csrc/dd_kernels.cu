@@ -14,16 +14,22 @@
 // the reference's own operations (the sums of integers below 2^53 are exact in
 // the reference's float64 too), which makes DD bit-exact.
 //
-// Per site, sum_j |s - ref_j| = sum_u c_u |s - u| + sum_{missing j} |s - raw_j|,
-// with c_u the number of individuals holding the called value u:
+// Per site, sum_j |s - ref_j| = sum_u c_u |s - u| + sum_{j not in c} |s - r_j|,
+// with c_u the number of individuals holding the called value u (u = 0..14); the rest are the
+// missing calls (raw values from the negative-value table) and, in populations of 5-8 planes,
+// the *wide* calls (values 15..127, read back from the planes):
 //   k_site_hist   one genotype pass over ref and tgt -> c_u per site (bit-plane
-//                 match masks + POPC; lane == site as in k_site)
+//                 match masks + POPC; lane == site as in k_site), plus the number of
+//                 wide calls of a 5-8-plane population
 //   k_site_dd     per site and source individual the two distances sum_j |src_a - ref_j|,
-//                 sum_j |src_a - tgt_j| (called part from c_u, missing calls from the
-//                 negative-value table: the bit-planes keep a single "missing" code, the table
-//                 restores the raw values) -- once per site, not once per overlapping window
+//                 sum_j |src_a - tgt_j| (called part from c_u, wide calls from the planes,
+//                 missing calls from the negative-value table: the bit-planes keep a single
+//                 "missing" code, the table restores the raw values) -- once per site, not once
+//                 per overlapping window
 //   k_window_dd   one warp per (source population, window): exact int64 sums of those
 //                 per-site integers over the window's site range.
+// The site and entry kernels come in two builds: kMaxB = 4 for layouts of 2-4 planes (the
+// common case, unchanged) and kMaxB = 8 as soon as one DD population has 5-8 planes.
 #include <algorithm>
 
 #include "common.cuh"
@@ -34,7 +40,14 @@ namespace sai {
 
 constexpr int kHistWarps = 8;
 constexpr int kDdWarps = 8;
-constexpr int kMaxCodes = 15;  // called values of a 4-plane population
+constexpr int kMaxCodes = 15;  // called values of a 4-plane population; histogram rows of values
+                               // 0..14 in wider populations, whose row kMaxCodes counts wide calls
+
+// histogram rows holding called values (2^B - 1, or 0..14 when the population is wider)
+template <int kMaxB>
+__device__ __forceinline__ int value_rows(int bits) {
+  return kMaxB > 4 && bits > 4 ? kMaxCodes : (1 << bits) - 1;
+}
 
 struct HistParams {
   const uint2* packed;
@@ -62,6 +75,7 @@ __device__ __forceinline__ unsigned long long warp_sum_u64(unsigned long long v)
 }
 
 // grid-stride over tiles, one warp per tile, lane == site
+template <int kMaxB>
 __global__ void __launch_bounds__(kHistWarps * 32, 4) k_site_hist(const __grid_constant__ HistParams P) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   // population by population (each one's pairs are a contiguous 256 B x n_pairs run of a tile)
@@ -104,6 +118,37 @@ __global__ void __launch_bounds__(kHistWarps * 32, 4) k_site_hist(const __grid_c
         out[0] = 32 * G - c1 - c2 - miss;
         out[P.stride] = c1;
         out[2 * P.stride] = c2;
+      } else if (kMaxB > 4 && B > 4) {
+        // values 0..14 as in a 4-plane population (planes 4.. clear), then one row of wide calls:
+        // not all-ones and either a high plane set or value 15 (planes 0..3 set, the rest clear)
+        int cnt[kMaxCodes];
+#pragma unroll
+        for (int u = 0; u < kMaxCodes; ++u) cnt[u] = 0;
+        int wide = 0;
+        for (int g = 0; g < G; ++g) {
+          uint32_t w[4];
+#pragma unroll
+          for (int b = 0; b < 4; ++b) w[b] = plane_word(col, g * B + b);
+          const uint32_t low_ones = w[0] & w[1] & w[2] & w[3];
+          uint32_t hi = 0, all = low_ones;
+          for (int b = 4; b < B; ++b) {
+            const uint32_t x = plane_word(col, g * B + b);
+            hi |= x;
+            all &= x;
+          }
+          miss += __popc(all);
+          wide += __popc((hi | low_ones) & ~all);
+#pragma unroll
+          for (int u = 0; u < kMaxCodes; ++u) {
+            uint32_t m = ~hi;
+#pragma unroll
+            for (int b = 0; b < 4; ++b) m &= ((u >> b) & 1) ? w[b] : ~w[b];
+            cnt[u] += __popc(m);
+          }
+        }
+#pragma unroll
+        for (int u = 0; u < kMaxCodes; ++u) out[(size_t)u * P.stride] = cnt[u];
+        out[(size_t)kMaxCodes * P.stride] = wide;
       } else {
         int cnt[kMaxCodes];
 #pragma unroll
@@ -198,12 +243,14 @@ __device__ __forceinline__ int64_t warp_lower_bound(const int32_t* __restrict__ 
 
 // ---- pass 2: per-site distances, once per site -------------------------------------------------
 // A site lies in win_len / win_step windows; its contribution
-//     dist[a][ref] = sum_j |src_a - ref_j| = sum_u c_u |s_a - u| + sum_{missing j} |s_a - raw_j|
+//     dist[a][ref] = sum_j |src_a - ref_j| = sum_u c_u |s_a - u| + sum_{j not in c} |s_a - r_j|
 // (s_a: the source individual's called value, or its raw negative value from the table when its
 // call is missing) does not depend on the window, so it is computed once and the window kernel
-// only adds integers.  Two launches, neither of which searches the tables per site:
+// only adds integers.  Two launches:
 //   k_site_dd    site-driven, lane == site: the called part sum_u c_u |s_a - u| of every CALLED
-//                source individual (0 for a missing one) -- plain stores;
+//                source individual (0 for a missing one) -- plain stores; then, only where a
+//                5-8-plane ref / tgt has wide calls at the site, |s_a - v| for each wide value v
+//                and every source individual, a missing one with its raw value from the table;
 //   k_entry_dd   entry-driven, one thread per table entry: a missing ref / tgt call adds
 //                |s_a - raw| for every source individual of its site; a missing source call adds
 //                its called part sum_u c_u |raw - u| -- integer atomics, order-free and exact.
@@ -215,59 +262,6 @@ __device__ __forceinline__ int called_part(const int (&cu)[kMaxCodes], int s) {
     d += cu[u] * (diff < 0 ? -diff : diff);  // cu is 0 beyond the population's called values
   }
   return d;
-}
-
-__global__ void __launch_bounds__(kDdWarps * 32) k_site_dd(const __grid_constant__ DdParams P) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int64_t T = (int64_t)blockIdx.x * kDdWarps + warp; T < P.n_tiles; T += (int64_t)gridDim.x * kDdWarps) {
-    const int site = (int)(T * kTile) + lane;
-    int cu[2][kMaxCodes];
-#pragma unroll
-    for (int t = 0; t < 2; ++t) {
-      const DdPop& pp = t == 0 ? P.ref : P.tgt;
-      const int32_t* h = P.hist + (size_t)pp.code_base * P.stride + site;
-      const int n_called = (1 << pp.bits) - 1;
-#pragma unroll
-      for (int u = 0; u < kMaxCodes; ++u) cu[t][u] = u < n_called ? __ldg(h + (size_t)u * P.stride) : 0;
-    }
-    for (int k = 0; k < P.n_src; ++k) {
-      const DdPop& sp = P.src[k];
-      const int s_missing = (1 << sp.bits) - 1;
-      const uint2* col = P.packed + ((size_t)T * P.pairs_per_site + sp.pair_off) * kTile + lane;
-      // called source values repeat (0, 1, 2 for two planes): their distances once per site
-      int dc[2][3];
-      if (sp.bits == 2) {
-#pragma unroll
-        for (int t = 0; t < 2; ++t)
-#pragma unroll
-          for (int v = 0; v < 3; ++v) dc[t][v] = called_part(cu[t], v);
-      }
-      for (int a0 = 0; a0 < sp.n_samples; a0 += 32) {
-        uint32_t w[4];
-#pragma unroll
-        for (int b = 0; b < 4; ++b) w[b] = b < sp.bits ? plane_word(col, (a0 >> 5) * sp.bits + b) : 0u;
-        const int cnt = sp.n_samples - a0 < 32 ? sp.n_samples - a0 : 32;
-        for (int bit = 0; bit < cnt; ++bit) {
-          int sv = 0;
-#pragma unroll
-          for (int b = 0; b < 4; ++b) sv |= (int)((w[b] >> bit) & 1u) << b;
-          int dr = 0, dt = 0;
-          if (sv != s_missing) {
-            if (sp.bits == 2) {
-              dr = sv == 0 ? dc[0][0] : (sv == 1 ? dc[0][1] : dc[0][2]);
-              dt = sv == 0 ? dc[1][0] : (sv == 1 ? dc[1][1] : dc[1][2]);
-            } else {
-              dr = called_part(cu[0], sv);
-              dt = called_part(cu[1], sv);
-            }
-          }
-          int32_t* o = P.dist + (size_t)(P.slot0[k] + a0 + bit) * 2 * P.stride + site;
-          o[0] = dr;
-          o[P.stride] = dt;
-        }
-      }
-    }
-  }
 }
 
 // raw value of a missing call: entry (site, ind) of the population's table slice
@@ -288,7 +282,133 @@ __device__ __forceinline__ bool raw_lookup(const DdParams& P, const DdPop& pp, i
   return false;
 }
 
+// n (<= 8) wide values of ref (t = 0) or tgt (t = 1) at this lane's site, one byte each in `vals`,
+// against every source individual.  In k_site_dd the lane owns its site's dist entries.
+template <int kMaxB>
+__device__ __forceinline__ void add_wide(const DdParams& P, int64_t T, int site, int lane, int t,
+                                         unsigned long long vals, int n) {
+  for (int k = 0; k < P.n_src; ++k) {
+    const DdPop& sp = P.src[k];
+    const int s_missing = (1 << sp.bits) - 1;
+    const uint2* col = P.packed + ((size_t)T * P.pairs_per_site + sp.pair_off) * kTile + lane;
+    for (int a0 = 0; a0 < sp.n_samples; a0 += 32) {
+      uint32_t w[kMaxB];
+#pragma unroll
+      for (int b = 0; b < kMaxB; ++b) w[b] = b < sp.bits ? plane_word(col, (a0 >> 5) * sp.bits + b) : 0u;
+      const int cnt = sp.n_samples - a0 < 32 ? sp.n_samples - a0 : 32;
+      for (int bit = 0; bit < cnt; ++bit) {
+        int sv = 0;
+#pragma unroll
+        for (int b = 0; b < kMaxB; ++b) sv |= (int)((w[b] >> bit) & 1u) << b;
+        if (sv == s_missing) {
+          sv = -1;
+          if (!raw_lookup(P, sp, site, a0 + bit, sv)) *P.err = 1;
+        }
+        int d = 0;
+        for (int i = 0; i < n; ++i) {
+          const int diff = sv - (int)((vals >> (8 * i)) & 0xffu);
+          d += diff < 0 ? -diff : diff;
+        }
+        P.dist[((size_t)(P.slot0[k] + a0 + bit) * 2 + t) * P.stride + site] += d;
+      }
+    }
+  }
+}
+
+// kMaxB = 8: a min-blocks hint of 1 lets ptxas use 80 registers instead of spilling at 64
+template <int kMaxB>
+__global__ void __launch_bounds__(kDdWarps * 32, kMaxB > 4 ? 1 : 0) k_site_dd(const __grid_constant__ DdParams P) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int64_t T = (int64_t)blockIdx.x * kDdWarps + warp; T < P.n_tiles; T += (int64_t)gridDim.x * kDdWarps) {
+    const int site = (int)(T * kTile) + lane;
+    int cu[2][kMaxCodes];
+#pragma unroll
+    for (int t = 0; t < 2; ++t) {
+      const DdPop& pp = t == 0 ? P.ref : P.tgt;
+      const int32_t* h = P.hist + (size_t)pp.code_base * P.stride + site;
+      const int n_called = value_rows<kMaxB>(pp.bits);
+#pragma unroll
+      for (int u = 0; u < kMaxCodes; ++u) cu[t][u] = u < n_called ? __ldg(h + (size_t)u * P.stride) : 0;
+    }
+    for (int k = 0; k < P.n_src; ++k) {
+      const DdPop& sp = P.src[k];
+      const int s_missing = (1 << sp.bits) - 1;
+      const uint2* col = P.packed + ((size_t)T * P.pairs_per_site + sp.pair_off) * kTile + lane;
+      // called source values repeat (0, 1, 2 for two planes): their distances once per site
+      int dc[2][3];
+      if (sp.bits == 2) {
+#pragma unroll
+        for (int t = 0; t < 2; ++t)
+#pragma unroll
+          for (int v = 0; v < 3; ++v) dc[t][v] = called_part(cu[t], v);
+      }
+      for (int a0 = 0; a0 < sp.n_samples; a0 += 32) {
+        uint32_t w[kMaxB];
+#pragma unroll
+        for (int b = 0; b < kMaxB; ++b) w[b] = b < sp.bits ? plane_word(col, (a0 >> 5) * sp.bits + b) : 0u;
+        const int cnt = sp.n_samples - a0 < 32 ? sp.n_samples - a0 : 32;
+        for (int bit = 0; bit < cnt; ++bit) {
+          int sv = 0;
+#pragma unroll
+          for (int b = 0; b < kMaxB; ++b) sv |= (int)((w[b] >> bit) & 1u) << b;
+          int dr = 0, dt = 0;
+          if (sv != s_missing) {
+            if (sp.bits == 2) {
+              dr = sv == 0 ? dc[0][0] : (sv == 1 ? dc[0][1] : dc[0][2]);
+              dt = sv == 0 ? dc[1][0] : (sv == 1 ? dc[1][1] : dc[1][2]);
+            } else {
+              dr = called_part(cu[0], sv);
+              dt = called_part(cu[1], sv);
+            }
+          }
+          int32_t* o = P.dist + (size_t)(P.slot0[k] + a0 + bit) * 2 * P.stride + site;
+          o[0] = dr;
+          o[P.stride] = dt;
+        }
+      }
+    }
+    if constexpr (kMaxB > 4) {
+      // wide ref / tgt calls: re-read the population's planes where its wide-call row is non-zero
+      for (int t = 0; t < 2; ++t) {
+        const DdPop& pp = t == 0 ? P.ref : P.tgt;
+        if (pp.bits <= 4) continue;
+        int left = __ldg(P.hist + (size_t)(pp.code_base + kMaxCodes) * P.stride + site);
+        const uint2* col = P.packed + ((size_t)T * P.pairs_per_site + pp.pair_off) * kTile + lane;
+        const int G = (pp.n_samples + 31) >> 5;
+        for (int g = 0; g < G && left > 0; ++g) {
+          uint32_t w[kMaxB];
+#pragma unroll
+          for (int b = 0; b < kMaxB; ++b) w[b] = b < pp.bits ? plane_word(col, g * pp.bits + b) : 0u;
+          const uint32_t low_ones = w[0] & w[1] & w[2] & w[3];
+          uint32_t hi = 0, all = low_ones;
+#pragma unroll
+          for (int b = 4; b < kMaxB; ++b) {
+            hi |= w[b];
+            if (b < pp.bits) all &= w[b];
+          }
+          uint32_t wm = (hi | low_ones) & ~all;  // as k_site_hist's wide row
+          left -= __popc(wm);
+          while (wm) {
+            unsigned long long vals = 0;
+            int n = 0;
+            for (; wm && n < 8; ++n) {
+              const int bit = __ffs(wm) - 1;
+              wm &= wm - 1;
+              int v = 0;
+#pragma unroll
+              for (int b = 0; b < kMaxB; ++b) v |= (int)((w[b] >> bit) & 1u) << b;
+              vals |= (unsigned long long)v << (8 * n);
+            }
+            add_wide<kMaxB>(P, T, site, lane, t, vals, n);
+          }
+        }
+      }
+    }
+  }
+}
+
 // one thread per entry of the ref table, the tgt table and the source tables, in that order
+template <int kMaxB>
 __global__ void __launch_bounds__(256) k_entry_dd(const __grid_constant__ DdParams P, int64_t n_ref, int64_t n_tgt,
                                                   int64_t n_total) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -304,14 +424,14 @@ __global__ void __launch_bounds__(256) k_entry_dd(const __grid_constant__ DdPara
         const int s_missing = (1 << sp.bits) - 1;
         const uint2* col = P.packed + ((size_t)(site >> 5) * P.pairs_per_site + sp.pair_off) * kTile + (site & 31);
         for (int a0 = 0; a0 < sp.n_samples; a0 += 32) {
-          uint32_t w[4];
+          uint32_t w[kMaxB];
 #pragma unroll
-          for (int b = 0; b < 4; ++b) w[b] = b < sp.bits ? plane_word(col, (a0 >> 5) * sp.bits + b) : 0u;
+          for (int b = 0; b < kMaxB; ++b) w[b] = b < sp.bits ? plane_word(col, (a0 >> 5) * sp.bits + b) : 0u;
           const int cnt = sp.n_samples - a0 < 32 ? sp.n_samples - a0 : 32;
           for (int bit = 0; bit < cnt; ++bit) {
             int sv = 0;
 #pragma unroll
-            for (int b = 0; b < 4; ++b) sv |= (int)((w[b] >> bit) & 1u) << b;
+            for (int b = 0; b < kMaxB; ++b) sv |= (int)((w[b] >> bit) & 1u) << b;
             if (sv == s_missing) {  // the source call is missing too: its raw value is in the table
               sv = -1;
               if (!raw_lookup(P, sp, site, a0 + bit, sv)) *P.err = 1;
@@ -322,7 +442,7 @@ __global__ void __launch_bounds__(256) k_entry_dd(const __grid_constant__ DdPara
         }
       }
     } else {
-      // a missing source call against the called ref / tgt values of its site
+      // a missing source call against the called ref / tgt values 0..14 of its site (wide ones: k_site_dd)
       int64_t r = i - n_ref - n_tgt;
       int k = 0;
       while (k + 1 < P.n_src && r >= P.src[k].neg_hi - P.src[k].neg_lo) {
@@ -336,7 +456,7 @@ __global__ void __launch_bounds__(256) k_entry_dd(const __grid_constant__ DdPara
       for (int t = 0; t < 2; ++t) {
         const DdPop& pp = t == 0 ? P.ref : P.tgt;
         const int32_t* h = P.hist + (size_t)pp.code_base * P.stride + site;
-        const int n_called = (1 << pp.bits) - 1;
+        const int n_called = value_rows<kMaxB>(pp.bits);
         int d = 0;
         for (int u = 0; u < n_called; ++u) {
           const int diff = v - u;
@@ -394,7 +514,20 @@ __global__ void __launch_bounds__(kDdWarps * 32) k_window_dd(const __grid_consta
   }
 }
 
-static int32_t code_rows(const sai_pop_layout& L) { return (1 << L.bits) - 1; }
+// histogram rows of a population: one per called value for 2-4 planes; values 0..14 plus the
+// wide-call row for 5-8 planes (a dense histogram of 255 values would take 6 GB per population
+// at chromosome-1 scale)
+static int32_t code_rows(const sai_pop_layout& L) { return L.bits > 4 ? kMaxCodes + 1 : (1 << L.bits) - 1; }
+
+// a per-site distance sum_j |s - r_j| is at most 254 n (values 0..127, raw values -127..-1) and is
+// kept in int32
+constexpr int32_t kMaxDdSamples = 2147483647 / 254;
+
+static bool any_wide(const sai_layout* lay, const int32_t* pops, int n) {
+  for (int q = 0; q < n; ++q)
+    if (lay->pop[pops[q]].bits > 4) return true;
+  return false;
+}
 
 }  // namespace sai
 
@@ -433,7 +566,6 @@ extern "C" int sai_site_hist(const sai_layout* lay, const void* d_packed, int64_
   for (int q = 0; q < n_hist_pops; ++q) {
     SAI_REQUIRE(pops[q] >= 0 && pops[q] < lay->n_pops, "bad population index");
     const sai_pop_layout& L = lay->pop[pops[q]];
-    SAI_REQUIRE(L.bits <= 4, "DD supports per-individual values up to 14 (population %d has %d bit-planes)", pops[q], L.bits);
     P.pair_off[q] = L.pair_off;
     P.n_groups[q] = L.n_groups;
     P.bits[q] = L.bits;
@@ -447,7 +579,8 @@ extern "C" int sai_site_hist(const sai_layout* lay, const void* d_packed, int64_
   if (d_missing) SAI_CUDA_CHECK(cudaMemsetAsync(d_missing, 0, sizeof(uint64_t) * n_hist_pops, st));
   const int64_t want = (n_tiles + kHistWarps - 1) / kHistWarps;
   const int64_t cap = (int64_t)sm_count() * 4;  // 56 registers: 4 resident blocks per SM, one wave
-  k_site_hist<<<(unsigned)(want < cap ? want : cap), kHistWarps * 32, 0, st>>>(P);
+  auto kernel = any_wide(lay, pops, n_hist_pops) ? k_site_hist<SAI_MAX_BITS> : k_site_hist<4>;
+  kernel<<<(unsigned)(want < cap ? want : cap), kHistWarps * 32, 0, st>>>(P);
   SAI_CUDA_CHECK(cudaGetLastError());
   return SAI_OK;
 }
@@ -470,10 +603,8 @@ extern "C" int sai_window_dd(const sai_layout* lay, const void* d_packed, const 
   SAI_REQUIRE(neg_off[0] == 0, "neg_off[0] must be 0");
   for (int p = 0; p < lay->n_pops; ++p) SAI_REQUIRE(neg_off[p + 1] >= neg_off[p], "neg_off must be non-decreasing");
   SAI_REQUIRE(neg_off[lay->n_pops] == 0 || (d_neg_site && d_neg_ind && d_neg_val), "NULL negative-value table");
-  for (int k = 0; k < n_src; ++k)
-    SAI_REQUIRE(src_pops[k] >= 0 && src_pops[k] < lay->n_pops && lay->pop[src_pops[k]].bits <= 4,
-                "DD supports per-individual values up to 14");
-  SAI_REQUIRE(lay->pop[ref_pop].bits <= 4 && lay->pop[tgt_pop].bits <= 4, "DD supports per-individual values up to 14");
+  SAI_REQUIRE(lay->pop[ref_pop].n_samples <= kMaxDdSamples && lay->pop[tgt_pop].n_samples <= kMaxDdSamples,
+              "DD supports at most %d individuals in ref and tgt", kMaxDdSamples);
   auto fill = [&](DdPop& d, int pop, int32_t code_base) {
     const sai_pop_layout& L = lay->pop[pop];
     d.pair_off = L.pair_off;
@@ -523,9 +654,11 @@ extern "C" int sai_window_dd(const sai_layout* lay, const void* d_packed, const 
   if (int rc = scratch_alloc(&scratch, sizeof(int32_t) * 2 * (size_t)slots * (size_t)std::max<int64_t>(stride, 32), st)) return rc;
   P.dist = static_cast<int32_t*>(scratch);
   if (P.n_tiles > 0) {
+    const int32_t ref_tgt[2] = {ref_pop, tgt_pop};
+    const bool wide = any_wide(lay, ref_tgt, 2) || any_wide(lay, src_pops, n_src);
     const int64_t wantt = (P.n_tiles + kDdWarps - 1) / kDdWarps;
     const int64_t capt = (int64_t)sm_count() * 16;
-    k_site_dd<<<(unsigned)(wantt < capt ? wantt : capt), kDdWarps * 32, 0, st>>>(P);
+    (wide ? k_site_dd<SAI_MAX_BITS> : k_site_dd<4>)<<<(unsigned)(wantt < capt ? wantt : capt), kDdWarps * 32, 0, st>>>(P);
     SAI_CUDA_CHECK(cudaGetLastError());
     const int64_t n_ref = P.ref.neg_hi - P.ref.neg_lo, n_tgt = P.tgt.neg_hi - P.tgt.neg_lo;
     int64_t n_total = n_ref + n_tgt;
@@ -533,7 +666,7 @@ extern "C" int sai_window_dd(const sai_layout* lay, const void* d_packed, const 
     if (n_total > 0) {
       const int64_t wante = (n_total + 255) / 256;
       const int64_t cape = (int64_t)sm_count() * 32;
-      k_entry_dd<<<(unsigned)(wante < cape ? wante : cape), 256, 0, st>>>(P, n_ref, n_tgt, n_total);
+      (wide ? k_entry_dd<SAI_MAX_BITS> : k_entry_dd<4>)<<<(unsigned)(wante < cape ? wante : cape), 256, 0, st>>>(P, n_ref, n_tgt, n_total);
       SAI_CUDA_CHECK(cudaGetLastError());
     }
   }
