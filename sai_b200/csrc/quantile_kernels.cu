@@ -220,7 +220,9 @@ __global__ void __cluster_dims__(kQCluster, 1, 1) __launch_bounds__(kQThreads, 1
     const double vi = __dmul_rn((double)(n - 1), P.q);
     long long cle;
     if (vi >= (double)(n - 1)) {
-      thr = key_value(kmax);
+      // numpy lerps the largest value with itself: b - (b - b) (1 - g) is b for a finite b, NaN for +inf
+      const double b = key_value(kmax);
+      thr = __dadd_rn(b, __dsub_rn(b, b));
     } else {
       const double fl = floor(vi);
       const long long k = (long long)fl;

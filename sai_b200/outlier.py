@@ -34,7 +34,10 @@ def linear_quantile_sorted(v: np.ndarray, q: float) -> float:
     n = v.size
     vi = np.float64(n - 1) * np.float64(q)
     if vi >= n - 1:
-        return float(v[-1])
+        # numpy lerps the last value with itself: top for a finite top, NaN for +inf
+        top = np.float64(v[-1])
+        with np.errstate(invalid="ignore"):
+            return float(top + (top - top))
     lo = int(np.floor(vi))
     g = np.float64(vi - lo)
     a, b = np.float64(v[lo]), np.float64(v[lo + 1])
