@@ -66,7 +66,8 @@ enum {
   SAI_E_DOMAIN = -3,   /* genotype value does not fit the bit-planes            */
   SAI_E_CAPACITY = -4, /* candidate buffers too small; totals were written      */
   SAI_E_NOMEM = -5,
-  SAI_E_CORRUPT = -6   /* a bgzip block inflated on the device is corrupt; see sai_last_error() */
+  SAI_E_CORRUPT = -6,  /* a bgzip block inflated on the device is corrupt; see sai_last_error() */
+  SAI_E_ORDER = -7     /* genome ingest: a chromosome's records resume after another chromosome's */
 };
 
 /* comparator of a source population, `"=", "<", ">", "<=", ">="`
@@ -615,6 +616,42 @@ int64_t sai_engine_vcf_slices(const sai_engine* e);
 int sai_engine_vcf_stats(const sai_engine* e, double* out, int32_t n);
 /* The resident tiles of the finished session (sai_packed_bytes(lay, n_sites) bytes) into HOST `out`. */
 int sai_engine_loaded_tiles(sai_engine* e, uint8_t* out, uint64_t cap);
+
+/* ---- genome ingest: every chromosome of a table from one pass over a multi-chromosome VCF ------
+ * sai_engine_vcf_genome_begin: as sai_engine_vcf_begin, with n_chrom (1..SAI_VCF_MAX_CHROMS) distinct
+ * chromosome names (names[name_off[c] .. name_off[c + 1]), 1..255 bytes each, HOST) instead of one
+ * name and no region, and the ancestral-allele tables of all of them concatenated: chromosome c's
+ * entries are anc_pos / anc_allele [anc_off[c], anc_off[c + 1]) (HOST; n_anc = anc_off[n_chrom];
+ * anc_off == NULL: no table, nothing is filtered).  A record's CHROM is hashed into a table in shared
+ * memory and compared once, so a record costs the same whatever n_chrom is.  The session is fed with
+ * sai_engine_vcf_feed / _feed_bgzf / _feed_bgzf_device.  Kept records become sites in file order, and
+ * each chromosome's first site lies on a tile boundary (the genome layout of sai_window_stats_pieces):
+ * the sites between a chromosome's last site and the next boundary are coded all-missing, so a
+ * chromosome's tiles equal sai_pack_i8_all's over that chromosome alone.
+ * sai_engine_vcf_genome_finish: as sai_engine_vcf_finish (*n_sites counts the padding sites, and so
+ * does the SAI_E_CAPACITY retry), plus chroms[c] for every chromosome of the table.  SAI_E_ORDER: a
+ * chromosome's kept records resume after another chromosome's (the tiles are not usable; read such a
+ * file one chromosome at a time). */
+#define SAI_VCF_MAX_CHROMS 1024
+typedef struct {
+  int64_t first_pos, last_pos; /* POS of the first / last record in file order (sai_vcf_chrom_span's  */
+  int64_t n_records;           /* semantics, every record: before the ancestral-allele filter); 0 none */
+  int64_t first_site, n_sites; /* kept sites [first_site, first_site + n_sites); first_site -1: none  */
+} sai_vcf_chrom;
+int sai_engine_vcf_genome_begin(sai_engine* e, const sai_layout* lay, const char* names, const int32_t* name_off,
+                                int32_t n_chrom, const int32_t* sample_column, int32_t n_out, const int32_t* anc_pos,
+                                const char* anc_allele, const int64_t* anc_off, int32_t n_file_samples,
+                                int64_t text_bytes_hint, int64_t min_sites);
+int sai_engine_vcf_genome_finish(sai_engine* e, int64_t* n_sites, int32_t* max_value, sai_vcf_chrom* chroms,
+                                 int32_t* pos_out, int64_t pos_cap);
+/* sai_engine_score_loaded over pieces of the resident tiles: piece p = pieces[3p .. 3p + 2] = (number of
+ * windows, first site (a multiple of 32), number of sites); the windows are given piece after piece.
+ * One genotype pass over all tiles, one sai_window_stats_pieces launch.  Afterwards
+ * sai_engine_score_resident / _rescore_windows / _pattern_sums (one sai_window_patterns per piece) work
+ * on the same pieces; sai_engine_dd_sums is refused. */
+int sai_engine_score_loaded_pieces(sai_engine* e, const int64_t* win_start, const int64_t* win_end,
+                                   const int64_t* pieces, int32_t n_pieces, const sai_job* jobs, int32_t n_jobs,
+                                   sai_host_results* out);
 
 /* ---- synthetic genotypes (bench / tests only) ---------------------------- */
 /* Fills tiles [tile0, tile0+n_tiles) of a packed matrix directly on the device

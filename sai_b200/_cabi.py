@@ -16,7 +16,8 @@ MAX_SRC = 8
 MAX_JOBS = 8
 TILE_SITES = 32
 
-OK, E_ARG, E_CUDA, E_DOMAIN, E_CAPACITY, E_NOMEM, E_CORRUPT = 0, -1, -2, -3, -4, -5, -6
+OK, E_ARG, E_CUDA, E_DOMAIN, E_CAPACITY, E_NOMEM, E_CORRUPT, E_ORDER = 0, -1, -2, -3, -4, -5, -6, -7
+MAX_CHROMS = 1024  # SAI_VCF_MAX_CHROMS: chromosomes of one genome ingest
 OPS = {"=": 0, "<": 1, ">": 2, "<=": 3, ">=": 4}
 
 
@@ -101,6 +102,16 @@ class VcfState(C.Structure):
         ("overflow", C.c_int32),
         ("pad_", C.c_int32),
         ("vmax", C.c_int32 * MAX_POPS),
+    ]
+
+
+class VcfChrom(C.Structure):
+    _fields_ = [
+        ("first_pos", C.c_int64),
+        ("last_pos", C.c_int64),
+        ("n_records", C.c_int64),
+        ("first_site", C.c_int64),
+        ("n_sites", C.c_int64),
     ]
 
 
@@ -203,6 +214,10 @@ SYMBOLS = {
     "sai_engine_set_vcf_slicing": (C.c_int, [_P, _I64, _I32]),
     "sai_engine_vcf_slices": (_I64, [_P]),
     "sai_engine_loaded_tiles": (C.c_int, [_P, _P, _U64]),
+    "sai_engine_vcf_genome_begin": (
+        C.c_int, [_P, _LAY, _P, _P, _I32, _P, _I32, _P, _P, _P, _I32, _I64, _I64]),
+    "sai_engine_vcf_genome_finish": (C.c_int, [_P, C.POINTER(_I64), _P, C.POINTER(VcfChrom), _P, _I64]),
+    "sai_engine_score_loaded_pieces": (C.c_int, [_P, _P, _P, _P, _I32, _JOB, _I32, C.POINTER(HostResults)]),
 }
 
 _lib = None

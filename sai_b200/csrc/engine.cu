@@ -24,6 +24,7 @@
 
 #include "common.cuh"
 #include "host_pack.h"
+#include "vcf_genome.cuh"
 #include "zt_format.cuh"
 #include "zt_simd.h"
 
@@ -116,10 +117,15 @@ struct sai_engine {
   int32_t n_jobs = 0;
   sai_job jobs[SAI_MAX_JOBS];
   sai_layout lay{};  // layout of the resident tiles (sai_engine_score_resident)
+  // sai_engine_score_loaded_pieces: (first window, windows, first site, sites) per piece; empty = one chunk.
+  // Per-window first / last sites follow the window bounds in `win`.
+  std::vector<std::array<int64_t, 4>> pieces;
   // ingest session (sai_engine_vcf_*): text ring (pinned + device), the query and its tables
   struct Vcf {
     int state = 0;                    // 0 none, 1 feeding, 2 finished (tiles resident)
     sai_vcf_query q{};
+    bool genome = false;              // sai_engine_vcf_genome_begin: the chromosome table of gq
+    sai::VcfGenomeQuery gq{};
     int64_t site_cap = 0;             // sites the tile / position buffers hold (multiple of 32)
     int64_t row_bytes = 64;           // lower bound of a record's length: sizes the tile buffer
     int64_t fed = 0, n_slices = 0;
@@ -145,6 +151,7 @@ struct sai_engine {
   } vcf;
   Buf vtext, vscratch, vcols, vanc_pos, vanc_all, vstate;
   Buf vcomp, vbad;  // device inflate: ring of compressed groups (+ block statuses), first corrupt block
+  Buf vgen;         // genome ingest: hash table, names, offsets, running state, per-chromosome records
 };
 
 namespace sai {
@@ -201,13 +208,22 @@ static int run_windows(sai_engine* e, sai_host_results* out) {
   int32_t* d_uc = static_cast<int32_t*>(e->cand.p);
   int32_t* d_qc = reinterpret_cast<int32_t*>(static_cast<char*>(e->cand.p) + cu);
   cudaStream_t st = e->s_comp;
-  if (int rc = sai_window_stats(
-          static_cast<const int32_t*>(e->pos.p), e->n_sites, d_ws, d_ws + W, W, e->jobs, n_jobs,
-          d_mask_u, d_mask_q, static_cast<const double*>(e->qval.p), stride,
-          reinterpret_cast<int32_t*>(res + rl.nsnps), reinterpret_cast<int64_t*>(res + rl.u),
-          reinterpret_cast<double*>(res + rl.q), reinterpret_cast<int32_t*>(res + rl.q_cnt),
-          reinterpret_cast<int64_t*>(res + rl.u_start), reinterpret_cast<int64_t*>(res + rl.q_start),
-          reinterpret_cast<int64_t*>(res + rl.totals), d_uc, out->cap_u, d_qc, out->cap_q, st))
+  const int32_t* d_first = reinterpret_cast<const int32_t*>(d_ws + 2 * W);
+  if (int rc = e->pieces.empty()
+                   ? sai_window_stats(
+                         static_cast<const int32_t*>(e->pos.p), e->n_sites, d_ws, d_ws + W, W, e->jobs, n_jobs,
+                         d_mask_u, d_mask_q, static_cast<const double*>(e->qval.p), stride,
+                         reinterpret_cast<int32_t*>(res + rl.nsnps), reinterpret_cast<int64_t*>(res + rl.u),
+                         reinterpret_cast<double*>(res + rl.q), reinterpret_cast<int32_t*>(res + rl.q_cnt),
+                         reinterpret_cast<int64_t*>(res + rl.u_start), reinterpret_cast<int64_t*>(res + rl.q_start),
+                         reinterpret_cast<int64_t*>(res + rl.totals), d_uc, out->cap_u, d_qc, out->cap_q, st)
+                   : sai_window_stats_pieces(
+                         static_cast<const int32_t*>(e->pos.p), e->n_sites, d_ws, d_ws + W, d_first, d_first + W, W,
+                         e->jobs, n_jobs, d_mask_u, d_mask_q, static_cast<const double*>(e->qval.p), stride,
+                         reinterpret_cast<int32_t*>(res + rl.nsnps), reinterpret_cast<int64_t*>(res + rl.u),
+                         reinterpret_cast<double*>(res + rl.q), reinterpret_cast<int32_t*>(res + rl.q_cnt),
+                         reinterpret_cast<int64_t*>(res + rl.u_start), reinterpret_cast<int64_t*>(res + rl.q_start),
+                         reinterpret_cast<int64_t*>(res + rl.totals), d_uc, out->cap_u, d_qc, out->cap_q, st))
     return rc;
   const size_t n = (size_t)n_jobs * (size_t)W;
   if (n > 0) {
@@ -562,6 +578,7 @@ static int score_host_impl(sai_engine* e, const sai_layout* lay, const uint8_t* 
   }
   e->n_sites = n_sites;
   e->W = W;
+  e->pieces.clear();
   e->n_jobs = n_jobs;
   e->lay = *lay;
   for (int j = 0; j < n_jobs; ++j) e->jobs[j] = jobs[j];
@@ -711,12 +728,25 @@ int sai_engine_pattern_sums(sai_engine* e, const sai_layout* lay, int32_t ref_po
   int32_t* d_called = d_num + (size_t)lay->n_pops * stride;
   if (int rc = sai_site_counts(lay, e->packed.p, 0, n_tiles, d_num, d_called, stride, 0, e->s_comp)) return rc;
   const int64_t* d_ws = static_cast<const int64_t*>(e->win.p);
-  if (int rc = sai_window_patterns(lay, static_cast<const int32_t*>(e->pos.p), e->n_sites, d_ws, d_ws + W, W,
-                                   d_num, d_called, stride, ref_pop, tgt_pop, out_pop, src_pops, n_src,
-                                   static_cast<double*>(e->sums.p), e->s_comp))
-    return rc;
-  SAI_CUDA_CHECK(cudaMemcpyAsync(sums, e->sums.p, sizeof(double) * 7 * (size_t)n_src * W,
-                                 cudaMemcpyDeviceToHost, e->s_comp));
+  const int32_t* d_pos = static_cast<const int32_t*>(e->pos.p);
+  double* d_sums = static_cast<double*>(e->sums.p);
+  if (e->pieces.empty()) {
+    if (int rc = sai_window_patterns(lay, d_pos, e->n_sites, d_ws, d_ws + W, W, d_num, d_called, stride, ref_pop, tgt_pop,
+                                     out_pop, src_pops, n_src, d_sums, e->s_comp))
+      return rc;
+    SAI_CUDA_CHECK(cudaMemcpyAsync(sums, d_sums, sizeof(double) * 7 * (size_t)n_src * W, cudaMemcpyDeviceToHost, e->s_comp));
+  } else {  // one sai_window_patterns per piece on its sites and counts; sums[k][w0 + i] <- piece's [k][i]
+    for (const auto& P : e->pieces) {
+      const int64_t w0 = P[0], nw = P[1], lo = P[2];
+      if (nw == 0) continue;
+      double* d_p = d_sums + 7 * (size_t)n_src * w0;
+      if (int rc = sai_window_patterns(lay, d_pos + lo, P[3], d_ws + w0, d_ws + W + w0, nw, d_num + lo, d_called + lo,
+                                       stride, ref_pop, tgt_pop, out_pop, src_pops, n_src, d_p, e->s_comp))
+        return rc;
+      SAI_CUDA_CHECK(cudaMemcpy2DAsync(sums + 7 * w0, sizeof(double) * 7 * W, d_p, sizeof(double) * 7 * nw,
+                                       sizeof(double) * 7 * nw, n_src, cudaMemcpyDeviceToHost, e->s_comp));
+    }
+  }
   SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));
   return SAI_OK;
 }
@@ -731,6 +761,7 @@ int sai_engine_dd_sums(sai_engine* e, const sai_layout* lay, int32_t ref_pop, in
   SAI_REQUIRE(ref_pop >= 0 && ref_pop < lay->n_pops && tgt_pop >= 0 && tgt_pop < lay->n_pops,
               "bad population index");
   SAI_REQUIRE(m_max >= 1, "m_max must be positive");
+  SAI_REQUIRE(e->pieces.empty(), "sai_engine_dd_sums: the resident tiles are scored in pieces");
   SAI_CUDA_CHECK(cudaSetDevice(e->device));
   const int64_t n_tiles = sai_num_tiles(e->n_sites);
   const int64_t stride = n_tiles * kTile;
@@ -833,6 +864,29 @@ int sai_engine_rescore_windows(sai_engine* e, sai_host_results* out) {
 // the slice in it has been parsed (`parsed`).
 namespace sai {
 
+// vgen (genome ingest): hash table | name_off | anc_off | state | chroms | names, 256-byte aligned parts
+struct GenLayout {
+  size_t hash, name_off, anc_off, state, chroms, names, total;
+};
+static GenLayout gen_layout(int n_chrom, size_t name_bytes) {
+  GenLayout g{};
+  size_t at = 0;
+  g.hash = at, at += align256(sizeof(uint32_t) * 2 * kChromHashSlots);
+  g.name_off = at, at += align256(sizeof(int32_t) * (n_chrom + 1));
+  g.anc_off = at, at += align256(sizeof(int64_t) * (n_chrom + 1));
+  g.state = at, at += align256(sizeof(VcfGenomeState));
+  g.chroms = at, at += align256(sizeof(VcfChromDev) * n_chrom);
+  g.names = at, at += align256(name_bytes);
+  g.total = at;
+  return g;
+}
+static VcfGenomeState* vcf_genome_state(sai_engine* e) {
+  return reinterpret_cast<VcfGenomeState*>(static_cast<char*>(e->vgen.p) + gen_layout(e->vcf.gq.n_chrom, 0).state);
+}
+static VcfChromDev* vcf_genome_chroms(sai_engine* e) {
+  return reinterpret_cast<VcfChromDev*>(static_cast<char*>(e->vgen.p) + gen_layout(e->vcf.gq.n_chrom, 0).chroms);
+}
+
 // tile / position buffers for `cap` sites; `keep`: the sites parsed so far move along
 static int vcf_grow_sites(sai_engine* e, int64_t cap, bool keep) {
   auto& V = e->vcf;
@@ -872,6 +926,11 @@ static int vcf_wait(cudaEvent_t ev) {
   }
 }
 
+// parse scratch of one slice of `len` bytes for the session's query
+static uint64_t vcf_scratch_need(const sai_engine* e, int64_t len) {
+  return e->vcf.genome ? vcf_genome_scratch_bytes(e->vcf.gq, len) : sai_vcf_scratch_bytes(&e->vcf.q, len);
+}
+
 static int stage_threads(const sai_engine* e) {
   return std::min(16, e->host_threads > 0 ? e->host_threads : (int)std::max(1u, std::thread::hardware_concurrency()));
 }
@@ -894,7 +953,7 @@ static int vcf_acquire_slot(sai_engine* e, int64_t n, char** h) {
     V.slot_bytes = 0;
     SAI_CUDA_CHECK(cudaHostAlloc(reinterpret_cast<void**>(&V.h_ring), slot * V.ring, cudaHostAllocDefault));
     if (int rc = grow(e->vtext, slot * V.ring)) return rc;
-    if (int rc = grow(e->vscratch, sai_vcf_scratch_bytes(&V.q, (int64_t)slot))) return rc;
+    if (int rc = grow(e->vscratch, vcf_scratch_need(e, (int64_t)slot))) return rc;
     V.slot_bytes = slot;
   }
   while ((int)V.copied.size() < V.ring) {
@@ -938,7 +997,8 @@ static int vcf_launch_slot(sai_engine* e, int64_t off, int64_t n, const DevGroup
 static int vcf_launch_slot_impl(sai_engine* e, int64_t off, int64_t n, const DevGroup* g) {
   auto& V = e->vcf;
   V.fed += n;
-  const int64_t need = V.fed / V.row_bytes + V.n_slices + 1 + 1024;  // records of normal width in the text so far
+  // records of normal width in the text so far (+ a tile of padding per chromosome of a genome parse)
+  const int64_t need = V.fed / V.row_bytes + V.n_slices + 1 + 1024 + (V.genome ? (int64_t)kTile * V.gq.n_chrom : 0);
   if (need > V.site_cap)
     if (int rc = vcf_grow_sites(e, std::max(need, 2 * V.site_cap), true)) return rc;
   while ((int64_t)V.tev.size() <= V.n_slices) {
@@ -984,8 +1044,13 @@ static int vcf_launch_slot_impl(sai_engine* e, int64_t off, int64_t n, const Dev
     SAI_CUDA_CHECK(cudaStreamWaitEvent(e->s_comp, V.copied[slot], 0));
   }
   SAI_CUDA_CHECK(cudaEventRecord(T[2], e->s_comp));
-  if (int rc = sai_vcf_tiles_device(&V.q, d, n, e->vscratch.p, e->vscratch.cap, e->packed.p, static_cast<int32_t*>(e->pos.p),
-                                    V.site_cap, static_cast<sai_vcf_state*>(e->vstate.p), e->s_comp))
+  if (int rc = V.genome ? vcf_tiles_genome(V.gq, d, n, e->vscratch.p, e->vscratch.cap, e->packed.p,
+                                            static_cast<int32_t*>(e->pos.p), V.site_cap,
+                                            static_cast<sai_vcf_state*>(e->vstate.p), vcf_genome_state(e),
+                                            vcf_genome_chroms(e), e->s_comp)
+                       : sai_vcf_tiles_device(&V.q, d, n, e->vscratch.p, e->vscratch.cap, e->packed.p,
+                                              static_cast<int32_t*>(e->pos.p), V.site_cap,
+                                              static_cast<sai_vcf_state*>(e->vstate.p), e->s_comp))
     return rc;
   SAI_CUDA_CHECK(cudaEventRecord(T[3], e->s_comp));
   SAI_CUDA_CHECK(cudaEventRecord(V.parsed[slot], e->s_comp));
@@ -1034,7 +1099,9 @@ int sai_engine_vcf_begin(sai_engine* e, const sai_layout* lay, const char* chrom
     SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));
   }
   V.state = 0;
+  V.genome = false;
   e->n_jobs = 0;  // the resident chunk is replaced
+  e->pieces.clear();
   sai_vcf_query& q = V.q;
   q = sai_vcf_query{};
   q.lay = *lay;
@@ -1061,7 +1128,7 @@ int sai_engine_vcf_begin(sai_engine* e, const sai_layout* lay, const char* chrom
   V.site_cap = 0;  // the buffers' content is not kept from an earlier chunk
   if (int rc = vcf_grow_sites(e, std::max(text_bytes_hint / V.row_bytes + 1024, min_sites), false)) return rc;
   if (V.slot_bytes > 0)  // the scratch depends on the query (max_column): resize for the ring's slots
-    if (int rc = grow(e->vscratch, sai_vcf_scratch_bytes(&q, (int64_t)V.slot_bytes))) return rc;
+    if (int rc = grow(e->vscratch, vcf_scratch_need(e, (int64_t)V.slot_bytes))) return rc;
   if (int rc = grow(e->vbad, sizeof(unsigned long long))) return rc;
   SAI_CUDA_CHECK(cudaMemsetAsync(e->vbad.p, 0xff, sizeof(unsigned long long), e->s_copy));  // no corrupt block
   V.fed = V.n_slices = 0;
@@ -1119,8 +1186,83 @@ static int vcf_feed_impl(sai_engine* e, const char* text, int64_t len, int64_t* 
   return SAI_OK;
 }
 
+static int vcf_finish_impl(sai_engine* e, int64_t* n_sites, int32_t* max_value, int32_t* pos_out, int64_t pos_cap);
 int sai_engine_vcf_finish(sai_engine* e, int64_t* n_sites, int32_t* max_value, int32_t* pos_out, int64_t pos_cap) {
   SAI_REQUIRE(e && n_sites && max_value, "sai_engine_vcf_finish: NULL argument");
+  SAI_REQUIRE(!e->vcf.genome, "sai_engine_vcf_finish: a genome session ends with sai_engine_vcf_genome_finish");
+  return vcf_finish_impl(e, n_sites, max_value, pos_out, pos_cap);
+}
+
+int sai_engine_vcf_genome_begin(sai_engine* e, const sai_layout* lay, const char* names, const int32_t* name_off,
+                                int32_t n_chrom, const int32_t* sample_column, int32_t n_out, const int32_t* anc_pos,
+                                const char* anc_allele, const int64_t* anc_off, int32_t n_file_samples,
+                                int64_t text_bytes_hint, int64_t min_sites) {
+  SAI_REQUIRE(e && names && name_off, "sai_engine_vcf_genome_begin: NULL argument");
+  std::vector<uint32_t> table(2 * kChromHashSlots);
+  if (int rc = vcf_chrom_table(names, name_off, n_chrom, table.data())) return rc;
+  const int64_t n_anc = anc_off ? anc_off[n_chrom] : 0;
+  for (int c = 0; anc_off && c < n_chrom; ++c)
+    SAI_REQUIRE(anc_off[0] == 0 && anc_off[c] <= anc_off[c + 1], "sai_engine_vcf_genome_begin: bad ancestral-table offsets");
+  const std::string first(names + name_off[0], names + name_off[1]);
+  if (int rc = sai_engine_vcf_begin(e, lay, first.c_str(), 1, 0, sample_column, n_out, anc_pos, anc_allele, n_anc,
+                                    n_file_samples, text_bytes_hint, min_sites))
+    return rc;
+  auto& V = e->vcf;
+  V.state = 0;  // until the table is in place
+  const GenLayout gl = gen_layout(n_chrom, (size_t)name_off[n_chrom]);
+  if (int rc = grow(e->vgen, gl.total)) return rc;
+  char* g = static_cast<char*>(e->vgen.p);
+  std::vector<int64_t> aoff(n_chrom + 1, 0);
+  if (anc_off) std::copy(anc_off, anc_off + n_chrom + 1, aoff.begin());
+  SAI_CUDA_CHECK(cudaMemcpyAsync(g + gl.hash, table.data(), sizeof(uint32_t) * table.size(), cudaMemcpyHostToDevice, e->s_comp));
+  SAI_CUDA_CHECK(cudaMemcpyAsync(g + gl.name_off, name_off, sizeof(int32_t) * (n_chrom + 1), cudaMemcpyHostToDevice, e->s_comp));
+  SAI_CUDA_CHECK(cudaMemcpyAsync(g + gl.anc_off, aoff.data(), sizeof(int64_t) * (n_chrom + 1), cudaMemcpyHostToDevice, e->s_comp));
+  SAI_CUDA_CHECK(cudaMemcpyAsync(g + gl.names, names, (size_t)name_off[n_chrom], cudaMemcpyHostToDevice, e->s_comp));
+  SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));  // the host vectors go out of scope
+  VcfGenomeQuery& gq = V.gq;
+  gq = VcfGenomeQuery{};
+  gq.q = V.q;
+  gq.anc_off = reinterpret_cast<const int64_t*>(g + gl.anc_off);
+  gq.names = g + gl.names;
+  gq.name_off = reinterpret_cast<const int32_t*>(g + gl.name_off);
+  gq.hash = reinterpret_cast<const uint32_t*>(g + gl.hash);
+  gq.n_chrom = n_chrom;
+  V.genome = true;
+  if (int rc = vcf_genome_state_init(vcf_genome_state(e), vcf_genome_chroms(e), n_chrom, e->s_comp)) return rc;
+  if (int rc = vcf_grow_sites(e, V.site_cap + (int64_t)kTile * n_chrom, false)) return rc;
+  if (V.slot_bytes > 0)
+    if (int rc = grow(e->vscratch, vcf_scratch_need(e, (int64_t)V.slot_bytes))) return rc;
+  V.state = 1;
+  return SAI_OK;
+}
+
+int sai_engine_vcf_genome_finish(sai_engine* e, int64_t* n_sites, int32_t* max_value, sai_vcf_chrom* chroms,
+                                 int32_t* pos_out, int64_t pos_cap) {
+  SAI_REQUIRE(e && n_sites && max_value && chroms, "sai_engine_vcf_genome_finish: NULL argument");
+  auto& V = e->vcf;
+  SAI_REQUIRE(V.genome, "sai_engine_vcf_genome_finish: no genome session (sai_engine_vcf_genome_begin)");
+  const int rc = vcf_finish_impl(e, n_sites, max_value, pos_out, pos_cap);
+  if (rc != SAI_OK && rc != SAI_E_CAPACITY && rc != SAI_E_DOMAIN) return rc;
+  const int n = V.gq.n_chrom;
+  VcfGenomeState gs;
+  std::vector<VcfChromDev> dev(n);
+  SAI_CUDA_CHECK(cudaMemcpy(&gs, vcf_genome_state(e), sizeof(gs), cudaMemcpyDeviceToHost));
+  SAI_CUDA_CHECK(cudaMemcpy(dev.data(), vcf_genome_chroms(e), sizeof(VcfChromDev) * n, cudaMemcpyDeviceToHost));
+  for (int c = 0; c < n; ++c) {
+    const VcfChromDev& d = dev[c];
+    const bool any = d.n_records > 0;
+    chroms[c] = sai_vcf_chrom{any ? (int64_t)(uint32_t)d.first_key : 0, any ? (int64_t)(uint32_t)d.last_key : 0,
+                              d.n_records, d.first_site, d.n_sites};
+  }
+  if (gs.noncontiguous) {
+    V.state = 0;
+    set_error("a chromosome's records resume after another chromosome's");
+    return SAI_E_ORDER;
+  }
+  return rc;
+}
+
+static int vcf_finish_impl(sai_engine* e, int64_t* n_sites, int32_t* max_value, int32_t* pos_out, int64_t pos_cap) {
   auto& V = e->vcf;
   SAI_REQUIRE(V.state == 1, "sai_engine_vcf_finish: no ingest session (sai_engine_vcf_begin)");
   SAI_CUDA_CHECK(cudaSetDevice(e->device));
@@ -1189,8 +1331,35 @@ int sai_engine_vcf_finish(sai_engine* e, int64_t* n_sites, int32_t* max_value, i
   return SAI_OK;
 }
 
+static int score_loaded_impl(sai_engine* e, const int64_t* win_start, const int64_t* win_end, int64_t n_windows,
+                             const sai_job* jobs, int32_t n_jobs, sai_host_results* out,
+                             const std::vector<std::array<int64_t, 4>>& pieces);
 int sai_engine_score_loaded(sai_engine* e, const int64_t* win_start, const int64_t* win_end, int64_t n_windows,
                             const sai_job* jobs, int32_t n_jobs, sai_host_results* out) {
+  return score_loaded_impl(e, win_start, win_end, n_windows, jobs, n_jobs, out, {});
+}
+
+int sai_engine_score_loaded_pieces(sai_engine* e, const int64_t* win_start, const int64_t* win_end,
+                                   const int64_t* pieces, int32_t n_pieces, const sai_job* jobs, int32_t n_jobs,
+                                   sai_host_results* out) {
+  SAI_REQUIRE(e && e->vcf.state == 2, "sai_engine_score_loaded_pieces: no finished ingest session");
+  SAI_REQUIRE(n_pieces >= 1 && pieces, "sai_engine_score_loaded_pieces: no pieces");
+  std::vector<std::array<int64_t, 4>> P((size_t)n_pieces);
+  int64_t W = 0;
+  for (int p = 0; p < n_pieces; ++p) {
+    const int64_t nw = pieces[3 * p], lo = pieces[3 * p + 1], n = pieces[3 * p + 2];
+    SAI_REQUIRE(nw >= 0 && lo >= 0 && lo % kTile == 0 && n >= 0 && lo + n <= e->n_sites,
+                "sai_engine_score_loaded_pieces: piece %d (%lld windows, sites %lld + %lld) outside the %lld resident sites",
+                p, (long long)nw, (long long)lo, (long long)n, (long long)e->n_sites);
+    P[p] = {W, nw, lo, n};
+    W += nw;
+  }
+  return score_loaded_impl(e, win_start, win_end, W, jobs, n_jobs, out, P);
+}
+
+static int score_loaded_impl(sai_engine* e, const int64_t* win_start, const int64_t* win_end, int64_t n_windows,
+                             const sai_job* jobs, int32_t n_jobs, sai_host_results* out,
+                             const std::vector<std::array<int64_t, 4>>& pieces) {
   SAI_REQUIRE(e && e->vcf.state == 2, "sai_engine_score_loaded: no finished ingest session");
   if (int rc = validate_jobs(&e->lay, jobs, n_jobs)) return rc;
   if (int rc = check_results(out)) return rc;
@@ -1200,17 +1369,29 @@ int sai_engine_score_loaded(sai_engine* e, const int64_t* win_start, const int64
   const int64_t n_tiles = sai_num_tiles(e->n_sites);
   const int64_t stride = n_tiles * kTile;
   const ResLayout rl = res_layout(W, n_jobs);
-  if (int rc = grow(e->win, sizeof(int64_t) * 2 * (size_t)W + 256)) return rc;
+  // window bounds, then (pieces) each window's first and last site
+  if (int rc = grow(e->win, (sizeof(int64_t) + sizeof(int32_t)) * 2 * (size_t)W + 256)) return rc;
   if (int rc = grow(e->mask, sizeof(uint32_t) * 2 * (size_t)n_jobs * n_tiles + 256)) return rc;
   if (int rc = grow(e->qval, sizeof(double) * (size_t)n_jobs * stride + 256)) return rc;
   if (int rc = grow(e->res, rl.total + 256)) return rc;
   e->W = W;
   e->n_jobs = n_jobs;
+  e->pieces = pieces;
   for (int j = 0; j < n_jobs; ++j) e->jobs[j] = jobs[j];
   int64_t* d_ws = static_cast<int64_t*>(e->win.p);
   if (W > 0) {
     SAI_CUDA_CHECK(cudaMemcpyAsync(d_ws, win_start, sizeof(int64_t) * W, cudaMemcpyHostToDevice, e->s_comp));
     SAI_CUDA_CHECK(cudaMemcpyAsync(d_ws + W, win_end, sizeof(int64_t) * W, cudaMemcpyHostToDevice, e->s_comp));
+  }
+  if (!pieces.empty() && W > 0) {
+    std::vector<int32_t> fl(2 * (size_t)W);
+    for (const auto& P : pieces)
+      for (int64_t i = P[0]; i < P[0] + P[1]; ++i) {
+        fl[i] = (int32_t)P[2];
+        fl[W + i] = (int32_t)(P[2] + P[3]);
+      }
+    SAI_CUDA_CHECK(cudaMemcpyAsync(d_ws + 2 * W, fl.data(), sizeof(int32_t) * 2 * W, cudaMemcpyHostToDevice, e->s_comp));
+    SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));  // fl goes out of scope
   }
   uint32_t* d_mask_u = static_cast<uint32_t*>(e->mask.p);
   if (n_tiles > 0)

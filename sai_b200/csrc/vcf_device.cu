@@ -21,7 +21,7 @@
 //      so after every call the tiles are exactly what sai_pack_i8_all writes for the sites so far.
 #include <string.h>
 
-#include "common.cuh"
+#include "vcf_genome.cuh"
 
 namespace sai {
 
@@ -35,6 +35,8 @@ struct SliceInfo {
   int32_t n_lines;
   int32_t n_kept;
   int64_t site_base;
+  int32_t n_bnd;  // genome: kept records whose chromosome differs from the one before (bnd)
+  int32_t n_seg;  // genome: runs of one chromosome's kept records in the slice (seg_*)
 };
 
 struct Scratch {
@@ -50,6 +52,13 @@ struct Scratch {
   int32_t* chunk_off; // [n_chunk]
   int32_t* kept;      // line index of the slice's k-th kept record: reuses line_end, which only the record pass reads
   int32_t* fields;    // [n_geno_warps][max_column + 1] field offsets of irregular records
+  // genome parse only
+  int32_t* rec_chrom; // [len] chromosome of the line, -1: not listed
+  uint32_t* rec_span; // [len] POS for the chromosome's span
+  int32_t* bnd;       // [n_chrom + 1] slice index of a kept record that starts a run (unordered)
+  int32_t* seg_k;     // [n_chrom + 2] first kept record (slice index) of run j, ascending
+  int64_t* seg_site;  // [n_chrom + 2] its site
+  int64_t* seg_gap;   // [n_chrom + 2] end of the run before it: [seg_gap, seg_site) are padding sites
 };
 
 inline size_t al(size_t x) { return (x + 255) & ~size_t(255); }
@@ -57,7 +66,7 @@ inline size_t al(size_t x) { return (x + 255) & ~size_t(255); }
 int geno_warps() { return sm_count() * 4 * kWarpsPerBlock; }
 
 // byte size of the scratch and, when base != null, its carving
-size_t carve(const sai_vcf_query& q, int64_t len, char* base, Scratch* s) {
+size_t carve(const sai_vcf_query& q, int64_t len, char* base, Scratch* s, int n_chrom = -1) {
   const size_t n_seg = (size_t)((len + kSegBytes - 1) / kSegBytes) + 1;
   const size_t n_line = (size_t)len + 1;
   const size_t n_chunk = n_line / kLinesPerChunk + 2;
@@ -80,6 +89,15 @@ size_t carve(const sai_vcf_query& q, int64_t len, char* base, Scratch* s) {
   t.chunk_off = reinterpret_cast<int32_t*>(take(4 * n_chunk));
   t.kept = t.line_end;
   t.fields = reinterpret_cast<int32_t*>(take(4 * (size_t)geno_warps() * (size_t)(q.max_column + 1)));
+  t.rec_chrom = nullptr, t.rec_span = nullptr, t.bnd = t.seg_k = nullptr, t.seg_site = t.seg_gap = nullptr;
+  if (n_chrom >= 0) {
+    t.rec_chrom = reinterpret_cast<int32_t*>(take(4 * n_line));
+    t.rec_span = reinterpret_cast<uint32_t*>(take(4 * n_line));
+    t.bnd = reinterpret_cast<int32_t*>(take(4 * ((size_t)n_chrom + 1)));
+    t.seg_k = reinterpret_cast<int32_t*>(take(4 * ((size_t)n_chrom + 2)));
+    t.seg_site = reinterpret_cast<int64_t*>(take(8 * ((size_t)n_chrom + 2)));
+    t.seg_gap = reinterpret_cast<int64_t*>(take(8 * ((size_t)n_chrom + 2)));
+  }
   if (s) *s = t;
   return at;
 }
@@ -170,6 +188,84 @@ __global__ void __launch_bounds__(256) k_nl_write(const char* __restrict__ text,
 }
 
 // ---- 2. record pass ---------------------------------------------------------------------------
+// the first nine tabs of the line [ls, le) into T (warp-cooperative); returns how many there are
+__device__ inline int find_tabs(const char* __restrict__ text, int32_t ls, int32_t le, int32_t* T, int lane) {
+  int n_tab = 0;
+  for (int32_t c = ls; c < le && n_tab < 9; c += 32) {
+    const bool t = c + lane < le && text[c + lane] == '\t';
+    const uint32_t m = __ballot_sync(0xffffffffu, t);
+    const int r = n_tab + __popc(m & ((1u << lane) - 1));
+    if (t && r < 9) T[r] = c + lane;
+    n_tab += __popc(m);
+  }
+  __syncwarp();
+  return n_tab;
+}
+
+__device__ inline int64_t parse_pos(const char* __restrict__ text, const int32_t* T) {
+  int64_t pos = 0;
+  for (int32_t p = T[0] + 1; p < T[1]; ++p)
+    pos = (int64_t)((uint64_t)pos * 10u + (uint64_t)(int64_t)((signed char)text[p] - '0'));
+  return pos;
+}
+
+// rec_meta of a record whose CHROM (and region) matched: the ancestral-allele entries
+// [anc_lo, anc_hi) of anc_pos / anc_allele decide keep and flip (no table: anc_lo == anc_hi == -1),
+// then the index of the first FORMAT key that is exactly "GT" (0 if none)
+__device__ inline int record_meta(const char* __restrict__ text, const int32_t* T, int64_t pos, const int32_t* anc_pos,
+                                  const char* anc_allele, int64_t anc_lo, int64_t anc_hi) {
+  bool keep = true, flip = false;
+  if (anc_lo >= 0) {
+    const int32_t key = (int32_t)pos;
+    int64_t lo = anc_lo, hi = anc_hi;  // lower_bound
+    while (lo < hi) {
+      const int64_t mid = (lo + hi) >> 1;
+      if (anc_pos[mid] < key) lo = mid + 1; else hi = mid;
+    }
+    if (lo == anc_hi || anc_pos[lo] != key) {
+      keep = false;
+    } else {
+      const char* a = anc_allele + 8 * lo;
+      int alen = 0;
+      while (alen < 8 && a[alen]) ++alen;
+      const int32_t ref = T[2] + 1, ref_len = T[3] - ref;
+      const int32_t alt = T[3] + 1;
+      int32_t alt_end = T[4];
+      for (int32_t p = alt; p < T[4]; ++p)
+        if (text[p] == ',') {
+          alt_end = p;
+          break;
+        }
+      bool is_ref = ref_len == alen, is_alt = alt_end - alt == alen;
+      for (int k = 0; k < alen; ++k) {
+        is_ref = is_ref && text[ref + k] == a[k];
+        is_alt = is_alt && text[alt + k] == a[k];
+      }
+      if (!is_ref && !is_alt) keep = false;
+      flip = is_alt;
+    }
+  }
+  if (!keep) return 0;
+  int gi = 0, k = 0;
+  for (int32_t p = T[7] + 1; p < T[8];) {
+    int32_t ke = p;
+    while (ke < T[8] && text[ke] != ':') ++ke;
+    if (ke - p == 2 && text[p] == 'G' && text[p + 1] == 'T') {
+      gi = k;
+      break;
+    }
+    p = ke + 1;
+    ++k;
+  }
+  return 1 | (flip ? 2 : 0) | (gi << 2);
+}
+
+__device__ inline void line_bounds(const char* __restrict__ text, const Scratch& s, int64_t i, int32_t* ls, int32_t* le) {
+  *ls = i > 0 ? s.line_end[i - 1] + 1 : 0;
+  *le = s.line_end[i];
+  if (*le > *ls && text[*le - 1] == '\r') --*le;
+}
+
 __global__ void __launch_bounds__(256) k_records(const char* __restrict__ text, const __grid_constant__ sai_vcf_query q,
                                                  Scratch s) {
   __shared__ int32_t tabs[kWarpsPerBlock][9];
@@ -177,75 +273,19 @@ __global__ void __launch_bounds__(256) k_records(const char* __restrict__ text, 
   const int n_lines = s.info->n_lines;
   const int64_t n_warps = (int64_t)gridDim.x * kWarpsPerBlock;
   for (int64_t i = (int64_t)blockIdx.x * kWarpsPerBlock + wib; i < n_lines; i += n_warps) {
-    const int32_t ls = i > 0 ? s.line_end[i - 1] + 1 : 0;
-    int32_t le = s.line_end[i];
-    if (le > ls && text[le - 1] == '\r') --le;
+    int32_t ls, le;
+    line_bounds(text, s, i, &ls, &le);
     int meta = 0, samp = 0, pos32 = 0;
     if (le > ls && text[ls] != '#') {
-      // the first nine tabs of the line
-      int n_tab = 0;
-      for (int32_t c = ls; c < le && n_tab < 9; c += 32) {
-        const bool t = c + lane < le && text[c + lane] == '\t';
-        const uint32_t m = __ballot_sync(0xffffffffu, t);
-        const int r = n_tab + __popc(m & ((1u << lane) - 1));
-        if (t && r < 9) tabs[wib][r] = c + lane;
-        n_tab += __popc(m);
-      }
-      __syncwarp();
+      const int n_tab = find_tabs(text, ls, le, tabs[wib], lane);
       if (lane == 0 && n_tab >= 9) {
         const int32_t* T = tabs[wib];
         bool keep = T[0] - ls == q.chrom_len;
         for (int k = 0; keep && k < q.chrom_len; ++k) keep = text[ls + k] == q.chrom[k];
-        int64_t pos = 0;
-        for (int32_t p = T[0] + 1; p < T[1]; ++p)
-          pos = (int64_t)((uint64_t)pos * 10u + (uint64_t)(int64_t)((signed char)text[p] - '0'));
+        const int64_t pos = parse_pos(text, T);
         if (keep && q.start <= q.end && (pos < q.start || pos > q.end)) keep = false;
-        bool flip = false;
-        if (keep && q.n_anc > 0) {
-          const int32_t key = (int32_t)pos;
-          int64_t lo = 0, hi = q.n_anc;  // lower_bound
-          while (lo < hi) {
-            const int64_t mid = (lo + hi) >> 1;
-            if (q.anc_pos[mid] < key) lo = mid + 1; else hi = mid;
-          }
-          if (lo == q.n_anc || q.anc_pos[lo] != key) {
-            keep = false;
-          } else {
-            const char* a = q.anc_allele + 8 * lo;
-            int alen = 0;
-            while (alen < 8 && a[alen]) ++alen;
-            const int32_t ref = T[2] + 1, ref_len = T[3] - ref;
-            const int32_t alt = T[3] + 1;
-            int32_t alt_end = T[4];
-            for (int32_t p = alt; p < T[4]; ++p)
-              if (text[p] == ',') {
-                alt_end = p;
-                break;
-              }
-            bool is_ref = ref_len == alen, is_alt = alt_end - alt == alen;
-            for (int k = 0; k < alen; ++k) {
-              is_ref = is_ref && text[ref + k] == a[k];
-              is_alt = is_alt && text[alt + k] == a[k];
-            }
-            if (!is_ref && !is_alt) keep = false;
-            flip = is_alt;
-          }
-        }
-        int gi = 0;
-        if (keep) {  // index of the first FORMAT key that is exactly "GT" (0 if none)
-          int k = 0;
-          for (int32_t p = T[7] + 1; p < T[8];) {
-            int32_t ke = p;
-            while (ke < T[8] && text[ke] != ':') ++ke;
-            if (ke - p == 2 && text[p] == 'G' && text[p + 1] == 'T') {
-              gi = k;
-              break;
-            }
-            p = ke + 1;
-            ++k;
-          }
-        }
-        meta = keep ? (1 | (flip ? 2 : 0) | (gi << 2)) : 0;
+        if (keep)
+          meta = record_meta(text, T, pos, q.anc_pos, q.anc_allele, q.n_anc > 0 ? 0 : -1, q.n_anc > 0 ? q.n_anc : -1);
         samp = T[8] + 1;
         pos32 = (int32_t)pos;
       }
@@ -260,8 +300,76 @@ __global__ void __launch_bounds__(256) k_records(const char* __restrict__ text, 
   }
 }
 
+// Genome record pass: CHROM looked up in the chromosome table (hashed into shared memory), every
+// record of a listed chromosome noted for its span (rec_chrom, rec_span: POS read as
+// sai_vcf_chrom_span reads it, any number of fields), the ancestral-allele search confined to the
+// chromosome's own entries.
+__global__ void __launch_bounds__(256) k_records_genome(const char* __restrict__ text,
+                                                        const __grid_constant__ VcfGenomeQuery g, Scratch s) {
+  __shared__ int32_t tabs[kWarpsPerBlock][9];
+  __shared__ uint2 table[kChromHashSlots];
+  for (int i = threadIdx.x; i < kChromHashSlots; i += blockDim.x)
+    table[i] = make_uint2(g.hash[2 * i], g.hash[2 * i + 1]);
+  __syncthreads();
+  const sai_vcf_query& q = g.q;
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int n_lines = s.info->n_lines;
+  const int64_t n_warps = (int64_t)gridDim.x * kWarpsPerBlock;
+  for (int64_t i = (int64_t)blockIdx.x * kWarpsPerBlock + wib; i < n_lines; i += n_warps) {
+    int32_t ls, le;
+    line_bounds(text, s, i, &ls, &le);
+    int meta = 0, samp = 0, pos32 = 0, chrom = -1;
+    uint32_t span = 0;
+    if (le > ls && text[ls] != '#') {
+      const int n_tab = find_tabs(text, ls, le, tabs[wib], lane);
+      if (lane == 0 && n_tab >= 1) {
+        const int32_t* T = tabs[wib];
+        const int n = T[0] - ls;
+        const uint32_t h = chrom_hash(text + ls, n);
+        for (uint32_t slot = h & (kChromHashSlots - 1);; slot = (slot + 1) & (kChromHashSlots - 1)) {
+          const uint2 e = table[slot];
+          if (e.y == 0) break;
+          if (e.x != h) continue;
+          const int c = (int)e.y - 1;
+          const int32_t a = g.name_off[c];
+          bool same = g.name_off[c + 1] - a == n;
+          for (int k = 0; same && k < n; ++k) same = text[ls + k] == g.names[a + k];
+          if (same) {
+            chrom = c;
+            break;
+          }
+        }
+        if (chrom >= 0) {
+          uint64_t sp = 0;  // sai_vcf_chrom_span: the digits behind the first tab
+          for (int32_t p = T[0] + 1; p < le && text[p] >= '0' && text[p] <= '9'; ++p) sp = sp * 10 + (text[p] - '0');
+          span = (uint32_t)sp;
+          if (n_tab >= 9) {
+            const int64_t pos = parse_pos(text, T);
+            meta = q.n_anc > 0 ? record_meta(text, T, pos, q.anc_pos, q.anc_allele, g.anc_off[chrom], g.anc_off[chrom + 1])
+                               : record_meta(text, T, pos, nullptr, nullptr, -1, -1);
+            samp = T[8] + 1;
+            pos32 = (int32_t)pos;
+          }
+        }
+      }
+    }
+    if (lane == 0) {
+      s.rec_meta[i] = meta;
+      s.rec_samp[i] = samp;
+      s.rec_end[i] = le;
+      s.rec_pos[i] = pos32;
+      s.rec_chrom[i] = chrom;
+      s.rec_span[i] = span;
+    }
+    __syncwarp();
+  }
+}
+
 // ---- 3. site numbering ------------------------------------------------------------------------
-__global__ void __launch_bounds__(kLinesPerChunk) k_keep_count(Scratch s) {
+// Genome parse: also the spans.  The lines of a warp are consecutive, so among the lanes of one
+// chromosome the lowest holds its first record and the highest its last: one atomic each per warp.
+template <bool kGenome = false>
+__global__ void __launch_bounds__(kLinesPerChunk) k_keep_count(Scratch s, const VcfGenomeState* gs, VcfChromDev* chroms) {
   const int n_lines = s.info->n_lines;
   const int n_chunk = (n_lines + kLinesPerChunk - 1) / kLinesPerChunk;
   for (int c = blockIdx.x; c < n_chunk; c += gridDim.x) {
@@ -269,9 +377,23 @@ __global__ void __launch_bounds__(kLinesPerChunk) k_keep_count(Scratch s) {
     int total;
     block_excl_scan(i < n_lines ? (s.rec_meta[i] & 1) : 0, &total);
     if (threadIdx.x == 0) s.chunk_cnt[c] = total;
+    if constexpr (kGenome) {
+      const int ch = i < n_lines ? s.rec_chrom[i] : -1;
+      const uint32_t same = __match_any_sync(0xffffffffu, ch);
+      const int lane = threadIdx.x & 31;
+      if (ch >= 0) {
+        const unsigned long long key = ((unsigned long long)(gs->lines + i) << 32) | s.rec_span[i];
+        if (lane == __ffs(same) - 1) {
+          atomicAdd(reinterpret_cast<unsigned long long*>(&chroms[ch].n_records), (unsigned long long)__popc(same));
+          atomicMin(&chroms[ch].first_key, key);
+        }
+        if (lane == 31 - __clz(same)) atomicMax(&chroms[ch].last_key, key);
+      }
+    }
   }
 }
 
+template <bool kGenome = false>
 __global__ void __launch_bounds__(1024) k_keep_scan(Scratch s, sai_vcf_state* st, int64_t site_cap) {
   const int n_chunk = (s.info->n_lines + kLinesPerChunk - 1) / kLinesPerChunk;
   scan_one_block(s.chunk_cnt, s.chunk_off, n_chunk, &s.info->n_kept);
@@ -279,11 +401,16 @@ __global__ void __launch_bounds__(1024) k_keep_scan(Scratch s, sai_vcf_state* st
   if (threadIdx.x == 0) {
     const int64_t base = st->n_sites;
     s.info->site_base = base;
-    st->n_sites = base + s.info->n_kept;
-    if (base + s.info->n_kept > site_cap) st->overflow = 1;
+    if constexpr (kGenome) {
+      s.info->n_bnd = 0;  // k_genome_plan numbers the sites
+    } else {
+      st->n_sites = base + s.info->n_kept;
+      if (base + s.info->n_kept > site_cap) st->overflow = 1;
+    }
   }
 }
 
+template <bool kGenome = false>
 __global__ void __launch_bounds__(kLinesPerChunk) k_keep_write(Scratch s, int32_t* __restrict__ pos, int64_t site_cap) {
   const int n_lines = s.info->n_lines;
   const int n_chunk = (n_lines + kLinesPerChunk - 1) / kLinesPerChunk;
@@ -295,9 +422,79 @@ __global__ void __launch_bounds__(kLinesPerChunk) k_keep_write(Scratch s, int32_
     const int k = s.chunk_off[c] + block_excl_scan(keep, &total);
     if (keep) {
       s.kept[k] = i;
-      if (base + k < site_cap) pos[base + k] = s.rec_pos[i];
+      if (!kGenome && base + k < site_cap) pos[base + k] = s.rec_pos[i];  // genome: k_genotypes writes pos
     }
   }
+}
+
+// genome: the kept records that start a run of one chromosome (the first of the slice continues the
+// last chromosome of the previous slices or starts one).  More starts than chromosomes: some
+// chromosome resumes, which k_genome_plan reports.
+__global__ void __launch_bounds__(256) k_genome_bounds(Scratch s, const VcfGenomeState* gs, int32_t n_chrom) {
+  const int n_kept = s.info->n_kept;
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_kept; k += gridDim.x * blockDim.x) {
+    const int c = s.rec_chrom[s.kept[k]];
+    const int prev = k > 0 ? s.rec_chrom[s.kept[k - 1]] : gs->last_chrom;
+    if (c != prev) {
+      const int r = atomicAdd(&s.info->n_bnd, 1);
+      if (r <= n_chrom) s.bnd[r] = k;
+    }
+  }
+}
+
+// genome: one thread lays the slice's runs out -- a run that starts a chromosome begins on the next
+// tile boundary -- and keeps the per-chromosome site ranges and the running state.  Runs are as rare
+// as chromosome changes, so this is a short sequential pass.
+__global__ void k_genome_plan(Scratch s, sai_vcf_state* st, VcfGenomeState* gs, VcfChromDev* chroms, int32_t n_chrom,
+                              int64_t site_cap) {
+  if (threadIdx.x != 0) return;
+  SliceInfo& I = *s.info;
+  gs->lines += I.n_lines;
+  I.n_seg = 0;
+  if (gs->noncontiguous || I.n_kept == 0) return;
+  const int nb = I.n_bnd;
+  if (nb > n_chrom) {
+    gs->noncontiguous = 1;
+    return;
+  }
+  for (int a = 1; a < nb; ++a) {  // insertion sort: the starts were appended in any order
+    const int v = s.bnd[a];
+    int b = a - 1;
+    for (; b >= 0 && s.bnd[b] > v; --b) s.bnd[b + 1] = s.bnd[b];
+    s.bnd[b + 1] = v;
+  }
+  int64_t end = st->n_sites;  // one past the last site so far
+  int cur = gs->last_chrom;
+  int n_seg = 0, at = 0;
+  if (nb == 0 || s.bnd[0] > 0) {  // the slice continues the last run
+    s.seg_k[0] = 0;
+    s.seg_site[0] = s.seg_gap[0] = end;
+    n_seg = 1;
+  }
+  for (int j = 0; j <= nb; ++j) {
+    const int k = j < nb ? s.bnd[j] : I.n_kept;
+    if (k > at && cur >= 0) {  // close the run [at, k) of `cur`
+      chroms[cur].n_sites += k - at;
+      end += k - at;
+    }
+    if (j == nb) break;
+    cur = s.rec_chrom[s.kept[k]];
+    if (chroms[cur].first_site >= 0) {
+      gs->noncontiguous = 1;
+      return;
+    }
+    s.seg_gap[n_seg] = end;
+    end = (end + kTile - 1) / kTile * kTile;
+    chroms[cur].first_site = end;
+    s.seg_k[n_seg] = k;
+    s.seg_site[n_seg] = end;
+    ++n_seg;
+    at = k;
+  }
+  I.n_seg = n_seg;
+  st->n_sites = end;
+  gs->last_chrom = cur;
+  if (end > site_cap) st->overflow = 1;
 }
 
 // ---- 4. genotype pass -------------------------------------------------------------------------
@@ -344,21 +541,34 @@ __device__ inline uint32_t* word_at(void* tiles, int pps, int64_t site, int w) {
   return reinterpret_cast<uint32_t*>(static_cast<char*>(tiles) + ((T * pps + (w >> 1)) * 32 + sl) * 8 + (w & 1) * 4);
 }
 
+// genome parse: the site of the slice's kept record k (its run's site plus its place in the run)
+__device__ inline int64_t genome_site(const Scratch& s, int n_seg, int64_t k) {
+  int lo = 0, hi = n_seg - 1;  // the last run that starts at or before k
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (s.seg_k[mid] <= k) lo = mid; else hi = mid - 1;
+  }
+  return s.seg_site[lo] + (k - s.seg_k[lo]);
+}
+
+template <bool kGenome = false>
 __global__ void __launch_bounds__(256) k_genotypes(const char* __restrict__ text, const __grid_constant__ sai_vcf_query q,
-                                                   Scratch s, void* __restrict__ tiles, int64_t site_cap,
-                                                   sai_vcf_state* st) {
+                                                   Scratch s, void* __restrict__ tiles, int32_t* __restrict__ pos,
+                                                   int64_t site_cap, sai_vcf_state* st) {
   const int lane = threadIdx.x & 31;
   const int64_t warp = (int64_t)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
   const int64_t n_warps = (int64_t)gridDim.x * kWarpsPerBlock;
-  const int n_kept = s.info->n_kept;
+  const int n_kept = kGenome && s.info->n_seg == 0 ? 0 : s.info->n_kept;  // genome: no runs = nothing to write
   const int64_t base = s.info->site_base;
+  const int n_seg = kGenome ? s.info->n_seg : 0;
   const int row = q.max_column + 1;
   int32_t* fo = s.fields + warp * row;
   const int pps = q.lay.pairs_per_site;
   for (int64_t k = warp; k < n_kept; k += n_warps) {
-    const int64_t site = base + k;
-    if (site >= site_cap) break;  // reported through st->overflow
+    const int64_t site = kGenome ? genome_site(s, n_seg, k) : base + k;
+    if (site >= site_cap) break;  // reported through st->overflow (sites grow with k)
     const int line = s.kept[k];
+    if (kGenome && lane == 0) pos[site] = s.rec_pos[line];
     const int meta = s.rec_meta[line];
     const bool flip = (meta & 2) != 0;
     const int gi = meta >> 2;
@@ -427,13 +637,10 @@ __global__ void __launch_bounds__(256) k_genotypes(const char* __restrict__ text
 }
 
 // ---- 5. padding sites behind the last site, to the end of its tile -----------------------------
-__global__ void k_pad_tail(const __grid_constant__ sai_layout lay, void* tiles, const sai_vcf_state* st, int64_t site_cap) {
-  const int64_t n = st->n_sites;
-  if (n > site_cap) return;
-  const int64_t end = (n + 31) & ~int64_t(31);
+__device__ inline void pad_sites(const sai_layout& lay, void* tiles, int64_t lo, int64_t hi) {
   const int n_words = 2 * lay.pairs_per_site;
-  for (int64_t x = threadIdx.x; x < (end - n) * n_words; x += blockDim.x) {
-    const int64_t site = n + x / n_words;
+  for (int64_t x = threadIdx.x; x < (hi - lo) * n_words; x += blockDim.x) {
+    const int64_t site = lo + x / n_words;
     const int w = (int)(x % n_words);
     int p = 0;
     while (p + 1 < lay.n_pops && w >= 2 * lay.pop[p + 1].pair_off) ++p;
@@ -442,7 +649,91 @@ __global__ void k_pad_tail(const __grid_constant__ sai_layout lay, void* tiles, 
   }
 }
 
+__global__ void k_pad_tail(const __grid_constant__ sai_layout lay, void* tiles, const sai_vcf_state* st, int64_t site_cap) {
+  const int64_t n = st->n_sites;
+  if (n > site_cap) return;
+  pad_sites(lay, tiles, n, (n + 31) & ~int64_t(31));
+}
+
+// genome: also the sites between a chromosome's last site and the tile boundary where the next run of
+// the slice starts
+__global__ void k_pad_genome(const __grid_constant__ sai_layout lay, void* tiles, const sai_vcf_state* st, Scratch s,
+                             int64_t site_cap) {
+  const int n_seg = s.info->n_seg;
+  for (int j = 0; j < n_seg; ++j)
+    if (s.seg_site[j] <= site_cap) pad_sites(lay, tiles, s.seg_gap[j], s.seg_site[j]);
+  const int64_t n = st->n_sites;
+  if (n <= site_cap) pad_sites(lay, tiles, n, (n + 31) & ~int64_t(31));
+}
+
+__global__ void k_genome_init(VcfGenomeState* gs, VcfChromDev* chroms, int32_t n_chrom) {
+  for (int c = threadIdx.x; c < n_chrom; c += blockDim.x) chroms[c] = VcfChromDev{~0ull, 0ull, 0, -1, 0};
+  if (threadIdx.x == 0) *gs = VcfGenomeState{0, -1, 0};
+}
+
 }  // namespace
+
+int vcf_chrom_table(const char* names, const int32_t* name_off, int32_t n, uint32_t* table) {
+  SAI_REQUIRE(names && name_off && table, "chromosome table: NULL argument");
+  SAI_REQUIRE(n >= 1 && n <= SAI_VCF_MAX_CHROMS, "chromosome table: %d names (1..%d)", n, SAI_VCF_MAX_CHROMS);
+  memset(table, 0, sizeof(uint32_t) * 2 * kChromHashSlots);
+  for (int c = 0; c < n; ++c) {
+    const int32_t a = name_off[c], len = name_off[c + 1] - a;
+    SAI_REQUIRE(len >= 1 && len <= 255, "chromosome table: name %d of %d bytes (1..255)", c, len);
+    const uint32_t h = chrom_hash(names + a, len);
+    uint32_t slot = h & (kChromHashSlots - 1);
+    for (; table[2 * slot + 1]; slot = (slot + 1) & (kChromHashSlots - 1)) {
+      const int o = (int)table[2 * slot + 1] - 1;
+      SAI_REQUIRE(!(table[2 * slot] == h && name_off[o + 1] - name_off[o] == len && !memcmp(names + name_off[o], names + a, len)),
+                  "chromosome table: %.*s is listed twice", len, names + a);
+    }
+    table[2 * slot] = h;
+    table[2 * slot + 1] = (uint32_t)c + 1;
+  }
+  return SAI_OK;
+}
+
+int vcf_genome_state_init(VcfGenomeState* d_gs, VcfChromDev* d_chroms, int32_t n_chrom, cudaStream_t stream) {
+  k_genome_init<<<1, 256, 0, stream>>>(d_gs, d_chroms, n_chrom);
+  SAI_CUDA_CHECK(cudaGetLastError());
+  return SAI_OK;
+}
+
+uint64_t vcf_genome_scratch_bytes(const VcfGenomeQuery& g, int64_t len) {
+  return (uint64_t)carve(g.q, len, nullptr, nullptr, g.n_chrom) + 256;
+}
+
+int vcf_tiles_genome(const VcfGenomeQuery& g, const char* d_text, int64_t len, void* d_scratch, uint64_t scratch_bytes,
+                     void* d_tiles, int32_t* d_pos, int64_t site_cap, sai_vcf_state* d_state, VcfGenomeState* d_gs,
+                     VcfChromDev* d_chroms, cudaStream_t st) {
+  SAI_REQUIRE(len >= 0 && len < (int64_t(1) << 31), "vcf_tiles_genome: slice of %lld bytes (at most 2^31 - 1)",
+              (long long)len);
+  SAI_REQUIRE(site_cap >= 0 && site_cap % kTile == 0, "vcf_tiles_genome: site_cap must be a multiple of 32");
+  Scratch s;
+  const size_t need = carve(g.q, len, static_cast<char*>(d_scratch), &s, g.n_chrom);
+  SAI_REQUIRE(scratch_bytes >= need, "vcf_tiles_genome: scratch of %llu bytes, %zu needed",
+              (unsigned long long)scratch_bytes, need);
+  const int n_seg = (int)((len + kSegBytes - 1) / kSegBytes);
+  const int grid = sm_count() * 4;
+  if (n_seg > 0) {
+    k_nl_count<<<n_seg, 256, 0, st>>>(d_text, len, s);
+    SAI_CUDA_CHECK(cudaGetLastError());
+    k_seg_scan<<<1, 1024, 0, st>>>(n_seg, s);
+    k_nl_write<<<n_seg, 256, 0, st>>>(d_text, len, s);
+  } else {
+    SAI_CUDA_CHECK(cudaMemsetAsync(&s.info->n_lines, 0, sizeof(int32_t), st));
+  }
+  k_records_genome<<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, g, s);
+  k_keep_count<true><<<grid, kLinesPerChunk, 0, st>>>(s, d_gs, d_chroms);
+  k_keep_scan<true><<<1, 1024, 0, st>>>(s, d_state, site_cap);
+  k_keep_write<true><<<grid, kLinesPerChunk, 0, st>>>(s, d_pos, site_cap);
+  k_genome_bounds<<<grid, 256, 0, st>>>(s, d_gs, g.n_chrom);
+  k_genome_plan<<<1, 32, 0, st>>>(s, d_state, d_gs, d_chroms, g.n_chrom, site_cap);
+  k_genotypes<true><<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, g.q, s, d_tiles, d_pos, site_cap, d_state);
+  k_pad_genome<<<1, 256, 0, st>>>(g.q.lay, d_tiles, d_state, s, site_cap);
+  SAI_CUDA_CHECK(cudaGetLastError());
+  return SAI_OK;
+}
 
 }  // namespace sai
 
@@ -485,10 +776,10 @@ int sai_vcf_tiles_device(const sai_vcf_query* q, const char* d_text, int64_t len
     SAI_CUDA_CHECK(cudaMemsetAsync(&s.info->n_lines, 0, sizeof(int32_t), st));
   }
   k_records<<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, *q, s);
-  k_keep_count<<<grid, kLinesPerChunk, 0, st>>>(s);
+  k_keep_count<<<grid, kLinesPerChunk, 0, st>>>(s, nullptr, nullptr);
   k_keep_scan<<<1, 1024, 0, st>>>(s, d_state, site_cap);
   k_keep_write<<<grid, kLinesPerChunk, 0, st>>>(s, d_pos, site_cap);
-  k_genotypes<<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, *q, s, d_tiles, site_cap, d_state);
+  k_genotypes<<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, *q, s, d_tiles, d_pos, site_cap, d_state);
   k_pad_tail<<<1, 256, 0, st>>>(q->lay, d_tiles, d_state, site_cap);
   SAI_CUDA_CHECK(cudaGetLastError());
   return SAI_OK;

@@ -63,7 +63,11 @@ def score_populations(
 
     ``loaded`` (a ``vcf_device.LoadedChunk``): the populations were parsed on the device into one
     layout resident in ``engine``; the ``*_data`` dicts then only name the populations (their
-    values are not read) and every combination is scored from that layout."""
+    values are not read) and every combination is scored from that layout.  A
+    ``vcf_device.LoadedGenome`` holds several chromosomes, each with its own windows
+    (``windows_by_tgt`` maps every target population to the list of them, one per chromosome;
+    ``chr_name`` is not used): all chromosomes are scored with one genotype pass and one window
+    launch per batch of combinations, and the items come out chromosome by chromosome."""
     stats = [s for s in stat_config.root.keys() if s in ("U", "Q")]
     four = [s for s in stat_config.root.keys() if s in ("Danc", "Dplus", "df", "fd") and stat_config.root[s] is True]
     dd = any(s == "DD" and stat_config.root[s] is True for s in stat_config.root.keys())
@@ -96,33 +100,35 @@ def score_populations(
     stat_order = [s for s in stat_config.root.keys() if s in stats or s in four or (dd and s == "DD")]
     empty_cdd = np.array([])
 
-    def emit(combo, windows, pos, res, j, four_vals, dd_vals):
+    def emit(combo, windows, pos, res, j, four_vals, dd_vals, chrom=chr_name, at=0):
         """One item dict per window (feature_preprocessor.py:119-191).  A chromosome-scale chunk has
         tens of thousands of windows, so the per-window work is kept to plain Python objects: the
         result columns are turned into lists once and the candidate lists are views into one
-        converted array."""
+        converted array.  ``windows`` are the result columns ``at, at + 1, ...``."""
         ref_pop, tgt_pop, src_comb, out_pop = combo
         n_src = len(src_comb)
         out_name = "NA" if out_pop is None else out_pop
         pos_dtype = np.asarray(pos).dtype
+        cols = slice(at, at + len(windows))
         if res is not None:
-            nsnps_l = res.nsnps[j].tolist()
+            nsnps_l = res.nsnps[j, cols].tolist()
         else:
             nsnps_l = [int(np.count_nonzero((pos >= s_) & (pos <= e_))) for s_, e_ in windows]
         want_u, want_q = "U" in stats, "Q" in stats
         if want_u:
-            u_l, us_l = res.u[j].tolist(), res.u_start[j].tolist()
+            u_l, us_l = res.u[j, cols].tolist(), res.u_start[j, cols].tolist()
             u_cand = res.u_cand[j].astype(pos_dtype, copy=False)
         if want_q:
-            q_col, qnan_l = res.q[j], np.isnan(res.q[j]).tolist()  # q_col[i] is a numpy.float64, like np.nanquantile's
-            qs_l, qc_l = res.q_start[j].tolist(), res.q_cnt[j].tolist()
+            q_col = res.q[j, cols]  # q_col[i] is a numpy.float64, like np.nanquantile's
+            qnan_l = np.isnan(q_col).tolist()
+            qs_l, qc_l = res.q_start[j, cols].tolist(), res.q_cnt[j, cols].tolist()
             q_cand = res.q_cand[j].astype(pos_dtype, copy=False)
         nan_list = [np.nan for _ in range(n_src)] if n_src > 1 else np.nan
         for i, (start, end) in enumerate(windows):
             nsnps = nsnps_l[i]
             cdd = {}
             item = {
-                "chr_name": chr_name,
+                "chr_name": chrom,
                 "start": start,
                 "end": end,
                 "ref_pop": ref_pop,
@@ -151,9 +157,9 @@ def score_populations(
                 elif nsnps == 0:  # feature_preprocessor.py:137-141
                     item[s] = list(nan_list) if n_src > 1 else np.nan
                 elif s == "DD":
-                    item[s] = [dd_vals[k][i] for k in range(n_src)]
+                    item[s] = [dd_vals[k][at + i] for k in range(n_src)]
                 else:
-                    item[s] = [four_vals[s][k][i] for k in range(n_src)]
+                    item[s] = [four_vals[s][k][at + i] for k in range(n_src)]
             items.append(item)
 
     def extras(pg, ref_idx, tgt_idx, src_idx, out_idx, n_ref, n_tgt, n_srcs):
@@ -164,6 +170,33 @@ def score_populations(
             ref_sum, tgt_sum = engine.dd_sums(pg, ref_idx, tgt_idx, src_idx)
             dd_vals = dd_values(ref_sum, tgt_sum, n_ref, n_tgt, n_srcs)
         return four_vals, dd_vals
+
+    if loaded is not None and hasattr(loaded, "first_site"):  # a LoadedGenome
+        win_lists = next(iter(windows_by_tgt.values()))
+        pieces = [(w, max(f, 0), n) for w, f, n in zip(win_lists, loaded.first_site, loaded.n_sites)]
+        at = np.cumsum([0] + [len(w) for w in win_lists]).tolist()
+        index, n_of = loaded.index, lambda i: int(loaded.layout.pop[i].n_samples)
+        use_out = bool(out_data) and bool(four)
+        batches = []
+        for b0 in range(0, len(combos), _cabi.MAX_JOBS):
+            batch = combos[b0 : b0 + _cabi.MAX_JOBS]
+            jobs = []
+            for r, t, sc, _ in batch:
+                src_ploidy_list(len(sc))  # same check as the host path
+                jobs.append(job_for(r, t, index[("ref", r)], index[("tgt", t)], [index[("src", s)] for s in sc]))
+            res = engine.score_loaded_pieces(pieces, jobs) if b0 == 0 else engine.score_resident(jobs)
+            four_by_job = []
+            for r, t, sc, o in batch:
+                src_idx = [index[("src", s)] for s in sc]
+                four_by_job.append(extras(loaded, index[("ref", r)], index[("tgt", t)], src_idx,
+                                          index[("out", o)] if (use_out and o is not None) else -1,
+                                          n_of(index[("ref", r)]), n_of(index[("tgt", t)]), [n_of(i) for i in src_idx]))
+            batches.append((batch, res, four_by_job))
+        for c, chrom in enumerate(loaded.names):
+            for batch, res, four_by_job in batches:
+                for j, combo in enumerate(batch):
+                    emit(combo, win_lists[c], loaded.pos[c], res, j, *four_by_job[j], chrom=chrom, at=at[c])
+        return items
 
     # ---- all populations in one packed matrix, the product as fused jobs ------------------
     use_out = bool(out_data) and bool(four)

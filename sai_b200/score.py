@@ -10,30 +10,22 @@ untouched and only the ``ChunkPreprocessor`` it constructs is swapped
 from __future__ import annotations
 
 import os
+import warnings
 from pathlib import Path
+from typing import Sequence
+
+import numpy as np
 
 from .configs import load_config
 from .preprocessors import ChunkPreprocessor
 from .generators import ChunkGenerator
 
 
-def score(
-    vcf_file: str,
-    chr_name: str,
-    win_len: int,
-    win_step: int,
-    anc_allele_file: str,
-    output_file: str,
-    config: str,
-    num_workers: int = 1,
-    device: int = 0,
-    ingest: str = "host",
-    inflate: str = "host",
-) -> None:
-    """``ingest="device"`` parses the VCF on the GPU (``ChunkPreprocessor(ingest=...)``), and
-    ``inflate="device"`` also inflates a bgzip file there; same output."""
+def _load_checked_config(config: str, anc_allele_file):
+    """The configuration, refused as the reference refuses it (sai/sai.py:79-84) and for statistics
+    this port does not compute."""
     cfg = load_config(config)
-    stat_config, ploidy_config, pop_config = cfg.statistics, cfg.ploidies, cfg.populations
+    stat_config = cfg.statistics
     others = [s for s in stat_config.root if s not in ("U", "Q", "Danc", "Dplus", "df", "fd", "DD") and stat_config.root[s] is not False]
     if others:
         raise NotImplementedError(
@@ -45,12 +37,12 @@ def score(
                 raise ValueError(
                     f"The {stat_name} statistic requires polarized data, please provide the ancestral allele information with `--anc-alleles`."
                 )
-    # ONE chunk, as sai.py:86-93 (num_chunks=1; `num_workers` is accepted and ignored there too):
-    # rows come out product-major / windows-inner, identical to the reference's text.  Real
-    # parallelism is sai_b200.multiprocessing.mp_pool (one worker per GPU) or sai_b200.distributed.
-    generator = ChunkGenerator(vcf_file=vcf_file, chr_name=chr_name, window_size=win_len, step_size=win_step,
-                               num_chunks=1)
-    pre = ChunkPreprocessor(
+    return cfg
+
+
+def _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file, device, ingest, inflate):
+    pop_config = cfg.populations
+    return ChunkPreprocessor(
         vcf_file=vcf_file,
         ref_ind_file=pop_config.get_population("ref"),
         tgt_ind_file=pop_config.get_population("tgt"),
@@ -59,13 +51,17 @@ def score(
         win_len=win_len,
         win_step=win_step,
         output_file=output_file,
-        ploidy_config=ploidy_config,
-        stat_config=stat_config,
+        ploidy_config=cfg.ploidies,
+        stat_config=cfg.statistics,
         anc_allele_file=anc_allele_file,
         device=device,
         ingest=ingest,
         inflate=inflate,
     )
+
+
+def _write_headers(output_file: str, stat_config, ploidy_config) -> None:
+    """The header lines of the score file and of the ``.U.log`` / ``.Q.log`` files (sai/sai.py:122-142)."""
     header = ["Chrom", "Start", "End", "Ref", "Tgt", "Src", "Outgroup", "N(Variants)"]
     src_pops = list(ploidy_config.root["src"].keys())
     for stat_name in stat_config.root.keys():  # sai/sai.py:122-129
@@ -84,7 +80,126 @@ def score(
         if key in stat_config.root:
             with open(Path(output_file).with_suffix(f".{key}.log"), "w") as f:
                 f.write(f"Chrom\tStart\tEnd\t{key}_SNP\n")
+
+
+def score(
+    vcf_file: str,
+    chr_name: str,
+    win_len: int,
+    win_step: int,
+    anc_allele_file: str,
+    output_file: str,
+    config: str,
+    num_workers: int = 1,
+    device: int = 0,
+    ingest: str = "host",
+    inflate: str = "host",
+) -> None:
+    """``ingest="device"`` parses the VCF on the GPU (``ChunkPreprocessor(ingest=...)``), and
+    ``inflate="device"`` also inflates a bgzip file there; same output."""
+    cfg = _load_checked_config(config, anc_allele_file)
+    # ONE chunk, as sai.py:86-93 (num_chunks=1; `num_workers` is accepted and ignored there too):
+    # rows come out product-major / windows-inner, identical to the reference's text.  Real
+    # parallelism is sai_b200.multiprocessing.mp_pool (one worker per GPU) or sai_b200.distributed.
+    generator = ChunkGenerator(vcf_file=vcf_file, chr_name=chr_name, window_size=win_len, step_size=win_step,
+                               num_chunks=1)
+    pre = _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file, device, ingest, inflate)
+    _write_headers(output_file, cfg.statistics, cfg.ploidies)
     items = []
     for params in generator.get():  # sai.py:148-149
         items.extend(pre.run(**params))
     pre.process_items(items)
+
+
+def score_genome(
+    vcf_file: str,
+    chr_names: Sequence[str],
+    win_len: int,
+    win_step: int,
+    anc_allele_file: str,
+    output_file: str,
+    config: str,
+    device: int = 0,
+    inflate: str = "host",
+) -> None:
+    """Scores every chromosome of ``chr_names`` of one (multi-chromosome) VCF: the score file and the
+    ``.U.log`` / ``.Q.log`` files are byte for byte those of ``score(vcf_file, c, ...)`` run for each
+    ``c`` in turn and concatenated (header lines once), and so are the errors -- but the file is read
+    once.  Its text is parsed on the GPU (``vcf_device.read_genome``; ``inflate="device"`` also
+    inflates a bgzip file there) into one resident layout in which every chromosome starts on a tile
+    boundary, and all chromosomes are scored with one genotype pass and one window launch.
+
+    Files the one-pass reader does not take -- where ``vcf_device.fallback_reason`` names a reason
+    (DD, more than 16 populations, long ancestral alleles, positional source ploidies), more than
+    ``SAI_VCF_MAX_CHROMS`` (1024) chromosomes, or chromosomes whose records are not contiguous in
+    the file -- are scored one chromosome at a time by the ``score`` path, with the same output."""
+    from . import _cabi
+    from .preprocessors import score_populations, write_items
+    from .vcf import read_anc_or_error
+    from .vcf_device import _wants_outgroup, fallback_reason, genome_tables, read_genome, read_plan
+    from .windows import chunk_windows, split_genome, split_windows_ranges
+
+    cfg = _load_checked_config(config, anc_allele_file)
+    stat_config, ploidy_config = cfg.statistics, cfg.ploidies
+    chr_names = list(chr_names)
+    pre = _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file, device, "device", inflate)
+
+    def each_chromosome() -> None:
+        generators = [ChunkGenerator(vcf_file=vcf_file, chr_name=c, window_size=win_len, step_size=win_step, num_chunks=1)
+                      for c in chr_names]
+        _write_headers(output_file, stat_config, ploidy_config)
+        for generator in generators:
+            items = []
+            for params in generator.get():
+                items.extend(pre.run(**params))
+            pre.process_items(items)
+
+    if not chr_names or len(set(chr_names)) != len(chr_names) or len(chr_names) > _cabi.MAX_CHROMS:
+        return each_chromosome()
+    with warnings.catch_warnings(record=True) as caught:  # warned once, by the read that is used
+        warnings.simplefilter("always")
+        plan, requests, out = read_plan(vcf_file, chr_names[0], ploidy_config, pre.ref_ind_file, pre.tgt_ind_file,
+                                        pre.src_ind_file, pre.out_ind_file)
+    if any(fallback_reason(stat_config, ploidy_config, plan, None, c, pre.num_src) is not None for c in chr_names):
+        return each_chromosome()
+    tables = genome_tables(chr_names, anc_allele_file)
+    if anc_allele_file and tables[2] is None:  # an ancestral allele longer than 7 bytes
+        return each_chromosome()
+    for w in caught:
+        warnings.warn_explicit(w.message, w.category, w.filename, w.lineno)
+    try:
+        loaded = read_genome(pre.engine, vcf_file, chr_names, plan, requests, out, tables,
+                             with_outgroup=_wants_outgroup(stat_config), inflate=inflate)
+    except (KeyError, OSError) as e:
+        raise ValueError(f"Failed to read VCF file {vcf_file} from {','.join(chr_names)}: {e}") from e
+    if loaded is None:  # no #CHROM line, or a chromosome's records are not contiguous
+        return each_chromosome()
+    windows = []
+    for c, name in enumerate(chr_names):
+        span = loaded.span[c]
+        if span is None:
+            raise ValueError(f"Chromosome {name} not found in VCF.")
+        chunks = split_windows_ranges(split_genome([span[0], span[1]], win_len, win_step), 1)
+        if not chunks:  # no window (last POS before the first): score() runs no chunk
+            return each_chromosome()
+        start, end = chunks[0]
+        pos = loaded.pos[c]
+        if pos.size and (int(pos.min()) < start or int(pos.max()) > end):  # score() reads [start, end] only
+            return each_chromosome()
+        if anc_allele_file:
+            anc_pos, _, anc_off = tables[2]
+            mine = anc_pos[anc_off[c] : anc_off[c + 1]]
+            if not np.any((mine >= start) & (mine <= end)):  # records but no ancestral allele: the reference raises
+                raise read_anc_or_error(anc_allele_file, name, start, end)[1]
+        windows.append(chunk_windows(start, end, win_len, win_step))
+    (ref_pops, _), (tgt_pops, tgt_samples) = loaded.groups["ref"], loaded.groups["tgt"]
+    (src_pops, _), (out_pops, _) = loaded.groups["src"], loaded.groups["outgroup"]
+    if ref_pops is None or tgt_pops is None or src_pops is None:
+        return each_chromosome()
+    _write_headers(output_file, stat_config, ploidy_config)
+    names = lambda pops: {p: None for p in pops} if pops else None
+    items = score_populations(
+        chr_names[0], {t: windows for t in tgt_samples}, names(ref_pops), names(tgt_pops), names(src_pops),
+        ploidy_config, stat_config, anc_allele_file is not None, pre.engine, out_data=names(out_pops),
+        num_src=pre.num_src, loaded=loaded)
+    write_items(output_file, items, stat_config)

@@ -273,6 +273,18 @@ class HostEngine:
         return self._resident_call("sai_engine_score_loaded", jobs, cap_u, cap_q,
                                    ws.ctypes.data if ws.size else None, we.ctypes.data if we.size else None, int(ws.shape[0]))
 
+    def score_loaded_pieces(self, pieces, jobs, cap_u=None, cap_q=None) -> WindowResults:
+        """``score_loaded`` over pieces of the resident tiles (``vcf_device.read_genome``): ``pieces``
+        = ``[(windows, first site, sites), ...]``, the results' windows piece after piece.  One genotype
+        pass and one window launch; ``score_resident`` / ``pattern_sums`` then work on the same pieces."""
+        ws = np.ascontiguousarray([w[0] for p in pieces for w in p[0]], dtype=np.int64)
+        we = np.ascontiguousarray([w[1] for p in pieces for w in p[0]], dtype=np.int64)
+        table = np.ascontiguousarray([[len(w), lo, n] for w, lo, n in pieces], dtype=np.int64)
+        self._last_W = int(ws.shape[0])
+        return self._resident_call("sai_engine_score_loaded_pieces", jobs, cap_u, cap_q,
+                                   ws.ctypes.data if ws.size else None, we.ctypes.data if we.size else None,
+                                   table.ctypes.data, int(table.shape[0]))
+
     def score_resident(self, jobs, cap_u=None, cap_q=None) -> WindowResults:
         """Another batch of jobs over the chunk of the last ``score*`` call, still resident on the
         device (no upload): a population product of more than 8 combinations costs one transfer."""
