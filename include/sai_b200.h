@@ -648,10 +648,34 @@ int sai_engine_vcf_genome_finish(sai_engine* e, int64_t* n_sites, int32_t* max_v
  * windows, first site (a multiple of 32), number of sites); the windows are given piece after piece.
  * One genotype pass over all tiles, one sai_window_stats_pieces launch.  Afterwards
  * sai_engine_score_resident / _rescore_windows / _pattern_sums (one sai_window_patterns per piece) work
- * on the same pieces; sai_engine_dd_sums is refused. */
+ * on the same pieces; sai_engine_dd_sums is refused (sai_engine_dd_sums_loaded is not). */
 int sai_engine_score_loaded_pieces(sai_engine* e, const int64_t* win_start, const int64_t* win_end,
                                    const int64_t* pieces, int32_t n_pieces, const sai_job* jobs, int32_t n_jobs,
                                    sai_host_results* out);
+
+/* ---- negative-value table of an ingest session (DD without a host copy) --------------------------
+ * sai_engine_set_vcf_neg_table: on != 0 makes the ingest sessions that follow (sai_engine_vcf_begin /
+ * _genome_begin) also keep the N4 negative-value table of their populations: the genotype pass keeps
+ * the raw value of every missing call it parses.  Its capacity is unknown until the text has been
+ * read: min_entries (0..2^31 - 1) is a lower bound of it (a repeat), and the finish returns
+ * SAI_E_CAPACITY when the text holds more entries; sai_engine_loaded_neg_table then returns how many.
+ * sai_engine_loaded_neg_table: the table of the last finished session into HOST memory, the entries of
+ * chromosome c (0 for a single-chromosome session) and population p at
+ *     neg_off[c * (n_pops + 1) + p] .. neg_off[c * (n_pops + 1) + p + 1] - 1
+ * of site / ind / val, sorted by (site, individual), site counted from the chromosome's first site --
+ * for every chromosome exactly sai_neg_table_i8 of its own int8 matrices.  neg_off (optional,
+ * [n_chrom][n_pops + 1]) is always written; the entries only when cap >= their number.  Returns that
+ * number (after SAI_E_CAPACITY: the number a repeat needs) or a negative SAI_E_* code.
+ * sai_engine_dd_sums_loaded: sai_engine_dd_sums on the resident tiles and the resident table (no copy
+ * to the device) after sai_engine_score_loaded or _score_loaded_pieces; with pieces one sai_site_hist +
+ * sai_window_dd per piece (a chromosome of the session), its results at ref_sum[k][w0 + i] as
+ * sai_engine_pattern_sums places them.  Fails with SAI_E_ARG when a population's missing calls and its
+ * table entries differ. */
+int sai_engine_set_vcf_neg_table(sai_engine* e, int32_t on, int64_t min_entries);
+int64_t sai_engine_loaded_neg_table(sai_engine* e, int64_t* neg_off, int32_t* site, int32_t* ind, int32_t* val,
+                                    int64_t cap);
+int sai_engine_dd_sums_loaded(sai_engine* e, int32_t ref_pop, int32_t tgt_pop, const int32_t* src_pops, int32_t n_src,
+                              int64_t* ref_sum, int64_t* tgt_sum, int32_t m_max);
 
 /* ---- synthetic genotypes (bench / tests only) ---------------------------- */
 /* Fills tiles [tile0, tile0+n_tiles) of a packed matrix directly on the device

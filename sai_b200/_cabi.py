@@ -218,6 +218,9 @@ SYMBOLS = {
         C.c_int, [_P, _LAY, _P, _P, _I32, _P, _I32, _P, _P, _P, _I32, _I64, _I64]),
     "sai_engine_vcf_genome_finish": (C.c_int, [_P, C.POINTER(_I64), _P, C.POINTER(VcfChrom), _P, _I64]),
     "sai_engine_score_loaded_pieces": (C.c_int, [_P, _P, _P, _P, _I32, _JOB, _I32, C.POINTER(HostResults)]),
+    "sai_engine_set_vcf_neg_table": (C.c_int, [_P, _I32, _I64]),
+    "sai_engine_loaded_neg_table": (_I64, [_P, _P, _P, _P, _P, _I64]),
+    "sai_engine_dd_sums_loaded": (C.c_int, [_P, _I32, _I32, _P, _I32, _P, _P, _I32]),
 }
 
 _lib = None

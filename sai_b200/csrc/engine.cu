@@ -148,10 +148,19 @@ struct sai_engine {
     double stats[14] = {0};           // sai_engine_vcf_stats of the last finished session
     int sticky_rc = SAI_OK;           // first failure of the session, reported by finish
     StagePool pool;
+    // negative-value table (DD): sai_engine_set_vcf_neg_table, then per session
+    bool neg_on = false;              // the sessions that follow keep the table
+    int64_t neg_min = 0;              // lower bound of its capacity (a repeat after SAI_E_CAPACITY)
+    bool neg = false;                 // the current / last session keeps it
+    sai::VcfNegSession negs{};        // its device buffers (vneg, vnega)
+    int64_t neg_n = -1;               // entries the last finished session found (-1: none)
+    std::vector<int64_t> neg_off;     // [n_chrom][n_pops + 1] offsets of the finished table (vnegt)
+    std::vector<std::array<int64_t, 2>> chrom_sites;  // genome session: (first site, sites) per chromosome
   } vcf;
   Buf vtext, vscratch, vcols, vanc_pos, vanc_all, vstate;
   Buf vcomp, vbad;  // device inflate: ring of compressed groups (+ block statuses), first corrupt block
   Buf vgen;         // genome ingest: hash table, names, offsets, running state, per-chromosome records
+  Buf vneg, vnega, vnegt;  // negative-value table: state + per-key counts, appended entries, finished table
 };
 
 namespace sai {
@@ -928,7 +937,70 @@ static int vcf_wait(cudaEvent_t ev) {
 
 // parse scratch of one slice of `len` bytes for the session's query
 static uint64_t vcf_scratch_need(const sai_engine* e, int64_t len) {
-  return e->vcf.genome ? vcf_genome_scratch_bytes(e->vcf.gq, len) : sai_vcf_scratch_bytes(&e->vcf.q, len);
+  return (e->vcf.genome ? vcf_genome_scratch_bytes(e->vcf.gq, len) : sai_vcf_scratch_bytes(&e->vcf.q, len)) +
+         (e->vcf.neg ? vcf_neg_scratch_bytes(e->vcf.q, len) : 0);
+}
+
+// The negative-value table of a session with n_chrom chromosomes (sai_engine_set_vcf_neg_table): its
+// capacity is unknown until the text has been read.  First estimate: 1/64 of the site capacity times the
+// individuals (about 1.6 % missing calls; the site capacity comes from the text size), at least 1024 and
+// at least neg_min; finish reports SAI_E_CAPACITY and the true count when the text holds more, and the
+// caller reads the text again.
+constexpr int64_t kNegMaxEntries = (int64_t(1) << 31) - 1;  // site / individual / index are int32
+static int vcf_neg_begin(sai_engine* e, int32_t n_chrom) {
+  auto& V = e->vcf;
+  V.neg = V.neg_on;
+  V.neg_n = -1;
+  V.neg_off.clear();
+  V.chrom_sites.clear();
+  if (!V.neg) return SAI_OK;
+  const sai_layout& lay = V.q.lay;
+  int64_t n_out = 0;
+  for (int p = 0; p < lay.n_pops; ++p) n_out += lay.pop[p].n_samples;
+  const int64_t cap = std::min(kNegMaxEntries, std::max(V.neg_min, std::max<int64_t>(1024, V.site_cap / 64 * n_out)));
+  const size_t part = align256(sizeof(int32_t) * (size_t)cap);
+  if (int rc = grow(e->vnega, 5 * part)) return rc;
+  const size_t count_bytes = sizeof(unsigned long long) * (size_t)n_chrom * lay.n_pops;
+  if (int rc = grow(e->vneg, align256(sizeof(VcfNegDev)) + count_bytes)) return rc;
+  VcfNegSession& t = V.negs;
+  char* a = static_cast<char*>(e->vnega.p);
+  t.site = reinterpret_cast<int32_t*>(a);
+  t.ind = reinterpret_cast<int32_t*>(a + part);
+  t.val = reinterpret_cast<int32_t*>(a + 2 * part);
+  t.key = reinterpret_cast<int32_t*>(a + 3 * part);
+  t.idx = reinterpret_cast<int32_t*>(a + 4 * part);
+  t.cap = cap;
+  t.state = static_cast<VcfNegDev*>(e->vneg.p);
+  t.count = reinterpret_cast<unsigned long long*>(static_cast<char*>(e->vneg.p) + align256(sizeof(VcfNegDev)));
+  SAI_CUDA_CHECK(cudaMemsetAsync(e->vneg.p, 0, align256(sizeof(VcfNegDev)) + count_bytes, e->s_comp));
+  return SAI_OK;
+}
+
+// After a successful finish: the appended entries placed key-major (chromosome, population; inside a
+// key by site and individual) into vnegt, and their offsets.
+static int vcf_neg_finish(sai_engine* e) {
+  auto& V = e->vcf;
+  const int n_chrom = V.genome ? V.gq.n_chrom : 1, n_pops = V.q.lay.n_pops;
+  const int64_t n = V.neg_n;
+  std::vector<unsigned long long> count((size_t)n_chrom * n_pops);
+  SAI_CUDA_CHECK(cudaMemcpy(count.data(), V.negs.count, sizeof(unsigned long long) * count.size(), cudaMemcpyDeviceToHost));
+  std::vector<int64_t> key_off(count.size() + 1, 0);
+  for (size_t k = 0; k < count.size(); ++k) key_off[k + 1] = key_off[k] + (int64_t)count[k];
+  SAI_REQUIRE(key_off.back() == n, "negative-value table: %lld entries appended, %lld counted", (long long)n,
+              (long long)key_off.back());
+  V.neg_off.assign((size_t)n_chrom * (n_pops + 1), 0);
+  for (int c = 0; c < n_chrom; ++c)
+    for (int p = 0; p <= n_pops; ++p) V.neg_off[(size_t)c * (n_pops + 1) + p] = key_off[(size_t)c * n_pops + p];
+  const size_t part = align256(sizeof(int32_t) * (size_t)std::max<int64_t>(n, 1));
+  if (int rc = grow(e->vnegt, 3 * part + sizeof(int64_t) * key_off.size())) return rc;
+  char* t = static_cast<char*>(e->vnegt.p);
+  int64_t* d_key_off = reinterpret_cast<int64_t*>(t + 3 * part);
+  SAI_CUDA_CHECK(cudaMemcpyAsync(d_key_off, key_off.data(), sizeof(int64_t) * key_off.size(), cudaMemcpyHostToDevice, e->s_comp));
+  if (int rc = vcf_neg_order(V.negs, n, d_key_off, reinterpret_cast<int32_t*>(t), reinterpret_cast<int32_t*>(t + part),
+                             reinterpret_cast<int32_t*>(t + 2 * part), e->s_comp))
+    return rc;
+  SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));  // key_off goes out of scope
+  return SAI_OK;
 }
 
 static int stage_threads(const sai_engine* e) {
@@ -1044,13 +1116,14 @@ static int vcf_launch_slot_impl(sai_engine* e, int64_t off, int64_t n, const Dev
     SAI_CUDA_CHECK(cudaStreamWaitEvent(e->s_comp, V.copied[slot], 0));
   }
   SAI_CUDA_CHECK(cudaEventRecord(T[2], e->s_comp));
+  const VcfNegSession* neg = V.neg ? &V.negs : nullptr;
   if (int rc = V.genome ? vcf_tiles_genome(V.gq, d, n, e->vscratch.p, e->vscratch.cap, e->packed.p,
                                             static_cast<int32_t*>(e->pos.p), V.site_cap,
                                             static_cast<sai_vcf_state*>(e->vstate.p), vcf_genome_state(e),
-                                            vcf_genome_chroms(e), e->s_comp)
-                       : sai_vcf_tiles_device(&V.q, d, n, e->vscratch.p, e->vscratch.cap, e->packed.p,
-                                              static_cast<int32_t*>(e->pos.p), V.site_cap,
-                                              static_cast<sai_vcf_state*>(e->vstate.p), e->s_comp))
+                                            vcf_genome_chroms(e), neg, e->s_comp)
+                       : vcf_tiles_single(V.q, d, n, e->vscratch.p, e->vscratch.cap, e->packed.p,
+                                          static_cast<int32_t*>(e->pos.p), V.site_cap,
+                                          static_cast<sai_vcf_state*>(e->vstate.p), neg, e->s_comp))
     return rc;
   SAI_CUDA_CHECK(cudaEventRecord(T[3], e->s_comp));
   SAI_CUDA_CHECK(cudaEventRecord(V.parsed[slot], e->s_comp));
@@ -1127,6 +1200,7 @@ int sai_engine_vcf_begin(sai_engine* e, const sai_layout* lay, const char* chrom
   V.row_bytes = std::max<int64_t>(64, 2 * (int64_t)n_file_samples + 18);
   V.site_cap = 0;  // the buffers' content is not kept from an earlier chunk
   if (int rc = vcf_grow_sites(e, std::max(text_bytes_hint / V.row_bytes + 1024, min_sites), false)) return rc;
+  if (int rc = vcf_neg_begin(e, 1)) return rc;
   if (V.slot_bytes > 0)  // the scratch depends on the query (max_column): resize for the ring's slots
     if (int rc = grow(e->vscratch, vcf_scratch_need(e, (int64_t)V.slot_bytes))) return rc;
   if (int rc = grow(e->vbad, sizeof(unsigned long long))) return rc;
@@ -1230,6 +1304,7 @@ int sai_engine_vcf_genome_begin(sai_engine* e, const sai_layout* lay, const char
   V.genome = true;
   if (int rc = vcf_genome_state_init(vcf_genome_state(e), vcf_genome_chroms(e), n_chrom, e->s_comp)) return rc;
   if (int rc = vcf_grow_sites(e, V.site_cap + (int64_t)kTile * n_chrom, false)) return rc;
+  if (int rc = vcf_neg_begin(e, n_chrom)) return rc;
   if (V.slot_bytes > 0)
     if (int rc = grow(e->vscratch, vcf_scratch_need(e, (int64_t)V.slot_bytes))) return rc;
   V.state = 1;
@@ -1254,6 +1329,8 @@ int sai_engine_vcf_genome_finish(sai_engine* e, int64_t* n_sites, int32_t* max_v
     chroms[c] = sai_vcf_chrom{any ? (int64_t)(uint32_t)d.first_key : 0, any ? (int64_t)(uint32_t)d.last_key : 0,
                               d.n_records, d.first_site, d.n_sites};
   }
+  V.chrom_sites.resize((size_t)n);
+  for (int c = 0; c < n; ++c) V.chrom_sites[c] = {dev[c].first_site, dev[c].n_sites};
   if (gs.noncontiguous) {
     V.state = 0;
     set_error("a chromosome's records resume after another chromosome's");
@@ -1312,9 +1389,19 @@ static int vcf_finish_impl(sai_engine* e, int64_t* n_sites, int32_t* max_value, 
     max_value[p] = std::max(lay.pop[p].ploidy, st.vmax[p]);
     if (max_value[p] > (1 << lay.pop[p].bits) - 2) fits = false;
   }
+  if (V.neg) {
+    VcfNegDev nd;
+    SAI_CUDA_CHECK(cudaMemcpy(&nd, V.negs.state, sizeof(nd), cudaMemcpyDeviceToHost));
+    V.neg_n = (int64_t)nd.n;
+  }
   if (st.overflow) {
     set_error("more records than the ingest buffers hold (%lld sites, room for %lld)", (long long)st.n_sites,
               (long long)V.site_cap);
+    return SAI_E_CAPACITY;
+  }
+  if (V.neg && V.neg_n > V.negs.cap) {
+    set_error("more missing calls than the negative-value table holds (%lld entries, room for %lld)",
+              (long long)V.neg_n, (long long)V.negs.cap);
     return SAI_E_CAPACITY;
   }
   if (!fits) {
@@ -1323,6 +1410,8 @@ static int vcf_finish_impl(sai_engine* e, int64_t* n_sites, int32_t* max_value, 
   }
   if (pos_out && pos_cap >= st.n_sites && st.n_sites > 0)
     SAI_CUDA_CHECK(cudaMemcpy(pos_out, e->pos.p, sizeof(int32_t) * (size_t)st.n_sites, cudaMemcpyDeviceToHost));
+  if (V.neg)
+    if (int rc = vcf_neg_finish(e)) return rc;
   e->n_sites = st.n_sites;
   e->lay = lay;
   e->n_jobs = 0;
@@ -1673,6 +1762,131 @@ int sai_engine_loaded_tiles(sai_engine* e, uint8_t* out, uint64_t cap) {
   SAI_REQUIRE(cap >= bytes && (bytes == 0 || out), "sai_engine_loaded_tiles: %llu bytes needed", (unsigned long long)bytes);
   SAI_CUDA_CHECK(cudaSetDevice(e->device));
   if (bytes) SAI_CUDA_CHECK(cudaMemcpy(out, e->packed.p, bytes, cudaMemcpyDeviceToHost));
+  return SAI_OK;
+}
+
+int sai_engine_set_vcf_neg_table(sai_engine* e, int32_t on, int64_t min_entries) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_REQUIRE(e->vcf.state != 1, "sai_engine_set_vcf_neg_table: an ingest session is feeding");
+  SAI_REQUIRE(min_entries >= 0 && min_entries <= sai::kNegMaxEntries,
+              "sai_engine_set_vcf_neg_table: min_entries %lld outside 0..2^31 - 1", (long long)min_entries);
+  e->vcf.neg_on = on != 0;
+  e->vcf.neg_min = min_entries;
+  return SAI_OK;
+}
+
+int64_t sai_engine_loaded_neg_table(sai_engine* e, int64_t* neg_off, int32_t* site, int32_t* ind, int32_t* val,
+                                    int64_t cap) {
+  SAI_REQUIRE(e, "NULL engine");
+  auto& V = e->vcf;
+  SAI_REQUIRE(V.neg && V.neg_n >= 0, "sai_engine_loaded_neg_table: the last ingest session kept no negative-value table");
+  if (V.state != 2) return V.neg_n;  // finished with SAI_E_CAPACITY: the count a repeat needs
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  if (neg_off) std::copy(V.neg_off.begin(), V.neg_off.end(), neg_off);
+  const int64_t n = V.neg_n;
+  if (cap >= n && n > 0 && site && ind && val) {
+    const size_t part = align256(sizeof(int32_t) * (size_t)n);
+    const char* t = static_cast<const char*>(e->vnegt.p);
+    SAI_CUDA_CHECK(cudaMemcpy(site, t, sizeof(int32_t) * n, cudaMemcpyDeviceToHost));
+    SAI_CUDA_CHECK(cudaMemcpy(ind, t + part, sizeof(int32_t) * n, cudaMemcpyDeviceToHost));
+    SAI_CUDA_CHECK(cudaMemcpy(val, t + 2 * part, sizeof(int32_t) * n, cudaMemcpyDeviceToHost));
+  }
+  return n;
+}
+
+int sai_engine_dd_sums_loaded(sai_engine* e, int32_t ref_pop, int32_t tgt_pop, const int32_t* src_pops, int32_t n_src,
+                              int64_t* ref_sum, int64_t* tgt_sum, int32_t m_max) {
+  SAI_REQUIRE(e && e->vcf.state == 2 && e->n_jobs > 0, "sai_engine_dd_sums_loaded: no scored ingest session");
+  SAI_REQUIRE(ref_sum && tgt_sum && src_pops, "NULL argument");
+  auto& V = e->vcf;
+  SAI_REQUIRE(V.neg, "sai_engine_dd_sums_loaded: the ingest session kept no negative-value table");
+  const sai_layout* lay = &e->lay;
+  SAI_REQUIRE(ref_pop >= 0 && ref_pop < lay->n_pops && tgt_pop >= 0 && tgt_pop < lay->n_pops, "bad population index");
+  SAI_REQUIRE(m_max >= 1, "m_max must be positive");
+  SAI_REQUIRE(n_src <= SAI_MAX_SRC, "n_src %d outside [1,%d]", n_src, SAI_MAX_SRC);
+  const int64_t W = e->W;
+  if (W == 0 || n_src <= 0) return SAI_OK;
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  const int n_pops = lay->n_pops;
+  // (first window, windows, first site, sites, chromosome) per piece: a genome session's piece is the
+  // chromosome whose sites it covers, the table's sites are chromosome-local
+  std::vector<std::array<int64_t, 5>> P;
+  if (e->pieces.empty()) {
+    SAI_REQUIRE(!V.genome || V.gq.n_chrom == 1, "sai_engine_dd_sums_loaded: a genome session is scored in pieces");
+    P.push_back({0, W, 0, e->n_sites, 0});
+  }
+  for (const auto& q : e->pieces) {
+    int64_t c = -1;
+    for (size_t k = 0; k < V.chrom_sites.size() && c < 0; ++k)
+      if (V.chrom_sites[k][0] == q[2] && V.chrom_sites[k][1] == q[3]) c = (int64_t)k;
+    SAI_REQUIRE(c >= 0 || q[3] == 0, "sai_engine_dd_sums_loaded: piece at site %lld (%lld sites) is not a chromosome",
+                (long long)q[2], (long long)q[3]);
+    P.push_back({q[0], q[1], q[2], q[3], c});
+  }
+  int32_t hp[2 + SAI_MAX_SRC] = {ref_pop, tgt_pop};
+  for (int k = 0; k < n_src; ++k) {
+    SAI_REQUIRE(src_pops[k] >= 0 && src_pops[k] < n_pops, "bad source population index");
+    hp[2 + k] = src_pops[k];
+  }
+  const int n_hp = 2 + n_src;
+  int64_t max_stride = kTile;
+  for (const auto& q : P) max_stride = std::max(max_stride, sai_num_tiles(q[3]) * kTile);
+  const int64_t rows = sai_hist_rows(lay, hp, n_hp);
+  const size_t out_n = (size_t)n_src * W * m_max;
+  const size_t hist_bytes = align256(sizeof(int32_t) * (size_t)rows * max_stride);
+  if (int rc = grow(e->hist, hist_bytes + sizeof(uint64_t) * n_hp * P.size() + 256)) return rc;
+  if (int rc = grow(e->dd, sizeof(int64_t) * 2 * out_n + 512)) return rc;
+  cudaStream_t st = e->s_comp;
+  int32_t* d_hist = static_cast<int32_t*>(e->hist.p);
+  uint64_t* d_missing = reinterpret_cast<uint64_t*>(static_cast<char*>(e->hist.p) + hist_bytes);
+  int32_t* d_err = reinterpret_cast<int32_t*>(d_missing + n_hp * P.size());
+  int64_t* d_r = static_cast<int64_t*>(e->dd.p);
+  int64_t* d_t = d_r + out_n;
+  // a piece without sites leaves its missing totals untouched (sai_site_hist returns early): zero all of them
+  SAI_CUDA_CHECK(cudaMemsetAsync(d_missing, 0, sizeof(uint64_t) * n_hp * P.size() + sizeof(int32_t), st));
+  SAI_CUDA_CHECK(cudaMemsetAsync(d_r, 0, sizeof(int64_t) * 2 * out_n, st));
+  const int64_t* d_ws = static_cast<const int64_t*>(e->win.p);
+  const int32_t* d_pos = static_cast<const int32_t*>(e->pos.p);
+  const size_t part = align256(sizeof(int32_t) * (size_t)std::max<int64_t>(V.neg_n, 1));
+  const int32_t* d_ns = static_cast<const int32_t*>(e->vnegt.p);
+  const int32_t* d_ni = reinterpret_cast<const int32_t*>(static_cast<const char*>(e->vnegt.p) + part);
+  const int32_t* d_nv = reinterpret_cast<const int32_t*>(static_cast<const char*>(e->vnegt.p) + 2 * part);
+  std::vector<int64_t> off((size_t)n_pops + 1);
+  for (size_t j = 0; j < P.size(); ++j) {
+    const int64_t w0 = P[j][0], nw = P[j][1], lo = P[j][2], n = P[j][3], c = P[j][4];
+    if (nw == 0) continue;
+    const int64_t base = c >= 0 ? V.neg_off[(size_t)c * (n_pops + 1)] : 0;
+    for (int p = 0; p <= n_pops; ++p) off[p] = c >= 0 ? V.neg_off[(size_t)c * (n_pops + 1) + p] - base : 0;
+    const void* packed = static_cast<const char*>(e->packed.p) + (size_t)(lo / kTile) * lay->pairs_per_site * kTile * 8;
+    const int64_t stride = sai_num_tiles(n) * kTile;
+    if (int rc = sai_site_hist(lay, packed, n, hp, n_hp, d_hist, stride, d_missing + n_hp * j, st)) return rc;
+    int64_t* r = d_r + (size_t)n_src * m_max * w0;
+    int64_t* t = d_t + (size_t)n_src * m_max * w0;
+    if (int rc = sai_window_dd(lay, packed, d_pos + lo, n, d_ws + w0, d_ws + W + w0, nw, d_hist, stride, ref_pop, tgt_pop,
+                               src_pops, n_src, off.data(), d_ns + base, d_ni + base, d_nv + base, r, t, m_max, d_err, st))
+      return rc;
+    const size_t row = sizeof(int64_t) * (size_t)nw * m_max, pitch = sizeof(int64_t) * (size_t)W * m_max;
+    SAI_CUDA_CHECK(cudaMemcpy2DAsync(ref_sum + w0 * m_max, pitch, r, row, row, n_src, cudaMemcpyDeviceToHost, st));
+    SAI_CUDA_CHECK(cudaMemcpy2DAsync(tgt_sum + w0 * m_max, pitch, t, row, row, n_src, cudaMemcpyDeviceToHost, st));
+  }
+  std::vector<uint64_t> h_missing((size_t)n_hp * P.size());
+  int32_t h_err = 0;
+  SAI_CUDA_CHECK(cudaMemcpyAsync(h_missing.data(), d_missing, sizeof(uint64_t) * h_missing.size(), cudaMemcpyDeviceToHost, st));
+  SAI_CUDA_CHECK(cudaMemcpyAsync(&h_err, d_err, sizeof(h_err), cudaMemcpyDeviceToHost, st));
+  SAI_CUDA_CHECK(cudaStreamSynchronize(st));
+  // the bit-planes keep one missing code: every missing call needs its raw value in the table
+  for (size_t j = 0; j < P.size(); ++j) {
+    const int64_t c = P[j][4];
+    if (P[j][1] == 0) continue;
+    for (int q = 0; q < n_hp; ++q) {
+      const size_t o = (size_t)c * (n_pops + 1) + hp[q];
+      const int64_t have = c >= 0 ? V.neg_off[o + 1] - V.neg_off[o] : 0;
+      SAI_REQUIRE((int64_t)h_missing[n_hp * j + q] == have,
+                  "population %d has %lld missing calls but %lld entries in the negative-value table", hp[q],
+                  (long long)h_missing[n_hp * j + q], (long long)have);
+    }
+  }
+  SAI_REQUIRE(h_err == 0, "a missing source call has no entry in the negative-value table");
   return SAI_OK;
 }
 

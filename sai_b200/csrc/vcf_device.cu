@@ -61,9 +61,48 @@ struct Scratch {
   int64_t* seg_gap;   // [n_chrom + 2] end of the run before it: [seg_gap, seg_site) are padding sites
 };
 
+// Slice scratch and session of the negative-value table (vcf_genome.cuh, VcfNegSession)
+struct NegArgs {
+  int32_t* cnt;        // [n_pops * n_kept + 1] missing calls of (population, kept record); then their exclusive scan
+  uint32_t* at;        // [n_pops * n_kept] first entry of (population, kept record), relative to slice_base
+  int2* pending;       // [n_geno_warps][row] (individual, value) of the record's population being parsed
+  int32_t* chunk_cnt;  // scan of cnt: per 1024 items
+  int32_t* chunk_off;
+  int32_t row;         // largest population
+  int32_t n_pops;
+  VcfNegSession t;
+};
+
 inline size_t al(size_t x) { return (x + 255) & ~size_t(255); }
 
 int geno_warps() { return sm_count() * 4 * kWarpsPerBlock; }
+
+// a kept record is at least 11 bytes (CHROM, nine tabs, newline)
+inline size_t max_kept(int64_t len) { return (size_t)len / 11 + 2; }
+
+// byte size of the negative-value scratch of a slice and, when base != null, its carving
+size_t carve_neg(const sai_vcf_query& q, int64_t len, char* base, NegArgs* a) {
+  int32_t row = 1;
+  for (int p = 0; p < q.lay.n_pops; ++p) row = row > q.lay.pop[p].n_samples ? row : q.lay.pop[p].n_samples;
+  const size_t n_item = (size_t)q.lay.n_pops * max_kept(len);
+  const size_t n_chunk = n_item / 1024 + 2;
+  size_t at = 0;
+  auto take = [&](size_t bytes) {
+    char* p = base ? base + at : nullptr;
+    at += al(bytes);
+    return p;
+  };
+  NegArgs t{};
+  t.cnt = reinterpret_cast<int32_t*>(take(4 * (n_item + 1)));
+  t.at = reinterpret_cast<uint32_t*>(take(4 * n_item));
+  t.pending = reinterpret_cast<int2*>(take(8 * (size_t)geno_warps() * (size_t)row));
+  t.chunk_cnt = reinterpret_cast<int32_t*>(take(4 * n_chunk));
+  t.chunk_off = reinterpret_cast<int32_t*>(take(4 * n_chunk));
+  t.row = row;
+  t.n_pops = q.lay.n_pops;
+  if (a) *a = t;
+  return at;
+}
 
 // byte size of the scratch and, when base != null, its carving
 size_t carve(const sai_vcf_query& q, int64_t len, char* base, Scratch* s, int n_chrom = -1) {
@@ -551,10 +590,13 @@ __device__ inline int64_t genome_site(const Scratch& s, int n_seg, int64_t k) {
   return s.seg_site[lo] + (k - s.seg_k[lo]);
 }
 
-template <bool kGenome = false>
+// kNeg: also the negative-value table.  Per (record, population) the lanes' missing calls are
+// ranked with one ballot per group (individual order), staged in the warp's `pending` row, and
+// copied to the session buffer at an offset reserved with one atomic; the count goes to `cnt`.
+template <bool kGenome = false, bool kNeg = false>
 __global__ void __launch_bounds__(256) k_genotypes(const char* __restrict__ text, const __grid_constant__ sai_vcf_query q,
                                                    Scratch s, void* __restrict__ tiles, int32_t* __restrict__ pos,
-                                                   int64_t site_cap, sai_vcf_state* st) {
+                                                   int64_t site_cap, sai_vcf_state* st, const NegArgs na) {
   const int lane = threadIdx.x & 31;
   const int64_t warp = (int64_t)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
   const int64_t n_warps = (int64_t)gridDim.x * kWarpsPerBlock;
@@ -563,6 +605,7 @@ __global__ void __launch_bounds__(256) k_genotypes(const char* __restrict__ text
   const int n_seg = kGenome ? s.info->n_seg : 0;
   const int row = q.max_column + 1;
   int32_t* fo = s.fields + warp * row;
+  int2* const pend = na.pending + warp * na.row;  // kNeg
   const int pps = q.lay.pairs_per_site;
   for (int64_t k = warp; k < n_kept; k += n_warps) {
     const int64_t site = kGenome ? genome_site(s, n_seg, k) : base + k;
@@ -604,9 +647,11 @@ __global__ void __launch_bounds__(256) k_genotypes(const char* __restrict__ text
       const sai_pop_layout& P = q.lay.pop[p];
       const int B = P.bits, miss = (1 << B) - 1;
       int vmax = 0;
+      int n_neg = 0;  // kNeg: missing calls of the record in this population so far
       for (int g = 0; g < P.n_groups; ++g) {
         const int ind = 32 * g + lane;
         uint32_t code = (uint32_t)miss;
+        int neg = 0;
         if (ind < P.n_samples) {
           const int col = q.sample_column[col_base + ind];
           int v;
@@ -620,12 +665,40 @@ __global__ void __launch_bounds__(256) k_genotypes(const char* __restrict__ text
             code = (uint32_t)v;
             vmax = max(vmax, v);
           }
+          if constexpr (kNeg) neg = min(v, 0);
         }
         const int w0 = 2 * P.pair_off + g * B;
         for (int b = 0; b < B; ++b) {
           const uint32_t word = __ballot_sync(0xffffffffu, (code >> b) & 1u);
           if (lane == b) *word_at(tiles, pps, site, w0 + b) = word;
         }
+        if constexpr (kNeg) {
+          const uint32_t m = __ballot_sync(0xffffffffu, neg < 0);
+          if (neg < 0) pend[n_neg + __popc(m & ((1u << lane) - 1))] = make_int2(ind, neg);
+          n_neg += __popc(m);
+        }
+      }
+      if constexpr (kNeg) {
+        const int64_t item = (int64_t)p * n_kept + k;
+        uint32_t rel = 0;
+        if (lane == 0) {
+          if (n_neg > 0)
+            rel = (uint32_t)(atomicAdd(&na.t.state->n, (unsigned long long)n_neg) - na.t.state->slice_base);
+          na.cnt[item] = n_neg;
+          na.at[item] = rel;
+        }
+        rel = __shfl_sync(0xffffffffu, rel, 0);
+        __syncwarp();  // the pending row is complete
+        const int64_t d0 = (int64_t)(na.t.state->slice_base + rel);
+        for (int e = lane; e < n_neg; e += 32) {
+          const int64_t d = d0 + e;
+          if (d < na.t.cap) {
+            const int2 x = pend[e];
+            na.t.ind[d] = x.x;
+            na.t.val[d] = x.y;
+          }
+        }
+        __syncwarp();  // the row is reused by the next population
       }
       if ((P.n_groups * B) & 1)
         if (lane == 0) *word_at(tiles, pps, site, 2 * P.pair_off + P.n_groups * B) = 0u;  // the pad word
@@ -671,6 +744,136 @@ __global__ void k_genome_init(VcfGenomeState* gs, VcfChromDev* chroms, int32_t n
   if (threadIdx.x == 0) *gs = VcfGenomeState{0, -1, 0};
 }
 
+// ---- 6. negative-value table: the slice's entries get their key and their index in it -------------
+// The kept records k_genotypes wrote (genome: none without runs) and, for record k, its site and the
+// first kept record of its chromosome's run in the slice.
+template <bool kGenome>
+__device__ inline int neg_kept(const Scratch& s) {
+  return kGenome && s.info->n_seg == 0 ? 0 : s.info->n_kept;
+}
+template <bool kGenome>
+__device__ inline int64_t neg_site(const Scratch& s, int64_t k, int* k0) {
+  if constexpr (kGenome) {
+    const int n_seg = s.info->n_seg;
+    int lo = 0, hi = n_seg - 1;
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (s.seg_k[mid] <= k) lo = mid; else hi = mid - 1;
+    }
+    *k0 = s.seg_k[lo];
+    return s.seg_site[lo] + (k - s.seg_k[lo]);
+  } else {
+    *k0 = 0;
+    return s.info->site_base + k;
+  }
+}
+
+__global__ void k_neg_begin(VcfNegDev* d) { d->slice_base = d->n; }
+
+// per 1024 (population, record) items: their count; records past site_cap (not parsed) count 0
+template <bool kGenome>
+__global__ void __launch_bounds__(1024) k_neg_count(Scratch s, const NegArgs na, int64_t site_cap) {
+  const int64_t n_kept = neg_kept<kGenome>(s);
+  const int64_t n = n_kept * na.n_pops;
+  for (int64_t c = blockIdx.x; c * 1024 < n; c += gridDim.x) {
+    const int64_t i = c * 1024 + threadIdx.x;
+    int v = 0;
+    if (i < n) {
+      int k0;
+      v = neg_site<kGenome>(s, i % n_kept, &k0) < site_cap ? na.cnt[i] : 0;
+      na.cnt[i] = v;
+    }
+    int total;
+    block_excl_scan(v, &total);
+    if (threadIdx.x == 0) na.chunk_cnt[c] = total;
+  }
+}
+
+template <bool kGenome>
+__global__ void __launch_bounds__(1024) k_neg_scan(Scratch s, const NegArgs na) {
+  const int64_t n = (int64_t)neg_kept<kGenome>(s) * na.n_pops;
+  scan_one_block(na.chunk_cnt, na.chunk_off, (int)((n + 1023) / 1024), na.cnt + n);
+}
+
+template <bool kGenome>
+__global__ void __launch_bounds__(1024) k_neg_excl(Scratch s, const NegArgs na) {
+  const int64_t n = (int64_t)neg_kept<kGenome>(s) * na.n_pops;
+  for (int64_t c = blockIdx.x; c * 1024 < n; c += gridDim.x) {
+    const int64_t i = c * 1024 + threadIdx.x;
+    const int v = i < n ? na.cnt[i] : 0;
+    int total;
+    const int ex = na.chunk_off[c] + block_excl_scan(v, &total);
+    if (i < n) na.cnt[i] = ex;
+  }
+}
+
+// every entry of (population p, record k): chromosome-local site, key, index inside the key =
+// entries of the key in earlier slices + entries of the key's earlier records in this slice + rank
+template <bool kGenome>
+__global__ void __launch_bounds__(256) k_neg_fix(Scratch s, const NegArgs na, const VcfChromDev* chroms) {
+  const int64_t n_kept = neg_kept<kGenome>(s);
+  const int64_t n = n_kept * na.n_pops;
+  const VcfNegSession& t = na.t;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int p = (int)(i / n_kept);
+    const int m = min(na.cnt[i + 1] - na.cnt[i], na.row);
+    if (m <= 0) continue;
+    const int64_t k = i - p * n_kept;
+    int k0;
+    int64_t site = neg_site<kGenome>(s, k, &k0);
+    int c = 0;
+    if constexpr (kGenome) {
+      c = s.rec_chrom[s.kept[k]];
+      site -= chroms[c].first_site;
+    }
+    const int key = c * na.n_pops + p;
+    const int64_t idx = (int64_t)t.count[key] + na.cnt[i] - na.cnt[p * n_kept + k0];
+    const int64_t d0 = (int64_t)(t.state->slice_base + na.at[i]);
+    for (int e = 0; e < m && d0 + e < t.cap; ++e) {
+      t.site[d0 + e] = (int32_t)site;
+      t.key[d0 + e] = key;
+      t.idx[d0 + e] = (int32_t)(idx + e);
+    }
+  }
+}
+
+// the slice's entries of each (run, population) added to its key's count
+template <bool kGenome>
+__global__ void k_neg_totals(Scratch s, const NegArgs na) {
+  const int64_t n_kept = neg_kept<kGenome>(s);
+  if (n_kept == 0) return;
+  const int n_run = kGenome ? s.info->n_seg : 1;
+  for (int r = threadIdx.x; r < n_run * na.n_pops; r += blockDim.x) {
+    const int j = r / na.n_pops, p = r % na.n_pops;
+    const int64_t k0 = kGenome ? s.seg_k[j] : 0, k1 = kGenome && j + 1 < n_run ? s.seg_k[j + 1] : n_kept;
+    const int c = kGenome ? s.rec_chrom[s.kept[k0]] : 0;
+    atomicAdd(&na.t.count[c * na.n_pops + p], (unsigned long long)(na.cnt[p * n_kept + k1] - na.cnt[p * n_kept + k0]));
+  }
+}
+
+__global__ void k_neg_order(const VcfNegSession t, int64_t n, const int64_t* __restrict__ key_off, int32_t* out_site,
+                            int32_t* out_ind, int32_t* out_val) {
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t d = key_off[t.key[e]] + t.idx[e];
+    if (d < 0 || d >= n) continue;
+    out_site[d] = t.site[e];
+    out_ind[d] = t.ind[e];
+    out_val[d] = t.val[e];
+  }
+}
+
+// the table's kernels of one slice, behind its genotype pass
+template <bool kGenome>
+int neg_slice(const Scratch& s, const NegArgs& na, const VcfChromDev* chroms, int64_t site_cap, int grid, cudaStream_t st) {
+  k_neg_count<kGenome><<<grid, 1024, 0, st>>>(s, na, site_cap);
+  k_neg_scan<kGenome><<<1, 1024, 0, st>>>(s, na);
+  k_neg_excl<kGenome><<<grid, 1024, 0, st>>>(s, na);
+  k_neg_fix<kGenome><<<grid * 4, 256, 0, st>>>(s, na, chroms);
+  k_neg_totals<kGenome><<<1, 256, 0, st>>>(s, na);
+  SAI_CUDA_CHECK(cudaGetLastError());
+  return SAI_OK;
+}
+
 }  // namespace
 
 int vcf_chrom_table(const char* names, const int32_t* name_off, int32_t n, uint32_t* table) {
@@ -703,9 +906,32 @@ uint64_t vcf_genome_scratch_bytes(const VcfGenomeQuery& g, int64_t len) {
   return (uint64_t)carve(g.q, len, nullptr, nullptr, g.n_chrom) + 256;
 }
 
+uint64_t vcf_neg_scratch_bytes(const sai_vcf_query& q, int64_t len) { return (uint64_t)carve_neg(q, len, nullptr, nullptr); }
+
+int vcf_neg_order(const VcfNegSession& neg, int64_t n, const int64_t* d_key_off, int32_t* out_site, int32_t* out_ind,
+                  int32_t* out_val, cudaStream_t st) {
+  if (n <= 0) return SAI_OK;
+  const int64_t want = (n + 255) / 256, cap = (int64_t)sm_count() * 8;
+  k_neg_order<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(neg, n, d_key_off, out_site, out_ind, out_val);
+  SAI_CUDA_CHECK(cudaGetLastError());
+  return SAI_OK;
+}
+
+// the scratch of the negative-value table behind the parse scratch (`need` bytes), checked against its size
+static int neg_args(const sai_vcf_query& q, int64_t len, void* d_scratch, uint64_t scratch_bytes, size_t need,
+                    const VcfNegSession* neg, NegArgs* na) {
+  *na = NegArgs{};
+  if (!neg) return SAI_OK;
+  const size_t extra = carve_neg(q, len, static_cast<char*>(d_scratch) + need, na);
+  SAI_REQUIRE(scratch_bytes >= need + extra, "device ingest: scratch of %llu bytes, %zu needed with the negative-value table",
+              (unsigned long long)scratch_bytes, need + extra);
+  na->t = *neg;
+  return SAI_OK;
+}
+
 int vcf_tiles_genome(const VcfGenomeQuery& g, const char* d_text, int64_t len, void* d_scratch, uint64_t scratch_bytes,
                      void* d_tiles, int32_t* d_pos, int64_t site_cap, sai_vcf_state* d_state, VcfGenomeState* d_gs,
-                     VcfChromDev* d_chroms, cudaStream_t st) {
+                     VcfChromDev* d_chroms, const VcfNegSession* neg, cudaStream_t st) {
   SAI_REQUIRE(len >= 0 && len < (int64_t(1) << 31), "vcf_tiles_genome: slice of %lld bytes (at most 2^31 - 1)",
               (long long)len);
   SAI_REQUIRE(site_cap >= 0 && site_cap % kTile == 0, "vcf_tiles_genome: site_cap must be a multiple of 32");
@@ -713,6 +939,8 @@ int vcf_tiles_genome(const VcfGenomeQuery& g, const char* d_text, int64_t len, v
   const size_t need = carve(g.q, len, static_cast<char*>(d_scratch), &s, g.n_chrom);
   SAI_REQUIRE(scratch_bytes >= need, "vcf_tiles_genome: scratch of %llu bytes, %zu needed",
               (unsigned long long)scratch_bytes, need);
+  NegArgs na;
+  if (int rc = neg_args(g.q, len, d_scratch, scratch_bytes, need, neg, &na)) return rc;
   const int n_seg = (int)((len + kSegBytes - 1) / kSegBytes);
   const int grid = sm_count() * 4;
   if (n_seg > 0) {
@@ -729,7 +957,13 @@ int vcf_tiles_genome(const VcfGenomeQuery& g, const char* d_text, int64_t len, v
   k_keep_write<true><<<grid, kLinesPerChunk, 0, st>>>(s, d_pos, site_cap);
   k_genome_bounds<<<grid, 256, 0, st>>>(s, d_gs, g.n_chrom);
   k_genome_plan<<<1, 32, 0, st>>>(s, d_state, d_gs, d_chroms, g.n_chrom, site_cap);
-  k_genotypes<true><<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, g.q, s, d_tiles, d_pos, site_cap, d_state);
+  if (neg) {
+    k_neg_begin<<<1, 1, 0, st>>>(neg->state);
+    k_genotypes<true, true><<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, g.q, s, d_tiles, d_pos, site_cap, d_state, na);
+    if (int rc = neg_slice<true>(s, na, d_chroms, site_cap, grid, st)) return rc;
+  } else {
+    k_genotypes<true><<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, g.q, s, d_tiles, d_pos, site_cap, d_state, na);
+  }
   k_pad_genome<<<1, 256, 0, st>>>(g.q.lay, d_tiles, d_state, s, site_cap);
   SAI_CUDA_CHECK(cudaGetLastError());
   return SAI_OK;
@@ -749,7 +983,18 @@ uint64_t sai_vcf_scratch_bytes(const sai_vcf_query* q, int64_t len) {
 int sai_vcf_tiles_device(const sai_vcf_query* q, const char* d_text, int64_t len, void* d_scratch,
                          uint64_t scratch_bytes, void* d_tiles, int32_t* d_pos, int64_t site_cap,
                          sai_vcf_state* d_state, void* stream) {
-  SAI_REQUIRE(q && d_state && d_scratch && d_tiles && d_pos, "sai_vcf_tiles_device: NULL argument");
+  SAI_REQUIRE(q, "sai_vcf_tiles_device: NULL argument");
+  return vcf_tiles_single(*q, d_text, len, d_scratch, scratch_bytes, d_tiles, d_pos, site_cap, d_state, nullptr,
+                          static_cast<cudaStream_t>(stream));
+}
+
+}  // extern "C"
+
+int sai::vcf_tiles_single(const sai_vcf_query& qr, const char* d_text, int64_t len, void* d_scratch,
+                          uint64_t scratch_bytes, void* d_tiles, int32_t* d_pos, int64_t site_cap,
+                          sai_vcf_state* d_state, const VcfNegSession* neg, cudaStream_t st) {
+  const sai_vcf_query* q = &qr;
+  SAI_REQUIRE(d_state && d_scratch && d_tiles && d_pos, "sai_vcf_tiles_device: NULL argument");
   if (int rc = validate_layout(&q->lay)) return rc;
   SAI_REQUIRE(len >= 0 && len < (int64_t(1) << 31), "sai_vcf_tiles_device: slice of %lld bytes (at most 2^31 - 1)",
               (long long)len);
@@ -764,7 +1009,8 @@ int sai_vcf_tiles_device(const sai_vcf_query* q, const char* d_text, int64_t len
   const size_t need = carve(*q, len, static_cast<char*>(d_scratch), &s);
   SAI_REQUIRE(scratch_bytes >= need, "sai_vcf_tiles_device: scratch of %llu bytes, %zu needed",
               (unsigned long long)scratch_bytes, need);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  NegArgs na;
+  if (int rc = neg_args(*q, len, d_scratch, scratch_bytes, need, neg, &na)) return rc;
   const int n_seg = (int)((len + kSegBytes - 1) / kSegBytes);
   const int grid = sm_count() * 4;
   if (n_seg > 0) {
@@ -779,10 +1025,14 @@ int sai_vcf_tiles_device(const sai_vcf_query* q, const char* d_text, int64_t len
   k_keep_count<<<grid, kLinesPerChunk, 0, st>>>(s, nullptr, nullptr);
   k_keep_scan<<<1, 1024, 0, st>>>(s, d_state, site_cap);
   k_keep_write<<<grid, kLinesPerChunk, 0, st>>>(s, d_pos, site_cap);
-  k_genotypes<<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, *q, s, d_tiles, d_pos, site_cap, d_state);
+  if (neg) {
+    k_neg_begin<<<1, 1, 0, st>>>(neg->state);
+    k_genotypes<false, true><<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, *q, s, d_tiles, d_pos, site_cap, d_state, na);
+    if (int rc = neg_slice<false>(s, na, nullptr, site_cap, grid, st)) return rc;
+  } else {
+    k_genotypes<<<grid, 32 * kWarpsPerBlock, 0, st>>>(d_text, *q, s, d_tiles, d_pos, site_cap, d_state, na);
+  }
   k_pad_tail<<<1, 256, 0, st>>>(q->lay, d_tiles, d_state, site_cap);
   SAI_CUDA_CHECK(cudaGetLastError());
   return SAI_OK;
 }
-
-}  // extern "C"

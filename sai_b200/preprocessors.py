@@ -343,6 +343,7 @@ class ChunkPreprocessor:
         device: int = 0,
         ingest: str = "host",
         inflate: str = "host",
+        dd_ingest: str = "host",
     ):
         """``ingest="device"`` parses the VCF on the GPU (``vcf_device``): the text is copied to the
         device and parsed there straight into the packed tiles, which all combinations are scored
@@ -350,7 +351,10 @@ class ChunkPreprocessor:
         more than 16 populations, ancestral alleles longer than 7 bytes, source ploidies that differ
         from their positions in a combination) are read on the host automatically.
         ``inflate="device"`` (with ``ingest="device"``) also inflates a bgzip file on the GPU: only
-        the compressed blocks cross PCIe.  Plain text and single-member gzip are read as before."""
+        the compressed blocks cross PCIe.  Plain text and single-member gzip are read as before.
+        ``dd_ingest="device"`` (with ``ingest="device"``) reads DD chunks on the device too: the
+        genotype pass keeps the raw values of missing calls DD needs (the negative-value table) in
+        HBM next to the tiles, so DD no longer sends the chunk to host ingest; same items."""
         from .vcf import parse_ind_file
 
         if ingest not in ("host", "device"):
@@ -359,8 +363,13 @@ class ChunkPreprocessor:
             raise ValueError(f"inflate must be 'host' or 'device', not {inflate!r}")
         if inflate == "device" and ingest != "device":
             raise ValueError("inflate='device' needs ingest='device'")
+        if dd_ingest not in ("host", "device"):
+            raise ValueError(f"dd_ingest must be 'host' or 'device', not {dd_ingest!r}")
+        if dd_ingest == "device" and ingest != "device":
+            raise ValueError("dd_ingest='device' needs ingest='device'")
         self.ingest = ingest
         self.inflate = inflate
+        self.dd_ingest = dd_ingest
 
         self.vcf_file = vcf_file
         self.ref_ind_file = ref_ind_file
@@ -425,26 +434,29 @@ class ChunkPreprocessor:
         plan, _, _ = read_plan(self.vcf_file, chr_name, self.ploidy_config, self.ref_ind_file, self.tgt_ind_file,
                                self.src_ind_file, self.out_ind_file)
         anc, _ = read_anc_or_error(self.anc_allele_file, chr_name, start, end)
-        return fallback_reason(self.stat_config, self.ploidy_config, plan, anc, chr_name, self.num_src)
+        return fallback_reason(self.stat_config, self.ploidy_config, plan, anc, chr_name, self.num_src,
+                               self.dd_ingest)
 
     def _run_device(self, chr_name, start, end):
         import warnings
 
         from .vcf import read_anc_or_error
-        from .vcf_device import _wants_outgroup, fallback_reason, read_loaded, read_plan
+        from .vcf_device import _wants_outgroup, fallback_reason, read_loaded, read_plan, wants_dd
 
         with warnings.catch_warnings(record=True) as caught:  # warned once, by the read that is used
             warnings.simplefilter("always")
             plan, requests, out = read_plan(self.vcf_file, chr_name, self.ploidy_config, self.ref_ind_file,
                                             self.tgt_ind_file, self.src_ind_file, self.out_ind_file)
         anc, anc_error = read_anc_or_error(self.anc_allele_file, chr_name, start, end)
-        if fallback_reason(self.stat_config, self.ploidy_config, plan, anc, chr_name, self.num_src) is not None:
+        if fallback_reason(self.stat_config, self.ploidy_config, plan, anc, chr_name, self.num_src,
+                           self.dd_ingest) is not None:
             return None
         for w in caught:
             warnings.warn_explicit(w.message, w.category, w.filename, w.lineno)
         try:
             loaded = read_loaded(self.engine, self.vcf_file, chr_name, plan, requests, out, anc, anc_error, start, end,
-                                 with_outgroup=_wants_outgroup(self.stat_config), inflate=self.inflate)
+                                 with_outgroup=_wants_outgroup(self.stat_config), inflate=self.inflate,
+                                 neg_table=self.dd_ingest == "device" and wants_dd(self.stat_config))
         except (KeyError, OSError) as e:
             region = chr_name if start is None and end is None else f"{chr_name}:{start}-{end}"
             raise ValueError(f"Failed to read VCF file {self.vcf_file} from {region}: {e}") from e

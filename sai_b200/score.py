@@ -40,7 +40,7 @@ def _load_checked_config(config: str, anc_allele_file):
     return cfg
 
 
-def _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file, device, ingest, inflate):
+def _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file, device, ingest, inflate, dd_ingest):
     pop_config = cfg.populations
     return ChunkPreprocessor(
         vcf_file=vcf_file,
@@ -57,6 +57,7 @@ def _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file
         device=device,
         ingest=ingest,
         inflate=inflate,
+        dd_ingest=dd_ingest,
     )
 
 
@@ -94,16 +95,19 @@ def score(
     device: int = 0,
     ingest: str = "host",
     inflate: str = "host",
+    dd_ingest: str = "host",
 ) -> None:
-    """``ingest="device"`` parses the VCF on the GPU (``ChunkPreprocessor(ingest=...)``), and
-    ``inflate="device"`` also inflates a bgzip file there; same output."""
+    """``ingest="device"`` parses the VCF on the GPU (``ChunkPreprocessor(ingest=...)``),
+    ``inflate="device"`` also inflates a bgzip file there, and ``dd_ingest="device"`` reads a DD
+    configuration there too (the raw values of missing calls are kept in HBM); same output."""
     cfg = _load_checked_config(config, anc_allele_file)
     # ONE chunk, as sai.py:86-93 (num_chunks=1; `num_workers` is accepted and ignored there too):
     # rows come out product-major / windows-inner, identical to the reference's text.  Real
     # parallelism is sai_b200.multiprocessing.mp_pool (one worker per GPU) or sai_b200.distributed.
     generator = ChunkGenerator(vcf_file=vcf_file, chr_name=chr_name, window_size=win_len, step_size=win_step,
                                num_chunks=1)
-    pre = _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file, device, ingest, inflate)
+    pre = _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file, device, ingest, inflate,
+                        dd_ingest)
     _write_headers(output_file, cfg.statistics, cfg.ploidies)
     items = []
     for params in generator.get():  # sai.py:148-149
@@ -121,6 +125,7 @@ def score_genome(
     config: str,
     device: int = 0,
     inflate: str = "host",
+    dd_ingest: str = "host",
 ) -> None:
     """Scores every chromosome of ``chr_names`` of one (multi-chromosome) VCF: the score file and the
     ``.U.log`` / ``.Q.log`` files are byte for byte those of ``score(vcf_file, c, ...)`` run for each
@@ -129,20 +134,26 @@ def score_genome(
     inflates a bgzip file there) into one resident layout in which every chromosome starts on a tile
     boundary, and all chromosomes are scored with one genotype pass and one window launch.
 
+    With ``dd_ingest="device"`` a DD configuration takes the one-pass read too: the genotype pass
+    keeps the raw values of missing calls (the negative-value table) per chromosome in HBM, and DD is
+    computed per chromosome from the resident tiles and table.
+
     Files the one-pass reader does not take -- where ``vcf_device.fallback_reason`` names a reason
-    (DD, more than 16 populations, long ancestral alleles, positional source ploidies), more than
+    (DD with ``dd_ingest="host"``, more than 16 populations, long ancestral alleles, positional
+    source ploidies), more than
     ``SAI_VCF_MAX_CHROMS`` (1024) chromosomes, or chromosomes whose records are not contiguous in
     the file -- are scored one chromosome at a time by the ``score`` path, with the same output."""
     from . import _cabi
     from .preprocessors import score_populations, write_items
     from .vcf import read_anc_or_error
-    from .vcf_device import _wants_outgroup, fallback_reason, genome_tables, read_genome, read_plan
+    from .vcf_device import _wants_outgroup, fallback_reason, genome_tables, read_genome, read_plan, wants_dd
     from .windows import chunk_windows, split_genome, split_windows_ranges
 
     cfg = _load_checked_config(config, anc_allele_file)
     stat_config, ploidy_config = cfg.statistics, cfg.ploidies
     chr_names = list(chr_names)
-    pre = _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file, device, "device", inflate)
+    pre = _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file, device, "device", inflate,
+                        dd_ingest)
 
     def each_chromosome() -> None:
         generators = [ChunkGenerator(vcf_file=vcf_file, chr_name=c, window_size=win_len, step_size=win_step, num_chunks=1)
@@ -160,7 +171,8 @@ def score_genome(
         warnings.simplefilter("always")
         plan, requests, out = read_plan(vcf_file, chr_names[0], ploidy_config, pre.ref_ind_file, pre.tgt_ind_file,
                                         pre.src_ind_file, pre.out_ind_file)
-    if any(fallback_reason(stat_config, ploidy_config, plan, None, c, pre.num_src) is not None for c in chr_names):
+    if any(fallback_reason(stat_config, ploidy_config, plan, None, c, pre.num_src, dd_ingest) is not None
+           for c in chr_names):
         return each_chromosome()
     tables = genome_tables(chr_names, anc_allele_file)
     if anc_allele_file and tables[2] is None:  # an ancestral allele longer than 7 bytes
@@ -169,7 +181,8 @@ def score_genome(
         warnings.warn_explicit(w.message, w.category, w.filename, w.lineno)
     try:
         loaded = read_genome(pre.engine, vcf_file, chr_names, plan, requests, out, tables,
-                             with_outgroup=_wants_outgroup(stat_config), inflate=inflate)
+                             with_outgroup=_wants_outgroup(stat_config), inflate=inflate,
+                             neg_table=dd_ingest == "device" and wants_dd(stat_config))
     except (KeyError, OSError) as e:
         raise ValueError(f"Failed to read VCF file {vcf_file} from {','.join(chr_names)}: {e}") from e
     if loaded is None:  # no #CHROM line, or a chromosome's records are not contiguous

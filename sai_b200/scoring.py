@@ -264,6 +264,21 @@ class HostEngine:
         _cabi.check(lib.sai_engine_loaded_tiles(self._handle(), out.ctypes.data, out.nbytes))
         return out[: int(lib.sai_packed_bytes(C.byref(layout), int(n_sites)))]
 
+    def loaded_neg_table(self, n_chrom: int, n_pops: int):
+        """Host copy of the negative-value table the last device ingest kept (``neg_table=True``):
+        ``(neg_off, site, ind, val)``, ``neg_off`` int64 ``[n_chrom, n_pops + 1]`` -- chromosome
+        ``c``'s population ``p`` holds entries ``neg_off[c, p] .. neg_off[c, p + 1] - 1`` (tests, tools)."""
+        lib = _cabi.load()
+        off = np.zeros((n_chrom, n_pops + 1), dtype=np.int64)
+        n = int(lib.sai_engine_loaded_neg_table(self._handle(), off.ctypes.data, None, None, None, 0))
+        if n < 0:
+            _cabi.check(n)
+        site, ind, val = (np.zeros(n, dtype=np.int32) for _ in range(3))
+        if n:
+            _cabi.check(min(0, int(lib.sai_engine_loaded_neg_table(self._handle(), off.ctypes.data, site.ctypes.data,
+                                                                    ind.ctypes.data, val.ctypes.data, n))))
+        return off, site, ind, val
+
     def score_loaded(self, windows, jobs, cap_u=None, cap_q=None) -> WindowResults:
         """K1 + K4 on the chunk the last device ingest (``vcf_device.read_loaded``) left resident;
         ``score_resident`` / ``pattern_sums`` then work on it like after ``score``."""
@@ -365,15 +380,21 @@ class HostEngine:
         the last ``score`` call: ``(ref_sum, tgt_sum)``, int64 ``[n_src, W, m_max]``
         with ``ref_sum[k, i, a] = sum_j sum_sites |src_a - ref_j|``
         (sai/stats/dd_statistic.py:70-71).  ``pg`` must carry the negative-value
-        table (``pack_populations(..., keep_negatives=True)``)."""
-        if pg.neg_off is None:
-            raise ValueError("DD needs the raw values of missing calls: pack with keep_negatives=True")
+        table (``pack_populations(..., keep_negatives=True)``), or be a device-parsed
+        chunk or genome whose table is resident (``LoadedChunk.neg``): then neither the
+        tiles nor the table cross PCIe (``sai_engine_dd_sums_loaded``)."""
         lib = _cabi.load()
         W = self._last_W
         m_max = max(int(pg.layout.pop[int(s)].n_samples) for s in src_pops)
         ref_sum = np.zeros((len(src_pops), W, m_max), dtype=np.int64)
         tgt_sum = np.zeros_like(ref_sum)
         src = (C.c_int32 * len(src_pops))(*[int(x) for x in src_pops])
+        if getattr(pg, "neg", False):
+            _cabi.check(lib.sai_engine_dd_sums_loaded(self._handle(), int(ref_pop), int(tgt_pop), src, len(src_pops),
+                                                      ref_sum.ctypes.data, tgt_sum.ctypes.data, m_max))
+            return ref_sum, tgt_sum
+        if getattr(pg, "neg_off", None) is None:
+            raise ValueError("DD needs the raw values of missing calls: pack with keep_negatives=True")
         ptr = lambda a: a.ctypes.data if a.size else None
         _cabi.check(lib.sai_engine_dd_sums(self._handle(), C.byref(pg.layout), int(ref_pop), int(tgt_pop), src,
                                            len(src_pops), pg.neg_off.ctypes.data, ptr(pg.neg_site), ptr(pg.neg_ind),

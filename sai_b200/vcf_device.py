@@ -9,6 +9,11 @@ a bgzip file's blocks go over compressed instead and are inflated on the device
 raises the host path's error.  The records and values
 are those of ``read_data`` (the host parser is the specification); the layout is the one the host
 path packs, so the tiles are comparable byte for byte.
+
+With ``neg_table=True`` (DD with ``dd_ingest="device"``) the genotype pass also keeps the raw value
+of every missing call: the negative-value table DD reads next to the tiles (``sai_b200.h``, N4),
+equal entry for entry to ``encode.negative_table`` of ``read_data``'s matrices and resident in the
+engine for ``HostEngine.dd_sums``.
 """
 
 from __future__ import annotations
@@ -28,23 +33,28 @@ GROUPS = ("ref", "tgt", "src", "outgroup")
 class LoadedChunk:
     """One VCF region parsed on the device: its tiles, positions and windows live in ``engine``.
     ``index[(group, population)]`` = population index in ``layout``; ``groups[group] =
-    (population names or None, samples)`` mirrors what ``read_data`` returns per group."""
+    (population names or None, samples)`` mirrors what ``read_data`` returns per group.  ``neg``:
+    the engine also holds the chunk's negative-value table (``read_loaded(..., neg_table=True)``)."""
 
-    def __init__(self, layout, pos, index, groups):
-        self.layout, self.pos, self.index, self.groups = layout, pos, index, groups
+    def __init__(self, layout, pos, index, groups, neg=False):
+        self.layout, self.pos, self.index, self.groups, self.neg = layout, pos, index, groups, neg
 
     @property
     def n_sites(self) -> int:
         return int(self.pos.shape[0])
 
 
-def fallback_reason(stat_config, ploidy_config, plan, anc, chr_name: str, num_src: int) -> Optional[str]:
+def fallback_reason(stat_config, ploidy_config, plan, anc, chr_name: str, num_src: int,
+                    dd_ingest: str = "host") -> Optional[str]:
     """Why a chunk has to be read on the host (``None``: it can be read on the device).
-    DD needs the raw values of missing calls, a table the host builds; one layout holds at most
-    ``SAI_MAX_POPS`` populations; the native parsers take ancestral alleles of at most 7 bytes;
+    DD needs the raw values of missing calls: with ``dd_ingest="host"`` that table is built by the
+    host, with ``"device"`` the genotype pass keeps it (``read_loaded(..., neg_table=True)``); one
+    layout holds at most ``SAI_MAX_POPS`` populations; the native parsers take ancestral alleles of at most 7 bytes;
     a source population is scored with the ploidy of its position in the combination
     (feature_preprocessor.py:160,168-170), which one layout can only hold when that is its own."""
-    if any(s == "DD" and stat_config.root[s] is True for s in stat_config.root):
+    if dd_ingest not in ("host", "device"):
+        raise ValueError(f"dd_ingest must be 'host' or 'device', not {dd_ingest!r}")
+    if dd_ingest == "host" and wants_dd(stat_config):
         return "DD is enabled"
     if sum(len(pops) for group, _, pops in plan if group != "outgroup" or _wants_outgroup(stat_config)) > _cabi.MAX_POPS:
         return f"more than {_cabi.MAX_POPS} populations"
@@ -61,6 +71,10 @@ def fallback_reason(stat_config, ploidy_config, plan, anc, chr_name: str, num_sr
             if [ploidy_config.get_ploidy("src", name) for name in comb] != positional[: len(comb)]:
                 return "source ploidies differ from their positions in a combination"
     return None
+
+
+def wants_dd(stat_config) -> bool:
+    return any(s == "DD" and stat_config.root[s] is True for s in stat_config.root)
 
 
 def _wants_outgroup(stat_config) -> bool:
@@ -84,11 +98,12 @@ def _pops_and_groups(plan, out, with_outgroup):
 
 
 def _ingest(engine, vcf_file: str, pops, requests, label: str, inflate: str, begin_session, finish_session,
-            region=None):
+            region=None, neg_table: bool = False):
     """The device parse shared by ``read_loaded`` and ``read_genome``: header columns, the text fed
     to the engine's session (``region = (chr_name, start, end)``: a sorted-region read when the file
     allows it), then the finish and its retries -- a wider layout (``SAI_E_DOMAIN``), more sites
-    (``SAI_E_CAPACITY``), host inflate after a corrupt block (``SAI_E_CORRUPT``).
+    (``SAI_E_CAPACITY``: and a larger negative-value table with ``neg_table``), host inflate after a
+    corrupt block (``SAI_E_CORRUPT``).
     ``begin_session(lay, cols, n_file_samples, text_bytes_hint, min_sites)`` opens the session;
     ``finish_session(pos)`` returns ``(rc, n_sites, vmax, extra)``.  Returns ``(layout, pos,
     extra)``; ``pos`` is ``None`` when the file has no ``#CHROM`` line, ``extra`` is ``None`` when it
@@ -99,7 +114,7 @@ def _ingest(engine, vcf_file: str, pops, requests, label: str, inflate: str, beg
     n_samples = [b - a for _, _, a, b in pops]
     ploidy = [requests[a][1] for _, _, a, _ in pops]
     empty = np.empty(0, dtype=np.int32)
-    bits, min_sites = None, 0
+    bits, min_sites, min_entries = None, 0, 0
     for _attempt in range(5):
         lay = make_layout(n_samples, ploidy, bits)
         state = {"cols": None, "n_file": 0, "hint": 0, "begun": False, "fed": 0}
@@ -121,6 +136,7 @@ def _ingest(engine, vcf_file: str, pops, requests, label: str, inflate: str, beg
 
         def begin(length: int) -> None:
             if not state["begun"]:
+                _cabi.check(lib.sai_engine_set_vcf_neg_table(engine._handle(), int(neg_table), min_entries))
                 begin_session(lay, state["cols"], state["n_file"], max(state["hint"], length), min_sites)
                 state["begun"] = True
 
@@ -170,6 +186,11 @@ def _ingest(engine, vcf_file: str, pops, requests, label: str, inflate: str, beg
             continue
         if rc == _cabi.E_CAPACITY:
             min_sites = int(n_sites)
+            if neg_table:  # the entries the table needs (its first capacity is an estimate)
+                need = int(lib.sai_engine_loaded_neg_table(engine._handle(), None, None, None, None, 0))
+                if need < 0:
+                    _cabi.check(need)
+                min_entries = max(min_entries, need)
             continue
         if rc == _cabi.E_CORRUPT:  # read again with host inflate: it raises the host path's error
             inflate = "host"
@@ -183,11 +204,12 @@ def _ingest(engine, vcf_file: str, pops, requests, label: str, inflate: str, beg
 
 
 def read_loaded(engine, vcf_file: str, chr_name: str, plan, requests, out, anc, anc_error, start=None, end=None,
-                with_outgroup: bool = True, inflate: str = "host") -> Optional[LoadedChunk]:
+                with_outgroup: bool = True, inflate: str = "host", neg_table: bool = False) -> Optional[LoadedChunk]:
     """Parses the records of ``chr_name`` (``start <= POS <= end`` when both are given) on the
     device into ``engine``'s resident tiles, one layout for every population of ``plan`` (the
     outgroup only with ``with_outgroup``).  ``None`` when the file has no ``#CHROM`` line.
-    ``inflate="device"``: bgzip blocks are inflated on the device."""
+    ``inflate="device"``: bgzip blocks are inflated on the device.  ``neg_table``: the engine also
+    keeps the negative-value table DD reads (``LoadedChunk.neg``)."""
     lib = _cabi.load()
     pops, groups, index = _pops_and_groups(plan, out, with_outgroup)
     if not pops:
@@ -207,15 +229,15 @@ def read_loaded(engine, vcf_file: str, chr_name: str, plan, requests, out, anc, 
         return rc, n_sites.value, vmax, True
 
     label = chr_name if start is None and end is None else f"{chr_name}:{start}-{end}"
-    lay, pos, _ = _ingest(engine, vcf_file, pops, requests, label, inflate, begin_session, finish_session,
-                          (chr_name, start, end) if (start is not None and end is not None) else None)
+    lay, pos, extra = _ingest(engine, vcf_file, pops, requests, label, inflate, begin_session, finish_session,
+                              (chr_name, start, end) if (start is not None and end is not None) else None, neg_table)
     if pos is None:
         return None
     if anc_error is not None and pos.size:  # records but no ancestral allele in the region: the reference raises
         raise anc_error
     if pos.size == 0:
         groups = {g: (None, v[1]) for g, v in groups.items()}
-    return LoadedChunk(lay, pos, index, groups)
+    return LoadedChunk(lay, pos, index, groups, neg=neg_table and extra is not None)
 
 
 class LoadedGenome:
@@ -223,10 +245,11 @@ class LoadedGenome:
     ``engine``, chromosome ``c``'s sites at ``[first_site[c], first_site[c] + n_sites[c])`` (a tile
     boundary; ``first_site`` -1: no site), ``pos[c]`` its positions.  ``span[c] = (first POS, last POS,
     records)`` in file order over all its records, as ``vcf.chromosome_span`` counts them (``None``:
-    no record).  ``index`` / ``groups`` as ``LoadedChunk``'s."""
+    no record).  ``index`` / ``groups`` / ``neg`` as ``LoadedChunk``'s; chromosome ``c``'s rows of
+    the negative-value table count sites from ``first_site[c]``."""
 
-    def __init__(self, layout, chroms, pos_all, index, groups, names):
-        self.layout, self.index, self.groups, self.names = layout, index, groups, list(names)
+    def __init__(self, layout, chroms, pos_all, index, groups, names, neg=False):
+        self.layout, self.index, self.groups, self.names, self.neg = layout, index, groups, list(names), neg
         self.first_site = [int(c.first_site) for c in chroms]
         self.n_sites = [int(c.n_sites) for c in chroms]
         self.span = [(int(c.first_pos), int(c.last_pos), int(c.n_records)) if c.n_records > 0 else None for c in chroms]
@@ -279,13 +302,13 @@ def genome_tables(chr_names, anc_allele_file):
 
 
 def read_genome(engine, vcf_file: str, chr_names, plan, requests, out, tables, with_outgroup: bool = True,
-                inflate: str = "host"):
+                inflate: str = "host", neg_table: bool = False):
     """Parses every chromosome of ``chr_names`` in one pass over ``vcf_file`` into ``engine``'s
     resident tiles (``sai_engine_vcf_genome_*``).  ``tables`` = ``genome_tables(chr_names, file)``
     (its ``anc`` ``None`` without an ancestral-allele file).  Returns a
     ``LoadedGenome``; ``None`` when the file has no ``#CHROM`` line, no populations are parsed, or a
     chromosome's records resume after another chromosome's (``SAI_E_ORDER``): such files are read
-    one chromosome at a time."""
+    one chromosome at a time.  ``neg_table`` as ``read_loaded``'s."""
     lib = _cabi.load()
     names, name_off, anc = tables
     pops, groups, index = _pops_and_groups(plan, out, with_outgroup)
@@ -309,12 +332,13 @@ def read_genome(engine, vcf_file: str, chr_names, plan, requests, out, tables, w
         return rc, n_sites.value, vmax, chroms
 
     lay, pos, extra = _ingest(engine, vcf_file, pops, requests, ",".join(chr_names), inflate, begin_session,
-                              finish_session)
+                              finish_session, neg_table=neg_table)
     if pos is None or extra == _cabi.E_ORDER:
         return None
+    neg = neg_table and extra is not None
     if extra is None:  # no record line: nothing found
         chroms = (_cabi.VcfChrom * n)(*[_cabi.VcfChrom(0, 0, 0, -1, 0) for _ in range(n)])
-    return LoadedGenome(lay, chroms, pos, index, groups, chr_names)
+    return LoadedGenome(lay, chroms, pos, index, groups, chr_names, neg=neg)
 
 
 def read_region(engine, vcf_file, chr_name, ploidy_config, ref_ind_file, tgt_ind_file, src_ind_file, out_ind_file,
