@@ -317,11 +317,12 @@ __global__ void __launch_bounds__(kSiteWarps * 32, MODE == 1 ? 3 : 4)
 // K1 without stored counts: the staged pass.  A site can be flagged only where its sources match
 // and its reference frequency is below w (site_gate), and the sources are the smallest operand
 // (bench layout: 1 of 80 pairs), so a tile is read in three stages -- the source populations of
-// all jobs, the references of the jobs still live on the tile, the targets of those still live --
-// and each population at most once.  On the bench spectrum 77 % of the tiles stop after the
-// source pair and 4.8x fewer bytes are read.  Decisions are unchanged: a tile that reaches the
-// third stage has every count its live jobs need and runs eval_site_fast as k_site does; a job
-// dead on a tile stores zero mask words (and no qval, which exists only at Q-flagged sites).
+// all jobs, the references of the jobs still live, the targets of those still live -- and each
+// population at most once.  Stages 2 and 3 read a population only at the sites where a job can
+// still hold (gather_sites), unless a tile has more than kGatherSites of them.  Decisions are
+// unchanged: the flags of a job come from eval_site_fast, as in k_site, at the sites that passed
+// its gates; a job dead on a tile stores zero mask words (and no qval, which exists only at
+// Q-flagged sites).
 //
 // A warp claims batches of batch_tiles consecutive tiles from a global counter (live tiles fall at
 // random, and a static tile-to-warp map leaves the busiest warp with ~2x the mean bytes) and reads
@@ -331,6 +332,101 @@ __global__ void __launch_bounds__(kSiteWarps * 32, MODE == 1 ? 3 : 4)
 // slower on the bench job (DESIGN section 4).
 constexpr int kGateTiles = 4;
 constexpr int kGateSmemPerWarp = 6144;  // 48 KB per 8-warp block: 4 blocks per SM
+// A tile with more live sites than this reads the population whole (n_pairs coalesced loads per
+// lane) instead of gathering (per site ceil(n_groups / 32) loads per lane, 32 sectors each).
+constexpr int kGatherSites = 8;
+
+// The B plane words of group g at one site (col: the population's first pair of the tile, as
+// words, plus 2 * site).  Word w of a group sits in pair w >> 1, half w & 1, as in count_wide.
+template <int BMAX>
+__device__ __forceinline__ void group_words(const uint32_t* col, int g, int B, uint32_t (&x)[BMAX]) {
+  if (BMAX == 2) {
+    const uint2 v = ld_stream(reinterpret_cast<const uint2*>(col + (size_t)g * 2 * kTile));
+    x[0] = v.x;
+    x[1] = v.y;
+  } else {
+#pragma unroll
+    for (int b = 0; b < BMAX; ++b) {
+      const int w = g * B + b;
+      if (b < B) x[b] = __ldg(col + (size_t)(w >> 1) * 2 * kTile + (w & 1));
+    }
+  }
+}
+
+// (num, called) of population L at the sites of a batch in lo:hi (bit 32 g + s = site s of tile g),
+// stored into those sites' slots of the shared counts.  Lanes stride over the population's groups;
+// the counts are those of count_wide, summed over the warp:
+//   num = sum_b popc(w_b) << b - (2^B - 1) popc(AND_b w_b),   missing = popc(AND_b w_b)
+// ROUND items and two groups per lane at a time, all their loads issued before any sum (a word
+// not loaded is 0 and adds nothing).  BMAX == 2 for 2-plane populations (one 8-byte load per
+// group), 8 for any other width.
+template <int BMAX, int ROUND>
+__device__ __noinline__ void gather_sites(const sai_pop_layout& L, const uint32_t* batch, int64_t pps,
+                                          uint64_t lo, uint64_t hi, int* s_pop, int per_tile, int n_pops,
+                                          int lane) {
+  const int B = BMAX == 2 ? 2 : L.bits, G = L.n_groups;
+  while (lo | hi) {
+    const uint32_t* col[ROUND];  // the item's population column at its site
+    int item[ROUND];             // 32 tile + site, -1: none
+#pragma unroll
+    for (int i = 0; i < ROUND; ++i) {
+      item[i] = -1;
+      if (lo) {
+        item[i] = __ffsll((long long)lo) - 1;
+        lo &= lo - 1;
+      } else if (hi) {
+        item[i] = 64 + __ffsll((long long)hi) - 1;
+        hi &= hi - 1;
+      }
+      const int it = item[i] < 0 ? item[0] : item[i];  // an empty slot loads nothing
+      col[i] = batch + ((size_t)(it >> 5) * pps + L.pair_off) * 2 * kTile + 2 * (it & 31);
+    }
+    int num[ROUND], miss[ROUND];
+#pragma unroll
+    for (int i = 0; i < ROUND; ++i) num[i] = miss[i] = 0;
+    for (int g = lane; g < G; g += 64) {
+      uint32_t x[2][ROUND][BMAX];
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+#pragma unroll
+        for (int i = 0; i < ROUND; ++i) {
+#pragma unroll
+          for (int b = 0; b < BMAX; ++b) x[h][i][b] = 0u;
+          if (item[i] >= 0 && g + 32 * h < G) group_words<BMAX>(col[i], g + 32 * h, B, x[h][i]);
+        }
+      }
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+#pragma unroll
+        for (int i = 0; i < ROUND; ++i) {
+          uint32_t andw = 0xffffffffu;
+          int s = 0;
+#pragma unroll
+          for (int b = 0; b < BMAX; ++b) {
+            if (b < B) {
+              s += __popc(x[h][i][b]) << b;
+              andw &= x[h][i][b];
+            }
+          }
+          const int m = __popc(andw);
+          num[i] += s - ((1 << B) - 1) * m;
+          miss[i] += m;
+        }
+      }
+    }
+#pragma unroll
+    for (int i = 0; i < ROUND; ++i) {
+      if (item[i] < 0) continue;
+      const int n = __reduce_add_sync(0xffffffffu, num[i]);
+      const int m = __reduce_add_sync(0xffffffffu, miss[i]);
+      if (lane == (item[i] & 31)) {
+        int* slot = s_pop + (item[i] >> 5) * per_tile + lane;
+        slot[0] = n;
+        slot[n_pops * kTile] = G * 32 - m;
+      }
+    }
+  }
+}
 
 __global__ void __launch_bounds__(kSiteWarps * 32, 4)
     k_site_gated(const __grid_constant__ SiteParams P, const __grid_constant__ JobBlock JB,
@@ -388,58 +484,114 @@ __global__ void __launch_bounds__(kSiteWarps * 32, 4)
       }
     }
 
-    for (int g = 0; g < n; ++g) {
-      const int64_t T = P.tile0 + t0 + g;
-      const uint2* tile = batch + (size_t)g * pps * kTile;
-      int* s_num = s_warp + g * per_tile;
-      int* s_cal = s_num + n_pops * kTile;
-      auto num_of = [&](int pop) { return s_num[pop * kTile + lane]; };
-      auto called_of = [&](int pop) { return s_cal[pop * kTile + lane]; };
-      auto read = [&](uint32_t pops) {
-        for (; pops; pops &= pops - 1) {
-          const int pi = __ffs(pops) - 1;
+    // Stages 2 and 3 run over the whole batch.  Per lane, bits 8 g + j of gate / still: job j's
+    // source gate / source and reference gates hold at this lane's site of tile g (SAI_MAX_JOBS
+    // == 8).  The counts of a population are valid at the sites it was read for: the source
+    // populations at every site, a population read in stage 2 at the sites where any job's source
+    // gate holds, one read in stage 3 where any job's reference gate holds too.  Every later use
+    // is within that set -- stage 3 sites are a subset of stage 2 sites, and the flags of job j
+    // are kept only where both its gates hold -- so a population needed by several stages or jobs
+    // is read once, by the first stage that needs it.
+    auto num_of_tile = [&](int g) {
+      return [=](int pop) { return s_warp[g * per_tile + pop * kTile + lane]; };
+    };
+    auto called_of_tile = [&](int g) {
+      return [=](int pop) { return s_warp[g * per_tile + (n_pops + pop) * kTile + lane]; };
+    };
+    auto pops_of = [&](uint32_t jobs, bool ref) {
+      uint32_t pops = 0;
+      for (; jobs; jobs &= jobs - 1) {
+        const sai_job& J = JB.job[__ffs(jobs) - 1];
+        pops |= 1u << (ref ? J.ref_pop : J.tgt_pop);
+      }
+      return pops;
+    };
+    // the sites of tile g where some job of lane_jobs is live
+    auto sites_of = [&](uint32_t lane_jobs, int g) {
+      return __ballot_sync(0xffffffffu, (lane_jobs >> (8 * g)) & 0xffu);
+    };
+    // reads population p of tile g for every bit 16 g + p of need (SAI_MAX_POPS == 16) at the sites
+    // of tile g where some job of lane_jobs is live: a tile with more than kGatherSites such sites
+    // whole, population after population; the others gathered, population by population across
+    // the batch
+    auto read_stage = [&](uint64_t need, uint32_t lane_jobs) {
+      for (int g = 0; g < n; ++g) {
+        if (__popc(sites_of(lane_jobs, g)) <= kGatherSites) continue;
+        for (uint32_t m = (uint32_t)(need >> (16 * g)) & 0xffffu; m; m &= m - 1) {
+          const int pi = __ffs(m) - 1;
           const sai_pop_layout& L = P.lay.pop[pi];
-          count_pop<0>(L, tile + (size_t)L.pair_off * kTile, s_num[pi * kTile + lane], s_cal[pi * kTile + lane]);
+          int* s_num = s_warp + g * per_tile + pi * kTile + lane;
+          count_pop<0>(L, batch + ((size_t)g * pps + L.pair_off) * kTile, s_num[0], s_num[n_pops * kTile]);
         }
-      };
-      // live: jobs whose U or Q can still hold at some site of the tile (warp-uniform)
-      uint32_t live = 0;
+        need &= ~(0xffffull << (16 * g));
+      }
+      uint32_t any = 0;
+      for (uint64_t m = need; m; m >>= 16) any |= (uint32_t)m & 0xffffu;
+      for (; any; any &= any - 1) {
+        const int pi = __ffs(any) - 1;
+        uint64_t lo = 0, hi = 0;  // gathered sites, bit 32 g + s (tiles 0, 1 | 2, 3)
+        for (int g = 0; g < n; ++g)
+          if ((need >> (16 * g + pi)) & 1u) (g < 2 ? lo : hi) |= (uint64_t)sites_of(lane_jobs, g) << (32 * (g & 1));
+        const sai_pop_layout& L = P.lay.pop[pi];
+        const uint32_t* words = reinterpret_cast<const uint32_t*>(batch - lane);
+        if (L.bits == 2)
+          gather_sites<2, 2>(L, words, pps, lo, hi, s_warp + pi * kTile, per_tile, n_pops, lane);
+        else
+          gather_sites<8, 1>(L, words, pps, lo, hi, s_warp + pi * kTile, per_tile, n_pops, lane);
+      }
+    };
+
+    uint32_t gate = 0;
+    for (int g = 0; g < n; ++g) {
       for (int j = 0; j < JB.n_jobs; ++j) {
         bool u, q;
-        site_gate(JF.job[j], JB.job[j], P.lay, false, num_of, called_of, u, q);
-        live |= (uint32_t)(u || q) << j;
+        site_gate(JF.job[j], JB.job[j], P.lay, false, num_of_tile(g), called_of_tile(g), u, q);
+        gate |= (uint32_t)(u || q) << (8 * g + j);
       }
-      live = __reduce_or_sync(0xffffffffu, live);
-      uint32_t have = P.gate_pops;
-      // stage 2: the references of the live jobs, then the reference gate
-      if (live) {
-        uint32_t need = 0;
-        for (uint32_t m = live; m; m &= m - 1) need |= 1u << JB.job[__ffs(m) - 1].ref_pop;
-        read(need & ~have);
-        have |= need;
-        uint32_t still = 0;
-        for (uint32_t m = live; m; m &= m - 1) {
-          const int j = __ffs(m) - 1;
-          bool u, q;
-          site_gate(JF.job[j], JB.job[j], P.lay, true, num_of, called_of, u, q);
-          still |= (uint32_t)(u || q) << j;
-        }
-        live = __reduce_or_sync(0xffffffffu, still);
-      }
-      // stage 3: the targets of the jobs still live
-      if (live) {
-        uint32_t need = 0;
-        for (uint32_t m = live; m; m &= m - 1) need |= 1u << JB.job[__ffs(m) - 1].tgt_pop;
-        read(need & ~have);
-      }
+    }
+    // stage 2: the references of the jobs live on each tile, then the reference gate.  A tile read
+    // whole reads the targets of those jobs with them: on a dense tile they are needed almost
+    // always, and one stage of whole-tile reads keeps the all-live case close to one pass (DESIGN 4).
+    const uint32_t live1 = __reduce_or_sync(0xffffffffu, gate);
+    uint64_t need2 = 0;
+    for (int g = 0; g < n; ++g) {
+      const uint32_t jobs = (live1 >> (8 * g)) & 0xffu;
+      uint32_t pops = pops_of(jobs, true);
+      if (__popc(sites_of(gate, g)) > kGatherSites) pops |= pops_of(jobs, false);
+      need2 |= (uint64_t)(pops & ~P.gate_pops) << (16 * g);
+    }
+    read_stage(need2, gate);
+    uint32_t still = 0;
+    for (uint32_t m = live1; m; m &= m - 1) {
+      const int g = (__ffs(m) - 1) >> 3, j = (__ffs(m) - 1) & 7;
+      bool u, q;
+      site_gate(JF.job[j], JB.job[j], P.lay, true, num_of_tile(g), called_of_tile(g), u, q);
+      still |= (uint32_t)(u || q) << (8 * g + j);
+    }
+    // stage 3: the targets of the jobs still live
+    const uint32_t live2 = __reduce_or_sync(0xffffffffu, still);
+    uint64_t need3 = 0;
+    for (int g = 0; g < n; ++g)
+      need3 |= (uint64_t)(pops_of((live2 >> (8 * g)) & 0xffu, false) & ~P.gate_pops) << (16 * g);
+    read_stage(need3 & ~need2, still);
+
+    for (int g = 0; g < n; ++g) {
+      const int64_t T = P.tile0 + t0 + g;
       const int64_t site = T * kTile + lane;
       for (int j = 0; j < JB.n_jobs; ++j) {
+        const int bit = 8 * g + j;
         uint32_t mu = 0, mq = 0;
-        if ((live >> j) & 1u) {
-          const SiteFlags f = eval_site_fast(JF.job[j], JB.job[j], P.lay, num_of, called_of);
-          mu = __ballot_sync(0xffffffffu, f.u);
-          mq = __ballot_sync(0xffffffffu, f.q);
-          if (f.q) P.qval[(size_t)j * P.qval_stride + site] = f.q_tgt_freq;
+        if ((live2 >> bit) & 1u) {
+          // lanes where job j's gates fail may hold counts never read for this tile: they are
+          // evaluated as fully called sites with a count of 0 (so they keep the warp on the
+          // integer path) and their flags dropped
+          const bool mine = (still >> bit) & 1u;
+          const SiteFlags f = eval_site_fast(
+              JF.job[j], JB.job[j], P.lay, [&](int pop) { return mine ? num_of_tile(g)(pop) : 0; },
+              [&](int pop) { return mine ? called_of_tile(g)(pop) : P.lay.pop[pop].n_samples; });
+          mu = __ballot_sync(0xffffffffu, f.u && mine);
+          mq = __ballot_sync(0xffffffffu, f.q && mine);
+          if (f.q && mine) P.qval[(size_t)j * P.qval_stride + site] = f.q_tgt_freq;
         }
         if (lane == 0) {
           P.mask_u[(size_t)j * P.n_tiles_total + T] = mu;

@@ -4,13 +4,20 @@ CUDA events.  Uses only the public DeviceScorer API, so the same script times an
 
     python tools/k1_gate_bench.py [--sites 6000000] [--reps 50] [--out FILE]
 
-Two jobs on bench.py's data (rank 0's shard):
+Three jobs on bench.py's data (rank 0's shard):
   bench     U + Q of bench.py (src "=1", w = 0.01, ancestral alleles): K1 time, the share of tiles
-            whose reference and target a pass that reads the sources first must read, and the
-            bytes such a pass reads over K1 time.  The shares come from `site_counts` on the same
-            data with the gate predicates in numpy (reporting only, not a correctness check).
+            on which the staged pass reads the reference and the target, and its bytes over K1 time.
+  sparse    src ">= y", w = 0.05, with y the smallest of 1, 7/8, ..., 1/8 for which at most half of
+            the tiles hold a source-live site: many tiles with a few live sites each, the middle of
+            the range between the bench job and the all-live job.
   all_live  src ">= 0", w = 1.0: every tile is live, so every byte is read as by a pass without
             gates; the worst case of the staged pass.
+The shares and bytes come from `site_counts` on the same data with the gate predicates in numpy
+(reporting only, not a correctness check).  Bytes are modelled for the pass as it reads: the source
+pairs of every tile, then per tile the reference at the sites where the source gate holds and the
+target where the reference gate holds too -- gathered (the distinct 32-byte sectors, 4 sites of
+one pair, or 64-byte blocks of 8 sites) at up to GATHER_SITES such sites, the whole tile above.
+`bytes_tile_granular` is the same pass reading every live tile whole.
 Prints the card's name, power limit and maximum SM clock, then one JSON line.
 """
 import argparse
@@ -26,6 +33,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.dont_write_bytecode = True
 from bench import WORKLOAD, make_job_for  # noqa: E402
+
+GATHER_SITES = 8  # kGatherSites, sai_b200/csrc/site_kernels.cu
 
 
 def card() -> str:
@@ -50,17 +59,37 @@ def time_k1(torch, sc, d_packed, job, reps: int, warmup: int = 5):
     return {"median_ms": float(np.median(ms)), "min_ms": float(ms.min()), "max_ms": float(ms.max()), "reps": reps}
 
 
-def gate_shares(num, called, lay, n_sites: int, wl):
-    """Tiles whose reference / target the staged pass reads for bench.py's job (one source, "=" y,
-    ancestral alleles): src_freq == y, then ref_freq < w, in float64 as the kernels decide."""
-    freq = lambda p: np.divide(num[p, :n_sites], called[p, :n_sites] * lay.pop[p].ploidy,
-                               out=np.full(n_sites, np.nan), where=called[p, :n_sites] > 0)
-    assert wl["y"][0] == "=" and wl["anc"]
-    src = freq(2) == wl["y"][1]
-    ref = src & (freq(0) < wl["w"])
+def freqs(num, called, lay, n_sites: int):
+    return [np.divide(num[p, :n_sites], called[p, :n_sites] * lay.pop[p].ploidy, out=np.full(n_sites, np.nan),
+                      where=called[p, :n_sites] > 0) for p in range(3)]
+
+
+def gates(f, op: str, y: float, w: float):
+    """Per site: the source gate, and the source + reference gates, of a one-source job with
+    ancestral alleles (src 2, ref 0), in float64 as the kernels decide."""
+    src = {"=": f[2] == y, ">=": f[2] >= y}[op]
+    return src, src & (f[0] < w)
+
+
+def pass_model(src, ref, lay, n_sites: int):
+    """Tile shares and modelled bytes of the staged pass for the per-site gate masks src, ref."""
     n_tiles = (n_sites + 31) // 32
-    tiles = lambda m: np.pad(m, (0, n_tiles * 32 - n_sites)).reshape(n_tiles, 32).any(1)
-    return float(tiles(src).mean()), float(tiles(ref).mean()), float(src.mean()), float(ref.mean())
+    tiles = lambda m: np.pad(m, (0, n_tiles * 32 - n_sites)).reshape(n_tiles, 32)
+    pair_bytes = [256 * lay.pop[p].n_pairs for p in range(3)]  # per tile: ref, tgt, src
+    out = {"tiles_reading_ref": float(tiles(src).any(1).mean()), "tiles_reading_tgt": float(tiles(ref).any(1).mean()),
+           "sites_src_pass": float(src.mean()), "sites_src_ref_pass": float(ref.mean())}
+    tile_gran = n_tiles * pair_bytes[2]
+    model = {32: tile_gran, 64: tile_gran}
+    for pop, m in ((0, tiles(src)), (1, tiles(ref))):
+        live = m.sum(1)
+        tile_gran += int((live > 0).sum()) * pair_bytes[pop]
+        whole = int((live > GATHER_SITES).sum()) * pair_bytes[pop]
+        g = m[(live > 0) & (live <= GATHER_SITES)]
+        for sector in (32, 64):
+            blocks = int(g.reshape(g.shape[0], 32 * 8 // sector, sector // 8).any(2).sum())
+            model[sector] += whole + blocks * lay.pop[pop].n_pairs * sector
+    out.update(bytes_read=int(model[32]), bytes_read_64B=int(model[64]), bytes_tile_granular=int(tile_gran))
+    return out
 
 
 def main():
@@ -90,21 +119,30 @@ def main():
     full_bytes = n_tiles * sum(pair_bytes)
 
     num, called = (t.cpu().numpy() for t in sc.site_counts(d_packed))
-    tile_ref, tile_tgt, site_src, site_ref = gate_shares(num, called, lay, S, wl)
-    gated_bytes = n_tiles * (pair_bytes[2] + tile_ref * pair_bytes[0] + tile_tgt * pair_bytes[1])
+    f = freqs(num, called, lay, S)
+    n_tiles = sc.n_tiles
+    full_bytes = n_tiles * sum(256 * lay.pop[p].n_pairs for p in range(3))
+    assert wl["y"][0] == "=" and wl["anc"]
+    bench_model = pass_model(*gates(f, "=", wl["y"][1], wl["w"]), lay, S)
+    sparse_y = next(y / 8 for y in range(8, 0, -1)
+                    if pass_model(*gates(f, ">=", (y - 1) / 8, 0.05), lay, S)["tiles_reading_ref"] > 0.5 or y == 1)
+    sparse_model = pass_model(*gates(f, ">=", sparse_y, 0.05), lay, S)
 
     bench = time_k1(torch, sc, d_packed, make_job_for(wl), args.reps)
+    sparse_job = make_job(0, 1, [2], wl["anc"], u=dict(w=0.05, x=wl["x"], y_list=[(">=", sparse_y)]),
+                          q=dict(w=0.05, quantile=wl["quantile"], y_list=[(">=", sparse_y)]))
+    sparse = time_k1(torch, sc, d_packed, sparse_job, args.reps)
     all_live_job = make_job(0, 1, [2], wl["anc"], u=dict(w=1.0, x=wl["x"], y_list=[(">=", 0.0)]),
                             q=dict(w=1.0, quantile=wl["quantile"], y_list=[(">=", 0.0)]))
     all_live = time_k1(torch, sc, d_packed, all_live_job, args.reps)
 
-    bench.update(tiles_reading_ref=tile_ref, tiles_reading_tgt=tile_tgt, sites_src_pass=site_src,
-                 sites_src_ref_pass=site_ref, bytes_read=int(gated_bytes),
-                 tb_s_bytes_read=gated_bytes / (bench["median_ms"] / 1e3) / 1e12,
-                 tb_s_all_bytes=full_bytes / (bench["median_ms"] / 1e3) / 1e12)
+    for r, model in ((bench, bench_model), (sparse, sparse_model)):
+        r.update(model, tb_s_bytes_read=model["bytes_read"] / (r["median_ms"] / 1e3) / 1e12,
+                 tb_s_all_bytes=full_bytes / (r["median_ms"] / 1e3) / 1e12)
+    sparse["src_y"] = sparse_y
     all_live.update(bytes_read=int(full_bytes), tb_s_bytes_read=full_bytes / (all_live["median_ms"] / 1e3) / 1e12)
     line = json.dumps({"sites": S, "tiles": n_tiles, "card": card().splitlines()[-1], "bench": bench,
-                       "all_live": all_live})
+                       "sparse": sparse, "all_live": all_live})
     print(line)
     if args.out:
         with open(args.out, "w") as f:
