@@ -184,7 +184,7 @@ __device__ __forceinline__ SiteFlags eval_site_fast(const JobFast& F, const sai_
 }
 
 // ---------------------------------------------------------------------------
-// Gates of the staged genotype pass (k_site_gated).  A site is flagged only if its sources
+// Gates of the staged genotype pass (k_site_live).  A site is flagged only if its sources
 // match (op(src_freq, y), or op(src_freq, 1 - y) without ancestral alleles) and its possibly
 // inverted ref_freq < w, so the pass reads the sources first and the reference and target only
 // where a job can still hold.  Each factor below is evaluated per lane exactly as eval_site /

@@ -249,6 +249,16 @@ void build_job_fast(const sai_layout& lay, const sai_job& J, JobFast& F) {
   F.ok = 1;
 }
 
+// k_site_scan's test of one job: a necessary condition of its source gate (site_gate with
+// with_ref == false) on its first source alone.  Where that population is fully called
+// (called * ploidy == den) the gate needs its count in one of the n intervals [lo, hi] -- the y and,
+// without ancestral alleles, 1 - y intervals of the enabled U / Q conditions; anywhere else the
+// site counts as live.
+struct ScanTest {
+  int32_t pop, den, n;
+  int32_t lo[4], hi[4];
+};
+
 struct SiteParams {
   sai_layout lay;
   const uint2* packed;  // tile 0
@@ -260,10 +270,15 @@ struct SiteParams {
   int32_t* num;
   int32_t* called;
   int64_t count_stride;
-  // k_site_gated only
-  unsigned long long* next_batch;  // batch counter, zero at launch
-  uint32_t gate_pops;              // populations that are a source of a job with U or Q enabled
-  int32_t batch_tiles;             // tiles per batch, 1..kGateTiles
+  // staged pass only (k_site_scan, k_site_live)
+  unsigned long long* counters;  // [0] queue length, [1] batches claimed; zero at launch
+  int32_t* queue;                // [n_tiles] live tiles (relative to tile0), in no particular order
+  uint32_t gate_pops;            // populations that are a source of a job with U or Q enabled
+  int32_t batch_tiles;           // live tiles per batch of k_site_live, 1..kGateTiles
+  uint32_t scan_pops;            // populations k_site_scan reads: the first source of each job in scan[]
+  int32_t scan_all;              // some job can be live at any site: every tile is queued, nothing read
+  int32_t n_scan;
+  ScanTest scan[SAI_MAX_JOBS];   // jobs with U or Q enabled and integer intervals
 };
 
 constexpr int kSiteWarps = 8;
@@ -324,17 +339,148 @@ __global__ void __launch_bounds__(kSiteWarps * 32, MODE == 1 ? 3 : 4)
 // its gates; a job dead on a tile stores zero mask words (and no qval, which exists only at
 // Q-flagged sites).
 //
-// A warp claims batches of batch_tiles consecutive tiles from a global counter (live tiles fall at
-// random, and a static tile-to-warp map leaves the busiest warp with ~2x the mean bytes) and reads
-// the source pairs of the whole batch at once, so a 1-pair source still has one load per tile in
-// flight.  Shared memory holds the counts of every tile of the batch: [warp][tile][2][n_pops][32].
-// 4 tiles per batch: on one B200, 8 was slower on both the bench job and the all-live job, and 2
-// slower on the bench job (DESIGN section 4).
+// Two kernels.  k_site_scan reads the first source of every job at every tile and tests it against
+// interval bounds the host computes in advance (ScanTest, a necessary condition of the source gate):
+// a tile where no job can be live gets its zero mask words there, any other is appended to a queue.
+// k_site_live runs the three stages on the queued tiles only.  Most tiles are dead (bench data: 77 %) and a live one usually holds a single live site, so
+// batching consecutive tiles paid a batch's whole chain of dependent DRAM round trips for about one
+// site; batching queued tiles gives each round trip several live tiles' worth of gathers.
+//
+// Live tiles fall at random and their cost varies, so k_site_live's warps claim batches of
+// batch_tiles queue entries from a counter (a static map leaves the busiest warp with ~2x the mean).
+// Shared memory holds the counts of every tile of a batch: [warp][tile][2][n_pops][32].
 constexpr int kGateTiles = 4;
-constexpr int kGateSmemPerWarp = 6144;  // 48 KB per 8-warp block: 4 blocks per SM
+constexpr int kScanTiles = 8;
+constexpr int kGateSmemPerWarp = 6144;  // bounds a batch's shared counts: 4 blocks per SM at any n_pops
 // A tile with more live sites than this reads the population whole (n_pairs coalesced loads per
 // lane) instead of gathering (per site ceil(n_groups / 32) loads per lane, 32 sectors each).
 constexpr int kGatherSites = 8;
+
+// Stage 1: (num, called) of the gate populations at this lane's site of n tiles into the counts of
+// each tile.  tile(g) is tile g's first pair at this lane's site and is called by the whole warp.
+// 2 planes: pair by pair across the tiles, n loads in flight per lane; other widths tile by tile.
+template <int NT, typename TileFn>
+__device__ __forceinline__ void count_sources(const SiteParams& P, int n, TileFn tile, int* s_warp, int per_tile,
+                                              int lane) {
+  const int n_pops = P.lay.n_pops;
+  for (uint32_t m = P.gate_pops; m; m &= m - 1) {
+    const int pi = __ffs(m) - 1;
+    const sai_pop_layout& L = P.lay.pop[pi];
+    int* s_num = s_warp + pi * kTile + lane;
+    int* s_cal = s_num + n_pops * kTile;
+    if (L.bits == 2) {
+      int num[NT], miss[NT];
+#pragma unroll
+      for (int g = 0; g < NT; ++g) num[g] = miss[g] = 0;
+      for (int i = 0; i < L.n_pairs; ++i) {
+        uint2 v[NT];
+#pragma unroll
+        for (int g = 0; g < NT; ++g)
+          v[g] = g < n ? ld_stream(tile(g) + (size_t)(L.pair_off + i) * kTile) : make_uint2(0u, 0u);
+#pragma unroll
+        for (int g = 0; g < NT; ++g) {
+          const int mm = __popc(v[g].x & v[g].y);
+          num[g] += __popc(v[g].x) + 2 * __popc(v[g].y) - 3 * mm;
+          miss[g] += mm;
+        }
+      }
+#pragma unroll
+      for (int g = 0; g < NT; ++g) {
+        if (g < n) {
+          s_num[g * per_tile] = num[g];
+          s_cal[g * per_tile] = L.n_groups * 32 - miss[g];
+        }
+      }
+    } else {
+      for (int g = 0; g < n; ++g)
+        count_pop<0>(L, tile(g) + (size_t)L.pair_off * kTile, s_num[g * per_tile], s_cal[g * per_tile]);
+    }
+  }
+}
+
+// Phase A over tiles [tile0, tile0 + n_tiles): one warp takes 32 consecutive tiles per trip, in
+// steps of kScanTiles tiles whose loads are in flight together.  Per step and lane, the counts of
+// each population in scan_pops at its site of every tile stay in registers, and bit g of site_live
+// says whether the ScanTest of some job holds at this lane's site of tile g; a warp-wide OR of it
+// gives the tiles of the step that may be live.  Lane g then owns tile g of the trip: it stores the
+// tile's zero mask words (32 tiles = one 128-byte store per array and job) or its queue entry, with
+// one atomic per trip reserving the trip's entries.  The tests only ever queue a superset of the
+// live tiles: k_site_live decides every queued tile exactly, so a tile queued for nothing stores
+// zero mask words there.  WIDE: some scanned population has more than two planes (count_pop, whose
+// inlined counters need more than 64 registers); otherwise one popcount path for 2-plane groups.
+template <bool WIDE>
+__global__ void __launch_bounds__(kSiteWarps * 32, WIDE ? 3 : 4)
+    k_site_scan(const __grid_constant__ SiteParams P, const __grid_constant__ JobBlock JB) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t pps = P.lay.pairs_per_site;
+  for (int64_t t0 = ((int64_t)blockIdx.x * kSiteWarps + warp) * kTile; t0 < P.n_tiles;
+       t0 += (int64_t)gridDim.x * kSiteWarps * kTile) {
+    const int n = (int)(P.n_tiles - t0 < kTile ? P.n_tiles - t0 : kTile);
+    uint32_t live = P.scan_all ? 0xffffffffu : 0u;  // bit g: a job may be live at a site of tile t0 + g
+    for (int s0 = 0; s0 < n && !P.scan_all; s0 += kScanTiles) {
+      const int ns = n - s0 < kScanTiles ? n - s0 : kScanTiles;
+      const uint2* first = P.packed + (size_t)(P.tile0 + t0 + s0) * pps * kTile + lane;
+      uint32_t site_live = 0;
+      for (uint32_t m = P.scan_pops; m; m &= m - 1) {
+        const int pi = __ffs(m) - 1;
+        const sai_pop_layout& L = P.lay.pop[pi];
+        int num[kScanTiles], called[kScanTiles];
+        if (WIDE) {
+#pragma unroll
+          for (int g = 0; g < kScanTiles; ++g) {
+            num[g] = called[g] = 0;
+            if (g < ns) count_pop<0>(L, first + ((size_t)g * pps + L.pair_off) * kTile, num[g], called[g]);
+          }
+        } else {
+          int miss[kScanTiles];
+#pragma unroll
+          for (int g = 0; g < kScanTiles; ++g) num[g] = miss[g] = 0;
+          for (int i = 0; i < L.n_pairs; ++i) {
+            uint2 v[kScanTiles];
+#pragma unroll
+            for (int g = 0; g < kScanTiles; ++g)
+              v[g] = g < ns ? ld_stream(first + ((size_t)g * pps + L.pair_off + i) * kTile) : make_uint2(0u, 0u);
+#pragma unroll
+            for (int g = 0; g < kScanTiles; ++g) {
+              const int mm = __popc(v[g].x & v[g].y);
+              num[g] += __popc(v[g].x) + 2 * __popc(v[g].y) - 3 * mm;
+              miss[g] += mm;
+            }
+          }
+#pragma unroll
+          for (int g = 0; g < kScanTiles; ++g) called[g] = L.n_groups * 32 - miss[g];
+        }
+        for (int j = 0; j < P.n_scan; ++j) {
+          const ScanTest& T = P.scan[j];
+          if (T.pop != pi) continue;
+#pragma unroll
+          for (int g = 0; g < kScanTiles; ++g) {
+            bool ok = called[g] * L.ploidy != T.den;
+#pragma unroll
+            for (int i = 0; i < 4; ++i) ok = ok || (i < T.n && num[g] >= T.lo[i] && num[g] <= T.hi[i]);
+            site_live |= (uint32_t)ok << g;
+          }
+        }
+      }
+      live |= (__reduce_or_sync(0xffffffffu, site_live) & ((1u << ns) - 1u)) << s0;
+    }
+    unsigned long long at = 0;
+    if (lane == 0 && (live & (n == kTile ? 0xffffffffu : (1u << n) - 1u)))
+      at = atomicAdd(P.counters, (unsigned long long)__popc(live & (n == kTile ? 0xffffffffu : (1u << n) - 1u)));
+    at = __shfl_sync(0xffffffffu, at, 0);
+    if (lane < n) {
+      if ((live >> lane) & 1u) {
+        P.queue[at + __popc(live & ((1u << lane) - 1u))] = (int32_t)(t0 + lane);
+      } else {
+        const int64_t T = P.tile0 + t0 + lane;
+        for (int j = 0; j < JB.n_jobs; ++j) {
+          P.mask_u[(size_t)j * P.n_tiles_total + T] = 0u;
+          P.mask_q[(size_t)j * P.n_tiles_total + T] = 0u;
+        }
+      }
+    }
+  }
+}
 
 // The B plane words of group g at one site (col: the population's first pair of the tile, as
 // words, plus 2 * site).  Word w of a group sits in pair w >> 1, half w & 1, as in count_wide.
@@ -353,16 +499,16 @@ __device__ __forceinline__ void group_words(const uint32_t* col, int g, int B, u
   }
 }
 
-// (num, called) of population L at the sites of a batch in lo:hi (bit 32 g + s = site s of tile g),
-// stored into those sites' slots of the shared counts.  Lanes stride over the population's groups;
-// the counts are those of count_wide, summed over the warp:
+// (num, called) of population L at the sites of a batch in lo:hi (bit 32 g + s = site s of tile g,
+// whose index lane g holds in my_tile), stored into those sites' slots of the shared counts.  Lanes
+// stride over the population's groups; the counts are those of count_wide, summed over the warp:
 //   num = sum_b popc(w_b) << b - (2^B - 1) popc(AND_b w_b),   missing = popc(AND_b w_b)
 // ROUND items and two groups per lane at a time, all their loads issued before any sum (a word
 // not loaded is 0 and adds nothing).  BMAX == 2 for 2-plane populations (one 8-byte load per
 // group), 8 for any other width.
 template <int BMAX, int ROUND>
-__device__ __noinline__ void gather_sites(const sai_pop_layout& L, const uint32_t* batch, int64_t pps,
-                                          uint64_t lo, uint64_t hi, int* s_pop, int per_tile, int n_pops,
+__device__ __noinline__ void gather_sites(const sai_pop_layout& L, const uint32_t* packed, int64_t my_tile,
+                                          int64_t pps, uint64_t lo, uint64_t hi, int* s_pop, int per_tile, int n_pops,
                                           int lane) {
   const int B = BMAX == 2 ? 2 : L.bits, G = L.n_groups;
   while (lo | hi) {
@@ -379,7 +525,8 @@ __device__ __noinline__ void gather_sites(const sai_pop_layout& L, const uint32_
         hi &= hi - 1;
       }
       const int it = item[i] < 0 ? item[0] : item[i];  // an empty slot loads nothing
-      col[i] = batch + ((size_t)(it >> 5) * pps + L.pair_off) * 2 * kTile + 2 * (it & 31);
+      const int64_t T = __shfl_sync(0xffffffffu, (long long)my_tile, it >> 5);
+      col[i] = packed + ((size_t)T * pps + L.pair_off) * 2 * kTile + 2 * (it & 31);
     }
     int num[ROUND], miss[ROUND];
 #pragma unroll
@@ -428,61 +575,37 @@ __device__ __noinline__ void gather_sites(const sai_pop_layout& L, const uint32_
   }
 }
 
+// Phase B: the three stages over batches of batch_tiles queued tiles.  Lane g holds the index of
+// the batch's tile g; the next batch's entries are loaded while this batch's stages 2 and 3 run.
 __global__ void __launch_bounds__(kSiteWarps * 32, 4)
-    k_site_gated(const __grid_constant__ SiteParams P, const __grid_constant__ JobBlock JB,
-                 const __grid_constant__ JobFastBlock JF) {
+    k_site_live(const __grid_constant__ SiteParams P, const __grid_constant__ JobBlock JB,
+                const __grid_constant__ JobFastBlock JF) {
   extern __shared__ int s_counts[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n_pops = P.lay.n_pops, G = P.batch_tiles;
   const int per_tile = 2 * n_pops * kTile;
   int* s_warp = s_counts + warp * G * per_tile;
   const int64_t pps = P.lay.pairs_per_site;
-  const int64_t n_batches = (P.n_tiles + G - 1) / G;
+  const int64_t n_live = (int64_t)P.counters[0];
+  const int64_t n_batches = (n_live + G - 1) / G;
   // lane 0 claims; the claim of the next batch is in flight while this one is read
-  auto claim = [&]() { return lane == 0 ? atomicAdd(P.next_batch, 1ull) : 0ull; };
-  unsigned long long claimed = claim();
-  for (int64_t b = (int64_t)__shfl_sync(0xffffffffu, claimed, 0); b < n_batches;
-       b = (int64_t)__shfl_sync(0xffffffffu, claimed, 0)) {
-    claimed = claim();
-    const int64_t t0 = b * G;
-    const int n = (int)(P.n_tiles - t0 < G ? P.n_tiles - t0 : G);
-    const uint2* batch = P.packed + (size_t)(P.tile0 + t0) * pps * kTile + lane;
+  auto claim = [&]() { return lane == 0 ? atomicAdd(P.counters + 1, 1ull) : 0ull; };
+  auto tiles_of = [&](int64_t b) {  // lane g: tile g of batch b (lanes past its end repeat its first)
+    const int64_t e = b * G + lane;
+    return P.tile0 + P.queue[lane < G && e < n_live ? e : b * G];
+  };
+  int64_t b = (int64_t)__shfl_sync(0xffffffffu, claim(), 0);
+  int64_t my_tile = b < n_batches ? tiles_of(b) : 0;
+  while (b < n_batches) {
+    const unsigned long long claimed = claim();
+    const int n = (int)(n_live - b * G < G ? n_live - b * G : G);
+    auto tile_at = [&](int g) {  // tile g's first pair at this lane's site
+      return P.packed + (size_t)__shfl_sync(0xffffffffu, (long long)my_tile, g) * pps * kTile + lane;
+    };
 
-    // stage 1: the source populations of the n tiles.  2 planes: pair by pair across the batch,
-    // n loads in flight per lane; other widths tile by tile.
-    for (uint32_t m = P.gate_pops; m; m &= m - 1) {
-      const int pi = __ffs(m) - 1;
-      const sai_pop_layout& L = P.lay.pop[pi];
-      int* s_num = s_warp + pi * kTile + lane;
-      int* s_cal = s_num + n_pops * kTile;
-      if (L.bits == 2) {
-        int num[kGateTiles], miss[kGateTiles];
-#pragma unroll
-        for (int g = 0; g < kGateTiles; ++g) num[g] = miss[g] = 0;
-        for (int i = 0; i < L.n_pairs; ++i) {
-          uint2 v[kGateTiles];
-#pragma unroll
-          for (int g = 0; g < kGateTiles; ++g)
-            v[g] = g < n ? ld_stream(batch + ((size_t)g * pps + L.pair_off + i) * kTile) : make_uint2(0u, 0u);
-#pragma unroll
-          for (int g = 0; g < kGateTiles; ++g) {
-            const int mm = __popc(v[g].x & v[g].y);
-            num[g] += __popc(v[g].x) + 2 * __popc(v[g].y) - 3 * mm;
-            miss[g] += mm;
-          }
-        }
-#pragma unroll
-        for (int g = 0; g < kGateTiles; ++g) {
-          if (g < n) {
-            s_num[g * per_tile] = num[g];
-            s_cal[g * per_tile] = L.n_groups * 32 - miss[g];
-          }
-        }
-      } else {
-        for (int g = 0; g < n; ++g)
-          count_pop<0>(L, batch + ((size_t)g * pps + L.pair_off) * kTile, s_num[g * per_tile], s_cal[g * per_tile]);
-      }
-    }
+    count_sources<kGateTiles>(P, n, tile_at, s_warp, per_tile, lane);
+    const int64_t next_b = (int64_t)__shfl_sync(0xffffffffu, claimed, 0);
+    const int64_t next_tile = next_b < n_batches ? tiles_of(next_b) : 0;
 
     // Stages 2 and 3 run over the whole batch.  Per lane, bits 8 g + j of gate / still: job j's
     // source gate / source and reference gates hold at this lane's site of tile g (SAI_MAX_JOBS
@@ -521,7 +644,7 @@ __global__ void __launch_bounds__(kSiteWarps * 32, 4)
           const int pi = __ffs(m) - 1;
           const sai_pop_layout& L = P.lay.pop[pi];
           int* s_num = s_warp + g * per_tile + pi * kTile + lane;
-          count_pop<0>(L, batch + ((size_t)g * pps + L.pair_off) * kTile, s_num[0], s_num[n_pops * kTile]);
+          count_pop<0>(L, tile_at(g) + (size_t)L.pair_off * kTile, s_num[0], s_num[n_pops * kTile]);
         }
         need &= ~(0xffffull << (16 * g));
       }
@@ -533,11 +656,11 @@ __global__ void __launch_bounds__(kSiteWarps * 32, 4)
         for (int g = 0; g < n; ++g)
           if ((need >> (16 * g + pi)) & 1u) (g < 2 ? lo : hi) |= (uint64_t)sites_of(lane_jobs, g) << (32 * (g & 1));
         const sai_pop_layout& L = P.lay.pop[pi];
-        const uint32_t* words = reinterpret_cast<const uint32_t*>(batch - lane);
+        const uint32_t* words = reinterpret_cast<const uint32_t*>(P.packed);
         if (L.bits == 2)
-          gather_sites<2, 2>(L, words, pps, lo, hi, s_warp + pi * kTile, per_tile, n_pops, lane);
+          gather_sites<2, 2>(L, words, my_tile, pps, lo, hi, s_warp + pi * kTile, per_tile, n_pops, lane);
         else
-          gather_sites<8, 1>(L, words, pps, lo, hi, s_warp + pi * kTile, per_tile, n_pops, lane);
+          gather_sites<8, 1>(L, words, my_tile, pps, lo, hi, s_warp + pi * kTile, per_tile, n_pops, lane);
       }
     };
 
@@ -576,7 +699,7 @@ __global__ void __launch_bounds__(kSiteWarps * 32, 4)
     read_stage(need3 & ~need2, still);
 
     for (int g = 0; g < n; ++g) {
-      const int64_t T = P.tile0 + t0 + g;
+      const int64_t T = __shfl_sync(0xffffffffu, (long long)my_tile, g);
       const int64_t site = T * kTile + lane;
       for (int j = 0; j < JB.n_jobs; ++j) {
         const int bit = 8 * g + j;
@@ -599,6 +722,8 @@ __global__ void __launch_bounds__(kSiteWarps * 32, 4)
         }
       }
     }
+    b = next_b;
+    my_tile = next_tile;
   }
 }
 
@@ -715,30 +840,64 @@ static int launch_site(const SiteParams& P, const JobBlock& JB, cudaStream_t st)
 
 static int launch_site_gated(SiteParams P, const JobBlock& JB, cudaStream_t st) {
   if (P.n_tiles == 0) return SAI_OK;
+  SAI_REQUIRE(P.n_tiles <= INT32_MAX, "too many tiles for one genotype pass (%lld)", (long long)P.n_tiles);
   P.gate_pops = 0;
   for (int j = 0; j < JB.n_jobs; ++j) {
     const sai_job& J = JB.job[j];
     if (J.u.enabled || J.q.enabled)
       for (int k = 0; k < J.n_src; ++k) P.gate_pops |= 1u << J.src_pop[k];
   }
-  const int tile_bytes = 2 * P.lay.n_pops * kTile * (int)sizeof(int);
-  P.batch_tiles = std::max(1, std::min(kGateTiles, kGateSmemPerWarp / tile_bytes));
-  const size_t smem = (size_t)kSiteWarps * P.batch_tiles * tile_bytes;
-  int occ = 0;
-  SAI_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_site_gated, kSiteWarps * 32, smem));
-  if (occ < 1) occ = 1;
-  const int64_t n_batches = (P.n_tiles + P.batch_tiles - 1) / P.batch_tiles;
-  const int64_t want = (n_batches + kSiteWarps - 1) / kSiteWarps;
-  const int64_t cap = (int64_t)sm_count() * occ;
   JobFastBlock JF;
   fill_job_fast(P.lay, JB, JF);
-  void* counter = nullptr;
-  if (int rc = scratch_alloc(&counter, sizeof(unsigned long long), st)) return rc;
-  P.next_batch = static_cast<unsigned long long*>(counter);
-  SAI_CUDA_CHECK(cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
-  k_site_gated<<<(int)(want < cap ? want : cap), kSiteWarps * 32, smem, st>>>(P, JB, JF);
+  P.scan_pops = 0;
+  P.scan_all = 0;
+  P.n_scan = 0;
+  bool wide = false;
+  for (int j = 0; j < JB.n_jobs; ++j) {
+    const sai_job& J = JB.job[j];
+    const JobFast& F = JF.job[j];
+    if (!(J.u.enabled || J.q.enabled)) continue;
+    if (!F.ok) {  // no integer intervals: the gate is decided by divisions only
+      P.scan_all = 1;
+      continue;
+    }
+    ScanTest& T = P.scan[P.n_scan++];
+    T.pop = J.src_pop[0];
+    T.den = F.den_src[0];
+    T.n = 0;
+    const CondFast* cf[2] = {&F.u, &F.q};
+    const bool en[2] = {J.u.enabled != 0, J.q.enabled != 0};
+    for (int c = 0; c < 2; ++c) {
+      if (!en[c]) continue;
+      T.lo[T.n] = cf[c]->y_lo[0], T.hi[T.n++] = cf[c]->y_hi[0];
+      if (!J.anc_allele_available) T.lo[T.n] = cf[c]->f_lo[0], T.hi[T.n++] = cf[c]->f_hi[0];
+    }
+    P.scan_pops |= 1u << T.pop;
+    wide = wide || P.lay.pop[T.pop].bits != 2;
+  }
+  const int tile_bytes = 2 * P.lay.n_pops * kTile * (int)sizeof(int);
+  P.batch_tiles = std::max(1, std::min(kGateTiles, kGateSmemPerWarp / tile_bytes));
+  const size_t smem_live = (size_t)kSiteWarps * P.batch_tiles * tile_bytes;
+  auto scan = wide ? k_site_scan<true> : k_site_scan<false>;
+  int occ_scan = 0, occ_live = 0;
+  SAI_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_scan, scan, kSiteWarps * 32, 0));
+  SAI_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_live, k_site_live, kSiteWarps * 32, smem_live));
+  const int64_t want_scan = (P.n_tiles + kSiteWarps * kTile - 1) / (kSiteWarps * kTile);
+  const int64_t want_live = ((P.n_tiles + P.batch_tiles - 1) / P.batch_tiles + kSiteWarps - 1) / kSiteWarps;
+  const int64_t cap_scan = (int64_t)sm_count() * std::max(occ_scan, 1);
+  const int64_t cap_live = (int64_t)sm_count() * std::max(occ_live, 1);
+  // counters, then the queue
+  void* scratch = nullptr;
+  if (int rc = scratch_alloc(&scratch, 2 * sizeof(unsigned long long) + (size_t)P.n_tiles * sizeof(int32_t), st))
+    return rc;
+  P.counters = static_cast<unsigned long long*>(scratch);
+  P.queue = reinterpret_cast<int32_t*>(P.counters + 2);
+  SAI_CUDA_CHECK(cudaMemsetAsync(scratch, 0, 2 * sizeof(unsigned long long), st));
+  scan<<<(int)std::min(want_scan, cap_scan), kSiteWarps * 32, 0, st>>>(P, JB);
   SAI_CUDA_CHECK(cudaGetLastError());
-  return scratch_free(counter, st);
+  k_site_live<<<(int)std::min(want_live, cap_live), kSiteWarps * 32, smem_live, st>>>(P, JB, JF);
+  SAI_CUDA_CHECK(cudaGetLastError());
+  return scratch_free(scratch, st);
 }
 
 

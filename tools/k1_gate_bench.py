@@ -2,7 +2,7 @@
 """K1 alone (the genotype pass, `DeviceScorer.site_flags`) at bench.py's layout and size, timed with
 CUDA events.  Uses only the public DeviceScorer API, so the same script times an older tree too.
 
-    python tools/k1_gate_bench.py [--sites 6000000] [--reps 50] [--out FILE]
+    python tools/k1_gate_bench.py [--sites 6000000] [--reps 50] [--out FILE] [--profile]
 
 Three jobs on bench.py's data (rank 0's shard):
   bench     U + Q of bench.py (src "=1", w = 0.01, ancestral alleles): K1 time, the share of tiles
@@ -17,7 +17,10 @@ The shares and bytes come from `site_counts` on the same data with the gate pred
 pairs of every tile, then per tile the reference at the sites where the source gate holds and the
 target where the reference gate holds too -- gathered (the distinct 32-byte sectors, 4 sites of
 one pair, or 64-byte blocks of 8 sites) at up to GATHER_SITES such sites, the whole tile above.
-`bytes_tile_granular` is the same pass reading every live tile whole.
+`bytes_tile_granular` is the same pass reading every live tile whole.  `live_tiles` is the number of
+tiles where the source gate holds at some site: the tiles on which the pass reads more than the sources.
+--profile times nothing with events; it runs each job under torch.profiler (CUDA activities) and
+reports the mean device time per launch of each kernel and memset of the pass (`split`).
 Prints the card's name, power limit and maximum SM clock, then one JSON line.
 """
 import argparse
@@ -59,6 +62,27 @@ def time_k1(torch, sc, d_packed, job, reps: int, warmup: int = 5):
     return {"median_ms": float(np.median(ms)), "min_ms": float(ms.min()), "max_ms": float(ms.max()), "reps": reps}
 
 
+def split_k1(torch, sc, d_packed, job, reps: int):
+    """Mean device time per K1 call of each kernel / memset it launches, from torch.profiler."""
+    from torch.profiler import ProfilerActivity, profile
+
+    for _ in range(5):
+        sc.site_flags(d_packed, [job])
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            sc.site_flags(d_packed, [job])
+        torch.cuda.synchronize()
+    out = {}
+    for e in prof.key_averages():
+        if e.device_type.name == "CUDA" and e.count > 0:
+            us = getattr(e, "device_time_total", None)
+            if us is None:
+                us = e.cuda_time_total
+            out[e.key[:60]] = {"us_per_call": us / reps, "launches_per_call": e.count / reps}
+    return out
+
+
 def freqs(num, called, lay, n_sites: int):
     return [np.divide(num[p, :n_sites], called[p, :n_sites] * lay.pop[p].ploidy, out=np.full(n_sites, np.nan),
                       where=called[p, :n_sites] > 0) for p in range(3)]
@@ -76,7 +100,8 @@ def pass_model(src, ref, lay, n_sites: int):
     n_tiles = (n_sites + 31) // 32
     tiles = lambda m: np.pad(m, (0, n_tiles * 32 - n_sites)).reshape(n_tiles, 32)
     pair_bytes = [256 * lay.pop[p].n_pairs for p in range(3)]  # per tile: ref, tgt, src
-    out = {"tiles_reading_ref": float(tiles(src).any(1).mean()), "tiles_reading_tgt": float(tiles(ref).any(1).mean()),
+    out = {"live_tiles": int(tiles(src).any(1).sum()),
+           "tiles_reading_ref": float(tiles(src).any(1).mean()), "tiles_reading_tgt": float(tiles(ref).any(1).mean()),
            "sites_src_pass": float(src.mean()), "sites_src_ref_pass": float(ref.mean())}
     tile_gran = n_tiles * pair_bytes[2]
     model = {32: tile_gran, 64: tile_gran}
@@ -97,6 +122,7 @@ def main():
     ap.add_argument("--sites", type=int, default=WORKLOAD["n_sites"])
     ap.add_argument("--reps", type=int, default=50)
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
+    ap.add_argument("--profile", action="store_true", help="per-kernel split from torch.profiler instead of events")
     args = ap.parse_args()
 
     import torch
@@ -128,19 +154,24 @@ def main():
                     if pass_model(*gates(f, ">=", (y - 1) / 8, 0.05), lay, S)["tiles_reading_ref"] > 0.5 or y == 1)
     sparse_model = pass_model(*gates(f, ">=", sparse_y, 0.05), lay, S)
 
-    bench = time_k1(torch, sc, d_packed, make_job_for(wl), args.reps)
+    timer = (lambda *a: {"split": split_k1(*a)}) if args.profile else time_k1
+    bench = timer(torch, sc, d_packed, make_job_for(wl), args.reps)
     sparse_job = make_job(0, 1, [2], wl["anc"], u=dict(w=0.05, x=wl["x"], y_list=[(">=", sparse_y)]),
                           q=dict(w=0.05, quantile=wl["quantile"], y_list=[(">=", sparse_y)]))
-    sparse = time_k1(torch, sc, d_packed, sparse_job, args.reps)
+    sparse = timer(torch, sc, d_packed, sparse_job, args.reps)
     all_live_job = make_job(0, 1, [2], wl["anc"], u=dict(w=1.0, x=wl["x"], y_list=[(">=", 0.0)]),
                             q=dict(w=1.0, quantile=wl["quantile"], y_list=[(">=", 0.0)]))
-    all_live = time_k1(torch, sc, d_packed, all_live_job, args.reps)
+    all_live = timer(torch, sc, d_packed, all_live_job, args.reps)
 
     for r, model in ((bench, bench_model), (sparse, sparse_model)):
-        r.update(model, tb_s_bytes_read=model["bytes_read"] / (r["median_ms"] / 1e3) / 1e12,
-                 tb_s_all_bytes=full_bytes / (r["median_ms"] / 1e3) / 1e12)
+        r.update(model)
+        if not args.profile:
+            r.update(tb_s_bytes_read=model["bytes_read"] / (r["median_ms"] / 1e3) / 1e12,
+                     tb_s_all_bytes=full_bytes / (r["median_ms"] / 1e3) / 1e12)
     sparse["src_y"] = sparse_y
-    all_live.update(bytes_read=int(full_bytes), tb_s_bytes_read=full_bytes / (all_live["median_ms"] / 1e3) / 1e12)
+    all_live.update(bytes_read=int(full_bytes), live_tiles=int(n_tiles))
+    if not args.profile:
+        all_live.update(tb_s_bytes_read=full_bytes / (all_live["median_ms"] / 1e3) / 1e12)
     line = json.dumps({"sites": S, "tiles": n_tiles, "card": card().splitlines()[-1], "bench": bench,
                        "sparse": sparse, "all_live": all_live})
     print(line)
