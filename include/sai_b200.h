@@ -544,13 +544,18 @@ int sai_engine_rescore_windows(sai_engine* e, sai_host_results* out);
 /* Site-pattern sums (see sai_window_patterns) for the chunk of the last
  * sai_engine_score_host call, whose packed tiles, positions and windows are
  * still resident on the device: runs the counting genotype pass + the pattern
- * kernel and copies sums[n_src][W][7] to the host. */
+ * kernel and copies sums[n_src][W][7] to the host.  The pattern kernel runs once per piece
+ * (sai_engine_score_loaded_pieces), a piece's window i landing at sums[k][w0 + i] for its first
+ * window w0; a chunk scored whole is the one piece of W windows from window 0 and all sites from
+ * site 0.  The DD sums below walk the pieces the same way. */
 int sai_engine_pattern_sums(sai_engine* e, const sai_layout* lay, int32_t ref_pop, int32_t tgt_pop,
                             int32_t out_pop, const int32_t* src_pops, int32_t n_src, double* sums);
 
 /* DD sums (see sai_window_dd) for the chunk of the last sai_engine_score_host call; the
- * negative-value table is HOST memory.  Fails with SAI_E_ARG when the table does not cover
- * every missing call of ref_pop / tgt_pop / the source populations.
+ * negative-value table is HOST memory, one row of offsets (neg_off[n_pops + 1]), copied to the
+ * device per call.  The chunk is one piece (see sai_engine_pattern_sums); tiles scored in pieces
+ * are refused (sai_engine_dd_sums_loaded takes them).  Fails with SAI_E_ARG when the table does not
+ * cover every missing call of ref_pop / tgt_pop / the source populations.
  * ref_sum / tgt_sum: host, [n_src][W][m_max]. */
 int sai_engine_dd_sums(sai_engine* e, const sai_layout* lay, int32_t ref_pop, int32_t tgt_pop,
                        const int32_t* src_pops, int32_t n_src, const int64_t* neg_off,
@@ -667,10 +672,11 @@ int sai_engine_score_loaded_pieces(sai_engine* e, const int64_t* win_start, cons
  * [n_chrom][n_pops + 1]) is always written; the entries only when cap >= their number.  Returns that
  * number (after SAI_E_CAPACITY: the number a repeat needs) or a negative SAI_E_* code.
  * sai_engine_dd_sums_loaded: sai_engine_dd_sums on the resident tiles and the resident table (no copy
- * to the device) after sai_engine_score_loaded or _score_loaded_pieces; with pieces one sai_site_hist +
- * sai_window_dd per piece (a chromosome of the session), its results at ref_sum[k][w0 + i] as
- * sai_engine_pattern_sums places them.  Fails with SAI_E_ARG when a population's missing calls and its
- * table entries differ. */
+ * to the device) after sai_engine_score_loaded or _score_loaded_pieces: one sai_site_hist +
+ * sai_window_dd per piece (see sai_engine_pattern_sums), which must be a chromosome of the session and
+ * reads that chromosome's row of the table (a single-chromosome session: its one row), its results at
+ * ref_sum[k][w0 + i].  Fails with SAI_E_ARG when a population's missing calls and its table entries
+ * differ. */
 int sai_engine_set_vcf_neg_table(sai_engine* e, int32_t on, int64_t min_entries);
 int64_t sai_engine_loaded_neg_table(sai_engine* e, int64_t* neg_off, int32_t* site, int32_t* ind, int32_t* val,
                                     int64_t cap);

@@ -200,6 +200,13 @@ static ResLayout res_layout(int64_t W, int n_jobs) {
   return r;
 }
 
+// The pieces the resident tiles were scored in: those of sai_engine_score_loaded_pieces, or one chunk as
+// the one piece (0, W, 0, n_sites).
+static std::vector<std::array<int64_t, 4>> scored_pieces(const sai_engine* e) {
+  if (!e->pieces.empty()) return e->pieces;
+  return {{0, e->W, 0, e->n_sites}};
+}
+
 // Window kernel on the device-resident flags + results back to the host.
 static int run_windows(sai_engine* e, sai_host_results* out) {
   const int64_t W = e->W;
@@ -739,24 +746,98 @@ int sai_engine_pattern_sums(sai_engine* e, const sai_layout* lay, int32_t ref_po
   const int64_t* d_ws = static_cast<const int64_t*>(e->win.p);
   const int32_t* d_pos = static_cast<const int32_t*>(e->pos.p);
   double* d_sums = static_cast<double*>(e->sums.p);
-  if (e->pieces.empty()) {
-    if (int rc = sai_window_patterns(lay, d_pos, e->n_sites, d_ws, d_ws + W, W, d_num, d_called, stride, ref_pop, tgt_pop,
-                                     out_pop, src_pops, n_src, d_sums, e->s_comp))
+  // one sai_window_patterns per piece on its sites and counts; sums[k][w0 + i] <- piece's [k][i]
+  for (const auto& P : scored_pieces(e)) {
+    const int64_t w0 = P[0], nw = P[1], lo = P[2];
+    if (nw == 0) continue;
+    double* d_p = d_sums + 7 * (size_t)n_src * w0;
+    if (int rc = sai_window_patterns(lay, d_pos + lo, P[3], d_ws + w0, d_ws + W + w0, nw, d_num + lo, d_called + lo,
+                                     stride, ref_pop, tgt_pop, out_pop, src_pops, n_src, d_p, e->s_comp))
       return rc;
-    SAI_CUDA_CHECK(cudaMemcpyAsync(sums, d_sums, sizeof(double) * 7 * (size_t)n_src * W, cudaMemcpyDeviceToHost, e->s_comp));
-  } else {  // one sai_window_patterns per piece on its sites and counts; sums[k][w0 + i] <- piece's [k][i]
-    for (const auto& P : e->pieces) {
-      const int64_t w0 = P[0], nw = P[1], lo = P[2];
-      if (nw == 0) continue;
-      double* d_p = d_sums + 7 * (size_t)n_src * w0;
-      if (int rc = sai_window_patterns(lay, d_pos + lo, P[3], d_ws + w0, d_ws + W + w0, nw, d_num + lo, d_called + lo,
-                                       stride, ref_pop, tgt_pop, out_pop, src_pops, n_src, d_p, e->s_comp))
-        return rc;
-      SAI_CUDA_CHECK(cudaMemcpy2DAsync(sums + 7 * w0, sizeof(double) * 7 * W, d_p, sizeof(double) * 7 * nw,
-                                       sizeof(double) * 7 * nw, n_src, cudaMemcpyDeviceToHost, e->s_comp));
-    }
+    SAI_CUDA_CHECK(cudaMemcpy2DAsync(sums + 7 * w0, sizeof(double) * 7 * W, d_p, sizeof(double) * 7 * nw,
+                                     sizeof(double) * 7 * nw, n_src, cudaMemcpyDeviceToHost, e->s_comp));
   }
   SAI_CUDA_CHECK(cudaStreamSynchronize(e->s_comp));
+  return SAI_OK;
+}
+
+// DD sums of both entry points over the pieces of the resident tiles.  P[j] = (first window, windows,
+// first site, sites, row): the piece's entries of the negative-value table (d_ns / d_ni / d_nv, device)
+// are those of offsets row `row` of neg_off ([rows][n_pops + 1], host), their sites counted from the
+// piece's first site; row -1: a piece without sites, which has no entries.
+static int dd_sums_impl(sai_engine* e, const sai_layout* lay, int32_t ref_pop, int32_t tgt_pop, const int32_t* src_pops,
+                        int32_t n_src, int32_t m_max, const int32_t* d_ns, const int32_t* d_ni, const int32_t* d_nv,
+                        const int64_t* neg_off, const std::vector<std::array<int64_t, 5>>& P, int64_t* ref_sum,
+                        int64_t* tgt_sum) {
+  const int n_pops = lay->n_pops;
+  SAI_REQUIRE(ref_pop >= 0 && ref_pop < n_pops && tgt_pop >= 0 && tgt_pop < n_pops, "bad population index");
+  SAI_REQUIRE(m_max >= 1, "m_max must be positive");
+  SAI_REQUIRE(n_src <= SAI_MAX_SRC, "n_src %d outside [1,%d]", n_src, SAI_MAX_SRC);
+  const int64_t W = e->W;
+  if (W == 0 || n_src <= 0) return SAI_OK;
+  // histograms of ref and tgt (what the distance kernels read) and, behind them, of the source
+  // populations: only their missing-call totals are used, to check the table against the tiles
+  int32_t hp[2 + SAI_MAX_SRC] = {ref_pop, tgt_pop};
+  for (int k = 0; k < n_src; ++k) {
+    SAI_REQUIRE(src_pops[k] >= 0 && src_pops[k] < n_pops, "bad source population index");
+    hp[2 + k] = src_pops[k];
+  }
+  const int n_hp = 2 + n_src;
+  int64_t max_stride = kTile;
+  for (const auto& q : P) max_stride = std::max(max_stride, sai_num_tiles(q[3]) * kTile);
+  const int64_t rows = sai_hist_rows(lay, hp, n_hp);
+  const size_t out_n = (size_t)n_src * W * m_max;
+  // [hist rows][uint64 missing totals per piece][int32 err] share the hist buffer
+  const size_t hist_bytes = align256(sizeof(int32_t) * (size_t)rows * max_stride);
+  if (int rc = grow(e->hist, hist_bytes + sizeof(uint64_t) * n_hp * P.size() + 256)) return rc;
+  if (int rc = grow(e->dd, sizeof(int64_t) * 2 * out_n + 512)) return rc;
+  cudaStream_t st = e->s_comp;
+  int32_t* d_hist = static_cast<int32_t*>(e->hist.p);
+  uint64_t* d_missing = reinterpret_cast<uint64_t*>(static_cast<char*>(e->hist.p) + hist_bytes);
+  int32_t* d_err = reinterpret_cast<int32_t*>(d_missing + n_hp * P.size());
+  int64_t* d_r = static_cast<int64_t*>(e->dd.p);
+  int64_t* d_t = d_r + out_n;
+  // a piece without sites leaves its missing totals untouched (sai_site_hist returns early): zero all of them
+  SAI_CUDA_CHECK(cudaMemsetAsync(d_missing, 0, sizeof(uint64_t) * n_hp * P.size() + sizeof(int32_t), st));
+  SAI_CUDA_CHECK(cudaMemsetAsync(d_r, 0, sizeof(int64_t) * 2 * out_n, st));
+  const int64_t* d_ws = static_cast<const int64_t*>(e->win.p);
+  const int32_t* d_pos = static_cast<const int32_t*>(e->pos.p);
+  std::vector<int64_t> off((size_t)n_pops + 1);
+  for (size_t j = 0; j < P.size(); ++j) {
+    const int64_t w0 = P[j][0], nw = P[j][1], lo = P[j][2], n = P[j][3], c = P[j][4];
+    if (nw == 0) continue;
+    const int64_t base = c >= 0 ? neg_off[(size_t)c * (n_pops + 1)] : 0;
+    for (int p = 0; p <= n_pops; ++p) off[p] = c >= 0 ? neg_off[(size_t)c * (n_pops + 1) + p] - base : 0;
+    const void* packed = static_cast<const char*>(e->packed.p) + (size_t)(lo / kTile) * lay->pairs_per_site * kTile * 8;
+    const int64_t stride = sai_num_tiles(n) * kTile;
+    if (int rc = sai_site_hist(lay, packed, n, hp, n_hp, d_hist, stride, d_missing + n_hp * j, st)) return rc;
+    int64_t* r = d_r + (size_t)n_src * m_max * w0;
+    int64_t* t = d_t + (size_t)n_src * m_max * w0;
+    if (int rc = sai_window_dd(lay, packed, d_pos + lo, n, d_ws + w0, d_ws + W + w0, nw, d_hist, stride, ref_pop, tgt_pop,
+                               src_pops, n_src, off.data(), d_ns + base, d_ni + base, d_nv + base, r, t, m_max, d_err, st))
+      return rc;
+    const size_t row = sizeof(int64_t) * (size_t)nw * m_max, pitch = sizeof(int64_t) * (size_t)W * m_max;
+    SAI_CUDA_CHECK(cudaMemcpy2DAsync(ref_sum + w0 * m_max, pitch, r, row, row, n_src, cudaMemcpyDeviceToHost, st));
+    SAI_CUDA_CHECK(cudaMemcpy2DAsync(tgt_sum + w0 * m_max, pitch, t, row, row, n_src, cudaMemcpyDeviceToHost, st));
+  }
+  std::vector<uint64_t> h_missing((size_t)n_hp * P.size());
+  int32_t h_err = 0;
+  SAI_CUDA_CHECK(cudaMemcpyAsync(h_missing.data(), d_missing, sizeof(uint64_t) * h_missing.size(), cudaMemcpyDeviceToHost, st));
+  SAI_CUDA_CHECK(cudaMemcpyAsync(&h_err, d_err, sizeof(h_err), cudaMemcpyDeviceToHost, st));
+  SAI_CUDA_CHECK(cudaStreamSynchronize(st));
+  // the bit-planes keep one missing code: every missing call needs its raw value in the table
+  for (size_t j = 0; j < P.size(); ++j) {
+    const int64_t c = P[j][4];
+    if (P[j][1] == 0) continue;
+    for (int q = 0; q < n_hp; ++q) {
+      const size_t o = (size_t)c * (n_pops + 1) + hp[q];
+      const int64_t have = c >= 0 ? neg_off[o + 1] - neg_off[o] : 0;
+      SAI_REQUIRE((int64_t)h_missing[n_hp * j + q] == have,
+                  "population %d has %lld missing calls but %lld entries in the negative-value table", hp[q],
+                  (long long)h_missing[n_hp * j + q], (long long)have);
+    }
+  }
+  SAI_REQUIRE(h_err == 0, "a missing source call has no entry in the negative-value table");
   return SAI_OK;
 }
 
@@ -767,71 +848,22 @@ int sai_engine_dd_sums(sai_engine* e, const sai_layout* lay, int32_t ref_pop, in
   SAI_REQUIRE(e && e->n_jobs > 0, "no previous sai_engine_score_host call");
   SAI_REQUIRE(ref_sum && tgt_sum && src_pops && neg_off, "NULL argument");
   if (int rc = validate_layout(lay)) return rc;
-  SAI_REQUIRE(ref_pop >= 0 && ref_pop < lay->n_pops && tgt_pop >= 0 && tgt_pop < lay->n_pops,
-              "bad population index");
-  SAI_REQUIRE(m_max >= 1, "m_max must be positive");
   SAI_REQUIRE(e->pieces.empty(), "sai_engine_dd_sums: the resident tiles are scored in pieces");
-  SAI_CUDA_CHECK(cudaSetDevice(e->device));
-  const int64_t n_tiles = sai_num_tiles(e->n_sites);
-  const int64_t stride = n_tiles * kTile;
-  const int64_t W = e->W;
-  if (W == 0 || n_src <= 0) return SAI_OK;
   const int64_t n_neg = neg_off[lay->n_pops];
   SAI_REQUIRE(n_neg >= 0 && (n_neg == 0 || (neg_site && neg_ind && neg_val)), "bad negative-value table");
-  // histograms of ref and tgt (what the distance kernels read) and, behind them, of the source
-  // populations: only their missing-call totals are used, to check the table against the tiles
-  SAI_REQUIRE(n_src <= SAI_MAX_SRC, "n_src %d outside [1,%d]", n_src, SAI_MAX_SRC);
-  int32_t hp[2 + SAI_MAX_SRC] = {ref_pop, tgt_pop};
-  for (int k = 0; k < n_src; ++k) {
-    SAI_REQUIRE(src_pops[k] >= 0 && src_pops[k] < lay->n_pops, "bad source population index");
-    hp[2 + k] = src_pops[k];
-  }
-  const int n_hp = 2 + n_src;
-  const int64_t rows = sai_hist_rows(lay, hp, n_hp);
-  const size_t out_n = (size_t)n_src * W * m_max;
-  if (int rc = grow(e->hist, sizeof(int32_t) * (size_t)rows * stride + 512)) return rc;
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
   if (int rc = grow(e->neg, sizeof(int32_t) * 3 * (size_t)n_neg + 256)) return rc;
-  if (int rc = grow(e->dd, sizeof(int64_t) * 2 * out_n + 512)) return rc;
-  cudaStream_t st = e->s_comp;
-  // [hist rows][uint64 missing totals][int32 err] share the hist buffer's tail
-  int32_t* d_hist = static_cast<int32_t*>(e->hist.p);
-  uint64_t* d_missing = reinterpret_cast<uint64_t*>(
-      static_cast<char*>(e->hist.p) + align256(sizeof(int32_t) * (size_t)rows * stride));
-  int32_t* d_err = reinterpret_cast<int32_t*>(d_missing + n_hp);
   int32_t* d_ns = static_cast<int32_t*>(e->neg.p);
   int32_t* d_ni = d_ns + n_neg;
   int32_t* d_nv = d_ni + n_neg;
   if (n_neg > 0) {
-    SAI_CUDA_CHECK(cudaMemcpyAsync(d_ns, neg_site, sizeof(int32_t) * n_neg, cudaMemcpyHostToDevice, st));
-    SAI_CUDA_CHECK(cudaMemcpyAsync(d_ni, neg_ind, sizeof(int32_t) * n_neg, cudaMemcpyHostToDevice, st));
-    SAI_CUDA_CHECK(cudaMemcpyAsync(d_nv, neg_val, sizeof(int32_t) * n_neg, cudaMemcpyHostToDevice, st));
+    SAI_CUDA_CHECK(cudaMemcpyAsync(d_ns, neg_site, sizeof(int32_t) * n_neg, cudaMemcpyHostToDevice, e->s_comp));
+    SAI_CUDA_CHECK(cudaMemcpyAsync(d_ni, neg_ind, sizeof(int32_t) * n_neg, cudaMemcpyHostToDevice, e->s_comp));
+    SAI_CUDA_CHECK(cudaMemcpyAsync(d_nv, neg_val, sizeof(int32_t) * n_neg, cudaMemcpyHostToDevice, e->s_comp));
   }
-  SAI_CUDA_CHECK(cudaMemsetAsync(d_err, 0, sizeof(int32_t), st));
-  if (int rc = sai_site_hist(lay, e->packed.p, e->n_sites, hp, n_hp, d_hist, stride, d_missing, st)) return rc;
-  int64_t* d_r = static_cast<int64_t*>(e->dd.p);
-  int64_t* d_t = d_r + out_n;
-  SAI_CUDA_CHECK(cudaMemsetAsync(d_r, 0, sizeof(int64_t) * 2 * out_n, st));
-  const int64_t* d_ws = static_cast<const int64_t*>(e->win.p);
-  if (int rc = sai_window_dd(lay, e->packed.p, static_cast<const int32_t*>(e->pos.p), e->n_sites, d_ws, d_ws + W,
-                             W, d_hist, stride, ref_pop, tgt_pop, src_pops, n_src, neg_off, d_ns, d_ni, d_nv,
-                             d_r, d_t, m_max, d_err, st))
-    return rc;
-  uint64_t h_missing[2 + SAI_MAX_SRC] = {0};
-  int32_t h_err = 0;
-  SAI_CUDA_CHECK(cudaMemcpyAsync(ref_sum, d_r, sizeof(int64_t) * out_n, cudaMemcpyDeviceToHost, st));
-  SAI_CUDA_CHECK(cudaMemcpyAsync(tgt_sum, d_t, sizeof(int64_t) * out_n, cudaMemcpyDeviceToHost, st));
-  SAI_CUDA_CHECK(cudaMemcpyAsync(h_missing, d_missing, sizeof(uint64_t) * n_hp, cudaMemcpyDeviceToHost, st));
-  SAI_CUDA_CHECK(cudaMemcpyAsync(&h_err, d_err, sizeof(h_err), cudaMemcpyDeviceToHost, st));
-  SAI_CUDA_CHECK(cudaStreamSynchronize(st));
-  // the bit-planes keep one missing code: every missing call needs its raw value in the table
-  for (int q = 0; q < n_hp; ++q) {
-    const int64_t have = neg_off[hp[q] + 1] - neg_off[hp[q]];
-    SAI_REQUIRE((int64_t)h_missing[q] == have,
-                "population %d has %lld missing calls but %lld entries in the negative-value table", hp[q],
-                (long long)h_missing[q], (long long)have);
-  }
-  SAI_REQUIRE(h_err == 0, "a missing source call has no entry in the negative-value table");
-  return SAI_OK;
+  const auto q = scored_pieces(e)[0];  // the chunk is one piece, its entries the table's only row
+  return dd_sums_impl(e, lay, ref_pop, tgt_pop, src_pops, n_src, m_max, d_ns, d_ni, d_nv, neg_off,
+                      {{q[0], q[1], q[2], q[3], 0}}, ref_sum, tgt_sum);
 }
 
 int sai_engine_score_resident(sai_engine* e, const sai_job* jobs, int32_t n_jobs, sai_host_results* out) {
@@ -1800,94 +1832,25 @@ int sai_engine_dd_sums_loaded(sai_engine* e, int32_t ref_pop, int32_t tgt_pop, c
   SAI_REQUIRE(ref_sum && tgt_sum && src_pops, "NULL argument");
   auto& V = e->vcf;
   SAI_REQUIRE(V.neg, "sai_engine_dd_sums_loaded: the ingest session kept no negative-value table");
-  const sai_layout* lay = &e->lay;
-  SAI_REQUIRE(ref_pop >= 0 && ref_pop < lay->n_pops && tgt_pop >= 0 && tgt_pop < lay->n_pops, "bad population index");
-  SAI_REQUIRE(m_max >= 1, "m_max must be positive");
-  SAI_REQUIRE(n_src <= SAI_MAX_SRC, "n_src %d outside [1,%d]", n_src, SAI_MAX_SRC);
-  const int64_t W = e->W;
-  if (W == 0 || n_src <= 0) return SAI_OK;
-  SAI_CUDA_CHECK(cudaSetDevice(e->device));
-  const int n_pops = lay->n_pops;
-  // (first window, windows, first site, sites, chromosome) per piece: a genome session's piece is the
-  // chromosome whose sites it covers, the table's sites are chromosome-local
+  SAI_REQUIRE(!e->pieces.empty() || !V.genome || V.gq.n_chrom == 1,
+              "sai_engine_dd_sums_loaded: a genome session is scored in pieces");
+  // each piece's row of the table: a genome session's piece is the chromosome whose sites it covers
+  // (the table's sites are chromosome-local); one chunk is the only row
   std::vector<std::array<int64_t, 5>> P;
-  if (e->pieces.empty()) {
-    SAI_REQUIRE(!V.genome || V.gq.n_chrom == 1, "sai_engine_dd_sums_loaded: a genome session is scored in pieces");
-    P.push_back({0, W, 0, e->n_sites, 0});
-  }
-  for (const auto& q : e->pieces) {
-    int64_t c = -1;
+  for (const auto& q : scored_pieces(e)) {
+    int64_t c = e->pieces.empty() ? 0 : -1;
     for (size_t k = 0; k < V.chrom_sites.size() && c < 0; ++k)
       if (V.chrom_sites[k][0] == q[2] && V.chrom_sites[k][1] == q[3]) c = (int64_t)k;
     SAI_REQUIRE(c >= 0 || q[3] == 0, "sai_engine_dd_sums_loaded: piece at site %lld (%lld sites) is not a chromosome",
                 (long long)q[2], (long long)q[3]);
     P.push_back({q[0], q[1], q[2], q[3], c});
   }
-  int32_t hp[2 + SAI_MAX_SRC] = {ref_pop, tgt_pop};
-  for (int k = 0; k < n_src; ++k) {
-    SAI_REQUIRE(src_pops[k] >= 0 && src_pops[k] < n_pops, "bad source population index");
-    hp[2 + k] = src_pops[k];
-  }
-  const int n_hp = 2 + n_src;
-  int64_t max_stride = kTile;
-  for (const auto& q : P) max_stride = std::max(max_stride, sai_num_tiles(q[3]) * kTile);
-  const int64_t rows = sai_hist_rows(lay, hp, n_hp);
-  const size_t out_n = (size_t)n_src * W * m_max;
-  const size_t hist_bytes = align256(sizeof(int32_t) * (size_t)rows * max_stride);
-  if (int rc = grow(e->hist, hist_bytes + sizeof(uint64_t) * n_hp * P.size() + 256)) return rc;
-  if (int rc = grow(e->dd, sizeof(int64_t) * 2 * out_n + 512)) return rc;
-  cudaStream_t st = e->s_comp;
-  int32_t* d_hist = static_cast<int32_t*>(e->hist.p);
-  uint64_t* d_missing = reinterpret_cast<uint64_t*>(static_cast<char*>(e->hist.p) + hist_bytes);
-  int32_t* d_err = reinterpret_cast<int32_t*>(d_missing + n_hp * P.size());
-  int64_t* d_r = static_cast<int64_t*>(e->dd.p);
-  int64_t* d_t = d_r + out_n;
-  // a piece without sites leaves its missing totals untouched (sai_site_hist returns early): zero all of them
-  SAI_CUDA_CHECK(cudaMemsetAsync(d_missing, 0, sizeof(uint64_t) * n_hp * P.size() + sizeof(int32_t), st));
-  SAI_CUDA_CHECK(cudaMemsetAsync(d_r, 0, sizeof(int64_t) * 2 * out_n, st));
-  const int64_t* d_ws = static_cast<const int64_t*>(e->win.p);
-  const int32_t* d_pos = static_cast<const int32_t*>(e->pos.p);
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
   const size_t part = align256(sizeof(int32_t) * (size_t)std::max<int64_t>(V.neg_n, 1));
-  const int32_t* d_ns = static_cast<const int32_t*>(e->vnegt.p);
-  const int32_t* d_ni = reinterpret_cast<const int32_t*>(static_cast<const char*>(e->vnegt.p) + part);
-  const int32_t* d_nv = reinterpret_cast<const int32_t*>(static_cast<const char*>(e->vnegt.p) + 2 * part);
-  std::vector<int64_t> off((size_t)n_pops + 1);
-  for (size_t j = 0; j < P.size(); ++j) {
-    const int64_t w0 = P[j][0], nw = P[j][1], lo = P[j][2], n = P[j][3], c = P[j][4];
-    if (nw == 0) continue;
-    const int64_t base = c >= 0 ? V.neg_off[(size_t)c * (n_pops + 1)] : 0;
-    for (int p = 0; p <= n_pops; ++p) off[p] = c >= 0 ? V.neg_off[(size_t)c * (n_pops + 1) + p] - base : 0;
-    const void* packed = static_cast<const char*>(e->packed.p) + (size_t)(lo / kTile) * lay->pairs_per_site * kTile * 8;
-    const int64_t stride = sai_num_tiles(n) * kTile;
-    if (int rc = sai_site_hist(lay, packed, n, hp, n_hp, d_hist, stride, d_missing + n_hp * j, st)) return rc;
-    int64_t* r = d_r + (size_t)n_src * m_max * w0;
-    int64_t* t = d_t + (size_t)n_src * m_max * w0;
-    if (int rc = sai_window_dd(lay, packed, d_pos + lo, n, d_ws + w0, d_ws + W + w0, nw, d_hist, stride, ref_pop, tgt_pop,
-                               src_pops, n_src, off.data(), d_ns + base, d_ni + base, d_nv + base, r, t, m_max, d_err, st))
-      return rc;
-    const size_t row = sizeof(int64_t) * (size_t)nw * m_max, pitch = sizeof(int64_t) * (size_t)W * m_max;
-    SAI_CUDA_CHECK(cudaMemcpy2DAsync(ref_sum + w0 * m_max, pitch, r, row, row, n_src, cudaMemcpyDeviceToHost, st));
-    SAI_CUDA_CHECK(cudaMemcpy2DAsync(tgt_sum + w0 * m_max, pitch, t, row, row, n_src, cudaMemcpyDeviceToHost, st));
-  }
-  std::vector<uint64_t> h_missing((size_t)n_hp * P.size());
-  int32_t h_err = 0;
-  SAI_CUDA_CHECK(cudaMemcpyAsync(h_missing.data(), d_missing, sizeof(uint64_t) * h_missing.size(), cudaMemcpyDeviceToHost, st));
-  SAI_CUDA_CHECK(cudaMemcpyAsync(&h_err, d_err, sizeof(h_err), cudaMemcpyDeviceToHost, st));
-  SAI_CUDA_CHECK(cudaStreamSynchronize(st));
-  // the bit-planes keep one missing code: every missing call needs its raw value in the table
-  for (size_t j = 0; j < P.size(); ++j) {
-    const int64_t c = P[j][4];
-    if (P[j][1] == 0) continue;
-    for (int q = 0; q < n_hp; ++q) {
-      const size_t o = (size_t)c * (n_pops + 1) + hp[q];
-      const int64_t have = c >= 0 ? V.neg_off[o + 1] - V.neg_off[o] : 0;
-      SAI_REQUIRE((int64_t)h_missing[n_hp * j + q] == have,
-                  "population %d has %lld missing calls but %lld entries in the negative-value table", hp[q],
-                  (long long)h_missing[n_hp * j + q], (long long)have);
-    }
-  }
-  SAI_REQUIRE(h_err == 0, "a missing source call has no entry in the negative-value table");
-  return SAI_OK;
+  const char* t = static_cast<const char*>(e->vnegt.p);
+  return dd_sums_impl(e, &e->lay, ref_pop, tgt_pop, src_pops, n_src, m_max, reinterpret_cast<const int32_t*>(t),
+                      reinterpret_cast<const int32_t*>(t + part), reinterpret_cast<const int32_t*>(t + 2 * part),
+                      V.neg_off.data(), P, ref_sum, tgt_sum);
 }
 
 }  // extern "C"

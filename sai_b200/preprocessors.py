@@ -171,12 +171,18 @@ def score_populations(
             dd_vals = dd_values(ref_sum, tgt_sum, n_ref, n_tgt, n_srcs)
         return four_vals, dd_vals
 
-    if loaded is not None and hasattr(loaded, "first_site"):  # a LoadedGenome
+    use_out = bool(out_data) and bool(four)
+
+    # ---- populations parsed on the device, resident in `engine`: one chunk, or a genome in pieces ----
+    if loaded is not None:
         win_lists = next(iter(windows_by_tgt.values()))
-        pieces = [(w, max(f, 0), n) for w, f, n in zip(win_lists, loaded.first_site, loaded.n_sites)]
-        at = np.cumsum([0] + [len(w) for w in win_lists]).tolist()
+        if hasattr(loaded, "first_site"):  # a LoadedGenome: one piece per chromosome
+            chroms = list(zip(loaded.names, win_lists, loaded.pos))
+            pieces = [(w, max(f, 0), n) for w, f, n in zip(win_lists, loaded.first_site, loaded.n_sites)]
+        else:
+            chroms, pieces = [(chr_name, win_lists, loaded.pos)], None
+        at = np.cumsum([0] + [len(w) for _, w, _ in chroms]).tolist()
         index, n_of = loaded.index, lambda i: int(loaded.layout.pop[i].n_samples)
-        use_out = bool(out_data) and bool(four)
         batches = []
         for b0 in range(0, len(combos), _cabi.MAX_JOBS):
             batch = combos[b0 : b0 + _cabi.MAX_JOBS]
@@ -184,7 +190,12 @@ def score_populations(
             for r, t, sc, _ in batch:
                 src_ploidy_list(len(sc))  # same check as the host path
                 jobs.append(job_for(r, t, index[("ref", r)], index[("tgt", t)], [index[("src", s)] for s in sc]))
-            res = engine.score_loaded_pieces(pieces, jobs) if b0 == 0 else engine.score_resident(jobs)
+            if b0 > 0:
+                res = engine.score_resident(jobs)
+            elif pieces is None:
+                res = engine.score_loaded(win_lists, jobs)
+            else:
+                res = engine.score_loaded_pieces(pieces, jobs)
             four_by_job = []
             for r, t, sc, o in batch:
                 src_idx = [index[("src", s)] for s in sc]
@@ -192,19 +203,18 @@ def score_populations(
                                           index[("out", o)] if (use_out and o is not None) else -1,
                                           n_of(index[("ref", r)]), n_of(index[("tgt", t)]), [n_of(i) for i in src_idx]))
             batches.append((batch, res, four_by_job))
-        for c, chrom in enumerate(loaded.names):
+        for (chrom, windows, pos), a in zip(chroms, at):
             for batch, res, four_by_job in batches:
                 for j, combo in enumerate(batch):
-                    emit(combo, win_lists[c], loaded.pos[c], res, j, *four_by_job[j], chrom=chrom, at=at[c])
+                    emit(combo, windows, pos, res, j, *four_by_job[j], chrom=chrom, at=a)
         return items
 
     # ---- all populations in one packed matrix, the product as fused jobs ------------------
-    use_out = bool(out_data) and bool(four)
     everyone = list(ref_data.values()) + list(tgt_data.values()) + list(src_data.values())
     if use_out:
         everyone += list(out_data.values())
     win_lists = list(windows_by_tgt.values())
-    fused = loaded is not None or (
+    fused = (
         len(combos) > 1
         and len(src_combos) == 1
         and len(everyone) <= _cabi.MAX_POPS
@@ -212,9 +222,7 @@ def score_populations(
         and all(w == win_lists[0] for w in win_lists[1:])
         and (stats or four or dd)
     )
-    if loaded is not None:
-        index, pos, pg = loaded.index, loaded.pos, loaded
-    elif fused:
+    if fused:
         index, mats, ploidy = {}, [], []
         for group, data in (("ref", ref_data), ("tgt", tgt_data)):
             for name, d in data.items():
@@ -233,19 +241,14 @@ def score_populations(
                 ploidy.append(ploidy_config.get_ploidy("outgroup", name))
         pos = everyone[0].POS
         pg = None
-    if fused:
         windows = win_lists[0]
         n_of = lambda i: int(pg.layout.pop[i].n_samples)
         for b0 in range(0, len(combos), _cabi.MAX_JOBS):
             batch = combos[b0 : b0 + _cabi.MAX_JOBS]
             jobs = []
             for r, t, sc, _ in batch:
-                if loaded is not None:
-                    src_ploidy_list(len(sc))  # same check as the host path
                 jobs.append(job_for(r, t, index[("ref", r)], index[("tgt", t)], [index[("src", s)] for s in sc]))
-            if b0 == 0 and loaded is not None:  # the device-parsed tiles are already resident
-                res = engine.score_loaded(windows, jobs)
-            elif pg is None:  # int8 matrices -> pack | copy | genotype pass, pipelined; ONE upload for all batches
+            if pg is None:  # int8 matrices -> pack | copy | genotype pass, pipelined; ONE upload for all batches
                 res, pg = engine.score_matrices(mats, ploidy, pos, windows, jobs, keep_negatives=dd)
             else:
                 res = engine.score_resident(jobs)

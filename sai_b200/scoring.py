@@ -79,6 +79,17 @@ def _job_array(jobs: Sequence["_cabi.Job"]):
     return (_cabi.Job * len(jobs))(*jobs)
 
 
+def _bounds(windows: Sequence[tuple[int, int]]) -> tuple[np.ndarray, np.ndarray]:
+    """The windows' starts and ends as two int64 arrays."""
+    ws = np.ascontiguousarray([w[0] for w in windows], dtype=np.int64)
+    we = np.ascontiguousarray([w[1] for w in windows], dtype=np.int64)
+    return ws, we
+
+
+def _ptr(a: np.ndarray):
+    return a.ctypes.data if a.size else None
+
+
 # --------------------------------------------------------------------------
 # results
 # --------------------------------------------------------------------------
@@ -152,9 +163,7 @@ class HostEngine:
         cap_u: Optional[int] = None,
         cap_q: Optional[int] = None,
     ) -> WindowResults:
-        ws = np.ascontiguousarray([w[0] for w in windows], dtype=np.int64)
-        we = np.ascontiguousarray([w[1] for w in windows], dtype=np.int64)
-        return self.score_arrays(pg, ws, we, jobs, cap_u, cap_q)
+        return self.score_arrays(pg, *_bounds(windows), jobs, cap_u, cap_q)
 
     def set_host_threads(self, n_threads: int) -> None:
         """Host threads of the int8 pipeline (``score_matrices``); <= 0: all cores."""
@@ -174,65 +183,22 @@ class HostEngine:
         """``pg``: ``PackedGenotypes`` (dense tiles), ``ZtGenotypes`` (zero-suppressed wire format)
         or ``MatrixGenotypes`` (int8 matrices: packed by host threads slice by slice while earlier
         slices are on the wire and in the genotype pass, ``sai_engine_score_host_i8``)."""
-        lib = _cabi.load()
-        J, W = len(jobs), int(ws.shape[0])
-        self._last_W = W
-        cap_u = max(1, 4 * W + 1024) if cap_u is None else int(cap_u)
-        cap_q = max(1, 4 * W + 1024) if cap_q is None else int(cap_q)
-        jarr = _job_array(jobs)
-        r = WindowResults(
-            nsnps=np.zeros((J, W), dtype=np.int32),
-            u=np.zeros((J, W), dtype=np.int64),
-            q=np.full((J, W), np.nan, dtype=np.float64),
-            q_cnt=np.zeros((J, W), dtype=np.int32),
-            u_start=np.zeros((J, W), dtype=np.int64),
-            q_start=np.zeros((J, W), dtype=np.int64),
-            totals=np.zeros((J, 2), dtype=np.int64),
-            u_cand=np.zeros((J, cap_u), dtype=np.int32),
-            q_cand=np.zeros((J, cap_q), dtype=np.int32),
-        )
-
-        def c_results():
-            h = _cabi.HostResults()
-            for name in ("nsnps", "u", "q", "q_cnt", "u_start", "q_start", "totals", "u_cand", "q_cand"):
-                setattr(h, name, getattr(r, name).ctypes.data)
-            h.cap_u, h.cap_q = r.u_cand.shape[1], r.q_cand.shape[1]
-            return h
-
         pos = np.ascontiguousarray(pg.pos, dtype=np.int32)
-        res = c_results()
         if isinstance(pg, ZtGenotypes):  # zero-suppressed wire format: expanded on the device
-            entry = lib.sai_engine_score_host_zt
-            tiles = (pg.stream.ctypes.data if pg.stream.size else None, pg.tile_off.ctypes.data)
+            entry = "sai_engine_score_host_zt"
+            tiles = (_ptr(pg.stream), pg.tile_off.ctypes.data)
         elif isinstance(pg, MatrixGenotypes):  # int8 matrices: host pack | copy | genotype pass, pipelined
-            entry = lib.sai_engine_score_host_i8
+            entry = "sai_engine_score_host_i8"
             n = len(pg.mats)
             ptrs = (C.c_void_p * n)(*[m.ctypes.data for m in pg.mats])
             strides = (C.c_int64 * n)(*[m.strides[0] if m.shape[0] > 1 else max(1, m.shape[1]) for m in pg.mats])
             tiles = (ptrs, strides)
         else:
-            entry = lib.sai_engine_score_host
-            tiles = (pg.packed.ctypes.data if pg.packed.size else None,)
-        rc = entry(
-            self._handle(),
-            C.byref(pg.layout),
-            *tiles,
-            pos.ctypes.data if pos.size else None,
-            pg.n_sites,
-            ws.ctypes.data if W else None,
-            we.ctypes.data if W else None,
-            W,
-            jarr,
-            J,
-            C.byref(res),
-        )
-        if rc == _cabi.E_CAPACITY:  # totals say what is needed: re-run the window kernel only
-            r.u_cand = np.zeros((J, max(1, int(r.totals[:, 0].max()))), dtype=np.int32)
-            r.q_cand = np.zeros((J, max(1, int(r.totals[:, 1].max()))), dtype=np.int32)
-            res = c_results()
-            rc = lib.sai_engine_rescore_windows(self._handle(), C.byref(res))
-        _cabi.check(rc)
-        return r
+            entry = "sai_engine_score_host"
+            tiles = (_ptr(pg.packed),)
+        W = int(ws.shape[0])
+        return self._score_call(entry, W, jobs, cap_u, cap_q, C.byref(pg.layout), *tiles, _ptr(pos), pg.n_sites,
+                                _ptr(ws), _ptr(we), W)
 
     def set_vcf_slicing(self, slice_bytes: int = 0, ring: int = 0) -> None:
         """Slice size and ring depth of device ingest (<= 0: default).  Tests force many slices."""
@@ -282,34 +248,33 @@ class HostEngine:
     def score_loaded(self, windows, jobs, cap_u=None, cap_q=None) -> WindowResults:
         """K1 + K4 on the chunk the last device ingest (``vcf_device.read_loaded``) left resident;
         ``score_resident`` / ``pattern_sums`` then work on it like after ``score``."""
-        ws = np.ascontiguousarray([w[0] for w in windows], dtype=np.int64)
-        we = np.ascontiguousarray([w[1] for w in windows], dtype=np.int64)
-        self._last_W = int(ws.shape[0])
-        return self._resident_call("sai_engine_score_loaded", jobs, cap_u, cap_q,
-                                   ws.ctypes.data if ws.size else None, we.ctypes.data if we.size else None, int(ws.shape[0]))
+        ws, we = _bounds(windows)
+        return self._score_call("sai_engine_score_loaded", len(ws), jobs, cap_u, cap_q, _ptr(ws), _ptr(we), len(ws))
 
     def score_loaded_pieces(self, pieces, jobs, cap_u=None, cap_q=None) -> WindowResults:
         """``score_loaded`` over pieces of the resident tiles (``vcf_device.read_genome``): ``pieces``
         = ``[(windows, first site, sites), ...]``, the results' windows piece after piece.  One genotype
         pass and one window launch; ``score_resident`` / ``pattern_sums`` then work on the same pieces."""
-        ws = np.ascontiguousarray([w[0] for p in pieces for w in p[0]], dtype=np.int64)
-        we = np.ascontiguousarray([w[1] for p in pieces for w in p[0]], dtype=np.int64)
+        ws, we = _bounds([w for p in pieces for w in p[0]])
         table = np.ascontiguousarray([[len(w), lo, n] for w, lo, n in pieces], dtype=np.int64)
-        self._last_W = int(ws.shape[0])
-        return self._resident_call("sai_engine_score_loaded_pieces", jobs, cap_u, cap_q,
-                                   ws.ctypes.data if ws.size else None, we.ctypes.data if we.size else None,
-                                   table.ctypes.data, int(table.shape[0]))
+        return self._score_call("sai_engine_score_loaded_pieces", len(ws), jobs, cap_u, cap_q, _ptr(ws), _ptr(we),
+                                table.ctypes.data, int(table.shape[0]))
 
     def score_resident(self, jobs, cap_u=None, cap_q=None) -> WindowResults:
         """Another batch of jobs over the chunk of the last ``score*`` call, still resident on the
         device (no upload): a population product of more than 8 combinations costs one transfer."""
-        return self._resident_call("sai_engine_score_resident", jobs, cap_u, cap_q)
+        return self._score_call("sai_engine_score_resident", self._last_W, jobs, cap_u, cap_q)
 
-    def _resident_call(self, entry: str, jobs, cap_u, cap_q, *head) -> WindowResults:
+    def _score_call(self, entry: str, W: int, jobs, cap_u, cap_q, *head) -> WindowResults:
+        """``entry(engine, *head, jobs, n_jobs, results)`` into new results of ``W`` windows, the windows
+        that ``pattern_sums`` / ``dd_sums`` then see.  After SAI_E_CAPACITY the totals say what is
+        needed: the candidate lists are regrown and only the window kernel is re-run."""
         lib = _cabi.load()
-        J, W = len(jobs), self._last_W
+        J = len(jobs)
+        self._last_W = W
         cap_u = max(1, 4 * W + 1024) if cap_u is None else int(cap_u)
         cap_q = max(1, 4 * W + 1024) if cap_q is None else int(cap_q)
+        jarr = _job_array(jobs)
         r = WindowResults(
             nsnps=np.zeros((J, W), dtype=np.int32), u=np.zeros((J, W), dtype=np.int64),
             q=np.full((J, W), np.nan, dtype=np.float64), q_cnt=np.zeros((J, W), dtype=np.int32),
@@ -326,7 +291,7 @@ class HostEngine:
             return h
 
         res = c_results()
-        rc = getattr(lib, entry)(self._handle(), *head, _job_array(jobs), J, C.byref(res))
+        rc = getattr(lib, entry)(self._handle(), *head, jarr, J, C.byref(res))
         if rc == _cabi.E_CAPACITY:
             r.u_cand = np.zeros((J, max(1, int(r.totals[:, 0].max()))), dtype=np.int32)
             r.q_cand = np.zeros((J, max(1, int(r.totals[:, 1].max()))), dtype=np.int32)
@@ -351,8 +316,7 @@ class HostEngine:
         for m in m8:
             if m.shape[0] != pos.shape[0]:
                 raise ValueError("every population must have one row per position")
-        ws = np.ascontiguousarray([w[0] for w in windows], dtype=np.int64)
-        we = np.ascontiguousarray([w[1] for w in windows], dtype=np.int64)
+        ws, we = _bounds(windows)
         lay = make_layout([m.shape[1] for m in m8], ploidy, bits)
         mg = MatrixGenotypes(lay, int(pos.shape[0]), pos, m8, [], *neg)
         try:
@@ -395,10 +359,9 @@ class HostEngine:
             return ref_sum, tgt_sum
         if getattr(pg, "neg_off", None) is None:
             raise ValueError("DD needs the raw values of missing calls: pack with keep_negatives=True")
-        ptr = lambda a: a.ctypes.data if a.size else None
         _cabi.check(lib.sai_engine_dd_sums(self._handle(), C.byref(pg.layout), int(ref_pop), int(tgt_pop), src,
-                                           len(src_pops), pg.neg_off.ctypes.data, ptr(pg.neg_site), ptr(pg.neg_ind),
-                                           ptr(pg.neg_val), ref_sum.ctypes.data, tgt_sum.ctypes.data, m_max))
+                                           len(src_pops), pg.neg_off.ctypes.data, _ptr(pg.neg_site), _ptr(pg.neg_ind),
+                                           _ptr(pg.neg_val), ref_sum.ctypes.data, tgt_sum.ctypes.data, m_max))
         return ref_sum, tgt_sum
 
 
