@@ -1,16 +1,29 @@
 // K4: per-window U, N(Variants), exact Q and the candidate position lists (one launch).
 //
-// One warp owns one (job, window).  A window [start, end] (inclusive,
-// sai/generators/window_generator.py:173-174) maps to the site range [lo, hi)
-// by a cooperative 32-ary search on the sorted positions; its U count is the
-// popcount of the tile masks over that range (sai/stats/u_statistic.py:94-96)
-// and Q is the numpy 'linear' quantile of the flagged sites' target frequencies
-// (sai/stats/q_statistic.py:96-101; numpy/lib/_function_base_impl.py _lerp).
-// Order statistics are selected exactly on the float64 bit patterns (all
-// values are non-negative, so unsigned order == numeric order).
+// A window [start, end] (inclusive, sai/generators/window_generator.py:173-174)
+// maps to the site range [lo, hi) = [lower_bound(start), lower_bound(end + 1))
+// on the sorted positions; its U count is the popcount of the tile masks over
+// that range (sai/stats/u_statistic.py:94-96) and Q is the numpy 'linear'
+// quantile of the flagged sites' target frequencies (sai/stats/q_statistic.py:96-101;
+// numpy/lib/_function_base_impl.py _lerp).  Order statistics are selected exactly
+// on the float64 bit patterns (all values are non-negative, so unsigned order ==
+// numeric order).
 //
-// The kernel is issue-bound (see profiles/), so all site / tile indices are
-// 32-bit (n_sites < 2^31 is checked on the host) and warp sums use REDUX.
+// One block owns a span of kSpan = 32 consecutive windows of one job.  When the
+// span's starts and ends are sorted, its windows share one piece and the sites of
+// all of them (R) fit the shared-memory budget, the span is scored from shared
+// memory: two searches for R, a coarse index (first position of every tile of R)
+// plus one 128-byte line of positions per window bound, R's masks read once with
+// a prefix of their popcounts (U and the number of Q-flagged sites of a window are
+// differences of it), the flagged sites of R compacted once (a window's candidates
+// are a contiguous slice), a quad of threads per window for Q and the candidate
+// writes, one atomic per span to reserve the candidate slices.
+// Any other span -- unsorted or overlapping window lists, a span crossing pieces,
+// R too long or too densely flagged -- runs the per-window code (window_batch):
+// one warp per window, a cooperative 32-ary search per bound.
+//
+// The per-window code is issue-bound (see profiles/), so all site / tile indices
+// are 32-bit (n_sites < 2^31 is checked on the host) and warp sums use REDUX.
 #include <math_constants.h>
 #include <stdlib.h>
 
@@ -483,30 +496,29 @@ __device__ __forceinline__ void warp_lower_bound_batch(const int32_t* __restrict
   for (int t = 0; t < 2 * kBatch; ++t) out[t] = lo[t];
 }
 
-// grid: x = window batches (kWinWarps * kBatch windows per block, grid-stride), y = job.
-// Each warp works on kBatch consecutive windows at once so that every dependent
-// memory round trip (window bounds, searches, masks, flagged values, slice
-// reservation) is shared by kBatch windows; windows that do not fit the fast
-// path (> 64 tiles or > 32 flagged sites) fall through to window_generic.
-template <int kBatch, int kMinBlocks>
-__global__ void __launch_bounds__(kWinWarps * 32, kMinBlocks)
-    k_window_stats(const __grid_constant__ WinParams P) {
-  __shared__ WarpScratch<kBatch> s_scratch[kWinWarps];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+__device__ __forceinline__ JobView job_view(const WinParams& P, int j) {
   JobView J;
-  J.j = blockIdx.y;
-  J.mu = P.mask_u + (size_t)J.j * P.n_tiles;
-  J.mq = P.mask_q + (size_t)J.j * P.n_tiles;
-  J.qv = P.qval + (size_t)J.j * P.qval_stride;
-  J.want_u = P.u_enabled[J.j] != 0;
-  J.want_q = P.q_enabled[J.j] != 0;
-  J.qq = P.quantile[J.j];
-  J.uc = P.u_cand + (size_t)J.j * P.cap_u;
-  J.qc = P.q_cand + (size_t)J.j * P.cap_q;
-  WarpScratch<kBatch>& SC = s_scratch[warp];
-  const unsigned lt_mask = (1u << lane) - 1u;
+  J.j = j;
+  J.mu = P.mask_u + (size_t)j * P.n_tiles;
+  J.mq = P.mask_q + (size_t)j * P.n_tiles;
+  J.qv = P.qval + (size_t)j * P.qval_stride;
+  J.want_u = P.u_enabled[j] != 0;
+  J.want_q = P.q_enabled[j] != 0;
+  J.qq = P.quantile[j];
+  J.uc = P.u_cand + (size_t)j * P.cap_u;
+  J.qc = P.q_cand + (size_t)j * P.cap_q;
+  return J;
+}
 
-  for (int i0 = (blockIdx.x * kWinWarps + warp) * kBatch; i0 < P.W; i0 += gridDim.x * kWinWarps * kBatch) {
+// The per-window code: one warp, kBatch consecutive windows from i0 at once, so
+// that every dependent memory round trip (window bounds, searches, masks, flagged
+// values, slice reservation) is shared by kBatch windows; windows that do not fit
+// the fast path (> 64 tiles or > 32 flagged sites) fall through to window_generic.
+// Takes any window list: unsorted, overlapping, end < start.
+template <int kBatch>
+__device__ void window_batch(const WinParams& P, const JobView& J, WarpScratch<kBatch>& SC, int i0, int lane) {
+  const unsigned lt_mask = (1u << lane) - 1u;
+  {
     // ---- A: window bounds as keys (one coalesced load for the whole batch) ----
     int64_t key[2 * kBatch];
     {
@@ -672,6 +684,376 @@ __global__ void __launch_bounds__(kWinWarps * 32, kMinBlocks)
   }
 }
 
+// grid: x = window batches (kWinWarps * kBatch windows per block, grid-stride), y = job.
+// Every window through window_batch: the -DSAI_EXPERIMENTS variants.
+template <int kBatch, int kMinBlocks>
+__global__ void __launch_bounds__(kWinWarps * 32, kMinBlocks)
+    k_window_stats(const __grid_constant__ WinParams P) {
+  __shared__ WarpScratch<kBatch> s_scratch[kWinWarps];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const JobView J = job_view(P, blockIdx.y);
+  for (int i0 = (blockIdx.x * kWinWarps + warp) * kBatch; i0 < P.W; i0 += gridDim.x * kWinWarps * kBatch)
+    window_batch<kBatch>(P, J, s_scratch[warp], i0, lane);
+}
+
+// ---------------------------------------------------------------------------
+// Span path: one block per span of kSpan consecutive windows of one job.
+// ---------------------------------------------------------------------------
+constexpr int kSpan = 32;          // windows per span: one per lane of warp 0
+constexpr int kSpanWarps = 4;
+constexpr int kSpanThreads = kSpanWarps * 32;
+constexpr int kSpanTiles = 512;    // tiles of the span's site range R held in shared memory
+constexpr int kSpanFlags = 1024;   // U-flagged and Q-flagged sites of R held in shared memory (each)
+constexpr int kSpanBlocksPerSM = 6;  // ~33 KB of shared memory per block
+constexpr int kTilesPerThread = kSpanTiles / kSpanThreads;
+constexpr int kKeysPerWarp = 2 * kSpan / kSpanWarps;
+static_assert(kSpan == 32 && kSpanThreads == 4 * kSpan && kSpanTiles % kSpanThreads == 0 && (2 * kSpan) % kSpanWarps == 0, "span shape");
+
+struct SpanCtl {  // outside the union: read by every warp after the fallback warps start writing their scratch
+  int ok, lo, hi, T0, nT, nu, nq;
+  int warp_u[kSpanWarps], warp_q[kSpanWarps];
+};
+struct SpanData {
+  int32_t first_pos[kSpanTiles];         // coarse index: position of the first site of R in every tile
+  uint32_t mu[kSpanTiles + 1], mq[kSpanTiles + 1];  // masks restricted to R (+ a zero past the end)
+  int32_t pu[kSpanTiles + 1], pq[kSpanTiles + 1];   // exclusive prefix of their popcounts
+  int32_t upos[kSpanFlags];              // U-flagged sites of R in site order (index, then position)
+  int32_t qpos[kSpanFlags];              // Q-flagged sites of R (index, then position)
+  unsigned long long qv[kSpanFlags];     // ... and their target frequencies (bit patterns)
+  int64_t key[2 * kSpan];                // window k: key 2k = start, 2k + 1 = end + 1
+  int32_t tile_of_key[2 * kSpan];
+  int32_t bnd[2 * kSpan];
+  int32_t u_a[kSpan], q_a[kSpan], n_u[kSpan], n_q[kSpan], q_c[kSpan], nsnps[kSpan];
+  double qres[kSpan];
+  long long u_st[kSpan], q_st[kSpan];
+  int hist[kSpanWarps][256];
+};
+union SpanSmem {
+  SpanData d;
+  WarpScratch<1> w[kSpanWarps];  // the per-window fallback
+};
+
+// flagged sites of R before site x (x in [lo, hi] of R): prefix of the tile + bits below x in its tile
+__device__ __forceinline__ int flags_before(const uint32_t* m, const int32_t* pre, int x, int T0) {
+  const int t = (x >> 5) - T0;
+  return pre[t] + __popc(m[t] & ((1u << (x & 31)) - 1u));
+}
+
+// grid: x = spans (grid-stride), y = job.  A span qualifies when its starts and its ends + 1 are
+// non-decreasing, all its windows share one piece, R (the sites of all its windows) spans at most
+// kSpanTiles tiles and holds at most kSpanFlags U- and Q-flagged sites.  Then every window's site
+// bounds, U, Q and candidates come out of shared memory with a fixed number of dependent memory trips
+// per span; any other span runs window_batch<1> per window, warp by warp.
+__global__ void __launch_bounds__(kSpanThreads, kSpanBlocksPerSM) k_window_spans(const __grid_constant__ WinParams P) {
+  __shared__ SpanSmem sm;
+  __shared__ SpanCtl ctl;
+  SpanData& S = sm.d;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const JobView J = job_view(P, blockIdx.y);
+  const int n_spans = (P.W + kSpan - 1) / kSpan;
+
+  for (int span = blockIdx.x; span < n_spans; span += gridDim.x) {
+    const int i0 = span * kSpan;
+    const int nw = min(kSpan, P.W - i0);
+    __syncthreads();  // the previous span is done with the shared memory
+    // ---- 1: qualify the span and find its site range R = [lo, hi) with two searches ----
+    if (warp == 0) {
+      const bool v = lane < nw;
+      const int64_t ks = v ? P.ws[i0 + lane] : 0, ke = v ? P.we[i0 + lane] + 1 : 0;
+      const int sl = (P.seg_lo != nullptr && v) ? P.seg_lo[i0 + lane] : 0;
+      const int sh = (P.seg_lo != nullptr && v) ? P.seg_hi[i0 + lane] : P.n_sites;
+      const int64_t ps = (int64_t)shfl64((unsigned long long)ks, lane - 1 < 0 ? 0 : lane - 1);
+      const int64_t pe = (int64_t)shfl64((unsigned long long)ke, lane - 1 < 0 ? 0 : lane - 1);
+      const int psl = __shfl_sync(0xffffffffu, sl, lane - 1 < 0 ? 0 : lane - 1);
+      const int psh = __shfl_sync(0xffffffffu, sh, lane - 1 < 0 ? 0 : lane - 1);
+      bool ok = !__any_sync(0xffffffffu, v && lane > 0 && (ks < ps || ke < pe || sl != psl || sh != psh));
+      S.key[2 * lane] = ks;
+      S.key[2 * lane + 1] = ke;
+      // every key of the span lies in [min(start, end + 1) of the first window, max(...) of the last]
+      const int64_t kmin = (int64_t)shfl64((unsigned long long)(ks < ke ? ks : ke), 0);
+      const int64_t kmax = (int64_t)shfl64((unsigned long long)(ks > ke ? ks : ke), nw - 1);
+      int lo = 0, hi = 0, T0 = 0, nT = 0;
+      if (ok) {
+        const int first[1] = {__shfl_sync(0xffffffffu, sl, 0)}, last[1] = {__shfl_sync(0xffffffffu, sh, 0)};
+        const int64_t key[2] = {kmin, kmax};
+        int out[2];
+        warp_lower_bound_batch<1>(P.pos, first, last, key, lane, out);
+        lo = out[0];
+        hi = out[1] > lo ? out[1] : lo;
+        T0 = lo >> 5;
+        nT = hi > lo ? ((hi - 1) >> 5) - T0 + 1 : 0;
+        ok = nT <= kSpanTiles;
+      }
+      if (lane == 0) {
+        ctl.ok = ok;
+        ctl.lo = lo;
+        ctl.hi = hi;
+        ctl.T0 = T0;
+        ctl.nT = nT;
+      }
+    }
+    __syncthreads();
+    if (!ctl.ok) {
+      for (int k = warp; k < nw; k += kSpanWarps) window_batch<1>(P, J, sm.w[warp], i0 + k, lane);
+      continue;
+    }
+    const int lo = ctl.lo, hi = ctl.hi, T0 = ctl.T0, nT = ctl.nT;
+
+    // ---- 2: masks of R's tiles and the coarse index, once; block-wide prefix of the popcounts ----
+    {
+      uint32_t a[kTilesPerThread], b[kTilesPerThread];
+      int fp[kTilesPerThread];
+      int su = 0, sq = 0;
+#pragma unroll
+      for (int r = 0; r < kTilesPerThread; ++r) {
+        const int t = tid * kTilesPerThread + r, T = T0 + t;
+        a[r] = b[r] = 0;
+        fp[r] = 0;
+        if (t < nT) {
+          const uint32_t rm = range_mask(T, lo, hi);
+          if (J.want_u) a[r] = __ldg(J.mu + T) & rm;
+          if (J.want_q) b[r] = __ldg(J.mq + T) & rm;
+          fp[r] = __ldg(P.pos + (T * kTile > lo ? T * kTile : lo));
+        }
+        su += __popc(a[r]);
+        sq += __popc(b[r]);
+      }
+      const int xu = warp_excl_scan(su, lane), xq = warp_excl_scan(sq, lane);
+      if (lane == 31) {
+        ctl.warp_u[warp] = xu + su;
+        ctl.warp_q[warp] = xq + sq;
+      }
+      __syncthreads();
+      int bu = xu, bq = xq;
+      for (int w = 0; w < warp; ++w) {
+        bu += ctl.warp_u[w];
+        bq += ctl.warp_q[w];
+      }
+#pragma unroll
+      for (int r = 0; r < kTilesPerThread; ++r) {
+        const int t = tid * kTilesPerThread + r;
+        S.mu[t] = a[r];
+        S.mq[t] = b[r];
+        S.pu[t] = bu;
+        S.pq[t] = bq;
+        S.first_pos[t] = fp[r];
+        bu += __popc(a[r]);
+        bq += __popc(b[r]);
+      }
+      if (tid == kSpanThreads - 1) {
+        S.mu[kSpanTiles] = S.mq[kSpanTiles] = 0;
+        S.pu[kSpanTiles] = bu;
+        S.pq[kSpanTiles] = bq;
+        ctl.nu = bu;
+        ctl.nq = bq;
+      }
+    }
+    __syncthreads();
+    if (ctl.nu > kSpanFlags || ctl.nq > kSpanFlags) {
+      for (int k = warp; k < nw; k += kSpanWarps) window_batch<1>(P, J, sm.w[warp], i0 + k, lane);
+      continue;
+    }
+    const int nu = ctl.nu, nq = ctl.nq;
+
+    // ---- 3: flagged sites of R in site order; each key's tile from the coarse index ----
+#pragma unroll
+    for (int r = 0; r < kTilesPerThread; ++r) {
+      const int t = tid * kTilesPerThread + r, site0 = (T0 + t) * kTile;
+      uint32_t m = S.mu[t];
+      for (int w = S.pu[t]; m; ++w, m &= m - 1) S.upos[w] = site0 + __ffs(m) - 1;
+      m = S.mq[t];
+      for (int w = S.pq[t]; m; ++w, m &= m - 1) S.qpos[w] = site0 + __ffs(m) - 1;
+    }
+    if (tid < 2 * nw) {
+      // number of tiles whose first site of R lies below the key; the key's bound is inside the last of them
+      const int k32 = clamp_key(S.key[tid]);
+      int a = 0, b = nT;
+      while (a < b) {
+        const int m = (a + b) >> 1;
+        if (S.first_pos[m] < k32) a = m + 1; else b = m;
+      }
+      S.tile_of_key[tid] = a;
+    }
+    __syncthreads();
+
+    // ---- 4: flagged positions / values and every window bound: every load issued before any is used ----
+    {
+      int kp[kKeysPerWarp];  // the key's tile line of positions (INT32_MAX outside R: never below a key)
+#pragma unroll
+      for (int r = 0; r < kKeysPerWarp; ++r) {
+        const int kk = warp * kKeysPerWarp + r;
+        const int c = kk < 2 * nw ? S.tile_of_key[kk] : 0;
+        const int idx = (T0 + c - 1) * kTile + lane;
+        kp[r] = c > 0 && idx >= lo && idx < hi ? __ldg(P.pos + idx) : 2147483647;
+      }
+      int pu = 0, pq = 0;
+      unsigned long long vq = 0;
+      if (tid < nu) pu = __ldg(P.pos + S.upos[tid]);
+      if (tid < nq) {
+        const int site = S.qpos[tid];
+        vq = (unsigned long long)__double_as_longlong(__ldg(J.qv + (size_t)site));
+        pq = __ldg(P.pos + site);
+      }
+#pragma unroll
+      for (int r = 0; r < kKeysPerWarp; ++r) {
+        const int kk = warp * kKeysPerWarp + r;
+        const int c = __popc(__ballot_sync(0xffffffffu, kk < 2 * nw && kp[r] < clamp_key(S.key[kk])));
+        if (lane == 0 && kk < 2 * nw) {
+          const int tc = S.tile_of_key[kk];
+          const int base = tc > 0 ? max((T0 + tc - 1) * kTile, lo) : lo;
+          // a key beyond INT32_MAX lies above every position: the end of the piece, which is hi
+          S.bnd[kk] = S.key[kk] > 2147483647ll ? hi : base + c;
+        }
+      }
+      if (tid < nu) S.upos[tid] = pu;
+      if (tid < nq) {
+        S.qv[tid] = vq;
+        S.qpos[tid] = pq;
+      }
+    }
+    for (int i = tid + kSpanThreads; i < nu; i += kSpanThreads) S.upos[i] = __ldg(P.pos + S.upos[i]);
+    for (int i = tid + kSpanThreads; i < nq; i += kSpanThreads) {
+      const int site = S.qpos[i];
+      S.qv[i] = (unsigned long long)__double_as_longlong(__ldg(J.qv + (size_t)site));
+      S.qpos[i] = __ldg(P.pos + site);
+    }
+    __syncthreads();
+
+    // ---- 5: U, N(Variants) and Q of every window: a quad of threads per window, all windows at once ----
+    {
+      const int k = tid >> 2, q = tid & 3;
+      const bool v = k < nw;
+      int wlo = 0, whi = 0, ua = 0, ub = 0, qa = 0, qn = 0;
+      if (v) {
+        wlo = S.bnd[2 * k];
+        whi = max(S.bnd[2 * k + 1], wlo);  // end < start selects nothing
+        ua = flags_before(S.mu, S.pu, wlo, T0);
+        ub = flags_before(S.mu, S.pu, whi, T0);
+        qa = flags_before(S.mq, S.pq, wlo, T0);
+        qn = flags_before(S.mq, S.pq, whi, T0) - qa;
+      }
+      // n <= 32: the two neighbouring order statistics by rank (ties broken by site order, as in
+      // warp_quantile_small), the ranks of the window's values split over the quad
+      const bool small = v && qn > 0 && qn <= 32;
+      int ka = 0, kb = 0;
+      double g = 0.0;
+      if (small) {
+        const double vi = __dmul_rn((double)(qn - 1), J.qq);
+        if (vi >= (double)(qn - 1)) {
+          ka = kb = qn - 1;
+        } else {
+          const double fl = floor(vi);
+          ka = (int)fl;
+          kb = ka + 1;
+          g = __dsub_rn(vi, fl);
+        }
+      }
+      unsigned long long va = 0, vb = 0;
+      if (small) {
+        for (int i = q; i < qn; i += 4) {
+          const unsigned long long key = S.qv[qa + i];
+          int r = 0;
+          for (int j = 0; j < qn; ++j) {
+            const unsigned long long o = S.qv[qa + j];
+            r += (o < key) || (o == key && j < i);
+          }
+          if (r == ka) va = key;
+          if (r == kb) vb = key;
+        }
+      }
+      // each rank belongs to exactly one value: OR over the quad collects it
+      va |= shfl64(va, lane ^ 1);
+      va |= shfl64(va, lane ^ 2);
+      vb |= shfl64(vb, lane ^ 1);
+      vb |= shfl64(vb, lane ^ 2);
+      double qres = CUDART_NAN;
+      int qc = 0;
+      if (small) {
+        const double da = __longlong_as_double((long long)va), db = __longlong_as_double((long long)vb);
+        qres = ka == kb ? da : lerp_numpy(da, db, g);
+        for (int i = q; i < qn; i += 4) qc += __longlong_as_double((long long)S.qv[qa + i]) >= qres;
+      }
+      qc += __shfl_xor_sync(0xffffffffu, qc, 1);
+      qc += __shfl_xor_sync(0xffffffffu, qc, 2);
+      if (v && q == 0) {
+        S.nsnps[k] = whi - wlo;
+        S.u_a[k] = ua;
+        S.n_u[k] = ub - ua;
+        S.q_a[k] = qa;
+        S.n_q[k] = qn;
+        S.q_c[k] = qc;
+        S.qres[k] = qres;
+      }
+    }
+    __syncthreads();
+    // windows above 32 Q-flagged sites: exact radix selection on the window's slice, warp per window
+    for (int k = warp; k < nw; k += kSpanWarps) {
+      const int qn = S.n_q[k];
+      if (qn <= 32) continue;
+      BufSource src{S.qv + S.q_a[k], qn, lane};
+      const double qres = warp_quantile(src, qn, J.qq, S.hist[warp], lane);
+      const int qc = warp_count_ge(src, qres);
+      if (lane == 0) {
+        S.qres[k] = qres;
+        S.q_c[k] = qc;
+      }
+    }
+    __syncthreads();
+
+    // ---- 6: one atomic per span and array, coalesced result stores ----
+    if (warp == 0) {
+      const bool v = lane < nw;
+      const int nu_k = v ? S.n_u[lane] : 0, qc_k = v ? S.q_c[lane] : 0;
+      const int xu = warp_excl_scan(nu_k, lane), xq = warp_excl_scan(qc_k, lane);
+      const int tu = warp_sum(nu_k), tq = warp_sum(qc_k);
+      unsigned long long base = 0;
+      if (lane < 2 && (lane ? tq : tu) > 0) base = atomicAdd(P.totals + 2 * J.j + lane, (unsigned long long)(lane ? tq : tu));
+      const long long ubase = (long long)shfl64(base, 0), qbase = (long long)shfl64(base, 1);
+      if (v) {
+        const size_t item = (size_t)J.j * P.W + i0 + lane;
+        const long long us = nu_k > 0 ? ubase + xu : 0, qs = qc_k > 0 ? qbase + xq : 0;
+        P.nsnps[item] = S.nsnps[lane];
+        P.u[item] = nu_k;
+        P.q[item] = S.qres[lane];
+        P.q_cnt[item] = qc_k;
+        P.u_start[item] = us;
+        P.q_start[item] = qs;
+        S.u_st[lane] = us;
+        S.q_st[lane] = qs;
+      }
+    }
+    __syncthreads();
+
+    // ---- 7: candidate positions in site order, a quad of threads per window ----
+    {
+      const int k = tid >> 2, q = tid & 3;
+      int ua = 0, un = 0, qa = 0, qn = 0;
+      long long us = 0, qw = 0;
+      double qres = 0.0;
+      if (k < nw) {
+        ua = S.u_a[k];
+        un = S.n_u[k];
+        us = S.u_st[k];
+        qa = S.q_a[k];
+        qn = S.n_q[k];
+        qw = S.q_st[k];
+        qres = S.qres[k];
+      }
+      for (int e = q; e < un; e += 4)
+        if (us + e < P.cap_u) J.uc[us + e] = S.upos[ua + e];
+      const int steps = (int)__reduce_max_sync(0xffffffffu, (unsigned)(qn + 3) >> 2);
+      for (int st = 0; st < steps; ++st) {
+        const int e = 4 * st + q;
+        const bool ge = e < qn && __longlong_as_double((long long)S.qv[qa + e]) >= qres;
+        const unsigned m = (__ballot_sync(0xffffffffu, ge) >> (lane & 28)) & 0xfu;  // this quad's 4 bits
+        const long long w = qw + __popc(m & ((1u << q) - 1u));
+        if (ge && w < P.cap_q) J.qc[w] = S.qpos[qa + e];
+        qw += __popc(m);
+      }
+    }
+  }
+}
+
 }  // namespace sai
 
 using namespace sai;
@@ -731,9 +1113,10 @@ static int window_stats_impl(const int32_t* d_pos, int64_t n_sites, const int64_
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   SAI_CUDA_CHECK(cudaMemsetAsync(d_totals, 0, sizeof(int64_t) * 2 * n_jobs, st));
   if (n_windows == 0) return SAI_OK;
-  const int64_t cap = (int64_t)sm_count() * 32;
 #ifdef SAI_EXPERIMENTS
-  // tuning knobs of tools/ builds: windows per warp and the occupancy bound
+  // tuning knobs of tools/ builds: every window on the per-window path, windows per warp and the
+  // occupancy bound
+  const int64_t cap = (int64_t)sm_count() * 32;
   static const int batch = [] {
     const char* e = getenv("SAI_WIN_BATCH");
     const int b = e ? atoi(e) : 1;
@@ -757,11 +1140,14 @@ static int window_stats_impl(const int32_t* d_pos, int64_t n_sites, const int64_
   else
     k_window_stats<4, 4><<<grid, kWinWarps * 32, 0, st>>>(P);
 #else
-  // one window per warp, 12 blocks per SM: the configuration that measured fastest
-  // (profiles/round1_notes.md); the batched variants live in -DSAI_EXPERIMENTS builds
-  const int64_t want = (n_windows + kWinWarps - 1) / kWinWarps;
-  const dim3 grid((unsigned)(want < cap ? want : cap), (unsigned)n_jobs);
-  k_window_stats<1, 12><<<grid, kWinWarps * 32, 0, st>>>(P);
+  // one block per span of kSpan windows, as many blocks as are resident at once (grid-stride)
+  const int64_t spans = (n_windows + kSpan - 1) / kSpan, span_cap = (int64_t)sm_count() * kSpanBlocksPerSM;
+  const dim3 grid((unsigned)(spans < span_cap ? spans : span_cap), (unsigned)n_jobs);
+  // kSpanBlocksPerSM blocks of ~33 KB need the largest shared-memory carveout
+  static const cudaError_t carveout = cudaFuncSetAttribute(
+      k_window_spans, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  SAI_CUDA_CHECK(carveout);
+  k_window_spans<<<grid, kSpanThreads, 0, st>>>(P);
 #endif
   SAI_CUDA_CHECK(cudaGetLastError());
   return SAI_OK;
