@@ -683,6 +683,59 @@ int64_t sai_engine_loaded_neg_table(sai_engine* e, int64_t* neg_off, int32_t* si
 int sai_engine_dd_sums_loaded(sai_engine* e, int32_t ref_pop, int32_t tgt_pop, const int32_t* src_pops, int32_t n_src,
                               int64_t* ref_sum, int64_t* tgt_sum, int32_t m_max);
 
+/* ---- score file text on the device (score(..., write="device")) ------------------------------------
+ * The rows of the score file and of the .U.log / .Q.log files, byte for byte what the host writer
+ * (sai_b200.preprocessors.write_items) prints from the item dicts, formatted in HBM.  Rows come in
+ * blocks: block b is one (chromosome, combination) run of windows, rows block_rows[b] ..
+ * block_rows[b + 1] - 1, and holds two strings of `strings`: its chromosome (block_str[4b], length
+ * block_str[4b + 1]) and "Ref\tTgt\tSrc\tOutgroup" (block_str[4b + 2], length block_str[4b + 3]).
+ * A score row is
+ *     chrom \t start \t end \t Ref \t Tgt \t Src \t Outgroup \t nsnps \t field_0 \t ... \t field_{n-1} \n
+ * field[f] = SAI_FMT_U (the integer u), SAI_FMT_Q (the float64 q) or a column k of vals[row][n_vals];
+ * every field of a row with nsnps == 0 prints "nan", a float64 prints as Python's repr(float).  A log
+ * row is "chrom \t start \t end \t " followed by "NA" or the window's candidate positions as
+ * "chrom:pos" joined by ",": u[row] positions from u_cand[u_start[row]] (none when nsnps == 0), and
+ * q_cnt[row] from q_cand[q_start[row]] (none when nsnps == 0 or q is NaN).  The .U.log text exists
+ * when a field is SAI_FMT_U (u, u_start, u_cand are then read), the .Q.log text likewise.
+ * sai_engine_format_scores copies the inputs to the device, formats the three texts there (a length
+ * pass, a scan of the lengths, a write pass) and keeps them resident; sizes[0..2] = bytes of the
+ * rows, the .U.log and the .Q.log text (0 for one that does not exist).  sai_engine_format_text
+ * copies text `which` (0..2) of the last call into HOST memory (cap >= its size).
+ * sai_engine_format_stats: seconds of the last call (CUDA events): input copy, length + scan
+ * kernels, write kernels.
+ * sai_format_double / sai_format_doubles: repr(float(x)) on the host (the device's code), the
+ * length returned; the batch writes 32 NUL-padded bytes per value.  sai_engine_format_doubles: the
+ * same batch formatted by the device in one launch (tests). */
+#define SAI_FMT_U (-1)
+#define SAI_FMT_Q (-2)
+typedef struct {
+  int64_t n_blocks, n_rows;
+  const int64_t* block_rows; /* [n_blocks + 1] */
+  const int64_t* block_str;  /* [n_blocks][4]  */
+  const char* strings;
+  int64_t strings_len;
+  const int64_t* start;      /* [n_rows] window bounds */
+  const int64_t* end;
+  const int32_t* nsnps;
+  const int64_t* u;          /* [n_rows], with u_start: NULL without SAI_FMT_U */
+  const int64_t* u_start;
+  const double* q;           /* [n_rows], with q_start, q_cnt: NULL without SAI_FMT_Q */
+  const int64_t* q_start;
+  const int32_t* q_cnt;
+  const int32_t* u_cand;     /* [n_u_cand] */
+  const int32_t* q_cand;     /* [n_q_cand] */
+  int64_t n_u_cand, n_q_cand;
+  const int32_t* field;      /* [n_fields] */
+  const double* vals;        /* [n_rows][n_vals] */
+  int32_t n_fields, n_vals;
+} sai_format_input;
+int sai_engine_format_scores(sai_engine* e, const sai_format_input* in, int64_t* sizes);
+int sai_engine_format_text(sai_engine* e, int32_t which, char* out, int64_t cap);
+int sai_engine_format_stats(const sai_engine* e, double* out, int32_t n);
+int sai_engine_format_doubles(sai_engine* e, const double* x, int64_t n, char* out);
+int32_t sai_format_double(double x, char* out);
+int sai_format_doubles(const double* x, int64_t n, char* out);
+
 /* ---- synthetic genotypes (bench / tests only) ---------------------------- */
 /* Fills tiles [tile0, tile0+n_tiles) of a packed matrix directly on the device
  * with the synthetic model of DESIGN.md (counter-based RNG, reproducible from

@@ -115,6 +115,37 @@ class VcfChrom(C.Structure):
     ]
 
 
+class FormatInput(C.Structure):
+    """``sai_format_input``: the blocks of score rows ``sai_engine_format_scores`` formats."""
+
+    _fields_ = [
+        ("n_blocks", C.c_int64),
+        ("n_rows", C.c_int64),
+        ("block_rows", C.c_void_p),
+        ("block_str", C.c_void_p),
+        ("strings", C.c_void_p),
+        ("strings_len", C.c_int64),
+        ("start", C.c_void_p),
+        ("end", C.c_void_p),
+        ("nsnps", C.c_void_p),
+        ("u", C.c_void_p),
+        ("u_start", C.c_void_p),
+        ("q", C.c_void_p),
+        ("q_start", C.c_void_p),
+        ("q_cnt", C.c_void_p),
+        ("u_cand", C.c_void_p),
+        ("q_cand", C.c_void_p),
+        ("n_u_cand", C.c_int64),
+        ("n_q_cand", C.c_int64),
+        ("field", C.c_void_p),
+        ("vals", C.c_void_p),
+        ("n_fields", C.c_int32),
+        ("n_vals", C.c_int32),
+    ]
+
+
+FMT_U, FMT_Q = -1, -2  # SAI_FMT_U / SAI_FMT_Q: the U and Q fields of a score row
+
 #: every symbol include/sai_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 _I32, _I64, _U64 = C.c_int32, C.c_int64, C.c_uint64
@@ -221,6 +252,12 @@ SYMBOLS = {
     "sai_engine_set_vcf_neg_table": (C.c_int, [_P, _I32, _I64]),
     "sai_engine_loaded_neg_table": (_I64, [_P, _P, _P, _P, _P, _I64]),
     "sai_engine_dd_sums_loaded": (C.c_int, [_P, _I32, _I32, _P, _I32, _P, _P, _I32]),
+    "sai_engine_format_scores": (C.c_int, [_P, C.POINTER(FormatInput), _P]),
+    "sai_engine_format_text": (C.c_int, [_P, _I32, _P, _I64]),
+    "sai_engine_format_stats": (C.c_int, [_P, _P, _I32]),
+    "sai_engine_format_doubles": (C.c_int, [_P, _P, _I64, _P]),
+    "sai_format_double": (_I32, [C.c_double, C.c_char_p]),
+    "sai_format_doubles": (C.c_int, [_P, _I64, _P]),
 }
 
 _lib = None

@@ -23,6 +23,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "format_kernels.cuh"
 #include "host_pack.h"
 #include "vcf_genome.cuh"
 #include "zt_format.cuh"
@@ -161,6 +162,7 @@ struct sai_engine {
   Buf vcomp, vbad;  // device inflate: ring of compressed groups (+ block statuses), first corrupt block
   Buf vgen;         // genome ingest: hash table, names, offsets, running state, per-chromosome records
   Buf vneg, vnega, vnegt;  // negative-value table: state + per-key counts, appended entries, finished table
+  sai::FormatState fmt;    // score file text (sai_engine_format_scores)
 };
 
 namespace sai {
@@ -319,6 +321,7 @@ void sai_engine_destroy(sai_engine* e) {
   for (auto s : e->vcf.s_infl) cudaStreamDestroy(s);
   if (e->ring) cudaFreeHost(e->ring);
   if (e->h_ztoff) cudaFreeHost(e->h_ztoff);
+  sai::format_release(e->fmt);
   if (e->s_copy) cudaStreamDestroy(e->s_copy);
   if (e->s_comp) cudaStreamDestroy(e->s_comp);
   delete e;
@@ -1854,3 +1857,27 @@ int sai_engine_dd_sums_loaded(sai_engine* e, int32_t ref_pop, int32_t tgt_pop, c
 }
 
 }  // extern "C"
+
+int sai_engine_format_scores(sai_engine* e, const sai_format_input* in, int64_t* sizes) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::format_scores(e->fmt, in, e->s_comp, sizes);
+}
+
+int sai_engine_format_text(sai_engine* e, int32_t which, char* out, int64_t cap) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::format_text(e->fmt, which, out, cap, e->s_comp);
+}
+
+int sai_engine_format_stats(const sai_engine* e, double* out, int32_t n) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::format_stats(const_cast<sai_engine*>(e)->fmt, out, n);
+}
+
+int sai_engine_format_doubles(sai_engine* e, const double* x, int64_t n, char* out) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::format_doubles_device(x, n, out, e->s_comp);
+}

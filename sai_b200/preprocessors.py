@@ -12,6 +12,7 @@ is replaced by one call into the CUDA library per chunk.
 
 from __future__ import annotations
 
+import locale
 from itertools import combinations, product
 from pathlib import Path
 from typing import Any, Optional
@@ -53,6 +54,7 @@ def score_populations(
     out_data: Optional[dict[str, PopData]] = None,
     num_src: Optional[int] = None,
     loaded=None,
+    sink=None,
 ) -> list[dict[str, Any]]:
     """Item dicts for every (ref, tgt, src-combination, outgroup) x window.
 
@@ -67,7 +69,11 @@ def score_populations(
     ``vcf_device.LoadedGenome`` holds several chromosomes, each with its own windows
     (``windows_by_tgt`` maps every target population to the list of them, one per chromosome;
     ``chr_name`` is not used): all chromosomes are scored with one genotype pass and one window
-    launch per batch of combinations, and the items come out chromosome by chromosome."""
+    launch per batch of combinations, and the items come out chromosome by chromosome.
+
+    ``sink`` (e.g. a ``DeviceRows``): each run of windows of one combination is handed to
+    ``sink(combo, windows, pos, res, j, four_vals, dd_vals, chrom, at)`` instead of being turned into
+    item dicts, and the returned list stays empty."""
     stats = [s for s in stat_config.root.keys() if s in ("U", "Q")]
     four = [s for s in stat_config.root.keys() if s in ("Danc", "Dplus", "df", "fd") and stat_config.root[s] is True]
     dd = any(s == "DD" and stat_config.root[s] is True for s in stat_config.root.keys())
@@ -105,6 +111,8 @@ def score_populations(
         tens of thousands of windows, so the per-window work is kept to plain Python objects: the
         result columns are turned into lists once and the candidate lists are views into one
         converted array.  ``windows`` are the result columns ``at, at + 1, ...``."""
+        if sink is not None:
+            return sink(combo, windows, pos, res, j, four_vals, dd_vals, chrom, at)
         ref_pop, tgt_pop, src_comb, out_pop = combo
         n_src = len(src_comb)
         out_name = "NA" if out_pop is None else out_pop
@@ -326,6 +334,138 @@ def write_items(output_file: str, items: list[dict[str, Any]], stat_config) -> N
             f.write("".join(rows))
 
 
+class DeviceRows:
+    """A ``score_populations`` sink for ``write="device"``: the score rows kept as numpy columns, one
+    block per (chromosome, combination) run of windows in the order ``write_items`` writes them, and
+    formatted on the GPU by ``write``.  No per-window Python object is made; the values are the ones
+    ``emit`` puts in the item dicts (``four_pop_values`` / ``dd_values`` lists as float64 arrays), so the
+    text is byte for byte that of ``write_items``."""
+
+    def __init__(self, stat_config):
+        root = stat_config.root
+        self.names = [s for s in root.keys() if s in ("U", "Q") or root[s] is True]  # write_items' columns
+        self.logs = [k for k in ("U", "Q") if k in root]
+        self.blocks: list[dict] = []
+        self._seen: dict = {}  # (id, what) -> (object, its array): a list or result converted once
+
+    def _once(self, obj, what, make):
+        hit = self._seen.get((id(obj), what))
+        if hit is None or hit[0] is not obj:
+            hit = self._seen[(id(obj), what)] = (obj, make())
+        return hit[1]
+
+    def __call__(self, combo, windows, pos, res, j, four_vals, dd_vals, chrom, at=0):
+        ref_pop, tgt_pop, src_comb, out_pop = combo
+        n = len(windows)
+        cols = slice(at, at + n)
+        out_name = "NA" if out_pop is None else out_pop
+        b = {"chrom": f"{chrom}", "combo": f"{ref_pop}\t{tgt_pop}\t{','.join(src_comb)}\t{out_name}",
+             "bounds": self._once(windows, "bounds", lambda: np.asarray(windows, dtype=np.int64).reshape(-1, 2))}
+        if res is not None:
+            b["nsnps"] = res.nsnps[j, cols]
+        else:  # as emit: no statistic scored, or a region without data (empty positions)
+            b["nsnps"] = np.array([int(np.count_nonzero((pos >= s_) & (pos <= e_))) for s_, e_ in windows], dtype=np.int32)
+        zeros = np.zeros(n, dtype=np.int64)
+        for key in ("u", "q"):
+            if key.upper() not in self.names:
+                continue
+            if res is None:  # every window has nsnps == 0: no candidates are read
+                b[key] = np.full(n, np.nan) if key == "q" else zeros
+                b[key + "_start"], b[key + "_pool"] = zeros, None
+                if key == "q":
+                    b["q_cnt"] = zeros
+                continue
+            b[key] = getattr(res, key)[j, cols]
+            b[key + "_start"] = getattr(res, key + "_start")[j, cols]
+            if key == "q":
+                b["q_cnt"] = res.q_cnt[j, cols]
+            cand = getattr(res, key + "_cand")
+            used = cand.shape[1]
+            if getattr(res, "totals", None) is not None:
+                used = min(int(res.totals[j, 0 if key == "u" else 1]), used)
+            # (identity of job j's list, the list, the results: kept alive so that no later results share the id)
+            b[key + "_pool"] = ((id(res), key, j), cand[j, :used], res)
+        n_src = len(src_comb)
+        field, vals = [], []
+        for s in self.names:
+            if s in ("U", "Q"):
+                field.append(_cabi.FMT_U if s == "U" else _cabi.FMT_Q)
+                continue
+            for k in range(max(n_src, 1)):  # one per source; a row with nsnps == 0 prints nan in each
+                src = dd_vals if s == "DD" else (four_vals[s] if four_vals is not None else None)
+                if src is None or k >= n_src:
+                    vals.append(np.full(n, np.nan))
+                else:
+                    vals.append(self._once(src[k], "f64", lambda: np.asarray(src[k], dtype=np.float64))[cols])
+                field.append(len(vals) - 1)
+        b["field"] = field
+        b["vals"] = np.stack(vals, axis=1) if vals else np.zeros((n, 0))
+        self.blocks.append(b)
+
+    def format(self, engine, encoding: str):
+        """The three texts (score rows, ``.U.log``, ``.Q.log``) as uint8 arrays, from the GPU."""
+        blocks = [b for b in self.blocks if len(b["bounds"])]
+        if not blocks:
+            return [np.zeros(0, dtype=np.uint8)] * 3
+        field = blocks[0]["field"]
+        if any(b["field"] != field for b in blocks):
+            raise ValueError("every combination of one score file has the same number of source populations")
+        strings, block_str, at = [], [], 0
+        for b in blocks:
+            for key in ("chrom", "combo"):
+                raw = b[key].encode(encoding)
+                block_str += [at, len(raw)]
+                strings.append(raw)
+                at += len(raw)
+        strings = b"".join(strings)
+        cat = lambda key, dt: np.ascontiguousarray(np.concatenate([b[key] for b in blocks]), dtype=dt)
+        bounds = np.concatenate([b["bounds"] for b in blocks])
+        keep = {
+            "block_rows": np.cumsum([0] + [len(b["bounds"]) for b in blocks], dtype=np.int64),
+            "block_str": np.asarray(block_str, dtype=np.int64),
+            "start": np.ascontiguousarray(bounds[:, 0]), "end": np.ascontiguousarray(bounds[:, 1]),
+            "nsnps": cat("nsnps", np.int32), "field": np.asarray(field, dtype=np.int32),
+            "vals": cat("vals", np.float64),
+        }
+        for key in ("u", "q"):
+            if key.upper() not in self.names:
+                continue
+            pools, base, n_pool = [], {}, 0
+            starts = []
+            for b in blocks:
+                p = b[key + "_pool"]
+                if p is not None and p[0] not in base:
+                    base[p[0]] = n_pool
+                    pools.append(p[1])
+                    n_pool += len(p[1])
+                starts.append(b[key + "_start"] + (0 if p is None else base[p[0]]))
+            keep[key] = cat(key, np.float64 if key == "q" else np.int64)
+            keep[key + "_start"] = np.ascontiguousarray(np.concatenate(starts), dtype=np.int64)
+            keep[key + "_cand"] = np.ascontiguousarray(np.concatenate(pools) if pools else np.zeros(0), dtype=np.int32)
+            if key == "q":
+                keep["q_cnt"] = cat("q_cnt", np.int32)
+        inp = _cabi.FormatInput()
+        inp.n_blocks, inp.n_rows = len(blocks), len(bounds)
+        keep["strings"] = np.frombuffer(strings, dtype=np.uint8)
+        inp.strings_len = len(strings)
+        for name, arr in keep.items():
+            setattr(inp, name, arr.ctypes.data if arr.size else None)
+        inp.n_u_cand = keep["u_cand"].size if "u_cand" in keep else 0
+        inp.n_q_cand = keep["q_cand"].size if "q_cand" in keep else 0
+        inp.n_fields, inp.n_vals = len(field), keep["vals"].shape[1]
+        return engine.format_scores(inp)
+
+    def write(self, output_file: str, engine) -> None:
+        """Appends the rows to the score file and the ``.U.log`` / ``.Q.log`` files: one write each."""
+        rows, u_log, q_log = self.format(engine, locale.getpreferredencoding(False))
+        with open(output_file, "ab") as f:
+            f.write(memoryview(rows))
+        for key, text in (("U", u_log), ("Q", q_log)):
+            if key in self.logs:
+                with open(Path(output_file).with_suffix(f".{key}.log"), "ab") as f:
+                    f.write(memoryview(text))
+
+
 class ChunkPreprocessor:
     """Drop-in for ``sai.preprocessors.ChunkPreprocessor`` on the U/Q path."""
 
@@ -390,6 +530,10 @@ class ChunkPreprocessor:
         self.engine = HostEngine(device)  # picklable; CUDA context created in run()
 
     def run(self, chr_name: str, start: int, end: int) -> list[dict[str, Any]]:
+        return self.run_into(chr_name, start, end, None)
+
+    def run_into(self, chr_name: str, start: int, end: int, sink) -> list[dict[str, Any]]:
+        """``run``, with the rows handed to ``sink`` (see ``score_populations``) when it is given."""
         from .vcf import read_data
 
         if self.win_len <= 0:
@@ -397,7 +541,7 @@ class ChunkPreprocessor:
         if self.win_step < 0:
             raise ValueError("`win_step` must be non-negative.")
         if self.ingest == "device":
-            items = self._run_device(chr_name, start, end)
+            items = self._run_device(chr_name, start, end, sink)
             if items is not None:
                 return items
         groups = read_data(
@@ -422,10 +566,10 @@ class ChunkPreprocessor:
             wins = chunk_windows(start, end, self.win_len, self.win_step)
             windows = {t: wins for t in tgt_samples}
         if ref_data is None or tgt_data is None or src_data is None:
-            return self._empty_items(chr_name, windows, ref_samples, tgt_samples, src_samples, out_samples)
+            return self._empty_items(chr_name, windows, ref_samples, tgt_samples, src_samples, out_samples, sink)
         return score_populations(
             chr_name, windows, ref_data, tgt_data, src_data, self.ploidy_config, self.stat_config,
-            self.anc_allele_available, self.engine, out_data=out_data, num_src=self.num_src,
+            self.anc_allele_available, self.engine, out_data=out_data, num_src=self.num_src, sink=sink,
         )
 
     def device_fallback(self, chr_name: str, start=None, end=None) -> Optional[str]:
@@ -440,7 +584,7 @@ class ChunkPreprocessor:
         return fallback_reason(self.stat_config, self.ploidy_config, plan, anc, chr_name, self.num_src,
                                self.dd_ingest)
 
-    def _run_device(self, chr_name, start, end):
+    def _run_device(self, chr_name, start, end, sink=None):
         import warnings
 
         from .vcf import read_anc_or_error
@@ -473,14 +617,15 @@ class ChunkPreprocessor:
             wins = chunk_windows(start, end, self.win_len, self.win_step)
             windows = {t: wins for t in tgt_samples}
         if ref_pops is None or tgt_pops is None or src_pops is None:
-            return self._empty_items(chr_name, windows, ref_samples, tgt_samples, src_samples, out_samples)
+            return self._empty_items(chr_name, windows, ref_samples, tgt_samples, src_samples, out_samples, sink)
         names = lambda pops: {p: None for p in pops} if pops else None
         return score_populations(
             chr_name, windows, names(ref_pops), names(tgt_pops), names(src_pops), self.ploidy_config, self.stat_config,
             self.anc_allele_available, self.engine, out_data=names(out_pops), num_src=self.num_src, loaded=loaded,
+            sink=sink,
         )
 
-    def _empty_items(self, chr_name, windows, ref_samples, tgt_samples, src_samples, out_samples=None):
+    def _empty_items(self, chr_name, windows, ref_samples, tgt_samples, src_samples, out_samples=None, sink=None):
         # no data in the region: window_generator.py:249-289 (product over the outgroup populations
         # too, :269-273) + feature_preprocessor.py:131-144
         stats = [s for s in self.stat_config.root.keys() if s in ("U", "Q")]
@@ -489,6 +634,10 @@ class ChunkPreprocessor:
         for ref_pop, tgt_pop, src_comb, out_pop in product(
             ref_samples, tgt_samples, list(combinations(src_samples.keys(), self.num_src)), out_samples or [None]
         ):
+            if sink is not None:  # no positions: every window has nsnps == 0
+                sink((ref_pop, tgt_pop, src_comb, out_pop), windows[tgt_pop], np.zeros(0, dtype=np.int64), None, 0,
+                     None, None, chr_name)
+                continue
             for start, end in windows[tgt_pop]:
                 it = {
                     "chr_name": chr_name, "start": start, "end": end, "ref_pop": ref_pop, "tgt_pop": tgt_pop,

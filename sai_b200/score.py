@@ -17,7 +17,7 @@ from typing import Sequence
 import numpy as np
 
 from .configs import load_config
-from .preprocessors import ChunkPreprocessor
+from .preprocessors import ChunkPreprocessor, DeviceRows
 from .generators import ChunkGenerator
 
 
@@ -61,6 +61,26 @@ def _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file
     )
 
 
+def _check_write(write: str) -> None:
+    if write not in ("host", "device"):
+        raise ValueError(f"write must be 'host' or 'device', not {write!r}")
+
+
+def _run_and_write(pre: ChunkPreprocessor, chunks, output_file: str, write: str) -> None:
+    """Scores the chunks and appends their rows: item dicts written by ``process_items``
+    (``write="host"``), or blocks of rows formatted on the GPU (``write="device"``)."""
+    if write == "host":
+        items = []
+        for params in chunks:
+            items.extend(pre.run(**params))
+        pre.process_items(items)
+        return
+    rows = DeviceRows(pre.stat_config)
+    for params in chunks:
+        pre.run_into(sink=rows, **params)
+    rows.write(output_file, pre.engine)
+
+
 def _write_headers(output_file: str, stat_config, ploidy_config) -> None:
     """The header lines of the score file and of the ``.U.log`` / ``.Q.log`` files (sai/sai.py:122-142)."""
     header = ["Chrom", "Start", "End", "Ref", "Tgt", "Src", "Outgroup", "N(Variants)"]
@@ -96,10 +116,15 @@ def score(
     ingest: str = "host",
     inflate: str = "host",
     dd_ingest: str = "host",
+    write: str = "host",
 ) -> None:
     """``ingest="device"`` parses the VCF on the GPU (``ChunkPreprocessor(ingest=...)``),
     ``inflate="device"`` also inflates a bgzip file there, and ``dd_ingest="device"`` reads a DD
-    configuration there too (the raw values of missing calls are kept in HBM); same output."""
+    configuration there too (the raw values of missing calls are kept in HBM); same output.
+    ``write="device"`` formats the score file and the ``.U.log`` / ``.Q.log`` files on the GPU from the
+    scoring results (``DeviceRows``: no per-window Python object, one copy back and one write per
+    file); same bytes."""
+    _check_write(write)
     cfg = _load_checked_config(config, anc_allele_file)
     # ONE chunk, as sai.py:86-93 (num_chunks=1; `num_workers` is accepted and ignored there too):
     # rows come out product-major / windows-inner, identical to the reference's text.  Real
@@ -109,10 +134,7 @@ def score(
     pre = _preprocessor(vcf_file, cfg, win_len, win_step, anc_allele_file, output_file, device, ingest, inflate,
                         dd_ingest)
     _write_headers(output_file, cfg.statistics, cfg.ploidies)
-    items = []
-    for params in generator.get():  # sai.py:148-149
-        items.extend(pre.run(**params))
-    pre.process_items(items)
+    _run_and_write(pre, generator.get(), output_file, write)  # sai.py:148-149
 
 
 def score_genome(
@@ -126,6 +148,7 @@ def score_genome(
     device: int = 0,
     inflate: str = "host",
     dd_ingest: str = "host",
+    write: str = "host",
 ) -> None:
     """Scores every chromosome of ``chr_names`` of one (multi-chromosome) VCF: the score file and the
     ``.U.log`` / ``.Q.log`` files are byte for byte those of ``score(vcf_file, c, ...)`` run for each
@@ -142,13 +165,17 @@ def score_genome(
     (DD with ``dd_ingest="host"``, more than 16 populations, long ancestral alleles, positional
     source ploidies), more than
     ``SAI_VCF_MAX_CHROMS`` (1024) chromosomes, or chromosomes whose records are not contiguous in
-    the file -- are scored one chromosome at a time by the ``score`` path, with the same output."""
+    the file -- are scored one chromosome at a time by the ``score`` path, with the same output.
+
+    ``write="device"`` formats the rows on the GPU as ``score(..., write="device")`` does, on both
+    paths."""
     from . import _cabi
     from .preprocessors import score_populations, write_items
     from .vcf import read_anc_or_error
     from .vcf_device import _wants_outgroup, fallback_reason, genome_tables, read_genome, read_plan, wants_dd
     from .windows import chunk_windows, split_genome, split_windows_ranges
 
+    _check_write(write)
     cfg = _load_checked_config(config, anc_allele_file)
     stat_config, ploidy_config = cfg.statistics, cfg.ploidies
     chr_names = list(chr_names)
@@ -160,10 +187,7 @@ def score_genome(
                       for c in chr_names]
         _write_headers(output_file, stat_config, ploidy_config)
         for generator in generators:
-            items = []
-            for params in generator.get():
-                items.extend(pre.run(**params))
-            pre.process_items(items)
+            _run_and_write(pre, generator.get(), output_file, write)
 
     if not chr_names or len(set(chr_names)) != len(chr_names) or len(chr_names) > _cabi.MAX_CHROMS:
         return each_chromosome()
@@ -211,8 +235,12 @@ def score_genome(
         return each_chromosome()
     _write_headers(output_file, stat_config, ploidy_config)
     names = lambda pops: {p: None for p in pops} if pops else None
+    rows = DeviceRows(stat_config) if write == "device" else None
     items = score_populations(
         chr_names[0], {t: windows for t in tgt_samples}, names(ref_pops), names(tgt_pops), names(src_pops),
         ploidy_config, stat_config, anc_allele_file is not None, pre.engine, out_data=names(out_pops),
-        num_src=pre.num_src, loaded=loaded)
-    write_items(output_file, items, stat_config)
+        num_src=pre.num_src, loaded=loaded, sink=rows)
+    if rows is not None:
+        rows.write(output_file, pre.engine)
+    else:
+        write_items(output_file, items, stat_config)

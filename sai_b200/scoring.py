@@ -364,6 +364,49 @@ class HostEngine:
                                            _ptr(pg.neg_val), ref_sum.ctypes.data, tgt_sum.ctypes.data, m_max))
         return ref_sum, tgt_sum
 
+    #: ``format_scores`` calls made by any engine of this process (which writer produced a file)
+    format_calls = 0
+
+    def format_scores(self, inp: "_cabi.FormatInput") -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """The score rows, ``.U.log`` and ``.Q.log`` text of ``inp`` formatted on the device
+        (``sai_engine_format_scores``), each copied back in one D2H copy: three uint8 arrays (empty for
+        a log that does not exist)."""
+        lib = _cabi.load()
+        sizes = np.zeros(3, dtype=np.int64)
+        _cabi.check(lib.sai_engine_format_scores(self._handle(), C.byref(inp), sizes.ctypes.data))
+        HostEngine.format_calls += 1
+        out = []
+        for k in range(3):
+            text = np.empty(int(sizes[k]), dtype=np.uint8)
+            if text.size:
+                _cabi.check(lib.sai_engine_format_text(self._handle(), k, text.ctypes.data, text.size))
+            out.append(text)
+        return tuple(out)
+
+    def format_stats(self) -> dict:
+        """Seconds of the last ``format_scores`` (CUDA events): input copy, length + scan kernels,
+        write kernels."""
+        out = (C.c_double * 3)()
+        _cabi.check(_cabi.load().sai_engine_format_stats(self._handle(), out, 3))
+        return dict(zip(("copy_s", "length_s", "write_s"), list(out)))
+
+    def format_doubles(self, x: np.ndarray) -> np.ndarray:
+        """``repr(float(v))`` of every value, formatted by the device in one launch: ``[n, 32]``
+        uint8, NUL-padded (tests)."""
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        out = np.zeros((x.size, 32), dtype=np.uint8)
+        _cabi.check(_cabi.load().sai_engine_format_doubles(self._handle(), x.ctypes.data, x.size, out.ctypes.data))
+        return out
+
+
+def format_doubles_host(x: np.ndarray) -> np.ndarray:
+    """``repr(float(v))`` of every value from the host build of the device formatter: ``[n, 32]``
+    uint8, NUL-padded."""
+    x = np.ascontiguousarray(x, dtype=np.float64)
+    out = np.zeros((x.size, 32), dtype=np.uint8)
+    _cabi.check(_cabi.load().sai_format_doubles(x.ctypes.data, x.size, out.ctypes.data))
+    return out
+
 
 def dd_values(ref_sum: np.ndarray, tgt_sum: np.ndarray, n_ref: int, n_tgt: int, n_src_samples: Sequence[int]) -> list:
     """DD per source population and window from the integer sums, with the
