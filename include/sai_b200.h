@@ -736,6 +736,60 @@ int sai_engine_format_doubles(sai_engine* e, const double* x, int64_t n, char* o
 int32_t sai_format_double(double x, char* out);
 int sai_format_doubles(const double* x, int64_t n, char* out);
 
+/* ---- outlier tables on the device (outlier(..., text="device")) ---------------------------------
+ * The tables of `sai outlier` (sai_b200.outlier.outlier) built from a score file in HBM, byte for byte
+ * what the host path prints after pandas.read_csv(sep="\t", na_values=["nan"], index_col=False).
+ * sai_engine_table_load copies the file (header line + data rows, '\n'-terminated, the last one
+ * optionally not) to the device, finds its lines and every data cell of n_cols (the header's field
+ * count, at most SAI_TABLE_MAX_COLS), and ORs the classes of the cells (SAI_CELL_*, as
+ * sai_classify_cells gives them) per column and per chunk of chunk_rows rows -- the rows pandas' C
+ * parser infers one dtype for.  info = {data rows, chunks, SAI_TABLE_* flags of what the device path
+ * does not reproduce}.  sai_engine_table_classes copies the masks, [chunks][n_cols] uint32.
+ * sai_engine_table_parse takes the dtype of every column (SAI_TABLE_TEXT / _INT / _FLOAT) and the
+ * columns first_metric.., Chrom, Start, End (int64): it writes the metric columns as float64 into
+ * the DEVICE array d_vals[n_metric][rows] (NaN for NA; what sai_column_quantiles reads), the first
+ * value of each metric column in file order into first_val (NaN when it has none), and the number of
+ * runs of equal Chrom text into *n_runs; sai_engine_table_runs gives each run's Chrom as a byte
+ * offset and length within the file.  sai_engine_table_order sorts the rows stably on (run_rank of
+ * the row's run, Start, End).  sai_engine_table_build makes one table per metric column m: the
+ * header line, then the sorted rows with value > thr[m] (strict[m] != 0) or >= thr[m] (NaN is never
+ * kept; thr NaN keeps nothing), printed as ScoreTable.format_cell prints them; table m is
+ * offsets[m] .. offsets[m + 1] of one text that sai_engine_table_text copies into HOST memory.
+ * sai_engine_table_stats: seconds of the last calls (CUDA events): copy in, tokenise + classify,
+ * parse, sort, format, copy back.
+ * sai_parse_doubles: pandas' precise_xstrtod of each string text[offs[i] .. offs[i + 1]) on the host
+ * (the device's code); ok[i] = 1 where pandas reads it as a float.  sai_engine_parse_doubles: the
+ * same on the device (tests).  sai_classify_cells: the class of each string as a score-file cell. */
+#define SAI_TABLE_MAX_COLS 128
+#define SAI_TABLE_TEXT 0
+#define SAI_TABLE_INT 1
+#define SAI_TABLE_FLOAT 2
+#define SAI_CELL_INT 1
+#define SAI_CELL_FLOAT 2
+#define SAI_CELL_NA 4
+#define SAI_CELL_TEXT 8
+#define SAI_CELL_UNSURE 16
+#define SAI_CELL_BIGINT 32  /* with SAI_CELL_INT: |value| > 2^53, or more than 17 digits */
+#define SAI_CELL_NEGZERO 64 /* with SAI_CELL_INT: a negative zero ("-0") */
+#define SAI_TABLE_QUOTE_CR 1
+#define SAI_TABLE_HIGH_BYTE 2
+#define SAI_TABLE_BLANK_LINE 4
+#define SAI_TABLE_RAGGED 8
+#define SAI_TABLE_LONG_LINE 16 /* a line longer than 65535 bytes */
+int sai_engine_table_load(sai_engine* e, const char* text, int64_t n_bytes, int32_t n_cols, int64_t chunk_rows,
+                          int64_t* info);
+int sai_engine_table_classes(sai_engine* e, uint32_t* out, int64_t cap);
+int sai_engine_table_parse(sai_engine* e, const int32_t* kinds, int32_t first_metric, int32_t chrom, int32_t start,
+                           int32_t end, double* d_vals, double* first_val, int64_t* n_runs);
+int sai_engine_table_runs(sai_engine* e, int64_t* off, int64_t* len, int64_t cap);
+int sai_engine_table_order(sai_engine* e, const int32_t* run_rank, int64_t n_runs);
+int sai_engine_table_build(sai_engine* e, const double* thr, const int32_t* strict, int64_t* offsets);
+int sai_engine_table_text(sai_engine* e, char* out, int64_t cap);
+int sai_engine_table_stats(const sai_engine* e, double* out, int32_t n);
+int sai_engine_parse_doubles(sai_engine* e, const char* text, const int64_t* offs, int64_t n, double* out, uint8_t* ok);
+int sai_parse_doubles(const char* text, const int64_t* offs, int64_t n, double* out, uint8_t* ok);
+int sai_classify_cells(const char* text, const int64_t* offs, int64_t n, uint8_t* cls);
+
 /* ---- synthetic genotypes (bench / tests only) ---------------------------- */
 /* Fills tiles [tile0, tile0+n_tiles) of a packed matrix directly on the device
  * with the synthetic model of DESIGN.md (counter-based RNG, reproducible from

@@ -146,6 +146,13 @@ class FormatInput(C.Structure):
 
 FMT_U, FMT_Q = -1, -2  # SAI_FMT_U / SAI_FMT_Q: the U and Q fields of a score row
 
+TABLE_MAX_COLS = 128  # SAI_TABLE_MAX_COLS
+TABLE_TEXT, TABLE_INT, TABLE_FLOAT = 0, 1, 2  # SAI_TABLE_*: a column's dtype
+CELL_INT, CELL_FLOAT, CELL_NA, CELL_TEXT, CELL_UNSURE, CELL_BIGINT, CELL_NEGZERO = 1, 2, 4, 8, 16, 32, 64  # SAI_CELL_*
+#: SAI_TABLE_* flags of sai_engine_table_load: what the device outlier path does not reproduce
+TABLE_FLAGS = {1: "a '\\r' or '\"' in the file", 2: "a byte >= 0x80", 4: "a blank line", 8: "a row without one field per column",
+               16: "a line longer than 65535 bytes"}
+
 #: every symbol include/sai_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 _I32, _I64, _U64 = C.c_int32, C.c_int64, C.c_uint64
@@ -258,6 +265,17 @@ SYMBOLS = {
     "sai_engine_format_doubles": (C.c_int, [_P, _P, _I64, _P]),
     "sai_format_double": (_I32, [C.c_double, C.c_char_p]),
     "sai_format_doubles": (C.c_int, [_P, _I64, _P]),
+    "sai_engine_table_load": (C.c_int, [_P, _P, _I64, _I32, _I64, _P]),
+    "sai_engine_table_classes": (C.c_int, [_P, _P, _I64]),
+    "sai_engine_table_parse": (C.c_int, [_P, _P, _I32, _I32, _I32, _I32, _P, _P, _P]),
+    "sai_engine_table_runs": (C.c_int, [_P, _P, _P, _I64]),
+    "sai_engine_table_order": (C.c_int, [_P, _P, _I64]),
+    "sai_engine_table_build": (C.c_int, [_P, _P, _P, _P]),
+    "sai_engine_table_text": (C.c_int, [_P, _P, _I64]),
+    "sai_engine_table_stats": (C.c_int, [_P, _P, _I32]),
+    "sai_engine_parse_doubles": (C.c_int, [_P, _P, _P, _I64, _P, _P]),
+    "sai_parse_doubles": (C.c_int, [_P, _P, _I64, _P, _P]),
+    "sai_classify_cells": (C.c_int, [_P, _P, _I64, _P]),
 }
 
 _lib = None

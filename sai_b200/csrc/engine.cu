@@ -24,6 +24,7 @@
 
 #include "common.cuh"
 #include "format_kernels.cuh"
+#include "table_kernels.cuh"
 #include "host_pack.h"
 #include "vcf_genome.cuh"
 #include "zt_format.cuh"
@@ -163,6 +164,7 @@ struct sai_engine {
   Buf vgen;         // genome ingest: hash table, names, offsets, running state, per-chromosome records
   Buf vneg, vnega, vnegt;  // negative-value table: state + per-key counts, appended entries, finished table
   sai::FormatState fmt;    // score file text (sai_engine_format_scores)
+  sai::TableState tab;     // outlier tables (sai_engine_table_*)
 };
 
 namespace sai {
@@ -322,6 +324,7 @@ void sai_engine_destroy(sai_engine* e) {
   if (e->ring) cudaFreeHost(e->ring);
   if (e->h_ztoff) cudaFreeHost(e->h_ztoff);
   sai::format_release(e->fmt);
+  sai::table_release(e->tab);
   if (e->s_copy) cudaStreamDestroy(e->s_copy);
   if (e->s_comp) cudaStreamDestroy(e->s_comp);
   delete e;
@@ -1880,4 +1883,60 @@ int sai_engine_format_doubles(sai_engine* e, const double* x, int64_t n, char* o
   SAI_REQUIRE(e, "NULL engine");
   SAI_CUDA_CHECK(cudaSetDevice(e->device));
   return sai::format_doubles_device(x, n, out, e->s_comp);
+}
+
+int sai_engine_table_load(sai_engine* e, const char* text, int64_t n_bytes, int32_t n_cols, int64_t chunk_rows,
+                          int64_t* info) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::table_load(e->tab, text, n_bytes, n_cols, chunk_rows, info, e->s_comp);
+}
+
+int sai_engine_table_classes(sai_engine* e, uint32_t* out, int64_t cap) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::table_classes(e->tab, out, cap, e->s_comp);
+}
+
+int sai_engine_table_parse(sai_engine* e, const int32_t* kinds, int32_t first_metric, int32_t chrom, int32_t start,
+                           int32_t end, double* d_vals, double* first_val, int64_t* n_runs) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::table_parse(e->tab, kinds, first_metric, chrom, start, end, d_vals, first_val, n_runs, e->s_comp);
+}
+
+int sai_engine_table_runs(sai_engine* e, int64_t* off, int64_t* len, int64_t cap) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::table_runs(e->tab, off, len, cap, e->s_comp);
+}
+
+int sai_engine_table_order(sai_engine* e, const int32_t* run_rank, int64_t n_runs) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::table_order(e->tab, run_rank, n_runs, e->s_comp);
+}
+
+int sai_engine_table_build(sai_engine* e, const double* thr, const int32_t* strict, int64_t* offsets) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::table_build(e->tab, thr, strict, offsets, e->s_comp);
+}
+
+int sai_engine_table_text(sai_engine* e, char* out, int64_t cap) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::table_text(e->tab, out, cap, e->s_comp);
+}
+
+int sai_engine_table_stats(const sai_engine* e, double* out, int32_t n) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::table_stats(const_cast<sai_engine*>(e)->tab, out, n);
+}
+
+int sai_engine_parse_doubles(sai_engine* e, const char* text, const int64_t* offs, int64_t n, double* out, uint8_t* ok) {
+  SAI_REQUIRE(e, "NULL engine");
+  SAI_CUDA_CHECK(cudaSetDevice(e->device));
+  return sai::parse_doubles_device(text, offs, n, out, ok, e->s_comp);
 }

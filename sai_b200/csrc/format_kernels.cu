@@ -24,6 +24,8 @@ namespace {
 using fmt::format_double;
 using fmt::format_int64;
 
+size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
+
 struct FmtArgs {
   int64_t n_blocks, n_rows;
   const int64_t* block_rows;
@@ -41,78 +43,6 @@ struct FmtArgs {
   const double* vals;
   int32_t n_fields, n_vals;
 };
-
-// ---- exclusive scan of int64 lengths, in place, total at v[n] ---------------------------------------
-// (the three-kernel scan of vcf_device.cu's negative-value table, on int64)
-__device__ int64_t block_excl_scan64(int64_t v, int64_t* total) {
-  __shared__ int64_t warp_sum[32];
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  int64_t x = v;
-  for (int d = 1; d < 32; d <<= 1) {
-    const int64_t y = __shfl_up_sync(0xffffffffu, x, d);
-    if (lane >= d) x += y;
-  }
-  if (lane == 31) warp_sum[w] = x;
-  __syncthreads();
-  if (w == 0) {
-    int64_t s = lane < nw ? warp_sum[lane] : 0;
-    for (int d = 1; d < 32; d <<= 1) {
-      const int64_t y = __shfl_up_sync(0xffffffffu, s, d);
-      if (lane >= d) s += y;
-    }
-    if (lane < nw) warp_sum[lane] = s;
-  }
-  __syncthreads();
-  const int64_t before = (w > 0 ? warp_sum[w - 1] : 0) + x - v;
-  *total = warp_sum[nw - 1];
-  __syncthreads();
-  return before;
-}
-
-__global__ void __launch_bounds__(1024) k_len_count(const int64_t* __restrict__ v, int64_t n, int64_t* chunk_sum) {
-  for (int64_t c = blockIdx.x; c * 1024 < n; c += gridDim.x) {
-    const int64_t i = c * 1024 + threadIdx.x;
-    int64_t total;
-    block_excl_scan64(i < n ? v[i] : 0, &total);
-    if (threadIdx.x == 0) chunk_sum[c] = total;
-  }
-}
-
-__global__ void __launch_bounds__(1024) k_len_scan(int64_t* chunk, int64_t n_chunks, int64_t* total) {
-  int64_t carry = 0;
-  for (int64_t base = 0; base < n_chunks; base += blockDim.x) {
-    const int64_t i = base + threadIdx.x;
-    const int64_t v = i < n_chunks ? chunk[i] : 0;
-    int64_t sum;
-    const int64_t ex = block_excl_scan64(v, &sum);
-    if (i < n_chunks) chunk[i] = carry + ex;
-    carry += sum;
-  }
-  if (threadIdx.x == 0) *total = carry;
-}
-
-__global__ void __launch_bounds__(1024) k_len_excl(int64_t* v, int64_t n, const int64_t* __restrict__ chunk_off) {
-  for (int64_t c = blockIdx.x; c * 1024 < n; c += gridDim.x) {
-    const int64_t i = c * 1024 + threadIdx.x;
-    int64_t total;
-    const int64_t ex = chunk_off[c] + block_excl_scan64(i < n ? v[i] : 0, &total);
-    if (i < n) v[i] = ex;
-  }
-}
-
-int grid_for(int64_t items, int per_block) {
-  const int64_t b = (items + per_block - 1) / per_block;
-  return (int)(b < 1 ? 1 : b > 8LL * sm_count() ? 8LL * sm_count() : b);
-}
-
-// v[0 .. n) -> exclusive offsets, v[n] = total; chunk: (n + 1023) / 1024 int64 of scratch
-void scan_lengths(int64_t* v, int64_t n, int64_t* chunk, cudaStream_t st) {
-  const int64_t n_chunks = (n + 1023) / 1024;
-  const int grid = grid_for(n, 1024);
-  if (n > 0) k_len_count<<<grid, 1024, 0, st>>>(v, n, chunk);
-  k_len_scan<<<1, 1024, 0, st>>>(chunk, n_chunks, v + n);
-  if (n > 0) k_len_excl<<<grid, 1024, 0, st>>>(v, n, chunk);
-}
 
 // ---- candidates: digit lengths --------------------------------------------------------------------
 __global__ void k_cand_digits(const int32_t* __restrict__ cand, int64_t n, int64_t* len) {
@@ -270,23 +200,6 @@ __global__ void k_format_doubles(const double* __restrict__ x, int64_t n, char* 
   }
 }
 
-size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
-
-int grow_dev(void** p, size_t* cap, size_t bytes) {
-  if (bytes <= *cap) return SAI_OK;
-  if (*p) SAI_CUDA_CHECK(cudaFree(*p));
-  *p = nullptr;
-  *cap = 0;
-  const size_t want = bytes + bytes / 8 + 256;
-  const cudaError_t e = cudaMalloc(p, want);
-  if (e != cudaSuccess) {
-    set_error("cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
-    return SAI_E_NOMEM;
-  }
-  *cap = want;
-  return SAI_OK;
-}
-
 // every pointer and range the kernels will read
 int check_input(const sai_format_input* in, bool* has_u, bool* has_q) {
   SAI_REQUIRE(in, "sai_engine_format_scores: NULL input");
@@ -337,6 +250,67 @@ int check_input(const sai_format_input* in, bool* has_u, bool* has_q) {
 }
 
 }  // namespace
+
+// ---- shared with table_kernels.cu: the int64 length scan and grow-only buffers ---------------------
+__global__ void __launch_bounds__(1024) k_len_count(const int64_t* __restrict__ v, int64_t n, int64_t* chunk_sum) {
+  for (int64_t c = blockIdx.x; c * 1024 < n; c += gridDim.x) {
+    const int64_t i = c * 1024 + threadIdx.x;
+    int64_t total;
+    block_excl_scan64(i < n ? v[i] : 0, &total);
+    if (threadIdx.x == 0) chunk_sum[c] = total;
+  }
+}
+
+__global__ void __launch_bounds__(1024) k_len_scan(int64_t* chunk, int64_t n_chunks, int64_t* total) {
+  int64_t carry = 0;
+  for (int64_t base = 0; base < n_chunks; base += blockDim.x) {
+    const int64_t i = base + threadIdx.x;
+    const int64_t v = i < n_chunks ? chunk[i] : 0;
+    int64_t sum;
+    const int64_t ex = block_excl_scan64(v, &sum);
+    if (i < n_chunks) chunk[i] = carry + ex;
+    carry += sum;
+  }
+  if (threadIdx.x == 0) *total = carry;
+}
+
+__global__ void __launch_bounds__(1024) k_len_excl(int64_t* v, int64_t n, const int64_t* __restrict__ chunk_off) {
+  for (int64_t c = blockIdx.x; c * 1024 < n; c += gridDim.x) {
+    const int64_t i = c * 1024 + threadIdx.x;
+    int64_t total;
+    const int64_t ex = chunk_off[c] + block_excl_scan64(i < n ? v[i] : 0, &total);
+    if (i < n) v[i] = ex;
+  }
+}
+
+int grid_for(int64_t items, int per_block) {
+  const int64_t b = (items + per_block - 1) / per_block;
+  return (int)(b < 1 ? 1 : b > 8LL * sm_count() ? 8LL * sm_count() : b);
+}
+
+// v[0 .. n) -> exclusive offsets, v[n] = total; chunk: (n + 1023) / 1024 int64 of scratch
+void scan_lengths(int64_t* v, int64_t n, int64_t* chunk, cudaStream_t st) {
+  const int64_t n_chunks = (n + 1023) / 1024;
+  const int grid = grid_for(n, 1024);
+  if (n > 0) k_len_count<<<grid, 1024, 0, st>>>(v, n, chunk);
+  k_len_scan<<<1, 1024, 0, st>>>(chunk, n_chunks, v + n);
+  if (n > 0) k_len_excl<<<grid, 1024, 0, st>>>(v, n, chunk);
+}
+
+int grow_dev(void** p, size_t* cap, size_t bytes) {
+  if (bytes <= *cap) return SAI_OK;
+  if (*p) SAI_CUDA_CHECK(cudaFree(*p));
+  *p = nullptr;
+  *cap = 0;
+  const size_t want = bytes + bytes / 8 + 256;
+  const cudaError_t e = cudaMalloc(p, want);
+  if (e != cudaSuccess) {
+    set_error("cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
+    return SAI_E_NOMEM;
+  }
+  *cap = want;
+  return SAI_OK;
+}
 
 int format_scores(FormatState& f, const sai_format_input* in, cudaStream_t st, int64_t* sizes) {
   SAI_REQUIRE(sizes, "sai_engine_format_scores: NULL sizes");

@@ -18,6 +18,7 @@ path (CPU tests) gathers U counts as a histogram and Q values as padded arrays.
 
 from __future__ import annotations
 
+import ctypes
 import re
 import warnings
 from typing import Optional, Sequence
@@ -211,12 +212,238 @@ class ScoreTable:
         return str(v)
 
 
-def outlier(score_file: str, output_prefix: str, quantile: float, group=None) -> None:
+TEXT_MODES = ("host", "device")
+
+
+def pandas_chunk_rows(n_cols: int) -> int:
+    """Rows per chunk of pandas' C parser (``low_memory=True``) for a table of ``n_cols`` columns: it
+    infers one dtype per chunk and column and concatenates the chunks, so a column that is int64 in
+    one chunk and text in another holds Python ints and strings (with a DtypeWarning)."""
+    heuristic = 2**20 // n_cols
+    rows = 1
+    while rows * 2 < heuristic:
+        rows *= 2
+    return rows
+
+
+def column_kinds(classes: np.ndarray) -> tuple[Optional[list[int]], Optional[str]]:
+    """pandas' dtype of every column (``_cabi.TABLE_TEXT`` / ``_INT`` / ``_FLOAT``) from the OR of its
+    cells' ``SAI_CELL_*`` classes per parse chunk, ``[chunks, columns]``; or the reason the device
+    path cannot reproduce it.  A chunk with a text cell is text, one of integers only int64, any
+    other float64 (an all-NA chunk too); int64 and float64 chunks concatenate to float64; text with
+    anything else is a column of mixed objects.  pandas reads the integers of a float64 column either
+    as int64 (cast) or with its float parser, which differ beyond 2^53, past 17 digits (leading zeros
+    included) and on "-0"; such a column is left to the host path."""
+    from . import _cabi
+
+    odd_int = _cabi.CELL_BIGINT | _cabi.CELL_NEGZERO
+    kinds = []
+    for c in range(classes.shape[1]):
+        col = classes[:, c]
+        if np.any(col & _cabi.CELL_UNSURE):
+            return None, f"column {c + 1} has a cell whose pandas type or value is not reproduced"
+        chunk = {(_cabi.TABLE_TEXT if m & _cabi.CELL_TEXT else
+                  _cabi.TABLE_INT if m & ~odd_int == _cabi.CELL_INT else _cabi.TABLE_FLOAT) for m in col.tolist()}
+        if chunk == {_cabi.TABLE_INT, _cabi.TABLE_FLOAT}:
+            chunk = {_cabi.TABLE_FLOAT}
+        if len(chunk) > 1:
+            return None, f"column {c + 1} has parse chunks of different pandas types"
+        kinds.append(chunk.pop())
+        if kinds[-1] == _cabi.TABLE_FLOAT and np.any(col & odd_int):
+            return None, f"column {c + 1} is float64 with an integer beyond 2^53, of more than 17 digits or -0"
+    return kinds, None
+
+
+class _DeviceFile:
+    """A score file loaded and classified on the device (``_load_device``)."""
+
+    def __init__(self, data: bytes, names: list[str], engine, n_rows: int, kinds: list[int]):
+        self.data, self.names, self.engine, self.n_rows, self.kinds = data, names, engine, n_rows, kinds
+        self.first_metric = names.index("N(Variants)") + 1
+        self.chrom, self.start, self.end = (names.index(c) for c in ("Chrom", "Start", "End"))
+
+
+def _load_device(data: bytes, quantile: float, group, device: int, timings: Optional[dict]):
+    """(reason, None) when the file has to be read on the host, else (None, ``_DeviceFile``)."""
+    import torch.distributed as dist
+
+    if not 0.0 <= quantile <= 1.0:
+        return "quantile outside [0, 1]", None
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1 \
+            and dist.get_backend(group) != "nccl":
+        return "a process group that is not NCCL", None
+    nl = data.find(b"\n")
+    if nl < 0:
+        return "no data rows", None
+    names_b = data[:nl].split(b"\t")
+    if any(not n for n in names_b):
+        return "an empty column name", None
+    if len(set(names_b)) != len(names_b):
+        return "duplicate column names", None
+    if any(b < 0x21 or b > 0x7E for n in names_b for b in n):
+        return "a column name with bytes outside printable ASCII", None
+    if len(names_b) > 128:
+        return "more than 128 columns", None
+    names = [n.decode() for n in names_b]
+    if "N(Variants)" not in names:
+        return "no N(Variants) column", None
+    if names[-1] == "N(Variants)":
+        return "no metric columns", None
+    if not {"Chrom", "Start", "End"} <= set(names):
+        return "no Chrom, Start or End column", None
+    from . import _cabi
+    from .scoring import HostEngine
+
+    eng = HostEngine(device)
+    n_rows, n_chunks, flags = eng.table_load(data, len(names), pandas_chunk_rows(len(names)))
+    if timings is not None:
+        timings.update(eng.table_stats())
+    reason = next((why for bit, why in _cabi.TABLE_FLAGS.items() if flags & bit), None)
+    if reason is None and n_rows == 0:
+        reason = "no data rows"
+    kinds = None
+    if reason is None:
+        classes = eng.table_classes(n_chunks, len(names))
+        kinds, reason = column_kinds(classes)
+    if reason is None:
+        f = _DeviceFile(data, names, eng, n_rows, kinds)
+        chrom_cls = int(np.bitwise_or.reduce(classes[:, f.chrom]))
+        if any(k == _cabi.TABLE_TEXT for k in kinds[f.first_metric:]):
+            reason = "a text metric column"
+        elif kinds[f.start] != _cabi.TABLE_INT or kinds[f.end] != _cabi.TABLE_INT:
+            reason = "Start or End is not int64"
+        elif kinds[f.chrom] == _cabi.TABLE_FLOAT or chrom_cls & _cabi.CELL_NA:
+            reason = "Chrom has NA cells or is float64"
+        else:
+            return None, f
+    eng.close()
+    return reason, None
+
+
+def fallback_reason(score_file: str, quantile: float, group=None, device: int = 0) -> Optional[str]:
+    """Why ``outlier(..., text="device")`` reads ``score_file`` on the host (``None``: it builds the
+    tables on the device), for this rank alone.  The host path takes every file whose pandas
+    dtypes, values or errors the device path does not reproduce exactly."""
+    with open(score_file, "rb") as fh:
+        data = fh.read()
+    reason, f = _load_device(data, quantile, group, device, None)
+    if f is not None:
+        f.engine.close()
+    return reason
+
+
+def _ranks_agree(ok: bool, header: bytes, group, device: int) -> bool:
+    """With an NCCL group of several ranks: True when every rank takes the device path and all read
+    the same column names (one MIN all-reduce), so that no rank waits in a collective another rank
+    never enters."""
+    import zlib
+
+    import torch
+    import torch.distributed as dist
+
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1 \
+            or dist.get_backend(group) != "nccl":
+        return ok
+    h = (zlib.crc32(header) << 20) | min(len(header), (1 << 20) - 1)
+    t = torch.tensor([int(ok), h, -h], dtype=torch.int64, device=torch.device("cuda", device))
+    dist.all_reduce(t, op=dist.ReduceOp.MIN, group=group)
+    ok_all, lo, neg_hi = t.tolist()
+    return ok_all == 1 and lo == -neg_hi
+
+
+def device_outlier(score_file: str, output_prefix: str, quantile: float, group=None, device: int = 0,
+                   timings: Optional[dict] = None) -> bool:
+    """``outlier`` with the score file parsed and the tables built as text on the GPU; returns False
+    (having written nothing) when the file needs the host path (``fallback_reason``).  ``timings``,
+    if given, receives the seconds of every phase."""
+    import time
+
+    import torch
+    import torch.distributed as dist
+
+    from . import _cabi
+
+    t0 = time.perf_counter()
+    with open(score_file, "rb") as fh:
+        data = fh.read()
+    t_read = time.perf_counter() - t0
+    reason, f = _load_device(data, quantile, group, device, timings)
+    nl = data.find(b"\n")
+    if not _ranks_agree(reason is None, data[:nl] if nl >= 0 else data, group, device):
+        if f is not None:
+            f.engine.close()
+        return False
+    eng = f.engine
+    try:
+        dev = torch.device("cuda", device)
+        metric = f.names[f.first_metric:]
+        n_metric = len(metric)
+        with torch.cuda.device(dev):
+            vals = torch.empty((n_metric, f.n_rows), dtype=torch.float64, device=dev)
+            first, n_runs = eng.table_parse(f.kinds, f.first_metric, f.chrom, f.start, f.end, vals)
+            # natural order of the chromosome names: ranked on the host with the host path's key
+            off, ln = eng.table_runs(n_runs)
+            names = [data[o:o + n].decode() for o, n in zip(off.tolist(), ln.tolist())]
+            if f.kinds[f.chrom] == _cabi.TABLE_INT:
+                names = [str(int(n)) for n in names]
+            keys = {n: _natural_key(n) for n in set(names)}
+            rank, last = {}, None
+            for n in sorted(keys, key=keys.get):
+                rank[n] = rank[last] + (keys[n] != keys[last]) if last is not None else 0
+                last = n
+            eng.table_order(np.array([rank[n] for n in names], dtype=np.int32))
+            t1 = time.perf_counter()
+            if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+                found = device_thresholds(vals, quantile, group)  # one all-gather for every column
+                none = [t is None for t in found]
+                thr = [np.nan if t is None else t for t in found]
+            else:
+                out = torch.empty((n_metric, 4), dtype=torch.float64, device=dev)
+                stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+                _cabi.check(_cabi.load().sai_column_quantiles(vals.data_ptr(), n_metric, 1, 0, f.n_rows, f.n_rows,
+                                                              float(quantile), out.data_ptr(), stream))
+                o = out.cpu().numpy()
+                # threshold_from_values: no threshold for an empty or single-valued column
+                none = [bool(o[m, 1] == 0 or o[m, 2] == o[m, 3]) for m in range(n_metric)]
+                thr = [np.nan if none[m] else float(o[m, 0]) for m in range(n_metric)]
+            t_thr = time.perf_counter() - t1
+            text, offs = eng.table_build(thr, [c.startswith("U") for c in metric])
+        if timings is not None:
+            timings.update(eng.table_stats())
+        t2 = time.perf_counter()
+        view = memoryview(text)
+        for m, col in enumerate(metric):
+            if none[m]:
+                if np.isnan(first[m]):
+                    warnings.warn(f"Column '{col}' has no numeric values; writing empty result.", UserWarning)
+                else:
+                    warnings.warn(f"Column '{col}' has only one unique value ({np.float64(first[m])}); writing empty result.",
+                                  UserWarning)
+            with open(f"{output_prefix}.{col}.{quantile}.outliers.tsv", "wb") as fh:
+                fh.write(view[offs[m]:offs[m + 1]])
+        if timings is not None:
+            timings.update(read_s=t_read, thresholds_s=t_thr, write_s=time.perf_counter() - t2)
+    finally:
+        eng.close()
+    return True
+
+
+def outlier(score_file: str, output_prefix: str, quantile: float, group=None, text: str = "host",
+            device: int = 0) -> None:
     """Reads a score TSV, writes one ``{prefix}.{column}.{quantile}.outliers.tsv``
     per metric column.  With an initialised process group every rank passes the
     score file of its own shard and all ranks use the same genome-wide
     thresholds (one small all-gather per column); each rank writes the outlier
-    rows of its own shard."""
+    rows of its own shard.
+
+    ``text="device"`` parses the file and builds the tables as text on GPU ``device``
+    (``device_outlier``): the same files, warnings and errors, with one all-gather for all
+    columns under NCCL.  A file whose pandas reading it does not reproduce exactly, and a gloo
+    group, take the host path (``fallback_reason``)."""
+    if text not in TEXT_MODES:
+        raise ValueError(f"text must be 'host' or 'device', not {text!r}")
+    if text == "device" and device_outlier(score_file, output_prefix, quantile, group, device):
+        return
     tab = ScoreTable(score_file)
     cols = tab.columns
     if "N(Variants)" in cols:

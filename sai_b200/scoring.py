@@ -398,6 +398,102 @@ class HostEngine:
         _cabi.check(_cabi.load().sai_engine_format_doubles(self._handle(), x.ctypes.data, x.size, out.ctypes.data))
         return out
 
+    #: ``table_build`` calls made by any engine of this process (which path wrote the outlier tables)
+    outlier_calls = 0
+
+    def table_load(self, data: bytes, n_cols: int, chunk_rows: int) -> tuple[int, int, int]:
+        """Copies a score file to the device, finds its cells and classifies them
+        (``sai_engine_table_load``): (data rows, parse chunks, ``SAI_TABLE_*`` flags)."""
+        info = np.zeros(3, dtype=np.int64)
+        _cabi.check(_cabi.load().sai_engine_table_load(self._handle(), data, len(data), int(n_cols), int(chunk_rows),
+                                                       info.ctypes.data))
+        return int(info[0]), int(info[1]), int(info[2])
+
+    def table_classes(self, n_chunks: int, n_cols: int) -> np.ndarray:
+        """``[n_chunks, n_cols]`` uint32: the OR of the ``SAI_CELL_*`` classes of every column's cells
+        per pandas parse chunk of the loaded file."""
+        out = np.zeros((n_chunks, n_cols), dtype=np.uint32)
+        _cabi.check(_cabi.load().sai_engine_table_classes(self._handle(), out.ctypes.data, out.size))
+        return out
+
+    def table_parse(self, kinds: Sequence[int], first_metric: int, chrom: int, start: int, end: int,
+                    vals) -> tuple[np.ndarray, int]:
+        """Parses the loaded file with the column dtypes ``kinds``: the metric columns into the float64
+        CUDA tensor ``vals`` ``[n_metric, rows]``.  Returns each metric column's first value in file
+        order (NaN: none) and the number of runs of equal Chrom text."""
+        k = np.ascontiguousarray(kinds, dtype=np.int32)
+        first = np.zeros(int(vals.shape[0]), dtype=np.float64)
+        n_runs = C.c_int64()
+        _cabi.check(_cabi.load().sai_engine_table_parse(self._handle(), k.ctypes.data, int(first_metric), int(chrom),
+                                                        int(start), int(end), vals.data_ptr(), first.ctypes.data,
+                                                        C.byref(n_runs)))
+        return first, int(n_runs.value)
+
+    def table_runs(self, n_runs: int) -> tuple[np.ndarray, np.ndarray]:
+        """Byte offset and length of each Chrom run's name within the loaded file."""
+        off = np.zeros(n_runs, dtype=np.int64)
+        ln = np.zeros(n_runs, dtype=np.int64)
+        _cabi.check(_cabi.load().sai_engine_table_runs(self._handle(), off.ctypes.data, ln.ctypes.data, n_runs))
+        return off, ln
+
+    def table_order(self, run_rank: np.ndarray) -> None:
+        """Sorts the rows stably on (rank of their Chrom run, Start, End)."""
+        r = np.ascontiguousarray(run_rank, dtype=np.int32)
+        _cabi.check(_cabi.load().sai_engine_table_order(self._handle(), r.ctypes.data, r.size))
+
+    def table_build(self, thr: Sequence[float], strict: Sequence[bool]) -> tuple[np.ndarray, np.ndarray]:
+        """Every metric column's outlier table as text, copied back in one D2H copy: (uint8 text,
+        int64 offsets ``[n_metric + 1]``; table m is ``text[offsets[m]:offsets[m + 1]]``)."""
+        lib = _cabi.load()
+        t = np.ascontiguousarray(thr, dtype=np.float64)
+        s = np.ascontiguousarray(strict, dtype=np.int32)
+        offs = np.zeros(t.size + 1, dtype=np.int64)
+        _cabi.check(lib.sai_engine_table_build(self._handle(), t.ctypes.data, s.ctypes.data, offs.ctypes.data))
+        HostEngine.outlier_calls += 1
+        text = np.empty(int(offs[-1]), dtype=np.uint8)
+        _cabi.check(lib.sai_engine_table_text(self._handle(), text.ctypes.data, text.size))
+        return text, offs
+
+    def table_stats(self) -> dict:
+        """Seconds of the last table calls (CUDA events)."""
+        out = (C.c_double * 6)()
+        _cabi.check(_cabi.load().sai_engine_table_stats(self._handle(), out, 6))
+        return dict(zip(("copy_in_s", "tokenise_s", "parse_s", "sort_s", "format_s", "copy_back_s"), list(out)))
+
+    def parse_doubles(self, strings: Sequence[bytes]) -> tuple[np.ndarray, np.ndarray]:
+        """pandas' float parser on every string, run by the device in one launch (tests): (values,
+        bool "pandas reads it as a float")."""
+        text, offs = _joined(strings)
+        out = np.zeros(len(strings), dtype=np.float64)
+        ok = np.zeros(len(strings), dtype=np.uint8)
+        _cabi.check(_cabi.load().sai_engine_parse_doubles(self._handle(), text, offs.ctypes.data, len(strings),
+                                                          out.ctypes.data, ok.ctypes.data))
+        return out, ok.astype(bool)
+
+
+def _joined(strings: Sequence[bytes]) -> tuple[bytes, np.ndarray]:
+    offs = np.zeros(len(strings) + 1, dtype=np.int64)
+    offs[1:] = np.cumsum([len(s) for s in strings])
+    return b"".join(strings), offs
+
+
+def parse_doubles_host(strings: Sequence[bytes]) -> tuple[np.ndarray, np.ndarray]:
+    """pandas' float parser (``precise_xstrtod``) on every string, from the host build of the device
+    parser: (values, bool "pandas reads it as a float")."""
+    text, offs = _joined(strings)
+    out = np.zeros(len(strings), dtype=np.float64)
+    ok = np.zeros(len(strings), dtype=np.uint8)
+    _cabi.check(_cabi.load().sai_parse_doubles(text, offs.ctypes.data, len(strings), out.ctypes.data, ok.ctypes.data))
+    return out, ok.astype(bool)
+
+
+def classify_cells_host(strings: Sequence[bytes]) -> np.ndarray:
+    """The ``SAI_CELL_*`` class of every string as a score-file cell (host build of the device code)."""
+    text, offs = _joined(strings)
+    out = np.zeros(len(strings), dtype=np.uint8)
+    _cabi.check(_cabi.load().sai_classify_cells(text, offs.ctypes.data, len(strings), out.ctypes.data))
+    return out
+
 
 def format_doubles_host(x: np.ndarray) -> np.ndarray:
     """``repr(float(v))`` of every value from the host build of the device formatter: ``[n, 32]``
